@@ -2,7 +2,7 @@
 """Headline benchmark: Mrays/s (ray segments per second) and frame time on a reference scene.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scene 3d_room]
-                    [--width 3840 --height 2160] [--pipeline wavefront|megakernel] [--no-configs]
+                    [--width 3840 --height 2160] [--pipeline wavefront|megakernel] [--no-configs] [--dump-outputs DIR]
 
 A "step" is one fixed-pose headless frame (Environment::render, src/universe/mod.rs:300-357).
  * value    : whole-job ray segments / second with the frame left in HBM (eucl_render_device)
@@ -359,8 +359,29 @@ def settle_frames(warmup: int) -> int:
     return max(warmup, 8)
 
 
-def measure(rig: Rig, steps: int, warmup: int, sample_clocks: bool):
-    """Device-timed value leg, profile pass, e2e leg.  Returns a dict on rank 0, None elsewhere."""
+DUMP_MAX_PIXELS = 1 << 21  # 24 MiB of float32 RGB, plus 16 MiB of float64 pixel indices when sampled
+
+
+def dump_outputs(out_dir: str, frame, stats: dict) -> None:
+    """Writes what the last timed step handed its caller: the RGB8 frame (row 0 = bottom) as float32 and the ray-tree
+    node count of every level as float64.  A frame of more than DUMP_MAX_PIXELS pixels is sampled: the same
+    seeded choice of pixels for the same frame size, their flat indices (y * width + x) in frame_pixel_index.npy."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    rgb = frame.cpu().numpy().reshape(-1, 3)
+    if rgb.shape[0] > DUMP_MAX_PIXELS:
+        index = np.sort(np.random.default_rng(0).choice(rgb.shape[0], DUMP_MAX_PIXELS, replace=False))
+        rgb = rgb[index]
+        np.save(out / "frame_pixel_index.npy", index.astype(np.float64))
+    else:
+        rgb = rgb.reshape(frame.shape)
+    np.save(out / "frame.npy", rgb.astype(np.float32))
+    np.save(out / "level_counts.npy", np.array(stats["level_counts"], dtype=np.float64))  # at N > 1: rank 0's rows
+
+
+def measure(rig: Rig, steps: int, warmup: int, sample_clocks: bool, dump_dir: str | None = None):
+    """Device-timed value leg, profile pass, e2e leg.  Returns a dict on rank 0, None elsewhere.
+    With `dump_dir`, rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     torch, dist = rig.torch, rig.dist
     world, rank = rig.world, rig.rank
     for _ in range(settle_frames(warmup)):
@@ -382,6 +403,8 @@ def measure(rig: Rig, steps: int, warmup: int, sample_clocks: bool):
     ev1.record(rig.stream)
     rig.sync_all()
     ms = ev0.elapsed_time(ev1)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, rig.frame, st)
     clocks = sampler.stop() if sampler else None
     prof = rig.step(profile=True)  # per-kernel-family device times (extra events; outside the timed region)
     rig.sync_all()
@@ -450,6 +473,8 @@ def main():
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: ranks store their rows into GPU 0's frame through CUDA IPC (peer) or NCCL gather")
     ap.add_argument("--check", action="store_true", help="N > 1: compare the gathered frames with a single-GPU render")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame and level counts of the last timed step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     width, height = DEFAULT_CONFIGS.get(args.scene, (3840, 2160))
     width, height = args.width or width, args.height or height
@@ -477,7 +502,7 @@ def main():
         dist.init_process_group("nccl", device_id=device)
 
     rig = Rig(args, args.scene, width, height, args.max_depth, world, rank, local_rank)
-    m = measure(rig, args.steps, args.warmup, sample_clocks=True)
+    m = measure(rig, args.steps, args.warmup, sample_clocks=True, dump_dir=args.dump_outputs)
     env = rig.env
 
     line = None

@@ -10,11 +10,11 @@ from ._capi import EuclCamera, EuclError, EuclRenderOpts, EuclStats, EUCL_PIPELI
 from .scene import Environment, Parser, ParserError, RawImage2d, SimulationContext
 
 ROOT = Path(__file__).resolve().parent.parent
-ASSET_ROOT = ROOT / "assets" / "_ref"  # reference scenes + textures (tools/fetch_assets.py)
+ASSET_ROOT = ROOT / "assets"  # the reference scenes, restated, and stand-in textures (assets/make_assets.py)
 
 
 def load_reference_scene(name: str) -> Environment:
-    """Parses assets/_ref/scenes/<name>.json with textures resolved under assets/_ref/."""
+    """Parses assets/scenes/<name>.json with textures resolved under assets/."""
     return Parser.default(resource_root=ASSET_ROOT).parse_file(ASSET_ROOT / "scenes" / f"{name}.json")
 
 

@@ -52,7 +52,6 @@ def _worker(rank, world, port, height, width, band, q):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(not (eb.ASSET_ROOT / "scenes").exists(), reason="assets/_ref missing")
 def test_two_rank_gather_gloo(oracle):
     import torch.multiprocessing as mp
 

@@ -11,7 +11,6 @@ import pytest
 import euclider_b200 as eb
 
 GOLDEN = sorted((Path(__file__).resolve().parent / "golden").glob("*.npz"))
-pytestmark = pytest.mark.skipif(not (eb.ASSET_ROOT / "scenes").exists(), reason="assets/_ref missing")
 
 
 @pytest.mark.parametrize("path", GOLDEN, ids=lambda p: p.stem)

@@ -7,8 +7,6 @@ import pytest
 import euclider_b200 as eb
 from euclider_b200 import _capi
 
-pytestmark = pytest.mark.skipif(not (eb.ASSET_ROOT / "scenes").exists(), reason="assets/_ref missing (tools/fetch_assets.py)")
-
 # scene -> (dim, surfaced primitives by kind {sphere, plane-like, cylinder}, entities)
 EXPECTED = {
     "3d_fresnel": (3, (1, 0, 0), 2),

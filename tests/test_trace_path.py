@@ -6,8 +6,6 @@ import pytest
 
 import euclider_b200 as eb
 
-pytestmark = pytest.mark.skipif(not (eb.ASSET_ROOT / "scenes").exists(), reason="assets/_ref missing")
-
 
 def test_straight_line_in_vacuum(oracle, built_lib):
     env = eb.load_reference_scene("3d_fresnel")  # sphere c (10,0,0) r 3 in a vacuum void

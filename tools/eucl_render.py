@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Headless renderer: scene JSON -> image file (the reference only renders into a window).
 
-    python tools/eucl_render.py assets/_ref/scenes/3d_room.json out.png --size 1920 1080 [--time 1.5]
-        [--resource-root assets/_ref] [--location x y z [w]] [--max-depth N] [--pipeline megakernel]
+    python tools/eucl_render.py assets/scenes/3d_room.json out.png --size 1920 1080 [--time 1.5]
+        [--resource-root assets] [--location x y z [w]] [--max-depth N] [--pipeline megakernel]
 """
 import argparse
 import sys

@@ -3,7 +3,7 @@
 
 The reference itself cannot run here (no Rust toolchain), so these fixtures pin the ORACLE (and,
 through the GPU parity tests, the CUDA path) against regressions; they are not outputs of the
-Rust binary.  Needs assets/_ref (tools/fetch_assets.py).  Run from the repo root:
+Rust binary.  Renders the scenes under assets/ (assets/make_assets.py).  Run from the repo root:
     python tools/make_golden.py
 """
 import sys
