@@ -71,6 +71,10 @@ class EuclCamera(C.Structure):
         return out
 
 
+class EuclFrame(C.Structure):
+    _fields_ = [("camera", EuclCamera), ("time_seconds", C.c_double)]
+
+
 class EuclFlatScene(C.Structure):
     _fields_ = [("dim", C.c_int32),
                 ("n_prims", C.c_int32), ("n_nodes", C.c_int32), ("n_entities", C.c_int32),
@@ -140,6 +144,10 @@ PROTOTYPES = {
                               C.POINTER(EuclStats)]),
     "eucl_render_device": (C.c_int, [C.c_void_p, C.POINTER(EuclCamera), C.POINTER(EuclRenderOpts), C.c_void_p,
                                      C.c_void_p, C.POINTER(EuclStats)]),
+    "eucl_render_frames": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts), C.c_void_p,
+                                     C.c_void_p, C.POINTER(EuclStats)]),
+    "eucl_render_frames_device": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts),
+                                            C.c_void_p, C.c_void_p, C.POINTER(EuclStats)]),
     "eucl_trace_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,
                                   C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "eucl_camera_rotate_yaw": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),

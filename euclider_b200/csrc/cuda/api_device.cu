@@ -138,6 +138,13 @@ struct EuclScene {
     DeviceBuffer order;    // per-bin node lists of the level being shaded
     DeviceBuffer path_io;  // eucl_trace_path staging
     DeviceBuffer rorder;   // per-reach-key node lists of the next level
+    // a batch of frames (eucl_render_frames*): the per-frame constants (leader only; its twins read them), their pinned
+    // host staging, and per pipeline the frames' camera entities and the frame tag of every node
+    DeviceBuffer frame_table;
+    FrameParams* h_frame_table = nullptr;
+    uint32_t h_frame_table_cap = 0;
+    DeviceBuffer frame_entity;
+    DeviceBuffer node_frame;
     int n_cull = 0;
     int light_capable = 0;
     // Grouping rays by reach key pays on scenes whose deep levels bounce around a few bounded objects
@@ -181,7 +188,8 @@ struct SmallLayout {                                        // one per chunk, in
     static constexpr int mega64 = undefined64 + 2;                    // (EUCL_MAX_LEVELS + 1) x u64
     static constexpr int bins = mega64 + 2 * (EUCL_MAX_LEVELS + 1);       // [level][kMaxBins]
     static constexpr int rbins = bins + (EUCL_MAX_LEVELS + 1) * kMaxBins; // [level][kRayBins]
-    static constexpr int total = rbins + (EUCL_MAX_LEVELS + 1) * kRayBins;
+    static constexpr int untraced = rbins + (EUCL_MAX_LEVELS + 1) * kRayBins; // Workspace::untraced
+    static constexpr int total = untraced + 1;
 };
 static_assert(SmallLayout::undefined64 % 2 == 0, "u64 counters must be 8-byte aligned");
 static_assert(SmallLayout::total <= kSmallInts, "small buffer layout");
@@ -665,6 +673,10 @@ void eucl_scene_destroy(EuclScene* s) {
     s->order.release();
     s->path_io.release();
     s->rorder.release();
+    s->frame_table.release();
+    s->frame_entity.release();
+    s->node_frame.release();
+    if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
     if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
     if (s->h_small) cudaFreeHost(s->h_small);
     for (auto& e : s->ev)
@@ -972,10 +984,29 @@ size_t arena_bytes(int dim, int real_bytes, size_t cap) {
     return per * cap + 16 * 16;
 }
 
-Workspace carve(EuclScene* s, int dim, int cap, int list_cap) {
+// The frames of one call.  A single frame (eucl_render*) is a batch of one and renders exactly as it always did;
+// K > 1 frames (eucl_render_frames*) are ONE virtual frame of K * rows rows -- chunks, bands and pipelines split it
+// like any other frame -- whose per-pixel constants the kernels look up in a device table by virtual row.
+struct FrameBatch {
+    const EuclFrame* frames;
+    uint32_t n;                      // K
+    uint32_t rows;                   // rows per frame
+    const FrameParams* d_table;      // K > 1: [K] frame constants on the device, uploaded before the first launch
+    uint64_t table_key;              // K > 1: hash of the table contents, part of the graph key
+};
+
+Workspace carve(EuclScene* s, int dim, int cap, int list_cap, const FrameBatch& fb) {
     Workspace ws{};
     ws.capacity = cap;
     ws.list_cap = list_cap;
+    ws.n_frames = (int32_t)fb.n;
+    ws.frame_rows = (int32_t)fb.rows;
+    if (fb.n > 1) {
+        ws.frames = fb.d_table;
+        ws.frame_entity = (int32_t*)s->frame_entity.ptr;
+        ws.node_frame = (int32_t*)s->node_frame.ptr;
+        ws.untraced = (int32_t*)s->small.ptr + SmallLayout::untraced;
+    }
     uint8_t* p = (uint8_t*)s->nodes.ptr;
     auto take = [&](size_t bytes) {
         uint8_t* r = p;
@@ -1035,16 +1066,24 @@ void tune_grouping(EuclScene* s, const EuclStats& st, int pipeline) {
 
 // Renders this rank's rows of `o` (all of them, or -- sub_stride > 1 -- the bands that `o` names, which are every
 // sub_stride-th band of the caller's rank starting at sub_offset: render_split).
-int render_impl(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
+// `o` describes the (virtual) frame: o->height = fb.n * fb.rows.
+int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
                 EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
     const int dim = s->dim;
+    const EuclCamera* cam = &fb.frames[0].camera; // (every frame of a batch has this max_depth)
     FrameParams fp;
-    frame_params(*cam, *o, s->real_bytes, &fp);
+    {
+        EuclRenderOpts first = *o;
+        first.height = fb.rows;
+        first.time_seconds = fb.frames[0].time_seconds;
+        frame_params(*cam, first, s->real_bytes, &fp);
+    }
     const int width = (int)o->width;
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
     EuclStats st{};
     st.levels = cam->max_depth + 1;
     if (!s->is_twin) choose_grouping(s); // a twin renders with its leader's setting
+    if (fb.n > 1) EUCL_CUDA(s->frame_entity.ensure(sizeof(int32_t) * fb.n));
     EUCL_CUDA(cudaEventRecord(s->ev[0], s->stream));
     if (my_rows > 0) {
         // chunking: whole local rows, about EUCL_CHUNK_PIXELS primaries per chunk.  Large chunks are faster (longer
@@ -1128,7 +1167,8 @@ int render_impl(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
                     rows_per_chunk = (rows_per_chunk + 1) / 2;
                     continue;
                 }
-                Workspace ws = carve(s, dim, s->arena_capacity, s->list_capacity);
+                if (fb.n > 1) EUCL_CUDA(s->node_frame.ensure(sizeof(int32_t) * (size_t)s->arena_capacity));
+                Workspace ws = carve(s, dim, s->arena_capacity, s->list_capacity, fb);
                 // profile mode: one event after every launch; family = 0 raygen, 1 intersect, 2 shade, 3 resolve
                 std::vector<int> prof_family;
                 auto mark = [&](int family) {
@@ -1172,6 +1212,11 @@ int render_impl(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
                         mark(1);
                         launches += 2;
                     } else {
+                        if (ws.frames) {
+                            EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
+                            dbg("k_camera_entity", 0);
+                            launches += 1;
+                        }
                         EUCL_PREC(launch_raygen)(dim, l, fp, cp, ws, d_hit);
                         dbg("k_raygen", 0);
                         mark(0);
@@ -1226,6 +1271,9 @@ int render_impl(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
                 mix(&pipeline_id, sizeof pipeline_id);
                 const uint32_t depth_id = cam->max_depth;
                 mix(&depth_id, sizeof depth_id);
+                // a batch: the graph reads the table the caller's poses were uploaded to, and it is keyed by its contents
+                // too, so that a changed pose or time is never taken for a repeated batch
+                if (fb.n > 1) mix(&fb.table_key, sizeof fb.table_key);
                 // (not while the scene is still choosing its ray-grouping mode: capture time would distort the comparison)
                 const bool graph_ok = env_int("EUCL_GRAPH", 1) && !o->profile && !debug_sync && !poison &&
                                       (s->ray_bins_mode >= 0 || o->pipeline != EUCL_PIPELINE_WAVEFRONT);
@@ -1306,12 +1354,14 @@ int render_impl(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
             }
             row0 += cp.n_rows;
             st.pixels += (uint64_t)cp.n_pixels;
-            // camera in no entity: checkerboard pixels, Universe::trace is never called (mod.rs:385-396)
+            // camera in no entity: checkerboard pixels, Universe::trace is never called (mod.rs:385-396).  In a batch with
+            // some frames traced, level 0 holds the checkerboard pixels of the others: they are not counted either.
             const bool traced = s->h_small[SmallLayout::cam_entity] >= 0;
             for (uint32_t lv = 0; traced && lv <= cam->max_depth; ++lv) {
                 uint64_t c = o->pipeline == EUCL_PIPELINE_MEGAKERNEL
                                  ? ((const unsigned long long*)(s->h_small + SmallLayout::mega64))[lv]
                                  : (uint64_t)s->h_small[SmallLayout::count + lv];
+                if (lv == 0) c -= (uint64_t)s->h_small[SmallLayout::untraced];
                 st.level_counts[lv] += c;
                 st.nodes += c;
                 if (lv < cam->max_depth) st.segments += c;
@@ -1397,7 +1447,7 @@ constexpr int kMaxSplit = 8;
 // 3d_room frame whatever its size (profiles/r2_band_scaling.txt) -- 3 % of a 4K frame on one GPU, 20 % of an
 // eighth of it.  Independent pipelines, each on every k-th 16-row band and on streams of its own, fill each other's
 // tails.  The picture cannot depend on it: pixels are independent (mod.rs:316-348).
-int render_split(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, EuclStats* stats) {
+int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, EuclStats* stats) {
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
     uint32_t world = o->band_world > 1 ? o->band_world : 1, rank = world > 1 ? o->band_rank : 0, band = o->band_rows;
     if (band == 0) { // one band: the frame belongs to rank 0
@@ -1408,7 +1458,7 @@ int render_split(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, u
     int k = std::min(kMaxSplit, env_int("EUCL_SPLIT", EUCL_SPLIT_DEFAULT));
     k = (int)std::min<uint32_t>((uint32_t)std::max(k, 1), my_rows / band); // a band or more for every pipeline
     if (o->pipeline != EUCL_PIPELINE_WAVEFRONT || (long long)my_rows * o->width < (long long)env_int("EUCL_SPLIT_MIN_PIXELS", 1 << 16)) k = 1;
-    if (k <= 1) return render_impl(s, cam, o, d_rgb, d_hit, stats);
+    if (k <= 1) return render_impl(s, fb, o, d_rgb, d_hit, stats);
     while ((int)s->twins.size() < k - 1) {
         int rc = add_twin(s);
         if (rc != EUCL_OK) return rc;
@@ -1433,7 +1483,7 @@ int render_split(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, u
     auto pipeline = [&](int p) {
         EuclScene* t = s->twins[p - 1];
         cudaSetDevice(t->device);
-        rc[p] = render_impl(t, cam, &opts[p], d_rgb, d_hit, &part[p], k, p);
+        rc[p] = render_impl(t, fb, &opts[p], d_rgb, d_hit, &part[p], k, p);
         if (rc[p] != EUCL_OK) err[p] = eucl_last_error();
     };
     for (int p = 1; p < k; ++p) {
@@ -1444,7 +1494,7 @@ int render_split(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, u
     }
     // (no early return between here and the last wait(): the helper threads work on this frame's locals)
     for (int p = 1; p < k && !serial; ++p) s->workers[p - 1]->run([&pipeline, p] { pipeline(p); });
-    rc[0] = render_impl(s, cam, &opts[0], d_rgb, d_hit, &part[0], k, 0);
+    rc[0] = render_impl(s, fb, &opts[0], d_rgb, d_hit, &part[0], k, 0);
     for (int p = 1; p < k; ++p) {
         if (serial) pipeline(p);
         else s->workers[p - 1]->wait();
@@ -1492,6 +1542,64 @@ int check_args(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o) {
     return EUCL_OK;
 }
 
+// eucl_render_frames*: every frame as eucl_render would take it, one max_depth, no band split, and a virtual frame whose
+// pixels the chunks can index with 32-bit integers.  Checked before any device is touched.
+int check_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o) {
+    if (!s || !frames || !o) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: null argument");
+    if (n_frames == 0) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: no frames");
+    for (uint32_t k = 0; k < n_frames; ++k) {
+        const int st = check_args(s, &frames[k].camera, o);
+        if (st != EUCL_OK) return st;
+        if (frames[k].camera.max_depth != frames[0].camera.max_depth)
+            return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: the frames of a batch must share max_depth");
+    }
+    if (o->band_world > 1) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: band-split batches are not supported");
+    if (o->compact_rows) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: compact_rows is not supported");
+    if ((uint64_t)n_frames * o->height * o->width > 0x7fffffffull)
+        return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: more than 2^31 - 1 pixels in one batch");
+    return EUCL_OK;
+}
+
+// The batch of `n` frames and the virtual frame they form.  K > 1: the frame constants are computed on the host like
+// a single frame's and uploaded, stream-ordered before the first launch (and outside any graph capture).
+int prepare_batch(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, FrameBatch* fb,
+                  EuclRenderOpts* virt) {
+    *fb = FrameBatch{frames, n, o->height, nullptr, 0};
+    *virt = *o;
+    virt->height = n * o->height;
+    if (n == 1) return EUCL_OK;
+    if (s->h_frame_table_cap < n) {
+        if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
+        s->h_frame_table = nullptr;
+        s->h_frame_table_cap = 0;
+        EUCL_CUDA(cudaMallocHost((void**)&s->h_frame_table, sizeof(FrameParams) * n));
+        s->h_frame_table_cap = n;
+    }
+    uint64_t key = 1469598103934665603ull;
+    for (uint32_t k = 0; k < n; ++k) {
+        EuclRenderOpts one = *o;
+        one.time_seconds = frames[k].time_seconds;
+        frame_params(frames[k].camera, one, s->real_bytes, &s->h_frame_table[k]);
+        const unsigned char* b = (const unsigned char*)&s->h_frame_table[k];
+        for (size_t i = 0; i < sizeof(FrameParams); ++i) key = (key ^ b[i]) * 1099511628211ull;
+    }
+    EUCL_CUDA(s->frame_table.ensure(sizeof(FrameParams) * n));
+    EUCL_CUDA(cudaMemcpyAsync(s->frame_table.ptr, s->h_frame_table, sizeof(FrameParams) * n, cudaMemcpyHostToDevice, s->stream));
+    fb->d_table = (const FrameParams*)s->frame_table.ptr;
+    fb->table_key = key;
+    return EUCL_OK;
+}
+
+// Device-output render of `n` frames (eucl_render_device: n = 1).
+int render_frames_to_device(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* d_rgb,
+                            int32_t* d_hit, EuclStats* stats) {
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    const int st = prepare_batch(s, frames, n, o, &fb, &virt);
+    if (st != EUCL_OK) return st;
+    return render_split(s, fb, &virt, d_rgb, d_hit, stats);
+}
+
 } // namespace
 
 extern "C" {
@@ -1502,7 +1610,38 @@ int eucl_render_device(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts
     if (st != EUCL_OK) return st;
     if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_device: null output");
     EUCL_CUDA(cudaSetDevice(s->device));
-    return render_split(s, cam, o, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
+    const EuclFrame frame{*cam, o->time_seconds};
+    return render_frames_to_device(s, &frame, 1, o, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
+}
+
+int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o,
+                              void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats) {
+    int st = check_frames(s, frames, n_frames, o);
+    if (st != EUCL_OK) return st;
+    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames_device: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
+    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
+                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
+}
+
+int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
+                       int32_t* out_hit_ids, EuclStats* stats) {
+    int st = check_frames(s, frames, n_frames, o);
+    if (st != EUCL_OK) return st;
+    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
+    const size_t pixels = (size_t)n_frames * o->height * o->width;
+    const bool want_hit = o->want_hit_ids && out_hit_ids;
+    EUCL_CUDA(s->frame.ensure(pixels * 3));
+    if (want_hit) EUCL_CUDA(s->hit_ids.ensure(pixels * 4));
+    EuclRenderOpts opts = *o;
+    opts.want_hit_ids = want_hit ? 1 : 0;
+    st = render_frames_to_device(s, frames, n_frames, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));
+    if (want_hit) EUCL_CUDA(cudaMemcpyAsync(out_hit_ids, s->hit_ids.ptr, pixels * 4, cudaMemcpyDeviceToHost, s->stream));
+    EUCL_CUDA(cudaStreamSynchronize(s->stream));
+    return EUCL_OK;
 }
 
 int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
@@ -1524,7 +1663,8 @@ int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
     EuclRenderOpts opts = *o;
     opts.want_hit_ids = want_hit ? 1 : 0;
     if (scatter) opts.compact_rows = 1;
-    st = render_split(s, cam, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
+    const EuclFrame frame{*cam, o->time_seconds};
+    st = render_frames_to_device(s, &frame, 1, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
     if (st != EUCL_OK) return st;
     if (!scatter) {
         EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));

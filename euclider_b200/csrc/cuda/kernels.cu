@@ -320,16 +320,38 @@ __device__ __forceinline__ Rgba checkerboard(int x, int y) { // mod.rs:387-395
 // ---------------------------------------------------------------------------------------------
 // kernels
 
-// material_at(camera location) is the same for every pixel of a frame: computed once.
+// material_at(camera location) is the same for every pixel of a frame: computed once (a batch: once per frame, and
+// cam_entity says whether any frame is traced at all).
 template <int D>
 __global__ void __launch_bounds__(32) k_camera_entity(const uint8_t* __restrict__ blob, FrameParams fp, Workspace ws) {
     const SceneView& sv = stage_scene(blob);
-    if (threadIdx.x == 0) {
+    if (!ws.frames) {
+        if (threadIdx.x == 0) {
+            Vec<D> loc;
+#pragma unroll
+            for (int k = 0; k < D; ++k) loc[k] = R(fp.location[k]);
+            *ws.cam_entity = material_at<D>(sv, loc);
+        }
+        return;
+    }
+    bool traced = false;
+    for (int f = threadIdx.x; f < ws.n_frames; f += blockDim.x) {
         Vec<D> loc;
 #pragma unroll
-        for (int k = 0; k < D; ++k) loc[k] = R(fp.location[k]);
-        *ws.cam_entity = material_at<D>(sv, loc);
+        for (int k = 0; k < D; ++k) loc[k] = R(ws.frames[f].location[k]);
+        const int e = material_at<D>(sv, loc);
+        ws.frame_entity[f] = e;
+        traced = traced || e >= 0;
     }
+    traced = __any_sync(0xffffffffu, traced);
+    if (threadIdx.x == 0) *ws.cam_entity = traced ? 0 : -1;
+}
+
+// Frame of virtual row `y` of a batch; `y` becomes the row within that frame.
+__device__ __forceinline__ int frame_of_row(const Workspace& ws, int& y) {
+    const int f = y / ws.frame_rows;
+    y -= f * ws.frame_rows;
+    return f;
 }
 
 // K1: one primary ray per pixel of the chunk; level 0 of the node arena is the pixel order.
@@ -337,44 +359,58 @@ template <int D>
 __global__ void __launch_bounds__(kBlock) k_raygen(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
                                                    Workspace ws, int32_t* __restrict__ hit_ids_out) {
     const SceneView& sv = stage_scene(blob);
+    const bool batch = ws.frames != nullptr;
     Vec<D> loc;
 #pragma unroll
     for (int k = 0; k < D; ++k) loc[k] = R(fp.location[k]);
     // material_at(camera location) is the same for every pixel of a frame: one thread per CTA evaluates it (a few hundred
-    // instructions) instead of a kernel of its own in front of this one
+    // instructions) instead of a kernel of its own in front of this one.  A batch reads its frames' entities from the
+    // table k_camera_entity filled (a CTA's pixels may belong to several frames).
     __shared__ int s_cam_entity;
     if (threadIdx.x == 0) {
-        s_cam_entity = material_at<D>(sv, loc);
+        if (!batch) s_cam_entity = material_at<D>(sv, loc);
         if (blockIdx.x == 0) {
-            *ws.cam_entity = s_cam_entity;
+            if (!batch) *ws.cam_entity = s_cam_entity;
             ws.count[0] = cp.n_pixels;
             ws.level_off[0] = 0;
         }
     }
     __syncthreads();
-    const int belongs_to = s_cam_entity;
     const unsigned lane = threadIdx.x & 31u;
     for (int base = blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < cp.n_pixels; base += gridDim.x * blockDim.x) {
         const int i = base + (int)lane;
         const bool valid = i < cp.n_pixels;
         const int local_row = cp.local_row0 + (valid ? i : 0) / fp.width;
         const int x = (valid ? i : 0) % fp.width;
-        const int y = frame_row_of_local(cp, local_row);
-        if (belongs_to < 0) { // the same for every pixel of the frame
+        int y = frame_row_of_local(cp, local_row);
+        int belongs_to = s_cam_entity, f = 0;
+        if (batch) {
+            f = frame_of_row(ws, y);
+            belongs_to = ws.frame_entity[f];
+#pragma unroll
+            for (int k = 0; k < D; ++k) loc[k] = R(ws.frames[f].location[k]);
+            if (valid) ws.node_frame[i] = f;
+            const unsigned untraced = __ballot_sync(0xffffffffu, valid && belongs_to < 0);
+            if (lane == 0 && untraced) atomicAdd(ws.untraced, __popc(untraced));
+        }
+        if (belongs_to < 0) { // a single frame: the same for every pixel
             if (valid) {
                 store_res(ws, i, checkerboard(x, y));
                 ws.meta[i] = NodeMeta{R(0.0), -1, -1, 0u, NODE_LEAF | NODE_FINAL_RGB};
                 ws.ray_cur[i] = -1;
                 if (hit_ids_out) hit_ids_out[(size_t)out_row_of_local(cp, local_row) * fp.width + x] = -2;
             }
-            continue;
+            // a batch goes on: the node gets a well-defined ray (k_intersect may walk it when the level is not grouped by
+            // reach key); ray_cur -1 keeps k_shade off it
+            if (!batch) continue;
         }
-        Vec<D> dir = camera_ray<D>(fp, x, y);
-        material_enter<D>(sv, belongs_to, dir);
-        if (valid) store_ray<D>(ws, i, loc, dir, belongs_to);
+        const bool traced = belongs_to >= 0;
+        Vec<D> dir = batch ? camera_ray<D>(ws.frames[f], x, y) : camera_ray<D>(fp, x, y);
+        if (traced) material_enter<D>(sv, belongs_to, dir);
+        if (valid) store_ray<D>(ws, i, loc, dir, traced ? belongs_to : -1);
         if (ws.ray_bins) { // group the primary rays by reach key like k_shade groups the children (one atomicAdd per warp and key)
-            const unsigned active = __ballot_sync(0xffffffffu, valid);
-            if (valid) {
+            const unsigned active = __ballot_sync(0xffffffffu, valid && traced);
+            if (valid && traced) {
                 const int key = reach_key<D>(sv, loc, dir);
                 const unsigned peers = __match_any_sync(active, key);
                 const int leader = __ffs(peers) - 1;
@@ -506,7 +542,10 @@ __global__ void __launch_bounds__(LIGHT ? kLightK2Block : kBlock, LIGHT ? EUCL_I
 // plus the rays that hit nothing; without the Fresnel / Snell / general_rotation code it needs far fewer registers
 // and keeps more warps resident.  The HEAVY one (GLASS = true) shades the remaining bins (and everything when the
 // level is not binned).  `bin_mask` selects the bins of a launch.
-template <int D, bool RAY_BINS, bool GLASS>
+//
+// FRAMES: a batch of frames (Workspace::node_frame): Perlin time from the node's frame, children tagged with it.  A build of
+// its own so that the single-frame builds carry none of it.
+template <int D, bool RAY_BINS, bool GLASS, bool FRAMES>
 __global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUCL_SHADE_MIN_BLOCKS : EUCL_SHADE_LIGHT_MIN_BLOCKS)
     k_shade(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp, Workspace ws, int level, unsigned long long bin_mask,
             int32_t* __restrict__ hit_ids_out) {
@@ -591,7 +630,8 @@ __global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUC
             } else {
                 const Vec<D> p = o + d * ei.t; // the intersectors' expression for the hit location (shape.rs:700,795,993)
                 Rgba sc;
-                shade_decide<D, GLASS>(sv, R(fp.time_millis), ei.entity, ei.exiting != 0, ei.cos_raw, ei.angle_raw, p, n, dec, sc);
+                const real time_millis = R(FRAMES ? ws.frames[ws.node_frame[node]].time_millis : fp.time_millis);
+                shade_decide<D, GLASS>(sv, time_millis, ei.entity, ei.exiting != 0, ei.cos_raw, ei.angle_raw, p, n, dec, sc);
                 if (dec.flags & NODE_HAS_SC) {
                     store_res(ws, node, sc);
                     if (!dec.r_emit) dec.flags |= NODE_LEAF; // opaque without a mirror term: the colour is final
@@ -633,12 +673,14 @@ __global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUC
                     tchild = next_off + slot + __popc(tmask & lt);
                     transmit_child<D, GLASS>(sv, d, cur, ei.entity, exiting, p, n, dec, child);
                     store_ray<D>(ws, tchild, child.o, child.d, child.cur);
+                    if (FRAMES) ws.node_frame[tchild] = ws.node_frame[node]; // a batch: the children belong to their parent's frame
                     if (RAY_BINS) tkey = reach_key<D>(sv, child.o, child.d);
                 }
                 if (dec.r_emit) {
                     rchild = next_off + slot + nt + __popc(rmask & lt);
                     reflect_child<D>(d, cur, exiting, p, n, child);
                     store_ray<D>(ws, rchild, child.o, child.d, child.cur);
+                    if (FRAMES) ws.node_frame[rchild] = ws.node_frame[node];
                     if (RAY_BINS) rkey = reach_key<D>(sv, child.o, child.d);
                 }
             }
@@ -759,25 +801,32 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
                                                        int32_t* __restrict__ hit_ids_out) {
     const SceneView& sv = stage_scene(blob);
     real* ts = plane_scratch(blob);
-    const int belongs_to = *ws.cam_entity;
+    const int cam_entity = *ws.cam_entity;
     unsigned long long local_counts[kMegaMaxDepth + 1];
     for (int l = 0; l <= kMegaMaxDepth; ++l) local_counts[l] = 0ull;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < cp.n_pixels; i += gridDim.x * blockDim.x) {
         const int local_row = cp.local_row0 + i / fp.width;
         const int x = i % fp.width;
-        const int y = frame_row_of_local(cp, local_row);
+        int y = frame_row_of_local(cp, local_row);
         const size_t opix = (size_t)out_row_of_local(cp, local_row) * fp.width + x;
+        int belongs_to = cam_entity, f = 0;
+        if (ws.frames) {
+            f = frame_of_row(ws, y);
+            belongs_to = ws.frame_entity[f];
+        }
         if (belongs_to < 0) {
             final_rgb8(checkerboard(x, y), false, out_rgb8 + opix * 3);
             if (hit_ids_out) hit_ids_out[opix] = -2;
             local_counts[0]++;
+            if (ws.frames) atomicAdd(ws.untraced, 1);
             continue;
         }
         MegaFrame<D> stack[kMegaMaxDepth];
         Vec<D> o, d;
 #pragma unroll
-        for (int k = 0; k < D; ++k) o[k] = R(fp.location[k]);
-        d = camera_ray<D>(fp, x, y);
+        for (int k = 0; k < D; ++k) o[k] = R(ws.frames ? ws.frames[f].location[k] : fp.location[k]);
+        d = ws.frames ? camera_ray<D>(ws.frames[f], x, y) : camera_ray<D>(fp, x, y);
+        const real time_millis = R(ws.frames ? ws.frames[f].time_millis : fp.time_millis);
         material_enter<D>(sv, belongs_to, d);
         int cur = belongs_to, level = 0;
         Rgba val{R(0.0), R(0.0), R(0.0), R(0.0)};
@@ -795,7 +844,7 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
                 val = mapped_color<D>(sv, sv.background, d);
             } else {
                 ShadeOut<D> so;
-                shade_hit<D, true>(sv, R(fp.time_millis), d, cur, ent, exiting, cos_raw, angle_raw, p, n, so);
+                shade_hit<D, true>(sv, time_millis, d, cur, ent, exiting, cos_raw, angle_raw, p, n, so);
                 if (so.flags & NODE_UNDEFINED) {
                     val = Rgba{R(0.0), R(0.0), R(0.0), R(0.0)};
                     atomicAdd(ws.undefined_count, 1ull);
@@ -968,6 +1017,7 @@ inline int grid_for(int n, int block, int grid_max) {
         else { CALL4; }                      \
     } while (0)
 
+// (a batch: in front of k_raygen as well, one thread per frame)
 void launch_camera_entity(int dim, const Launch& l, const FrameParams& fp, const Workspace& ws) {
     EUCL_DISPATCH_DIM(dim, (k_camera_entity<3><<<1, 32, l.smem_scene, l.stream>>>(l.blob, fp, ws)),
                       (k_camera_entity<4><<<1, 32, l.smem_scene, l.stream>>>(l.blob, fp, ws)));
@@ -1013,11 +1063,17 @@ int launch_intersect(int dim, const Launch& l, const Workspace& ws, int level) {
     if (fork) join_side(l);
     return launches;
 }
+template <int D, bool RAY_BINS, bool GLASS, bool FRAMES>
+static void launch_shade_build(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
+                               int level, unsigned long long mask, int32_t* hit_ids_out) {
+    if (GLASS) k_shade<D, RAY_BINS, true, FRAMES><<<l.grid_shade, kShadeBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
+    else k_shade<D, RAY_BINS, false, FRAMES><<<l.grid_light, kLightBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
+}
 template <int D, bool RAY_BINS, bool GLASS>
 static void launch_shade_one(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
                              int level, unsigned long long mask, int32_t* hit_ids_out) {
-    if (GLASS) k_shade<D, RAY_BINS, true><<<l.grid_shade, kShadeBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
-    else k_shade<D, RAY_BINS, false><<<l.grid_light, kLightBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
+    if (ws.node_frame) launch_shade_build<D, RAY_BINS, GLASS, true>(l, stream, fp, cp, ws, level, mask, hit_ids_out);
+    else launch_shade_build<D, RAY_BINS, GLASS, false>(l, stream, fp, cp, ws, level, mask, hit_ids_out);
 }
 template <int D, bool GLASS>
 static void launch_shade_dim(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
@@ -1114,14 +1170,22 @@ cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene) {
     const size_t smem_light = smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block;
     EUCL_CONF((k_intersect<3, true>), smem_light, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
     EUCL_CONF((k_intersect<4, true>), smem_light, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
-    EUCL_CONF((k_shade<3, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, false, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, false, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, true, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, true, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<3, false, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, false, false>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<3, true, true, false>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<4, true, true, false>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<3, false, true, false>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<4, false, true, false>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<3, true, false, false>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<4, true, false, false>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<3, false, false, false>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<4, false, false, false>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<3, true, true, true>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<4, true, true, true>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<3, false, true, true>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<4, false, true, true>), smem_scene, kShadeResidentBlocks);
+    EUCL_CONF((k_shade<3, true, false, true>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<4, true, false, true>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<3, false, false, true>), smem_scene, kLightResidentBlocks);
+    EUCL_CONF((k_shade<4, false, false, true>), smem_scene, kLightResidentBlocks);
     EUCL_CONF(k_background<3>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
     EUCL_CONF(k_background<4>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
     EUCL_CONF(k_megakernel<3>, smem_bytes, heavy);

@@ -95,17 +95,23 @@ struct Workspace {
     int32_t* count;     // [EUCL_MAX_LEVELS + 1] nodes per level
     int32_t* level_off; // [EUCL_MAX_LEVELS + 1] first node id of each level
     int32_t* overflow;  // 1: a child could not be appended (arena); 3: a level outgrew the index lists; 2: internal error
-    int32_t* cam_entity; // material_at(camera location), -1 if none
+    int32_t* cam_entity; // material_at(camera location), -1 if none; a batch: -1 when no frame's camera is in an entity
     int32_t n_bins;      // 1: shade in node order; else kBinsPerEntity * n_entities + 1 bins keyed by (hit entity, class), 0 = miss
-    int32_t _pad2;
+    int32_t frame_rows;  // a batch of frames (frames != nullptr): rows per frame of the virtual frame
     int32_t* bin_count;  // [EUCL_MAX_LEVELS + 1][kMaxBins] nodes per (level, hit-entity bin)
     int32_t* order;      // [n_bins][list_cap] node ids of the current level grouped by bin (reused per level)
     int32_t ray_bins;    // 1: the rays of a level are walked grouped by reach key (see SceneHeader::cull_root)
-    int32_t _pad3;
+    int32_t n_frames;    // frames of a batch (1: a single frame)
     int32_t* rbin_count; // [EUCL_MAX_LEVELS + 1][kRayBins]
     int32_t* rorder;     // [kRayBins][list_cap] node ids of the NEXT level grouped by reach key
     unsigned long long* undefined_count;   // nodes that touched a corner the reference leaves undefined
     unsigned long long* mega_level_counts; // [EUCL_MAX_LEVELS + 1] nodes per level, megakernel pipeline only
+    // A batch of frames rendered as ONE virtual frame of n_frames * frame_rows rows: virtual row r is row r % frame_rows
+    // of frame r / frame_rows.  All four are null for a single frame, which reads FrameParams / cam_entity instead.
+    const FrameParams* frames; // [n_frames] per-frame constants (pose, time)
+    int32_t* frame_entity;     // [n_frames] material_at(camera location of the frame), -1 if none
+    int32_t* node_frame;       // [capacity] frame of every node (Perlin time): level 0 by k_raygen, children by k_shade
+    int32_t* untraced;         // level-0 nodes of this chunk whose frame's camera is in no entity (checkerboard pixels)
 };
 
 struct Launch {

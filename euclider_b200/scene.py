@@ -17,7 +17,7 @@ from typing import Dict, Optional, Sequence, Tuple, Union
 import numpy as np
 
 from . import _capi
-from ._capi import (EuclCamera, EuclError, EuclFlatScene, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL,
+from ._capi import (EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL,
                     EUCL_PIPELINE_WAVEFRONT, check, lib)
 
 ParserError = EuclError  # the reference's `ParserError` (src/scene.rs:524-552); see EuclError.status
@@ -56,6 +56,43 @@ class RawImage2d:
             from PIL import Image
 
             Image.fromarray(np.ascontiguousarray(self.to_top_down())).save(path)
+
+
+@dataclass
+class RawFrames:
+    """The frames of one Environment.render_frames call: frame k is data[k], RGB8, row 0 = bottom."""
+    data: np.ndarray  # uint8, shape (K, height, width, 3)
+    width: int
+    height: int
+    hit_ids: Optional[np.ndarray] = None  # int32 (K, height, width), as RawImage2d.hit_ids
+    stats: Optional[dict] = None  # summed over the K frames
+
+    def __len__(self) -> int:
+        return int(self.data.shape[0])
+
+    def frame(self, k: int) -> RawImage2d:
+        """Frame k as a RawImage2d (a view, no copy)."""
+        return RawImage2d(self.data[k], self.width, self.height, hit_ids=None if self.hit_ids is None else self.hit_ids[k])
+
+
+def _frame_table(cameras: Sequence[EuclCamera], times) -> C.Array:
+    """EuclFrame[K] from K cameras and a time per frame (or one time for all)."""
+    cameras = list(cameras)
+    if not cameras:
+        raise ValueError("render_frames needs at least one camera")
+    if any(not isinstance(c, EuclCamera) for c in cameras):
+        raise TypeError("cameras must be EuclCamera poses (e.g. Environment.camera.copy())")
+    if np.ndim(times) == 0:
+        times = [float(times)] * len(cameras)
+    else:
+        times = [float(t) for t in times]
+        if len(times) != len(cameras):
+            raise ValueError(f"{len(cameras)} cameras but {len(times)} times")
+    table = (EuclFrame * len(cameras))()
+    for k, (cam, t) in enumerate(zip(cameras, times)):
+        table[k].camera = cam
+        table[k].time_seconds = t
+    return table
 
 
 def _decode_image(path: Path) -> Tuple[int, int, bytes]:
@@ -130,6 +167,42 @@ class Environment:
         check(lib().eucl_render_device(self._device_scene(device), C.byref(self.camera), C.byref(opts),
                                        C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
                                        C.byref(stats)))
+        return stats_to_dict(stats)
+
+    # -- many frames per call: camera paths and animations -------------------------------------------
+    def render_frames(self, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera], times=0.0,
+                      context: Optional[SimulationContext] = None, *, device: int = 0, want_hit_ids: bool = False,
+                      out: Optional[np.ndarray] = None, profile: bool = False) -> RawFrames:
+        """Renders one frame per camera pose in ONE call (eucl_render_frames): frame k equals
+        `render(dimensions, times[k])` with `self.camera` set to `cameras[k]`, bit for bit.  `times` is one time for
+        every frame or a sequence of one per frame.  Batching pays the fixed cost of a frame once per call."""
+        table = _frame_table(cameras, times)
+        context = context or SimulationContext()
+        width, height = int(dimensions[0]) // context.resolution, int(dimensions[1]) // context.resolution
+        k = len(table)
+        if out is None:
+            out = np.zeros((k, height, width, 3), dtype=np.uint8)
+        if out.dtype != np.uint8 or out.shape != (k, height, width, 3) or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {(k, height, width, 3)}")
+        opts = EuclRenderOpts(width=width, height=height, pipeline=self.pipeline, want_hit_ids=int(want_hit_ids),
+                              profile=int(profile))
+        hit = np.full((k, height, width), -3, dtype=np.int32) if want_hit_ids else None
+        stats = EuclStats()
+        check(lib().eucl_render_frames(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
+                                       hit.ctypes.data if hit is not None else None, C.byref(stats)))
+        return RawFrames(out, width, height, hit_ids=hit, stats=stats_to_dict(stats))
+
+    def render_frames_device(self, d_out_rgb8: int, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera],
+                             times=0.0, *, device: int = 0, d_out_hit_ids: int = 0, profile: bool = False) -> dict:
+        """render_frames into device buffers: K * height * width * 3 bytes (and K * height * width int32 hit ids)."""
+        table = _frame_table(cameras, times)
+        width, height = int(dimensions[0]), int(dimensions[1])
+        opts = EuclRenderOpts(width=width, height=height, pipeline=self.pipeline, want_hit_ids=int(bool(d_out_hit_ids)),
+                              profile=int(profile))
+        stats = EuclStats()
+        check(lib().eucl_render_frames_device(self._device_scene(device), table, len(table), C.byref(opts),
+                                              C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
+                                              C.byref(stats)))
         return stats_to_dict(stats)
 
     def trace_path_unknown(self, location: Sequence[float], direction: Sequence[float], distance: float, *,

@@ -326,6 +326,32 @@ int eucl_render(EuclScene* scene, const EuclCamera* camera, const EuclRenderOpts
 int eucl_render_device(EuclScene* scene, const EuclCamera* camera, const EuclRenderOpts* opts,
                        void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats);
 
+/* One frame of a batch: the pose (fov, max_depth) as for eucl_render, and the time that EuclRenderOpts.time_seconds
+ * would carry (Perlin only, truncated to whole ms). */
+typedef struct EuclFrame {
+    EuclCamera camera;
+    double time_seconds;
+} EuclFrame;
+
+/* K = n_frames frames of opts->width x opts->height -- a camera path, a turntable, an animation -- rendered as ONE
+ * wavefront: the fixed cost of a frame (its ~30 dependent kernel launches) is paid once per batch, not per frame.
+ * Output frame k occupies rows [k*height, (k+1)*height) of a K*height-row RGB8 buffer (each frame bottom-up, as
+ * eucl_render); hit ids likewise K*height*width int32.  Frame k is bit-identical to eucl_render(scene,
+ * &frames[k].camera, opts with time_seconds = frames[k].time_seconds).  EuclStats are the sums over the frames
+ * (ms_total: the whole batch).  Synchronous.
+ * Frames may differ in location, axes, fov and time; every frame must have the scene's dim and the same max_depth.
+ * opts->time_seconds is ignored.  EUCL_ERR_INVALID_ARGUMENT, before any device work, for n_frames == 0, a null
+ * `frames`, differing max_depth, band_world > 1 or compact_rows = 1 (band-split batches are not supported), and
+ * batches of more than 2^31 - 1 pixels.  A batch of identical frames replays its CUDA graph like a repeated
+ * eucl_render; a batch with any pose or time changed is launched anew. */
+int eucl_render_frames(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
+                       uint8_t* out_rgb8, int32_t* out_hit_ids, EuclStats* stats);
+
+/* Same, with DEVICE output buffers on the scene's device (K*height*width*3 bytes, and K*height*width int32 hit ids
+ * when opts->want_hit_ids).  Synchronous. */
+int eucl_render_frames_device(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
+                              void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats);
+
 /* Universe::trace_path_unknown (src/universe/mod.rs:273-286): moves `location` by `distance` along
  * `direction` THROUGH the universe -- surfaces are crossed with the material transitions of the
  * entities on either side, so a step through a LinearSpace void is stretched or shrunk.  The

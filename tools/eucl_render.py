@@ -3,6 +3,13 @@
 
     python tools/eucl_render.py assets/scenes/3d_room.json out.png --size 1920 1080 [--time 1.5]
         [--resource-root assets] [--location x y z [w]] [--max-depth N] [--pipeline megakernel]
+
+Image sequences -- a camera path, a turntable, a Perlin animation -- with --frames N: frame k is the pose after k steps
+of the per-frame motion and the time --time + k * --time-step; the output name takes a printf pattern.  Frames are
+rendered --batch at a time (default: all in one call, Environment.render_frames).
+
+    python tools/eucl_render.py assets/scenes/3d_room.json out_%04d.ppm --size 128 96 --frames 64 \\
+        --move 0 0.05 0 --yaw 0.02 --time-step 0.04
 """
 import argparse
 import sys
@@ -14,10 +21,10 @@ sys.path.insert(0, str(ROOT))
 import euclider_b200 as eb  # noqa: E402
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("scene")
-    ap.add_argument("output")
+    ap.add_argument("output", help="image path; with --frames > 1 a printf pattern such as out_%%04d.ppm")
     ap.add_argument("--size", type=int, nargs=2, default=(1920, 1080))
     ap.add_argument("--time", type=float, default=0.0)
     ap.add_argument("--resource-root", default=str(eb.ASSET_ROOT))
@@ -25,7 +32,53 @@ def main():
     ap.add_argument("--max-depth", type=int)
     ap.add_argument("--resolution", type=int, default=1, help="the reference's resolution divisor")
     ap.add_argument("--pipeline", default="wavefront", choices=["wavefront", "megakernel"])
-    args = ap.parse_args()
+    seq = ap.add_argument_group("image sequences (per-frame motion; angles in radians)")
+    seq.add_argument("--frames", type=int, default=1, help="frames to render")
+    seq.add_argument("--batch", type=int, help="frames per render call (default: all)")
+    seq.add_argument("--move", type=float, nargs="+", metavar="D",
+                     help="dx dy dz [dw]: camera step per frame through the universe (Environment.move_camera)")
+    seq.add_argument("--yaw", type=float, default=0.0, help="3-D: yaw per frame")
+    seq.add_argument("--pitch", type=float, default=0.0, help="3-D: pitch per frame")
+    seq.add_argument("--roll", type=float, default=0.0, help="3-D: roll per frame")
+    seq.add_argument("--plane4", type=float, nargs=3, metavar=("A", "B", "ANGLE"),
+                     help="4-D: rotation per frame in the plane of camera axes A and B (0 forward, 1 left, 2 up, 3 ana)")
+    seq.add_argument("--time-step", type=float, default=0.0, help="seconds added to the time per frame")
+    args = ap.parse_args(argv)
+    if args.frames < 1:
+        ap.error("--frames must be at least 1")
+    if args.batch is not None and args.batch < 1:
+        ap.error("--batch must be at least 1")
+    if args.move is not None and len(args.move) not in (3, 4):
+        ap.error("--move takes 3 or 4 components")
+    if args.plane4 is not None and (args.plane4[0] != int(args.plane4[0]) or args.plane4[1] != int(args.plane4[1])):
+        ap.error("--plane4: A and B are axis indices")
+    if args.frames > 1 and "%" not in args.output:
+        ap.error("--frames > 1 needs an output pattern such as out_%04d.ppm")
+    return args
+
+
+def is_sequence(args) -> bool:
+    """True when the new per-frame options are in use; otherwise the tool renders one frame with Environment.render."""
+    return (args.frames > 1 or args.batch is not None or args.move is not None or args.yaw or args.pitch or args.roll
+            or args.plane4 is not None or args.time_step or "%" in args.output)
+
+
+def step_camera(env, args) -> None:
+    """One frame's motion: the translation through the universe, then the turns."""
+    if args.move is not None and not env.move_camera(args.move, 1.0):
+        print("warning: the camera is in no entity; it stays where it is", file=sys.stderr)
+    if args.yaw:
+        env.rotate_yaw(args.yaw)
+    if args.pitch:
+        env.rotate_pitch(args.pitch)
+    if args.roll:
+        env.rotate_roll(args.roll)
+    if args.plane4 is not None:
+        env.rotate_plane4(int(args.plane4[0]), int(args.plane4[1]), args.plane4[2])
+
+
+def main(argv=None):
+    args = parse_args(argv)
     env = eb.Parser.default(resource_root=args.resource_root).parse_file(args.scene)
     if args.location:
         for k, v in enumerate(args.location[:env.dim]):
@@ -33,10 +86,29 @@ def main():
     if args.max_depth is not None:
         env.camera.max_depth = args.max_depth
     env.pipeline = eb.EUCL_PIPELINE_MEGAKERNEL if args.pipeline == "megakernel" else eb.EUCL_PIPELINE_WAVEFRONT
-    img = env.render(tuple(args.size), args.time, context=eb.SimulationContext(resolution=args.resolution))
-    img.save(args.output)
-    st = img.stats
-    print(f"{args.output}: {img.width}x{img.height}, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
+    context = eb.SimulationContext(resolution=args.resolution)
+    if not is_sequence(args):
+        img = env.render(tuple(args.size), args.time, context=context)
+        img.save(args.output)
+        st = img.stats
+        print(f"{args.output}: {img.width}x{img.height}, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
+        return
+    cameras, times = [], []
+    for k in range(args.frames):
+        if k > 0:
+            step_camera(env, args)
+        cameras.append(env.camera.copy())
+        times.append(args.time + k * args.time_step)
+    batch = args.batch or args.frames
+    segments, ms = 0, 0.0
+    for k0 in range(0, args.frames, batch):
+        frames = env.render_frames(tuple(args.size), cameras[k0:k0 + batch], times[k0:k0 + batch], context=context)
+        for j in range(len(frames)):
+            frames.frame(j).save(args.output % (k0 + j))
+        segments += frames.stats["segments"]
+        ms += frames.stats["ms_total"]
+    print(f"{args.output}: {args.frames} frames of {frames.width}x{frames.height} in calls of {batch}, {segments} ray segments, "
+          f"{ms:.2f} ms on the device")
 
 
 if __name__ == "__main__":
