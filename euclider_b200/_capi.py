@@ -75,6 +75,11 @@ class EuclFrame(C.Structure):
     _fields_ = [("camera", EuclCamera), ("time_seconds", C.c_double)]
 
 
+class EuclAovs(C.Structure):
+    _fields_ = [("depth", C.c_void_p), ("position", C.c_void_p), ("normal", C.c_void_p), ("segments", C.c_void_p),
+                ("levels", C.c_void_p)]
+
+
 class EuclFlatScene(C.Structure):
     _fields_ = [("dim", C.c_int32),
                 ("n_prims", C.c_int32), ("n_nodes", C.c_int32), ("n_entities", C.c_int32),
@@ -148,6 +153,10 @@ PROTOTYPES = {
                                      C.c_void_p, C.POINTER(EuclStats)]),
     "eucl_render_frames_device": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts),
                                             C.c_void_p, C.c_void_p, C.POINTER(EuclStats)]),
+    "eucl_render_aovs": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts), C.c_void_p,
+                                   C.c_void_p, C.POINTER(EuclAovs), C.POINTER(EuclStats)]),
+    "eucl_render_aovs_device": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts),
+                                          C.c_void_p, C.c_void_p, C.POINTER(EuclAovs), C.POINTER(EuclStats)]),
     "eucl_trace_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,
                                   C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "eucl_camera_rotate_yaw": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),

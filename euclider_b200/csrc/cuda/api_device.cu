@@ -145,6 +145,8 @@ struct EuclScene {
     uint32_t h_frame_table_cap = 0;
     DeviceBuffer frame_entity;
     DeviceBuffer node_frame;
+    DeviceBuffer node_cost; // (segments, levels) per node of this pipeline's arena: AOV renders that want either plane
+    DeviceBuffer aov_stage; // device copies of the AOV planes for eucl_render_aovs (host output)
     int n_cull = 0;
     int light_capable = 0;
     // Grouping rays by reach key pays on scenes whose deep levels bounce around a few bounded objects
@@ -676,6 +678,8 @@ void eucl_scene_destroy(EuclScene* s) {
     s->frame_table.release();
     s->frame_entity.release();
     s->node_frame.release();
+    s->node_cost.release();
+    s->aov_stage.release();
     if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
     if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
     if (s->h_small) cudaFreeHost(s->h_small);
@@ -1068,7 +1072,7 @@ void tune_grouping(EuclScene* s, const EuclStats& st, int pipeline) {
 // sub_stride-th band of the caller's rank starting at sub_offset: render_split).
 // `o` describes the (virtual) frame: o->height = fb.n * fb.rows.
 int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
-                EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
+                const AovPlanes& aov_out, EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
     const int dim = s->dim;
     const EuclCamera* cam = &fb.frames[0].camera; // (every frame of a batch has this max_depth)
     FrameParams fp;
@@ -1112,7 +1116,11 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
         // shade-coherence bins: one node list per hit entity (+ miss), each able to hold a whole level
         const bool want_order = o->pipeline == EUCL_PIPELINE_WAVEFRONT && kBinsPerEntity * s->n_entities + 1 <= kMaxBins && env_int("EUCL_BIN_SHADE", 1);
         const size_t n_lists = (want_rorder ? (size_t)kRayBins : 0) + (want_order ? (size_t)(kBinsPerEntity * s->n_entities + 1) : 0);
-        auto workspace_bytes = [&](size_t cap, size_t list_cap) { return arena_bytes(dim, s->real_bytes, cap) + sizeof(int32_t) * n_lists * list_cap; };
+        // the COST builds keep a (segments, levels) pair per node next to the arena
+        const bool want_cost = o->pipeline == EUCL_PIPELINE_WAVEFRONT && (aov_out.segments || aov_out.levels);
+        auto workspace_bytes = [&](size_t cap, size_t list_cap) {
+            return arena_bytes(dim, s->real_bytes, cap) + sizeof(int32_t) * n_lists * list_cap + (want_cost ? sizeof(uint2) * cap : 0);
+        };
 
         for (int row0 = 0; row0 < (int)my_rows;) {
             ChunkParams cp{};
@@ -1137,7 +1145,7 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                     want_list = std::max<long long>(want_list, s->list_capacity);
                     size_t free_b = 0, total_b = 0;
                     EUCL_CUDA(cudaMemGetInfo(&free_b, &total_b));
-                    const size_t held = s->nodes.bytes + s->order.bytes + s->rorder.bytes;
+                    const size_t held = s->nodes.bytes + s->order.bytes + s->rorder.bytes + s->node_cost.bytes;
                     size_t budget = (size_t)((double)(free_b + held) * 0.85);
                     const int cap_mb = env_int("EUCL_ARENA_MAX_MB", 0);
                     if (cap_mb > 0) budget = std::min(budget, (size_t)cap_mb << 20);
@@ -1154,6 +1162,7 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                             s->nodes.release();
                             s->rorder.release();
                             s->order.release();
+                            s->node_cost.release();
                             s->arena_capacity = 0;
                             s->list_capacity = 0;
                             if (e != cudaErrorMemoryAllocation) return fail(EUCL_ERR_CUDA, std::string("workspace allocation: ") + cudaGetErrorString(e));
@@ -1168,7 +1177,10 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                     continue;
                 }
                 if (fb.n > 1) EUCL_CUDA(s->node_frame.ensure(sizeof(int32_t) * (size_t)s->arena_capacity));
+                if (want_cost) EUCL_CUDA(s->node_cost.ensure(sizeof(uint2) * (size_t)s->arena_capacity));
                 Workspace ws = carve(s, dim, s->arena_capacity, s->list_capacity, fb);
+                AovPlanes aov = aov_out;
+                aov.cost = want_cost ? (uint2*)s->node_cost.ptr : nullptr;
                 // profile mode: one event after every launch; family = 0 raygen, 1 intersect, 2 shade, 3 resolve
                 std::vector<int> prof_family;
                 auto mark = [&](int family) {
@@ -1208,7 +1220,7 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                     if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL) {
                         EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
                         dbg("k_camera_entity", 0);
-                        EUCL_PREC(launch_megakernel)(dim, l, fp, cp, ws, d_rgb, d_hit);
+                        EUCL_PREC(launch_megakernel)(dim, l, fp, cp, ws, d_rgb, d_hit, aov);
                         mark(1);
                         launches += 2;
                     } else {
@@ -1235,7 +1247,7 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                         launches += EUCL_PREC(launch_shade)(dim, l, fp, cp, ws, (int)cam->max_depth, d_hit);
                         dbg("k_shade", (int)cam->max_depth);
                         mark(2);
-                        launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fp, cp, ws, d_rgb);
+                        launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fp, cp, ws, d_rgb, aov);
                         dbg("k_resolve / k_final", 0);
                         mark(3);
                         launches += 1; // raygen
@@ -1267,6 +1279,9 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                 }
                 mix(&d_rgb, sizeof d_rgb);
                 mix(&d_hit, sizeof d_hit);
+                // the AOV planes a chunk writes (null = not wanted) and the cost buffer: a graph captured with or without
+                // them never stands in for the other
+                mix(&aov, sizeof aov);
                 const int pipeline_id = o->pipeline;
                 mix(&pipeline_id, sizeof pipeline_id);
                 const uint32_t depth_id = cam->max_depth;
@@ -1385,6 +1400,7 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
             s->nodes.release();
             s->order.release();
             s->rorder.release();
+            s->node_cost.release();
             s->arena_capacity = 0;
             s->list_capacity = 0;
             if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
@@ -1447,7 +1463,8 @@ constexpr int kMaxSplit = 8;
 // 3d_room frame whatever its size (profiles/r2_band_scaling.txt) -- 3 % of a 4K frame on one GPU, 20 % of an
 // eighth of it.  Independent pipelines, each on every k-th 16-row band and on streams of its own, fill each other's
 // tails.  The picture cannot depend on it: pixels are independent (mod.rs:316-348).
-int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, EuclStats* stats) {
+int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, const AovPlanes& aov,
+                 EuclStats* stats) {
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
     uint32_t world = o->band_world > 1 ? o->band_world : 1, rank = world > 1 ? o->band_rank : 0, band = o->band_rows;
     if (band == 0) { // one band: the frame belongs to rank 0
@@ -1458,7 +1475,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     int k = std::min(kMaxSplit, env_int("EUCL_SPLIT", EUCL_SPLIT_DEFAULT));
     k = (int)std::min<uint32_t>((uint32_t)std::max(k, 1), my_rows / band); // a band or more for every pipeline
     if (o->pipeline != EUCL_PIPELINE_WAVEFRONT || (long long)my_rows * o->width < (long long)env_int("EUCL_SPLIT_MIN_PIXELS", 1 << 16)) k = 1;
-    if (k <= 1) return render_impl(s, fb, o, d_rgb, d_hit, stats);
+    if (k <= 1) return render_impl(s, fb, o, d_rgb, d_hit, aov, stats);
     while ((int)s->twins.size() < k - 1) {
         int rc = add_twin(s);
         if (rc != EUCL_OK) return rc;
@@ -1483,7 +1500,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     auto pipeline = [&](int p) {
         EuclScene* t = s->twins[p - 1];
         cudaSetDevice(t->device);
-        rc[p] = render_impl(t, fb, &opts[p], d_rgb, d_hit, &part[p], k, p);
+        rc[p] = render_impl(t, fb, &opts[p], d_rgb, d_hit, aov, &part[p], k, p);
         if (rc[p] != EUCL_OK) err[p] = eucl_last_error();
     };
     for (int p = 1; p < k; ++p) {
@@ -1494,7 +1511,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     }
     // (no early return between here and the last wait(): the helper threads work on this frame's locals)
     for (int p = 1; p < k && !serial; ++p) s->workers[p - 1]->run([&pipeline, p] { pipeline(p); });
-    rc[0] = render_impl(s, fb, &opts[0], d_rgb, d_hit, &part[0], k, 0);
+    rc[0] = render_impl(s, fb, &opts[0], d_rgb, d_hit, aov, &part[0], k, 0);
     for (int p = 1; p < k; ++p) {
         if (serial) pipeline(p);
         else s->workers[p - 1]->wait();
@@ -1592,83 +1609,68 @@ int prepare_batch(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclR
 
 // Device-output render of `n` frames (eucl_render_device: n = 1).
 int render_frames_to_device(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* d_rgb,
-                            int32_t* d_hit, EuclStats* stats) {
+                            int32_t* d_hit, const AovPlanes& aov, EuclStats* stats) {
     FrameBatch fb;
     EuclRenderOpts virt;
     const int st = prepare_batch(s, frames, n, o, &fb, &virt);
     if (st != EUCL_OK) return st;
-    return render_split(s, fb, &virt, d_rgb, d_hit, stats);
+    return render_split(s, fb, &virt, d_rgb, d_hit, aov, stats);
 }
 
-} // namespace
-
-extern "C" {
-
-int eucl_render_device(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, void* d_out_rgb8, void* d_out_hit_ids,
-                       EuclStats* stats) {
-    int st = check_args(s, cam, o);
-    if (st != EUCL_OK) return st;
-    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_device: null output");
-    EUCL_CUDA(cudaSetDevice(s->device));
-    const EuclFrame frame{*cam, o->time_seconds};
-    return render_frames_to_device(s, &frame, 1, o, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
-}
-
-int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o,
-                              void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats) {
-    int st = check_frames(s, frames, n_frames, o);
-    if (st != EUCL_OK) return st;
-    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames_device: null output");
-    EUCL_CUDA(cudaSetDevice(s->device));
-    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
-                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
-}
-
-int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
-                       int32_t* out_hit_ids, EuclStats* stats) {
-    int st = check_frames(s, frames, n_frames, o);
-    if (st != EUCL_OK) return st;
-    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: null output");
-    EUCL_CUDA(cudaSetDevice(s->device));
-    const size_t pixels = (size_t)n_frames * o->height * o->width;
-    const bool want_hit = o->want_hit_ids && out_hit_ids;
-    EUCL_CUDA(s->frame.ensure(pixels * 3));
-    if (want_hit) EUCL_CUDA(s->hit_ids.ensure(pixels * 4));
-    EuclRenderOpts opts = *o;
-    opts.want_hit_ids = want_hit ? 1 : 0;
-    st = render_frames_to_device(s, frames, n_frames, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
-    if (st != EUCL_OK) return st;
-    EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));
-    if (want_hit) EUCL_CUDA(cudaMemcpyAsync(out_hit_ids, s->hit_ids.ptr, pixels * 4, cudaMemcpyDeviceToHost, s->stream));
-    EUCL_CUDA(cudaStreamSynchronize(s->stream));
+// eucl_render_aovs*: at least one plane.  Checked before any device is touched.
+int check_aovs(const EuclAovs* a, const char* fn) {
+    if (!a || !(a->depth || a->position || a->normal || a->segments || a->levels))
+        return fail(EUCL_ERR_INVALID_ARGUMENT, std::string(fn) + ": no AOV plane requested (use the plain entry point)");
     return EUCL_OK;
 }
+AovPlanes aov_planes(const EuclAovs* a) {
+    if (!a) return AovPlanes{};
+    return AovPlanes{a->depth, a->position, a->normal, a->segments, a->levels, nullptr};
+}
 
-int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
-                EuclStats* stats) {
-    int st = check_args(s, cam, o);
-    if (st != EUCL_OK) return st;
-    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render: null output");
+// Host-output render of `n` frames (arguments already checked): rendered into the scene's device buffers, then copied out.
+// A rank of a band-split render (band_world > 1, a single frame) renders its rows compactly on the device and then copies
+// each band to its place in the caller's frame: rows of other ranks are never read or written, so N ranks can fill ONE
+// host frame (shared pinned memory) over their own PCIe links at the same time.  The AOV planes go the same way.
+int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* out_rgb8,
+                   int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats) {
     EUCL_CUDA(cudaSetDevice(s->device));
-    // A rank of a band-split render (band_world > 1) renders its rows compactly on the device and then copies
-    // each band to its place in the caller's frame: rows of other ranks are never read or written, so N ranks can
-    // fill ONE host frame (shared pinned memory) over their own PCIe links at the same time.
     const bool scatter = !o->compact_rows && o->band_world > 1;
     const size_t my_rows = eucl_band_rows_for_rank(o);
-    const size_t rows = (o->compact_rows || scatter) ? my_rows : o->height;
+    const size_t rows = (o->compact_rows || scatter) ? my_rows : (size_t)n * o->height;
     const size_t pixels = rows * (size_t)o->width;
     const bool want_hit = o->want_hit_ids && out_hit_ids;
     EUCL_CUDA(s->frame.ensure(std::max<size_t>(pixels, 1) * 3));
     if (want_hit) EUCL_CUDA(s->hit_ids.ensure(std::max<size_t>(pixels, 1) * 4));
+    // AOV planes: host pointer, bytes per pixel, device copy carved from one staging buffer
+    const AovPlanes want = aov_planes(aovs);
+    void* host[5] = {want.depth, want.position, want.normal, want.segments, want.levels};
+    const size_t px_bytes[5] = {4, 4 * (size_t)s->dim, 4 * (size_t)s->dim, 4, 4};
+    void* dev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    size_t stage_bytes = 0;
+    for (int k = 0; k < 5; ++k)
+        if (host[k]) stage_bytes += align16(std::max<size_t>(pixels, 1) * px_bytes[k]);
+    if (stage_bytes) {
+        EUCL_CUDA(s->aov_stage.ensure(stage_bytes));
+        uint8_t* p = (uint8_t*)s->aov_stage.ptr;
+        for (int k = 0; k < 5; ++k)
+            if (host[k]) {
+                dev[k] = p;
+                p += align16(std::max<size_t>(pixels, 1) * px_bytes[k]);
+            }
+    }
+    const AovPlanes d_aov{(float*)dev[0], (float*)dev[1], (float*)dev[2], (uint32_t*)dev[3], (uint32_t*)dev[4], nullptr};
     EuclRenderOpts opts = *o;
     opts.want_hit_ids = want_hit ? 1 : 0;
     if (scatter) opts.compact_rows = 1;
-    const EuclFrame frame{*cam, o->time_seconds};
-    st = render_frames_to_device(s, &frame, 1, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
+    const int st = render_frames_to_device(s, frames, n, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr,
+                                           d_aov, stats);
     if (st != EUCL_OK) return st;
     if (!scatter) {
         EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));
         if (want_hit) EUCL_CUDA(cudaMemcpyAsync(out_hit_ids, s->hit_ids.ptr, pixels * 4, cudaMemcpyDeviceToHost, s->stream));
+        for (int k = 0; k < 5; ++k)
+            if (host[k]) EUCL_CUDA(cudaMemcpyAsync(host[k], dev[k], pixels * px_bytes[k], cudaMemcpyDeviceToHost, s->stream));
     } else if (my_rows > 0) {
         // band k of this rank: compact rows [k * band, ...) -> frame rows [(k * world + rank) * band, ...)
         const size_t band = o->band_rows ? o->band_rows : o->height, world = o->band_world;
@@ -1685,9 +1687,79 @@ int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
         };
         EUCL_CUDA(copy_bands(out_rgb8, s->frame.ptr, 3));
         if (want_hit) EUCL_CUDA(copy_bands(out_hit_ids, s->hit_ids.ptr, 4));
+        for (int k = 0; k < 5; ++k)
+            if (host[k]) EUCL_CUDA(copy_bands(host[k], dev[k], px_bytes[k]));
     }
     EUCL_CUDA(cudaStreamSynchronize(s->stream));
     return EUCL_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int eucl_render_device(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, void* d_out_rgb8, void* d_out_hit_ids,
+                       EuclStats* stats) {
+    int st = check_args(s, cam, o);
+    if (st != EUCL_OK) return st;
+    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_device: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
+    const EuclFrame frame{*cam, o->time_seconds};
+    return render_frames_to_device(s, &frame, 1, o, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr,
+                                   AovPlanes{}, stats);
+}
+
+int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o,
+                              void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats) {
+    int st = check_frames(s, frames, n_frames, o);
+    if (st != EUCL_OK) return st;
+    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames_device: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
+    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
+                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
+}
+
+int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
+                       int32_t* out_hit_ids, EuclStats* stats) {
+    int st = check_frames(s, frames, n_frames, o);
+    if (st != EUCL_OK) return st;
+    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: null output");
+    return render_to_host(s, frames, n_frames, o, out_rgb8, out_hit_ids, nullptr, stats);
+}
+
+int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
+                EuclStats* stats) {
+    int st = check_args(s, cam, o);
+    if (st != EUCL_OK) return st;
+    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render: null output");
+    const EuclFrame frame{*cam, o->time_seconds};
+    return render_to_host(s, &frame, 1, o, out_rgb8, out_hit_ids, nullptr, stats);
+}
+
+// One frame: what eucl_render accepts; K > 1 frames: what eucl_render_frames accepts.
+static int check_aov_call(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, const EuclAovs* aovs,
+                          const char* fn) {
+    int st = n_frames == 1 ? check_args(s, frames ? &frames[0].camera : nullptr, o) : check_frames(s, frames, n_frames, o);
+    if (st == EUCL_OK) st = check_aovs(aovs, fn);
+    return st;
+}
+
+int eucl_render_aovs(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
+                     int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats) {
+    const int st = check_aov_call(s, frames, n_frames, o, aovs, "eucl_render_aovs");
+    if (st != EUCL_OK) return st;
+    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_aovs: null output");
+    return render_to_host(s, frames, n_frames, o, out_rgb8, out_hit_ids, aovs, stats);
+}
+
+int eucl_render_aovs_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, void* d_out_rgb8,
+                            void* d_out_hit_ids, const EuclAovs* d_aovs, EuclStats* stats) {
+    const int st = check_aov_call(s, frames, n_frames, o, d_aovs, "eucl_render_aovs_device");
+    if (st != EUCL_OK) return st;
+    if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_aovs_device: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
+    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
+                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, aov_planes(d_aovs), stats);
 }
 
 int eucl_scene_memory(const EuclScene* s, uint64_t* arena_bytes, uint64_t* list_bytes, uint64_t* node_capacity) {

@@ -141,9 +141,10 @@ __device__ __forceinline__ real* plane_scratch(const uint8_t* __restrict__ blob)
 // and its orientation relative to the ray (mod.rs:114-125).
 template <int D>
 __device__ __forceinline__ int intersect_ray(const SceneView& sv, const Vec<D>& o, const Vec<D>& d, bool& exiting, Vec<D>& p,
-                                             Vec<D>& n_raw, real& cos_raw, real& angle_raw, real* ts, int ts_stride) {
+                                             Vec<D>& n_raw, real& cos_raw, real& angle_raw, real& t, real* ts, int ts_stride) {
     const ClosestHit h = closest_hit<D>(sv, o, d, ts, ts_stride);
     if (h.entity < 0) return -1;
+    t = h.t;
     hit_geometry<D>(sv, h.prim, h.flags, o, d, h.t, p, n_raw);
     cos_raw = angle_cos(d, n_raw);
     angle_raw = angle_from_cos(cos_raw);
@@ -755,8 +756,32 @@ __device__ __forceinline__ Rgba node_color(const Workspace& ws, const NodeMeta& 
     return out;
 }
 
-// K4: colour of the inner nodes of one level from the colours of level + 1.
-__global__ void __launch_bounds__(256) k_resolve(Workspace ws, int level) {
+// Tree cost (segments, levels) of a node at `level` (AovPlanes::segments / levels): the node itself is one Universe::trace
+// call with depth > 0 when level < max_depth, and reaches level + 1 levels; an inner node adds its children's segments and
+// takes the maximum of their levels.  Every node of levels 1 .. max_depth - 1 gets its cost from k_resolve_cost of its own
+// level -- leaves included, although their colour needs no resolving.  The nodes of level max_depth (background lookups,
+// leaves all) are never resolved: their parents derive the cost from the level.
+__device__ __forceinline__ uint2 leaf_cost(int level, int max_depth) {
+    return make_uint2(level < max_depth ? 1u : 0u, (unsigned)level + 1u);
+}
+__device__ __forceinline__ uint2 tree_cost(const NodeMeta& m, int level, int max_depth, const uint2* __restrict__ cost) {
+    uint2 c = leaf_cost(level, max_depth);
+    if (m.flags & NODE_LEAF) return c;
+    const int child[2] = {m.tchild, m.rchild};
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+        if (child[k] < 0) continue;
+        const uint2 cc = level + 1 >= max_depth ? leaf_cost(level + 1, max_depth) : cost[child[k]];
+        c.x += cc.x;
+        c.y = max(c.y, cc.y);
+    }
+    return c;
+}
+
+// K4: colour of the inner nodes of one level from the colours of level + 1.  COST (k_resolve_cost): also the tree cost of
+// every node of the level.  Two kernels over one body so that the plain one keeps its symbol and its code.
+template <bool COST>
+__device__ __forceinline__ void resolve_level(const Workspace& ws, int level, int max_depth, const AovPlanes& aov) {
     __shared__ real s_unit[256];
     if (*ws.overflow) return;
     fill_unit_table(s_unit);
@@ -764,13 +789,21 @@ __global__ void __launch_bounds__(256) k_resolve(Workspace ws, int level) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < cnt; i += gridDim.x * blockDim.x) {
         const int node = off + i;
         const NodeMeta m = ws.meta[node];
+        if (COST) aov.cost[node] = tree_cost(m, level, max_depth, aov.cost);
         if (m.flags & NODE_LEAF) continue;
         store_res(ws, node, node_color(ws, m, node, s_unit));
     }
 }
+__global__ void __launch_bounds__(256) k_resolve(Workspace ws, int level) { resolve_level<false>(ws, level, 0, AovPlanes{}); }
+__global__ void __launch_bounds__(256) k_resolve_cost(Workspace ws, int level, int max_depth, AovPlanes aov) {
+    resolve_level<true>(ws, level, max_depth, aov);
+}
 
-// K5: resolve level 0, composite over white, quantise and pack RGB8 rows (row 0 = bottom).
-__global__ void __launch_bounds__(256) k_final(FrameParams fp, ChunkParams cp, Workspace ws, uint8_t* __restrict__ out_rgb8) {
+// K5: resolve level 0, composite over white, quantise and pack RGB8 rows (row 0 = bottom).  COST (k_final_cost): also the
+// segments / levels planes from the tree cost of level 0 (0 / 0 for checkerboard pixels).
+template <bool COST>
+__device__ __forceinline__ void final_pixels(const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
+                                             uint8_t* __restrict__ out_rgb8, const AovPlanes& aov) {
     __shared__ real s_unit[256];
     if (*ws.overflow) return;
     fill_unit_table(s_unit);
@@ -779,7 +812,66 @@ __global__ void __launch_bounds__(256) k_final(FrameParams fp, ChunkParams cp, W
         const Rgba c = node_color(ws, m, i, s_unit);
         const int local_row = cp.local_row0 + i / fp.width;
         const int orow = out_row_of_local(cp, local_row);
-        final_rgb8(c, !(m.flags & NODE_FINAL_RGB), out_rgb8 + ((size_t)orow * fp.width + i % fp.width) * 3);
+        const size_t opix = (size_t)orow * fp.width + i % fp.width;
+        final_rgb8(c, !(m.flags & NODE_FINAL_RGB), out_rgb8 + opix * 3);
+        if (COST) {
+            const uint2 cost = (m.flags & NODE_FINAL_RGB) ? make_uint2(0u, 0u) : tree_cost(m, 0, fp.max_depth, aov.cost);
+            if (aov.segments) aov.segments[opix] = cost.x;
+            if (aov.levels) aov.levels[opix] = cost.y;
+        }
+    }
+}
+__global__ void __launch_bounds__(256) k_final(FrameParams fp, ChunkParams cp, Workspace ws, uint8_t* __restrict__ out_rgb8) {
+    final_pixels<false>(fp, cp, ws, out_rgb8, AovPlanes{});
+}
+__global__ void __launch_bounds__(256) k_final_cost(FrameParams fp, ChunkParams cp, Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                    AovPlanes aov) {
+    final_pixels<true>(fp, cp, ws, out_rgb8, aov);
+}
+
+// The primary-hit planes of one level-0 node (AovPlanes::depth / position / normal), narrowed once to float:
+// t, o + d * t (the intersectors' expression) and normal_closer.  hit = false: the primary ray hit nothing or max_depth
+// is 0 (depth +inf); traced = false: checkerboard pixel (everything NaN).
+template <int D>
+__device__ __forceinline__ void write_primary(const AovPlanes& aov, size_t opix, bool traced, bool hit, real t, const Vec<D>& p,
+                                              const Vec<D>& n_closer) {
+    const float nan = __int_as_float(0x7fc00000);
+    const float depth = !traced ? nan : (hit ? (float)t : __int_as_float(0x7f800000));
+    const bool finite = isfinite(depth);
+    if (aov.depth) aov.depth[opix] = depth;
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+        if (aov.position) aov.position[opix * D + k] = finite ? (float)p[k] : nan;
+        if (aov.normal) aov.normal[opix * D + k] = hit ? (float)n_closer[k] : nan;
+    }
+}
+
+// K6 (AOVs only): the primary-hit planes from level 0 of the arena -- the ray record, ray_cur and the hit record, all still
+// there when the chunk ends.  No hit record exists for max_depth 0, nor for checkerboard nodes (ray_cur -1: a camera in
+// no entity, or an untraced frame of a batch).
+template <int D>
+__global__ void __launch_bounds__(256) k_aov_primary(FrameParams fp, ChunkParams cp, Workspace ws, AovPlanes aov) {
+    if (*ws.overflow) return;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < cp.n_pixels; i += gridDim.x * blockDim.x) {
+        const bool traced = ws.ray_cur[i] >= 0;
+        bool hit = false;
+        real t = R(0.0);
+        Vec<D> p, n;
+#pragma unroll
+        for (int k = 0; k < D; ++k) p[k] = n[k] = R(0.0);
+        if (traced && fp.max_depth > 0) {
+            const HitHead h = load_hit<D>(ws, i, n);
+            if (h.entity >= 0) {
+                Vec<D> o, d;
+                load_ray<D>(ws, i, o, d);
+                hit = true;
+                t = h.t;
+                p = o + d * h.t;
+                if (h.exiting) n = -n;
+            }
+        }
+        const int local_row = cp.local_row0 + i / fp.width;
+        write_primary<D>(aov, (size_t)out_row_of_local(cp, local_row) * fp.width + i % fp.width, traced, hit, t, p, n);
     }
 }
 
@@ -795,10 +887,12 @@ struct MegaFrame {
     ChildRay<D> r;
 };
 
-template <int D>
-__global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
-                                                       Workspace ws, uint8_t* __restrict__ out_rgb8,
-                                                       int32_t* __restrict__ hit_ids_out) {
+// AOV (k_megakernel_aov): also the AOV planes -- the level-0 geometry, and the segments and levels counted along the walk.
+// The cross-check of k_aov_primary and the COST builds of the wavefront.
+template <int D, bool AOV>
+__device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ blob, const FrameParams& fp, const ChunkParams& cp,
+                                                  const Workspace& ws, uint8_t* __restrict__ out_rgb8,
+                                                  int32_t* __restrict__ hit_ids_out, const AovPlanes& aov) {
     const SceneView& sv = stage_scene(blob);
     real* ts = plane_scratch(blob);
     const int cam_entity = *ws.cam_entity;
@@ -819,8 +913,15 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
             if (hit_ids_out) hit_ids_out[opix] = -2;
             local_counts[0]++;
             if (ws.frames) atomicAdd(ws.untraced, 1);
+            if (AOV) {
+                const Vec<D> zero{};
+                write_primary<D>(aov, opix, false, false, R(0.0), zero, zero);
+                if (aov.segments) aov.segments[opix] = 0u;
+                if (aov.levels) aov.levels[opix] = 0u;
+            }
             continue;
         }
+        unsigned aov_segments = 0u, aov_levels = 0u;
         MegaFrame<D> stack[kMegaMaxDepth];
         Vec<D> o, d;
 #pragma unroll
@@ -837,9 +938,14 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
             int ent = -1;
             bool exiting = false;
             Vec<D> p, n;
-            real cos_raw = R(0.0), angle_raw = R(0.0);
-            if (level < fp.max_depth) ent = intersect_ray<D>(sv, o, d, exiting, p, n, cos_raw, angle_raw, ts, (int)blockDim.x);
+            real cos_raw = R(0.0), angle_raw = R(0.0), t_hit = R(0.0);
+            if (level < fp.max_depth) ent = intersect_ray<D>(sv, o, d, exiting, p, n, cos_raw, angle_raw, t_hit, ts, (int)blockDim.x);
             if (level == 0 && hit_ids_out) hit_ids_out[opix] = ent;
+            if (AOV) {
+                aov_segments += level < fp.max_depth ? 1u : 0u;
+                aov_levels = max(aov_levels, (unsigned)level + 1u);
+                if (level == 0) write_primary<D>(aov, opix, true, ent >= 0, t_hit, p, exiting ? -n : n);
+            }
             if (ent < 0) {
                 val = mapped_color<D>(sv, sv.background, d);
             } else {
@@ -906,6 +1012,10 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
             if (done) break;
         }
         final_rgb8(val, true, out_rgb8 + opix * 3);
+        if (AOV) {
+            if (aov.segments) aov.segments[opix] = aov_segments;
+            if (aov.levels) aov.levels[opix] = aov_levels;
+        }
     }
     for (int l = 0; l <= fp.max_depth && l <= kMegaMaxDepth; ++l) {
         // per-level node counts, warp-reduced
@@ -913,6 +1023,18 @@ __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict
         for (int s = 16; s > 0; s >>= 1) v += __shfl_down_sync(0xffffffffu, v, s);
         if ((threadIdx.x & 31) == 0 && v) atomicAdd(ws.mega_level_counts + l, v);
     }
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                       Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                       int32_t* __restrict__ hit_ids_out) {
+    megakernel_pixels<D, false>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{});
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel_aov(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                           Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                           int32_t* __restrict__ hit_ids_out, AovPlanes aov) {
+    megakernel_pixels<D, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, aov);
 }
 
 // Universe::trace_path_unknown / trace_path (mod.rs:186-227,273-286) with Surface::get_path
@@ -1113,20 +1235,36 @@ int launch_shade(int dim, const Launch& l, const FrameParams& fp, const ChunkPar
 }
 // Bottom-up resolve of the ray tree (level max_depth holds leaves only) and the RGB8 pack of level 0.
 // Returns the number of kernels launched.
+// With AOVs: the COST builds when segments or levels are wanted, and k_aov_primary for the primary-hit planes.
 int launch_resolve_and_final(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                             uint8_t* out_rgb8) {
-    (void)dim;
+                             uint8_t* out_rgb8, const AovPlanes& aov) {
+    const bool cost = aov.segments || aov.levels;
     int launches = 0;
     for (int level = fp.max_depth - 1; level >= 1; --level) {
-        k_resolve<<<l.grid_mem, 256, 0, l.stream>>>(ws, level);
+        if (cost) k_resolve_cost<<<l.grid_mem, 256, 0, l.stream>>>(ws, level, fp.max_depth, aov);
+        else k_resolve<<<l.grid_mem, 256, 0, l.stream>>>(ws, level);
         ++launches;
     }
-    k_final<<<grid_for(cp.n_pixels, 256, l.grid_mem), 256, 0, l.stream>>>(fp, cp, ws, out_rgb8);
-    return launches + 1;
+    const int grid = grid_for(cp.n_pixels, 256, l.grid_mem);
+    if (cost) k_final_cost<<<grid, 256, 0, l.stream>>>(fp, cp, ws, out_rgb8, aov);
+    else k_final<<<grid, 256, 0, l.stream>>>(fp, cp, ws, out_rgb8);
+    ++launches;
+    if (aov.depth || aov.position || aov.normal) {
+        EUCL_DISPATCH_DIM(dim, (k_aov_primary<3><<<grid, 256, 0, l.stream>>>(fp, cp, ws, aov)),
+                          (k_aov_primary<4><<<grid, 256, 0, l.stream>>>(fp, cp, ws, aov)));
+        ++launches;
+    }
+    return launches;
 }
 void launch_megakernel(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                       uint8_t* out_rgb8, int32_t* hit_ids_out) {
+                       uint8_t* out_rgb8, int32_t* hit_ids_out, const AovPlanes& aov) {
     const int grid = grid_for(cp.n_pixels, kBlock, 1 << 30);
+    if (aov.depth || aov.position || aov.normal || aov.segments || aov.levels) {
+        EUCL_DISPATCH_DIM(
+            dim, (k_megakernel_aov<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)),
+            (k_megakernel_aov<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)));
+        return;
+    }
     EUCL_DISPATCH_DIM(
         dim, (k_megakernel<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)),
         (k_megakernel<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)));
@@ -1190,6 +1328,8 @@ cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene) {
     EUCL_CONF(k_background<4>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
     EUCL_CONF(k_megakernel<3>, smem_bytes, heavy);
     EUCL_CONF(k_megakernel<4>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_aov<3>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_aov<4>, smem_bytes, heavy);
     EUCL_CONF(k_trace_path<3>, smem_bytes, 1);
     EUCL_CONF(k_trace_path<4>, smem_bytes, 1);
 #undef EUCL_CONF

@@ -114,6 +114,20 @@ struct Workspace {
     int32_t* untraced;         // level-0 nodes of this chunk whose frame's camera is in no entity (checkerboard pixels)
 };
 
+// Per-pixel auxiliary outputs of the primary ray and its tree (eucl_render_aovs*, definitions in DESIGN.md §6): device planes
+// addressed like the hit ids (out_row_of_local), each null when not wanted.  The kernels that write them are builds of
+// their own (k_aov_primary, k_resolve_cost, k_final_cost, k_megakernel_aov): a render without AOVs runs none of this code.
+struct AovPlanes {
+    float* depth;       // [pixels] parametric distance t of the primary hit
+    float* position;    // [pixels][dim] o + d * t
+    float* normal;      // [pixels][dim] normal_closer of the primary hit
+    uint32_t* segments; // [pixels] Universe::trace calls with depth > 0 in the pixel's ray tree
+    uint32_t* levels;   // [pixels] deepest level of the tree + 1
+    // [capacity] (segments, levels) of every node of the chunk, filled bottom-up by k_resolve_cost; the pipeline's own
+    // buffer, set (wavefront only) when segments or levels are wanted
+    uint2* cost;
+};
+
 struct Launch {
     cudaStream_t stream;
     const uint8_t* blob;
@@ -183,9 +197,9 @@ constexpr int kMaxBins = 64; // shade-coherence bins (miss, then kBinsPerEntity 
     int launch_shade(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,                \
                      const eucl::Workspace& ws, int level, int32_t* hit_ids_out);                                              \
     int launch_resolve_and_final(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,    \
-                                 const eucl::Workspace& ws, uint8_t* out_rgb8);                                                \
+                                 const eucl::Workspace& ws, uint8_t* out_rgb8, const eucl::AovPlanes& aov);                    \
     void launch_megakernel(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
-                           const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out);                                \
+                           const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out, const eucl::AovPlanes& aov);    \
     void launch_trace_path(int dim, const eucl::Launch& l, const double* d_in, double distance, double* d_out, int* d_found); \
     cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);                                                       \
     }

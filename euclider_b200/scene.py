@@ -12,13 +12,13 @@ import ctypes as C
 import os
 from dataclasses import dataclass, field
 from pathlib import Path
-from typing import Dict, Optional, Sequence, Tuple, Union
+from typing import Dict, Mapping, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
 from . import _capi
-from ._capi import (EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL,
-                    EUCL_PIPELINE_WAVEFRONT, check, lib)
+from ._capi import (EuclAovs, EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRenderOpts, EuclStats,
+                    EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, check, lib)
 
 ParserError = EuclError  # the reference's `ParserError` (src/scene.rs:524-552); see EuclError.status
 
@@ -43,6 +43,7 @@ class RawImage2d:
     format: str = "U8U8U8"
     hit_ids: Optional[np.ndarray] = None  # int32 (height, width): primary hit entity, -1 background, -2 checkerboard
     stats: Optional[dict] = None
+    aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name (AOV_NAMES), rows as `data`
 
     def to_top_down(self) -> np.ndarray:
         return self.data[::-1]
@@ -66,13 +67,61 @@ class RawFrames:
     height: int
     hit_ids: Optional[np.ndarray] = None  # int32 (K, height, width), as RawImage2d.hit_ids
     stats: Optional[dict] = None  # summed over the K frames
+    aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name, frame k at index k
 
     def __len__(self) -> int:
         return int(self.data.shape[0])
 
     def frame(self, k: int) -> RawImage2d:
         """Frame k as a RawImage2d (a view, no copy)."""
-        return RawImage2d(self.data[k], self.width, self.height, hit_ids=None if self.hit_ids is None else self.hit_ids[k])
+        return RawImage2d(self.data[k], self.width, self.height, hit_ids=None if self.hit_ids is None else self.hit_ids[k],
+                          aovs=None if self.aovs is None else {name: a[k] for name, a in self.aovs.items()})
+
+
+# Per-pixel auxiliary outputs (include/euclider_b200.h, EuclAovs): name -> (dtype, one value per pixel or `dim` values).
+# depth / position / normal: the primary hit (float32, NaN / +inf where there is none); segments / levels: the cost of the
+# pixel's ray tree (uint32).  Host planes the library does not write (other ranks' rows of a band-split render) keep
+# their fill: NaN for the float planes, 0xFFFFFFFF for the counts.
+AOV_NAMES = ("depth", "position", "normal", "segments", "levels")
+_AOV_TYPES = {"depth": (np.float32, False), "position": (np.float32, True), "normal": (np.float32, True),
+              "segments": (np.uint32, False), "levels": (np.uint32, False)}
+
+
+def _aov_names(aovs) -> Tuple[str, ...]:
+    """The requested plane names, in AOV_NAMES order; ValueError for an unknown one."""
+    names = [aovs] if isinstance(aovs, str) else list(aovs)
+    unknown = [n for n in names if n not in _AOV_TYPES]
+    if unknown:
+        raise ValueError(f"unknown AOV plane(s) {unknown}: choose from {AOV_NAMES}")
+    return tuple(n for n in AOV_NAMES if n in names)
+
+
+def _aov_arrays(aovs, lead: Tuple[int, ...], dim: int) -> Dict[str, np.ndarray]:
+    """Host planes for `aovs`: a sequence of names (allocated here) or a mapping name -> array to render into (None:
+    allocated).  A given array must have the plane's dtype and shape and be C-contiguous."""
+    given = dict(aovs) if isinstance(aovs, Mapping) else {}
+    out = {}
+    for name in _aov_names(list(aovs)):
+        dtype, per_dim = _AOV_TYPES[name]
+        shape = lead + ((dim,) if per_dim else ())
+        a = given.get(name)
+        if a is None:
+            a = np.full(shape, np.nan if dtype == np.float32 else 0xFFFFFFFF, dtype=dtype)
+        elif not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags["C_CONTIGUOUS"]:
+            raise ValueError(f"AOV plane {name!r} must be a C-contiguous {np.dtype(dtype).name} array of shape {shape}")
+        out[name] = a
+    return out
+
+
+def _aov_struct(pointers: Mapping[str, int]) -> EuclAovs:
+    return EuclAovs(**{name: C.c_void_p(int(ptr)) for name, ptr in pointers.items() if ptr})
+
+
+def _device_aovs(d_aovs: Mapping[str, int]) -> EuclAovs:
+    _aov_names(list(d_aovs))
+    if not any(d_aovs.values()):
+        raise ValueError("d_aovs names no device plane")
+    return _aov_struct(d_aovs)
 
 
 def _frame_table(cameras: Sequence[EuclCamera], times) -> C.Array:
@@ -136,9 +185,11 @@ class Environment:
     def render(self, dimensions: Tuple[int, int], time: float = 0.0, threads: int = 0,
                context: Optional[SimulationContext] = None, *, device: int = 0, want_hit_ids: bool = False,
                band_rows: int = 0, band_rank: int = 0, band_world: int = 1, out: Optional[np.ndarray] = None,
-               profile: bool = False) -> RawImage2d:
+               profile: bool = False, aovs=None) -> RawImage2d:
         """Environment::render.  `time` is seconds since start (the reference passes a Duration);
-        `threads` is accepted for signature parity and ignored (the GPU schedules the pixels)."""
+        `threads` is accepted for signature parity and ignored (the GPU schedules the pixels).
+        `aovs`: per-pixel auxiliary planes to return in `.aovs` (names from AOV_NAMES, or a mapping name -> array to
+        render into); the frame, hit ids and stats are the same with or without them."""
         del threads
         context = context or SimulationContext()
         width, height = int(dimensions[0]) // context.resolution, int(dimensions[1]) // context.resolution
@@ -149,33 +200,48 @@ class Environment:
             out = np.zeros((height, width, 3), dtype=np.uint8)
         assert out.dtype == np.uint8 and out.size == height * width * 3 and out.flags["C_CONTIGUOUS"]
         hit = np.full((height, width), -3, dtype=np.int32) if want_hit_ids else None
+        planes = _aov_arrays(aovs, (height, width), self.dim) if aovs else None
         stats = EuclStats()
-        check(lib().eucl_render(self._device_scene(device), C.byref(self.camera), C.byref(opts), out.ctypes.data,
-                                hit.ctypes.data if hit is not None else None, C.byref(stats)))
-        return RawImage2d(out, width, height, hit_ids=hit, stats=stats_to_dict(stats))
+        if planes:
+            table = _frame_table([self.camera], float(time))
+            check(lib().eucl_render_aovs(self._device_scene(device), table, 1, C.byref(opts), out.ctypes.data,
+                                         hit.ctypes.data if hit is not None else None,
+                                         C.byref(_aov_struct({n: a.ctypes.data for n, a in planes.items()})), C.byref(stats)))
+        else:
+            check(lib().eucl_render(self._device_scene(device), C.byref(self.camera), C.byref(opts), out.ctypes.data,
+                                    hit.ctypes.data if hit is not None else None, C.byref(stats)))
+        return RawImage2d(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
 
     # -- device-resident variant (inputs and outputs stay in HBM) --------------------------------
     def render_device(self, d_out_rgb8: int, dimensions: Tuple[int, int], time: float = 0.0, *, device: int = 0,
                       d_out_hit_ids: int = 0, band_rows: int = 0, band_rank: int = 0, band_world: int = 1,
-                      compact_rows: bool = False, profile: bool = False) -> dict:
+                      compact_rows: bool = False, profile: bool = False, d_aovs: Optional[Mapping[str, int]] = None) -> dict:
+        """render into device buffers.  `d_aovs`: name -> device pointer of each wanted AOV plane (layout of the hit ids)."""
         width, height = int(dimensions[0]), int(dimensions[1])
         opts = EuclRenderOpts(width=width, height=height, time_seconds=float(time), band_rows=band_rows,
                               band_rank=band_rank, band_world=band_world, pipeline=self.pipeline,
                               compact_rows=int(compact_rows), want_hit_ids=int(bool(d_out_hit_ids)),
                               profile=int(profile))
         stats = EuclStats()
-        check(lib().eucl_render_device(self._device_scene(device), C.byref(self.camera), C.byref(opts),
-                                       C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
-                                       C.byref(stats)))
+        if d_aovs:
+            aov = _device_aovs(d_aovs)
+            check(lib().eucl_render_aovs_device(self._device_scene(device), _frame_table([self.camera], float(time)), 1,
+                                                C.byref(opts), C.c_void_p(d_out_rgb8),
+                                                C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None, C.byref(aov), C.byref(stats)))
+        else:
+            check(lib().eucl_render_device(self._device_scene(device), C.byref(self.camera), C.byref(opts),
+                                           C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
+                                           C.byref(stats)))
         return stats_to_dict(stats)
 
     # -- many frames per call: camera paths and animations -------------------------------------------
     def render_frames(self, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera], times=0.0,
                       context: Optional[SimulationContext] = None, *, device: int = 0, want_hit_ids: bool = False,
-                      out: Optional[np.ndarray] = None, profile: bool = False) -> RawFrames:
+                      out: Optional[np.ndarray] = None, profile: bool = False, aovs=None) -> RawFrames:
         """Renders one frame per camera pose in ONE call (eucl_render_frames): frame k equals
         `render(dimensions, times[k])` with `self.camera` set to `cameras[k]`, bit for bit.  `times` is one time for
-        every frame or a sequence of one per frame.  Batching pays the fixed cost of a frame once per call."""
+        every frame or a sequence of one per frame.  Batching pays the fixed cost of a frame once per call.
+        `aovs` as for `render`; plane k of the result belongs to frame k."""
         table = _frame_table(cameras, times)
         context = context or SimulationContext()
         width, height = int(dimensions[0]) // context.resolution, int(dimensions[1]) // context.resolution
@@ -187,22 +253,36 @@ class Environment:
         opts = EuclRenderOpts(width=width, height=height, pipeline=self.pipeline, want_hit_ids=int(want_hit_ids),
                               profile=int(profile))
         hit = np.full((k, height, width), -3, dtype=np.int32) if want_hit_ids else None
+        planes = _aov_arrays(aovs, (k, height, width), self.dim) if aovs else None
         stats = EuclStats()
-        check(lib().eucl_render_frames(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
-                                       hit.ctypes.data if hit is not None else None, C.byref(stats)))
-        return RawFrames(out, width, height, hit_ids=hit, stats=stats_to_dict(stats))
+        if planes:
+            check(lib().eucl_render_aovs(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
+                                         hit.ctypes.data if hit is not None else None,
+                                         C.byref(_aov_struct({n: a.ctypes.data for n, a in planes.items()})), C.byref(stats)))
+        else:
+            check(lib().eucl_render_frames(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
+                                           hit.ctypes.data if hit is not None else None, C.byref(stats)))
+        return RawFrames(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
 
     def render_frames_device(self, d_out_rgb8: int, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera],
-                             times=0.0, *, device: int = 0, d_out_hit_ids: int = 0, profile: bool = False) -> dict:
-        """render_frames into device buffers: K * height * width * 3 bytes (and K * height * width int32 hit ids)."""
+                             times=0.0, *, device: int = 0, d_out_hit_ids: int = 0, profile: bool = False,
+                             d_aovs: Optional[Mapping[str, int]] = None) -> dict:
+        """render_frames into device buffers: K * height * width * 3 bytes (and K * height * width int32 hit ids, and the
+        AOV planes of `d_aovs`, name -> device pointer)."""
         table = _frame_table(cameras, times)
         width, height = int(dimensions[0]), int(dimensions[1])
         opts = EuclRenderOpts(width=width, height=height, pipeline=self.pipeline, want_hit_ids=int(bool(d_out_hit_ids)),
                               profile=int(profile))
         stats = EuclStats()
-        check(lib().eucl_render_frames_device(self._device_scene(device), table, len(table), C.byref(opts),
-                                              C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
-                                              C.byref(stats)))
+        if d_aovs:
+            aov = _device_aovs(d_aovs)
+            check(lib().eucl_render_aovs_device(self._device_scene(device), table, len(table), C.byref(opts),
+                                                C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
+                                                C.byref(aov), C.byref(stats)))
+        else:
+            check(lib().eucl_render_frames_device(self._device_scene(device), table, len(table), C.byref(opts),
+                                                  C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
+                                                  C.byref(stats)))
         return stats_to_dict(stats)
 
     def trace_path_unknown(self, location: Sequence[float], direction: Sequence[float], distance: float, *,

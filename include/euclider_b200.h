@@ -352,6 +352,43 @@ int eucl_render_frames(EuclScene* scene, const EuclFrame* frames, uint32_t n_fra
 int eucl_render_frames_device(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
                               void* d_out_rgb8, void* d_out_hit_ids, EuclStats* stats);
 
+/* Per-pixel auxiliary outputs (AOVs) of a render: what the primary ray hit and what the pixel's ray tree cost.  Every
+ * plane has the layout of the hit ids -- row 0 at the bottom, frame k of a batch in rows [k*height, (k+1)*height),
+ * band-split and compact rows exactly as the hit ids -- and is optional.  `dim` is the scene's dimension (3 or 4).
+ *   depth     float32          the primary hit's parametric distance t (Intersection::distance, mod.rs:127-142);
+ *                              +inf when the primary ray hits nothing or max_depth == 0; NaN for checkerboard pixels
+ *                              (camera in no entity)
+ *   position  float32 x dim    o + d * t in the scene's precision (the intersectors' expression), narrowed once;
+ *                              NaN where depth is not finite
+ *   normal    float32 x dim    the primary hit's normal_closer (exiting ? -n : n, mod.rs:117-125), not renormalised;
+ *                              NaN where there is no hit
+ *   segments  uint32           Universe::trace calls with depth > 0 in the pixel's ray tree (the pixel's share of
+ *                              EuclStats.segments); 0 for checkerboard pixels
+ *   levels    uint32           deepest level of the pixel's tree + 1 (1: the primary ray ended there); 0 for
+ *                              checkerboard pixels
+ * Float planes are float32 for both precisions: an f64 scene narrows once.  Asking for AOVs never changes the RGB8
+ * frame, the hit ids or EuclStats. */
+typedef struct EuclAovs {      /* each pointer NULL = plane not wanted */
+    float* depth;              /* [pixels]       */
+    float* position;           /* [pixels][dim]  */
+    float* normal;             /* [pixels][dim]  */
+    uint32_t* segments;        /* [pixels]       */
+    uint32_t* levels;          /* [pixels]       */
+} EuclAovs;
+
+/* eucl_render / eucl_render_frames with AOVs, HOST buffers.  n_frames == 1 renders frames[0] (its time replaces
+ * opts->time_seconds) and accepts everything eucl_render accepts: bands, compact_rows (the planes then hold this
+ * rank's rows only), a band-split rank with compact_rows == 0 writing only its own rows of every full-frame plane,
+ * both pipelines.  n_frames > 1 follows the rules of eucl_render_frames.  EUCL_ERR_INVALID_ARGUMENT, before any device
+ * work, for a null `aovs` or one without any plane (the plain entry points cover that case).  Synchronous. */
+int eucl_render_aovs(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
+                     uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats);
+
+/* Same, with DEVICE buffers on the scene's device: the output, the hit ids and every plane of `d_aovs` (the struct
+ * itself is read on the host). */
+int eucl_render_aovs_device(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
+                            void* d_out_rgb8, void* d_out_hit_ids, const EuclAovs* d_aovs, EuclStats* stats);
+
 /* Universe::trace_path_unknown (src/universe/mod.rs:273-286): moves `location` by `distance` along
  * `direction` THROUGH the universe -- surfaces are crossed with the material transitions of the
  * entities on either side, so a step through a LinearSpace void is stretched or shrunk.  The

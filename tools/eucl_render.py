@@ -10,10 +10,17 @@ rendered --batch at a time (default: all in one call, Environment.render_frames)
 
     python tools/eucl_render.py assets/scenes/3d_room.json out_%04d.ppm --size 128 96 --frames 64 \\
         --move 0 0.05 0 --yaw 0.02 --time-step 0.04
+
+Per-pixel auxiliary outputs with --aov depth,position,normal,segments,levels: next to each image `out.png` the tool writes
+`out.<plane>.npy` (the plane as the library returns it, row 0 = bottom) and, for the scalar planes, a greyscale preview
+`out.<plane>.png` (top-down; depth and levels linear, segments on a log scale; pixels without a value black).
 """
 import argparse
+import os
 import sys
 from pathlib import Path
+
+import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
@@ -43,6 +50,8 @@ def parse_args(argv=None):
     seq.add_argument("--plane4", type=float, nargs=3, metavar=("A", "B", "ANGLE"),
                      help="4-D: rotation per frame in the plane of camera axes A and B (0 forward, 1 left, 2 up, 3 ana)")
     seq.add_argument("--time-step", type=float, default=0.0, help="seconds added to the time per frame")
+    ap.add_argument("--aov", type=aov_list, default=[], metavar="P,Q,..",
+                    help=f"also write these per-pixel planes, from {','.join(eb.AOV_NAMES)}")
     args = ap.parse_args(argv)
     if args.frames < 1:
         ap.error("--frames must be at least 1")
@@ -55,6 +64,39 @@ def parse_args(argv=None):
     if args.frames > 1 and "%" not in args.output:
         ap.error("--frames > 1 needs an output pattern such as out_%04d.ppm")
     return args
+
+
+def aov_list(text: str) -> list:
+    names = text.split(",")
+    bad = [n for n in names if n not in eb.AOV_NAMES]
+    if bad:
+        raise argparse.ArgumentTypeError(f"unknown plane(s) {bad}: choose from {','.join(eb.AOV_NAMES)}")
+    return names
+
+
+def aov_path(image_path: str, name: str, ext: str) -> str:
+    """out.png -> out.<name><ext>"""
+    return f"{os.path.splitext(image_path)[0]}.{name}{ext}"
+
+
+def preview(name: str, plane: np.ndarray) -> np.ndarray:
+    """Greyscale u8 image of a scalar plane, top-down: linear in depth and levels, log in segments; no value -> black."""
+    v = plane.astype(np.float64)
+    if name == "segments":
+        v = np.log1p(v)
+    ok = np.isfinite(v)
+    lo, hi = (v[ok].min(), v[ok].max()) if ok.any() else (0.0, 0.0)
+    scaled = np.where(ok, (v - lo) / (hi - lo) if hi > lo else 1.0, 0.0)
+    return np.round(scaled * 255.0).astype(np.uint8)[::-1]
+
+
+def write_aovs(image_path: str, aovs: dict) -> None:
+    from PIL import Image
+
+    for name, plane in aovs.items():
+        np.save(aov_path(image_path, name, ".npy"), plane)
+        if plane.ndim == 2:
+            Image.fromarray(preview(name, plane)).save(aov_path(image_path, name, ".png"))
 
 
 def is_sequence(args) -> bool:
@@ -88,8 +130,10 @@ def main(argv=None):
     env.pipeline = eb.EUCL_PIPELINE_MEGAKERNEL if args.pipeline == "megakernel" else eb.EUCL_PIPELINE_WAVEFRONT
     context = eb.SimulationContext(resolution=args.resolution)
     if not is_sequence(args):
-        img = env.render(tuple(args.size), args.time, context=context)
+        img = env.render(tuple(args.size), args.time, context=context, aovs=args.aov or None)
         img.save(args.output)
+        if args.aov:
+            write_aovs(args.output, img.aovs)
         st = img.stats
         print(f"{args.output}: {img.width}x{img.height}, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
         return
@@ -102,9 +146,12 @@ def main(argv=None):
     batch = args.batch or args.frames
     segments, ms = 0, 0.0
     for k0 in range(0, args.frames, batch):
-        frames = env.render_frames(tuple(args.size), cameras[k0:k0 + batch], times[k0:k0 + batch], context=context)
+        frames = env.render_frames(tuple(args.size), cameras[k0:k0 + batch], times[k0:k0 + batch], context=context,
+                                   aovs=args.aov or None)
         for j in range(len(frames)):
             frames.frame(j).save(args.output % (k0 + j))
+            if args.aov:
+                write_aovs(args.output % (k0 + j), frames.frame(j).aovs)
         segments += frames.stats["segments"]
         ms += frames.stats["ms_total"]
     print(f"{args.output}: {args.frames} frames of {frames.width}x{frames.height} in calls of {batch}, {segments} ray segments, "
