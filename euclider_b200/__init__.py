@@ -6,8 +6,9 @@ include/euclider_b200.h).  No CPU rendering fallback exists in this package.
 """
 from pathlib import Path
 
-from ._capi import EuclAovs, EuclCamera, EuclError, EuclFrame, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, lib
-from .scene import AOV_NAMES, Environment, Parser, ParserError, RawFrames, RawImage2d, SimulationContext
+from ._capi import EuclAovs, EuclCamera, EuclError, EuclFrame, EuclRays, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, lib
+from .scene import (AOV_NAMES, Environment, Parser, ParserError, RawFrames, RawImage2d, RawRays, SimulationContext,
+                    equirect_rays)
 
 ROOT = Path(__file__).resolve().parent.parent
 ASSET_ROOT = ROOT / "assets"  # the reference scenes, restated, and stand-in textures (assets/make_assets.py)
@@ -18,6 +19,6 @@ def load_reference_scene(name: str) -> Environment:
     return Parser.default(resource_root=ASSET_ROOT).parse_file(ASSET_ROOT / "scenes" / f"{name}.json")
 
 
-__all__ = ["Parser", "Environment", "SimulationContext", "RawImage2d", "RawFrames", "EuclFrame", "EuclAovs", "AOV_NAMES", "ParserError", "EuclError", "EuclCamera",
+__all__ = ["Parser", "Environment", "SimulationContext", "RawImage2d", "RawFrames", "RawRays", "EuclFrame", "EuclAovs", "EuclRays", "equirect_rays", "AOV_NAMES", "ParserError", "EuclError", "EuclCamera",
            "EuclRenderOpts", "EuclStats", "EUCL_PIPELINE_WAVEFRONT", "EUCL_PIPELINE_MEGAKERNEL", "lib",
            "load_reference_scene", "ASSET_ROOT", "ROOT"]

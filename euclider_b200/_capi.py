@@ -80,6 +80,12 @@ class EuclAovs(C.Structure):
                 ("levels", C.c_void_p)]
 
 
+class EuclRays(C.Structure):
+    _fields_ = [("origins", C.c_void_p), ("directions", C.c_void_p), ("n", C.c_uint32), ("width", C.c_uint32),
+                ("max_depth", C.c_uint32), ("pipeline", C.c_int32), ("time_seconds", C.c_double), ("profile", C.c_int32),
+                ("_pad", C.c_int32)]
+
+
 class EuclFlatScene(C.Structure):
     _fields_ = [("dim", C.c_int32),
                 ("n_prims", C.c_int32), ("n_nodes", C.c_int32), ("n_entities", C.c_int32),
@@ -157,6 +163,10 @@ PROTOTYPES = {
                                    C.c_void_p, C.POINTER(EuclAovs), C.POINTER(EuclStats)]),
     "eucl_render_aovs_device": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts),
                                           C.c_void_p, C.c_void_p, C.POINTER(EuclAovs), C.POINTER(EuclStats)]),
+    "eucl_trace_rays": (C.c_int, [C.c_void_p, C.POINTER(EuclRays), C.c_void_p, C.c_void_p, C.POINTER(EuclAovs),
+                                  C.POINTER(EuclStats)]),
+    "eucl_trace_rays_device": (C.c_int, [C.c_void_p, C.POINTER(EuclRays), C.c_void_p, C.c_void_p, C.POINTER(EuclAovs),
+                                         C.POINTER(EuclStats)]),
     "eucl_trace_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,
                                   C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "eucl_camera_rotate_yaw": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),

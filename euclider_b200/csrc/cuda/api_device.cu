@@ -147,6 +147,7 @@ struct EuclScene {
     DeviceBuffer node_frame;
     DeviceBuffer node_cost; // (segments, levels) per node of this pipeline's arena: AOV renders that want either plane
     DeviceBuffer aov_stage; // device copies of the AOV planes for eucl_render_aovs (host output)
+    DeviceBuffer ray_stage; // device copy of the rays of eucl_trace_rays (host input), refilled by every call
     int n_cull = 0;
     int light_capable = 0;
     // Grouping rays by reach key pays on scenes whose deep levels bounce around a few bounded objects
@@ -680,6 +681,7 @@ void eucl_scene_destroy(EuclScene* s) {
     s->node_frame.release();
     s->node_cost.release();
     s->aov_stage.release();
+    s->ray_stage.release();
     if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
     if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
     if (s->h_small) cudaFreeHost(s->h_small);
@@ -997,6 +999,10 @@ struct FrameBatch {
     uint32_t rows;                   // rows per frame
     const FrameParams* d_table;      // K > 1: [K] frame constants on the device, uploaded before the first launch
     uint64_t table_key;              // K > 1: hash of the table contents, part of the graph key
+    // eucl_trace_rays*: the rays on the device ([n][dim] each) in place of a camera (K = 1; frames[0] carries only
+    // max_depth and the time), null for camera frames.  The virtual frame has n / width rows of width rays.
+    const double* ray_origins = nullptr;
+    const double* ray_directions = nullptr;
 };
 
 Workspace carve(EuclScene* s, int dim, int cap, int list_cap, const FrameBatch& fb) {
@@ -1009,8 +1015,8 @@ Workspace carve(EuclScene* s, int dim, int cap, int list_cap, const FrameBatch& 
         ws.frames = fb.d_table;
         ws.frame_entity = (int32_t*)s->frame_entity.ptr;
         ws.node_frame = (int32_t*)s->node_frame.ptr;
-        ws.untraced = (int32_t*)s->small.ptr + SmallLayout::untraced;
     }
+    if (fb.n > 1 || fb.ray_origins) ws.untraced = (int32_t*)s->small.ptr + SmallLayout::untraced;
     uint8_t* p = (uint8_t*)s->nodes.ptr;
     auto take = [&](size_t bytes) {
         uint8_t* r = p;
@@ -1075,8 +1081,16 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                 const AovPlanes& aov_out, EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
     const int dim = s->dim;
     const EuclCamera* cam = &fb.frames[0].camera; // (every frame of a batch has this max_depth)
+    const bool rays = fb.ray_origins != nullptr;
     FrameParams fp;
-    {
+    if (rays) { // no camera: the grid, the depth and the time (truncated as for a frame, then `as F`)
+        std::memset(&fp, 0, sizeof fp);
+        const double millis = std::floor(fb.frames[0].time_seconds * 1000.0) / 1000.0;
+        fp.time_millis = s->real_bytes == 4 ? (double)(float)millis : millis;
+        fp.width = (int)o->width;
+        fp.height = (int)o->height;
+        fp.max_depth = (int)cam->max_depth;
+    } else {
         EuclRenderOpts first = *o;
         first.height = fb.rows;
         first.time_seconds = fb.frames[0].time_seconds;
@@ -1218,18 +1232,22 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                     }
                     mark(-1);
                     if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL) {
-                        EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
-                        dbg("k_camera_entity", 0);
-                        EUCL_PREC(launch_megakernel)(dim, l, fp, cp, ws, d_rgb, d_hit, aov);
+                        if (!rays) {
+                            EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
+                            dbg("k_camera_entity", 0);
+                            launches += 1;
+                        }
+                        EUCL_PREC(launch_megakernel)(dim, l, fp, cp, ws, d_rgb, d_hit, aov, fb.ray_origins, fb.ray_directions);
                         mark(1);
-                        launches += 2;
+                        launches += 1;
                     } else {
                         if (ws.frames) {
                             EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
                             dbg("k_camera_entity", 0);
                             launches += 1;
                         }
-                        EUCL_PREC(launch_raygen)(dim, l, fp, cp, ws, d_hit);
+                        if (rays) EUCL_PREC(launch_raygen_rays)(dim, l, fp, cp, ws, d_hit, fb.ray_origins, fb.ray_directions);
+                        else EUCL_PREC(launch_raygen)(dim, l, fp, cp, ws, d_hit);
                         dbg("k_raygen", 0);
                         mark(0);
                         for (int level = 0; level < (int)cam->max_depth; ++level) {
@@ -1289,9 +1307,17 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
                 // a batch: the graph reads the table the caller's poses were uploaded to, and it is keyed by its contents
                 // too, so that a changed pose or time is never taken for a repeated batch
                 if (fb.n > 1) mix(&fb.table_key, sizeof fb.table_key);
-                // (not while the scene is still choosing its ray-grouping mode: capture time would distort the comparison)
+                // a ray call: tagged, so that a ray call and a render whose other parameters coincide never stand in for
+                // each other, and keyed by the arrays it reads (their contents are read at replay time)
+                if (rays) {
+                    const uint64_t ray_id[] = {0x52415953ull /* "RAYS" */, (uint64_t)(uintptr_t)fb.ray_origins,
+                                               (uint64_t)(uintptr_t)fb.ray_directions, (uint64_t)o->height * o->width, o->width};
+                    mix(ray_id, sizeof ray_id);
+                }
+                // (not while the scene is still choosing its ray-grouping mode: capture time would distort the comparison;
+                // ray calls take no part in that choice)
                 const bool graph_ok = env_int("EUCL_GRAPH", 1) && !o->profile && !debug_sync && !poison &&
-                                      (s->ray_bins_mode >= 0 || o->pipeline != EUCL_PIPELINE_WAVEFRONT);
+                                      (s->ray_bins_mode >= 0 || o->pipeline != EUCL_PIPELINE_WAVEFRONT || rays);
                 if (graph_ok && s->graph_exec && s->graph_key == key) {
                     EUCL_CUDA(cudaGraphLaunch(s->graph_exec, s->stream));
                     st.launches += s->graph_launches;
@@ -1408,8 +1434,11 @@ int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uin
             s->graph_key = s->seen_key = 0;
         }
     }
-    if (sub_stride <= 1) tune_grouping(s, st, o->pipeline); // (a split frame is judged as a whole: render_split)
-    s->warm_frames++;
+    // (a split frame is judged as a whole: render_split).  A ray batch is not a frame of its size: it never tunes.
+    if (!rays) {
+        if (sub_stride <= 1) tune_grouping(s, st, o->pipeline);
+        s->warm_frames++;
+    }
     st.ray_grouping = s->ray_bins_now && s->rorder.ptr != nullptr && o->pipeline == EUCL_PIPELINE_WAVEFRONT ? 1u : 0u;
     if (stats) *stats = st;
     return EUCL_OK;
@@ -1542,7 +1571,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
         st.ms_shade += b.ms_shade;
         st.ms_resolve += b.ms_resolve;
     }
-    tune_grouping(s, st, o->pipeline);
+    if (!fb.ray_origins) tune_grouping(s, st, o->pipeline);
     if (stats) *stats = st;
     return EUCL_OK;
 }
@@ -1607,9 +1636,11 @@ int prepare_batch(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclR
     return EUCL_OK;
 }
 
-// Device-output render of `n` frames (eucl_render_device: n = 1).
+// Device-output render of `n` frames (eucl_render_device: n = 1), or -- `rays` -- of a ray call's virtual frame (`o` then
+// is that frame and `frames` is rays->frames).
 int render_frames_to_device(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* d_rgb,
-                            int32_t* d_hit, const AovPlanes& aov, EuclStats* stats) {
+                            int32_t* d_hit, const AovPlanes& aov, EuclStats* stats, const FrameBatch* rays = nullptr) {
+    if (rays) return render_split(s, *rays, o, d_rgb, d_hit, aov, stats);
     FrameBatch fb;
     EuclRenderOpts virt;
     const int st = prepare_batch(s, frames, n, o, &fb, &virt);
@@ -1633,7 +1664,7 @@ AovPlanes aov_planes(const EuclAovs* a) {
 // each band to its place in the caller's frame: rows of other ranks are never read or written, so N ranks can fill ONE
 // host frame (shared pinned memory) over their own PCIe links at the same time.  The AOV planes go the same way.
 int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* out_rgb8,
-                   int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats) {
+                   int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats, const FrameBatch* rays = nullptr) {
     EUCL_CUDA(cudaSetDevice(s->device));
     const bool scatter = !o->compact_rows && o->band_world > 1;
     const size_t my_rows = eucl_band_rows_for_rank(o);
@@ -1664,7 +1695,7 @@ int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const Eucl
     opts.want_hit_ids = want_hit ? 1 : 0;
     if (scatter) opts.compact_rows = 1;
     const int st = render_frames_to_device(s, frames, n, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr,
-                                           d_aov, stats);
+                                           d_aov, stats, rays);
     if (st != EUCL_OK) return st;
     if (!scatter) {
         EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));
@@ -1760,6 +1791,85 @@ int eucl_render_aovs_device(EuclScene* s, const EuclFrame* frames, uint32_t n_fr
     EUCL_CUDA(cudaSetDevice(s->device));
     return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
                                    o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, aov_planes(d_aovs), stats);
+}
+
+} // extern "C"
+
+namespace {
+
+static_assert(sizeof(EuclRays) == 48, "EuclRays is part of the C ABI");
+
+// eucl_trace_rays*: checked before any device is touched.
+int check_rays(EuclScene* s, const EuclRays* r, const void* out, const char* fn) {
+    const std::string f(fn);
+    if (!s || !r) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null argument");
+    if (r->n == 0 || r->n > 0x7fffffffu) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n must be 1 .. 2^31 - 1");
+    if (!r->origins || !r->directions) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null ray array");
+    if (!out) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null output");
+    if (r->width > 1 && r->n % r->width != 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": width does not divide n");
+    if (r->max_depth + 1ull > EUCL_MAX_LEVELS) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": max_depth too large");
+    if (r->pipeline != EUCL_PIPELINE_WAVEFRONT && r->pipeline != EUCL_PIPELINE_MEGAKERNEL)
+        return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": unknown pipeline");
+    return EUCL_OK;
+}
+
+// The virtual frame of a ray call (n / width rows of width) and its batch: one "frame" that carries the depth and the
+// time, and the device rays.
+struct RayCall {
+    EuclFrame frame;
+    EuclRenderOpts opts;
+    FrameBatch fb;
+    RayCall(const EuclScene* s, const EuclRays* r, const double* d_origins, const double* d_directions, bool want_hit) {
+        std::memset(&frame, 0, sizeof frame);
+        frame.camera.dim = s->dim;
+        frame.camera.max_depth = r->max_depth;
+        frame.time_seconds = r->time_seconds;
+        const uint32_t w = r->width > 1 ? r->width : 1;
+        opts = EuclRenderOpts{};
+        opts.width = w;
+        opts.height = r->n / w;
+        opts.time_seconds = r->time_seconds;
+        opts.pipeline = r->pipeline;
+        opts.want_hit_ids = want_hit ? 1 : 0;
+        opts.profile = r->profile;
+        fb = FrameBatch{&frame, 1, opts.height, nullptr, 0};
+        fb.ray_origins = d_origins;
+        fb.ray_directions = d_directions;
+    }
+};
+
+const EuclAovs* any_plane(const EuclAovs* a) {
+    return a && (a->depth || a->position || a->normal || a->segments || a->levels) ? a : nullptr;
+}
+
+} // namespace
+
+extern "C" {
+
+int eucl_trace_rays(EuclScene* s, const EuclRays* r, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs,
+                    EuclStats* stats) {
+    const int st = check_rays(s, r, out_rgb8, "eucl_trace_rays");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    // staged before the first launch, on the scene's stream and outside any graph capture: a replayed graph reads them
+    const size_t bytes = sizeof(double) * (size_t)s->dim * r->n;
+    EUCL_CUDA(s->ray_stage.ensure(2 * bytes));
+    double* d_o = (double*)s->ray_stage.ptr;
+    double* d_d = (double*)((uint8_t*)s->ray_stage.ptr + bytes);
+    EUCL_CUDA(cudaMemcpyAsync(d_o, r->origins, bytes, cudaMemcpyHostToDevice, s->stream));
+    EUCL_CUDA(cudaMemcpyAsync(d_d, r->directions, bytes, cudaMemcpyHostToDevice, s->stream));
+    RayCall call(s, r, d_o, d_d, out_hit_ids != nullptr);
+    return render_to_host(s, &call.frame, 1, &call.opts, out_rgb8, out_hit_ids, any_plane(aovs), stats, &call.fb);
+}
+
+int eucl_trace_rays_device(EuclScene* s, const EuclRays* r, void* d_out_rgb8, void* d_out_hit_ids, const EuclAovs* d_aovs,
+                           EuclStats* stats) {
+    const int st = check_rays(s, r, d_out_rgb8, "eucl_trace_rays_device");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    RayCall call(s, r, r->origins, r->directions, d_out_hit_ids != nullptr);
+    return render_frames_to_device(s, &call.frame, 1, &call.opts, (uint8_t*)d_out_rgb8, (int32_t*)d_out_hit_ids,
+                                   aov_planes(any_plane(d_aovs)), stats, &call.fb);
 }
 
 int eucl_scene_memory(const EuclScene* s, uint64_t* arena_bytes, uint64_t* list_bytes, uint64_t* node_capacity) {

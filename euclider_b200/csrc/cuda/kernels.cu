@@ -424,6 +424,62 @@ __global__ void __launch_bounds__(kBlock) k_raygen(const uint8_t* __restrict__ b
     }
 }
 
+// K1 of eucl_trace_rays*: the caller's rays instead of a camera.  Node i of the chunk is cell (x, y) of the call's virtual
+// frame of n / width rows, i.e. ray y * width + x of the [n][dim] f64 arrays, narrowed once to `real`.  Every ray has an
+// origin of its own, so every thread evaluates material_at (k_raygen does it once per CTA).  A ray whose origin lies in no
+// entity is a checkerboard leaf of its cell, like a pixel of an untraced frame of a batch, and is counted in ws.untraced;
+// *ws.cam_entity keeps the 0 of the counter reset, so the level is intersected whenever any of its rays is traced.
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_raygen_rays(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                        Workspace ws, int32_t* __restrict__ hit_ids_out,
+                                                        const double* __restrict__ origins, const double* __restrict__ directions) {
+    const SceneView& sv = stage_scene(blob);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        ws.count[0] = cp.n_pixels;
+        ws.level_off[0] = 0;
+    }
+    const unsigned lane = threadIdx.x & 31u;
+    for (int base = blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < cp.n_pixels; base += gridDim.x * blockDim.x) {
+        const int i = base + (int)lane;
+        const bool valid = i < cp.n_pixels;
+        const int local_row = cp.local_row0 + (valid ? i : 0) / fp.width;
+        const int x = (valid ? i : 0) % fp.width;
+        const int y = frame_row_of_local(cp, local_row);
+        const size_t ray = ((size_t)y * fp.width + x) * D;
+        Vec<D> o, dir;
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            o[k] = R(origins[ray + k]);
+            dir[k] = R(directions[ray + k]);
+        }
+        const int belongs_to = valid ? material_at<D>(sv, o) : -1;
+        const bool traced = belongs_to >= 0;
+        const unsigned untraced = __ballot_sync(0xffffffffu, valid && !traced);
+        if (lane == 0 && untraced) atomicAdd(ws.untraced, __popc(untraced));
+        if (valid && !traced) {
+            store_res(ws, i, checkerboard(x, y));
+            ws.meta[i] = NodeMeta{R(0.0), -1, -1, 0u, NODE_LEAF | NODE_FINAL_RGB};
+            if (hit_ids_out) hit_ids_out[(size_t)out_row_of_local(cp, local_row) * fp.width + x] = -2;
+        }
+        // an untraced node keeps its ray as given (k_intersect may walk it when the level is not grouped by reach key);
+        // ray_cur -1 keeps k_shade off it
+        if (traced) material_enter<D>(sv, belongs_to, dir);
+        if (valid) store_ray<D>(ws, i, o, dir, traced ? belongs_to : -1);
+        if (ws.ray_bins) { // as k_raygen
+            const unsigned active = __ballot_sync(0xffffffffu, valid && traced);
+            if (valid && traced) {
+                const int key = reach_key<D>(sv, o, dir);
+                const unsigned peers = __match_any_sync(active, key);
+                const int leader = __ffs(peers) - 1;
+                int s2 = 0;
+                if ((int)lane == leader) s2 = atomicAdd(&ws.rbin_count[key], __popc(peers));
+                s2 = __shfl_sync(peers, s2, leader);
+                ws.rorder[(size_t)key * ws.list_cap + s2 + __popc(peers & ((1u << lane) - 1u))] = i;
+            }
+        }
+    }
+}
+
 // K2: closest hit of every ray of one level.
 //
 // Two builds share a level when its rays are grouped by reach key and the scene allows it (SceneHeader::light_capable):
@@ -889,10 +945,12 @@ struct MegaFrame {
 
 // AOV (k_megakernel_aov): also the AOV planes -- the level-0 geometry, and the segments and levels counted along the walk.
 // The cross-check of k_aov_primary and the COST builds of the wavefront.
-template <int D, bool AOV>
+// RAYS (k_megakernel_rays*): the caller's rays of eucl_trace_rays* instead of a camera, addressed as in k_raygen_rays.
+template <int D, bool AOV, bool RAYS>
 __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ blob, const FrameParams& fp, const ChunkParams& cp,
                                                   const Workspace& ws, uint8_t* __restrict__ out_rgb8,
-                                                  int32_t* __restrict__ hit_ids_out, const AovPlanes& aov) {
+                                                  int32_t* __restrict__ hit_ids_out, const AovPlanes& aov,
+                                                  const double* __restrict__ origins, const double* __restrict__ directions) {
     const SceneView& sv = stage_scene(blob);
     real* ts = plane_scratch(blob);
     const int cam_entity = *ws.cam_entity;
@@ -904,7 +962,16 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
         int y = frame_row_of_local(cp, local_row);
         const size_t opix = (size_t)out_row_of_local(cp, local_row) * fp.width + x;
         int belongs_to = cam_entity, f = 0;
-        if (ws.frames) {
+        Vec<D> ray_o, ray_d;
+        if (RAYS) {
+            const size_t ray = ((size_t)y * fp.width + x) * D;
+#pragma unroll
+            for (int k = 0; k < D; ++k) {
+                ray_o[k] = R(origins[ray + k]);
+                ray_d[k] = R(directions[ray + k]);
+            }
+            belongs_to = material_at<D>(sv, ray_o);
+        } else if (ws.frames) {
             f = frame_of_row(ws, y);
             belongs_to = ws.frame_entity[f];
         }
@@ -912,7 +979,7 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
             final_rgb8(checkerboard(x, y), false, out_rgb8 + opix * 3);
             if (hit_ids_out) hit_ids_out[opix] = -2;
             local_counts[0]++;
-            if (ws.frames) atomicAdd(ws.untraced, 1);
+            if (RAYS || ws.frames) atomicAdd(ws.untraced, 1);
             if (AOV) {
                 const Vec<D> zero{};
                 write_primary<D>(aov, opix, false, false, R(0.0), zero, zero);
@@ -924,10 +991,15 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
         unsigned aov_segments = 0u, aov_levels = 0u;
         MegaFrame<D> stack[kMegaMaxDepth];
         Vec<D> o, d;
+        if (RAYS) {
+            o = ray_o;
+            d = ray_d;
+        } else {
 #pragma unroll
-        for (int k = 0; k < D; ++k) o[k] = R(ws.frames ? ws.frames[f].location[k] : fp.location[k]);
-        d = ws.frames ? camera_ray<D>(ws.frames[f], x, y) : camera_ray<D>(fp, x, y);
-        const real time_millis = R(ws.frames ? ws.frames[f].time_millis : fp.time_millis);
+            for (int k = 0; k < D; ++k) o[k] = R(ws.frames ? ws.frames[f].location[k] : fp.location[k]);
+            d = ws.frames ? camera_ray<D>(ws.frames[f], x, y) : camera_ray<D>(fp, x, y);
+        }
+        const real time_millis = R(!RAYS && ws.frames ? ws.frames[f].time_millis : fp.time_millis);
         material_enter<D>(sv, belongs_to, d);
         int cur = belongs_to, level = 0;
         Rgba val{R(0.0), R(0.0), R(0.0), R(0.0)};
@@ -1028,13 +1100,28 @@ template <int D>
 __global__ void __launch_bounds__(kBlock) k_megakernel(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
                                                        Workspace ws, uint8_t* __restrict__ out_rgb8,
                                                        int32_t* __restrict__ hit_ids_out) {
-    megakernel_pixels<D, false>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{});
+    megakernel_pixels<D, false, false>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{}, nullptr, nullptr);
 }
 template <int D>
 __global__ void __launch_bounds__(kBlock) k_megakernel_aov(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
                                                            Workspace ws, uint8_t* __restrict__ out_rgb8,
                                                            int32_t* __restrict__ hit_ids_out, AovPlanes aov) {
-    megakernel_pixels<D, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, aov);
+    megakernel_pixels<D, true, false>(blob, fp, cp, ws, out_rgb8, hit_ids_out, aov, nullptr, nullptr);
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel_rays(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                            Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                            int32_t* __restrict__ hit_ids_out, const double* __restrict__ origins,
+                                                            const double* __restrict__ directions) {
+    megakernel_pixels<D, false, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{}, origins, directions);
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel_rays_aov(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                                Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                                int32_t* __restrict__ hit_ids_out, AovPlanes aov,
+                                                                const double* __restrict__ origins,
+                                                                const double* __restrict__ directions) {
+    megakernel_pixels<D, true, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, aov, origins, directions);
 }
 
 // Universe::trace_path_unknown / trace_path (mod.rs:186-227,273-286) with Surface::get_path
@@ -1150,6 +1237,13 @@ void launch_raygen(int dim, const Launch& l, const FrameParams& fp, const ChunkP
     EUCL_DISPATCH_DIM(dim, (k_raygen<3><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out)),
                       (k_raygen<4><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out)));
 }
+void launch_raygen_rays(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
+                        int32_t* hit_ids_out, const double* origins, const double* directions) {
+    const int grid = grid_for(cp.n_pixels, kBlock, l.grid_mem);
+    EUCL_DISPATCH_DIM(
+        dim, (k_raygen_rays<3><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out, origins, directions)),
+        (k_raygen_rays<4><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out, origins, directions)));
+}
 // fork: the side stream waits for everything enqueued on the main stream so far; join: the main stream waits for the side
 static void fork_side(const Launch& l) {
     cudaEventRecord(l.ev_fork, l.stream);
@@ -1257,9 +1351,27 @@ int launch_resolve_and_final(int dim, const Launch& l, const FrameParams& fp, co
     return launches;
 }
 void launch_megakernel(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                       uint8_t* out_rgb8, int32_t* hit_ids_out, const AovPlanes& aov) {
+                       uint8_t* out_rgb8, int32_t* hit_ids_out, const AovPlanes& aov, const double* origins,
+                       const double* directions) {
     const int grid = grid_for(cp.n_pixels, kBlock, 1 << 30);
-    if (aov.depth || aov.position || aov.normal || aov.segments || aov.levels) {
+    const bool want_aov = aov.depth || aov.position || aov.normal || aov.segments || aov.levels;
+    if (origins && want_aov) {
+        EUCL_DISPATCH_DIM(dim,
+                          (k_megakernel_rays_aov<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                             aov, origins, directions)),
+                          (k_megakernel_rays_aov<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                             aov, origins, directions)));
+        return;
+    }
+    if (origins) {
+        EUCL_DISPATCH_DIM(dim,
+                          (k_megakernel_rays<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                         origins, directions)),
+                          (k_megakernel_rays<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                         origins, directions)));
+        return;
+    }
+    if (want_aov) {
         EUCL_DISPATCH_DIM(
             dim, (k_megakernel_aov<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)),
             (k_megakernel_aov<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)));
@@ -1330,6 +1442,12 @@ cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene) {
     EUCL_CONF(k_megakernel<4>, smem_bytes, heavy);
     EUCL_CONF(k_megakernel_aov<3>, smem_bytes, heavy);
     EUCL_CONF(k_megakernel_aov<4>, smem_bytes, heavy);
+    EUCL_CONF(k_raygen_rays<3>, smem_scene, 2);
+    EUCL_CONF(k_raygen_rays<4>, smem_scene, 2);
+    EUCL_CONF(k_megakernel_rays<3>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_rays<4>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_rays_aov<3>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_rays_aov<4>, smem_bytes, heavy);
     EUCL_CONF(k_trace_path<3>, smem_bytes, 1);
     EUCL_CONF(k_trace_path<4>, smem_bytes, 1);
 #undef EUCL_CONF

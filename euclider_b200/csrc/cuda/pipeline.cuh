@@ -111,7 +111,8 @@ struct Workspace {
     const FrameParams* frames; // [n_frames] per-frame constants (pose, time)
     int32_t* frame_entity;     // [n_frames] material_at(camera location of the frame), -1 if none
     int32_t* node_frame;       // [capacity] frame of every node (Perlin time): level 0 by k_raygen, children by k_shade
-    int32_t* untraced;         // level-0 nodes of this chunk whose frame's camera is in no entity (checkerboard pixels)
+    int32_t* untraced;         // level-0 nodes of this chunk whose frame's camera (eucl_trace_rays*: whose ray's origin) is in
+                               // no entity (checkerboard pixels); also carved for ray calls, which have no frame table
 };
 
 // Per-pixel auxiliary outputs of the primary ray and its tree (eucl_render_aovs*, definitions in DESIGN.md §6): device planes
@@ -193,13 +194,16 @@ constexpr int kMaxBins = 64; // shade-coherence bins (miss, then kBinsPerEntity 
     void launch_camera_entity(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::Workspace& ws);        \
     void launch_raygen(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,              \
                        const eucl::Workspace& ws, int32_t* hit_ids_out);                                                       \
+    void launch_raygen_rays(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,         \
+                            const eucl::Workspace& ws, int32_t* hit_ids_out, const double* origins, const double* directions); \
     int launch_intersect(int dim, const eucl::Launch& l, const eucl::Workspace& ws, int level);                                \
     int launch_shade(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,                \
                      const eucl::Workspace& ws, int level, int32_t* hit_ids_out);                                              \
     int launch_resolve_and_final(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,    \
                                  const eucl::Workspace& ws, uint8_t* out_rgb8, const eucl::AovPlanes& aov);                    \
     void launch_megakernel(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
-                           const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out, const eucl::AovPlanes& aov);    \
+                           const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out, const eucl::AovPlanes& aov,     \
+                           const double* origins, const double* directions);                                               \
     void launch_trace_path(int dim, const eucl::Launch& l, const double* d_in, double distance, double* d_out, int* d_found); \
     cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);                                                       \
     }

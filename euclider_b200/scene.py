@@ -17,7 +17,7 @@ from typing import Dict, Mapping, Optional, Sequence, Tuple, Union
 import numpy as np
 
 from . import _capi
-from ._capi import (EuclAovs, EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRenderOpts, EuclStats,
+from ._capi import (EuclAovs, EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRays, EuclRenderOpts, EuclStats,
                     EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, check, lib)
 
 ParserError = EuclError  # the reference's `ParserError` (src/scene.rs:524-552); see EuclError.status
@@ -76,6 +76,67 @@ class RawFrames:
         """Frame k as a RawImage2d (a view, no copy)."""
         return RawImage2d(self.data[k], self.width, self.height, hit_ids=None if self.hit_ids is None else self.hit_ids[k],
                           aovs=None if self.aovs is None else {name: a[k] for name, a in self.aovs.items()})
+
+
+@dataclass
+class RawRays:
+    """The outputs of one Environment.trace_rays call, in ray order with the rays' leading shape."""
+    data: np.ndarray  # uint8, shape (..., 3): RGB8 of each ray (the checkerboard of its grid cell when its origin is in no entity)
+    hit_ids: Optional[np.ndarray] = None  # int32 (...): primary hit entity, -1 a miss, -2 an origin in no entity
+    stats: Optional[dict] = None
+    aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name, leading shape as `data`
+
+
+def equirect_rays(camera: EuclCamera, width: int, height: int) -> Tuple[np.ndarray, np.ndarray]:
+    """Equirectangular (360 x 180 degree) panorama rays of a camera pose for Environment.trace_rays: (origins, directions),
+    both float64 of shape (height, width, dim), row 0 at the bottom.  Every origin is the camera location; cell (x, y) looks
+    at longitude phi = 2 pi ((x + 0.5) / width - 0.5) and latitude theta = pi ((y + 0.5) / height - 0.5) in the 3-space the
+    perspective camera's screen spans: cos(theta) (cos(phi) F - sin(phi) L) + sin(theta) U, with F forward, U up and L
+    `left` (4-D) or -normalize(F x U) (3-D).  The centre column looks forward, the first and last columns look back."""
+    dim = int(camera.dim)
+    if dim not in (3, 4):
+        raise ValueError("camera.dim must be 3 or 4")
+    if int(width) < 1 or int(height) < 1:
+        raise ValueError("width and height must be positive")
+    f = np.array(camera.forward[:dim], dtype=np.float64)
+    u = np.array(camera.up[:dim], dtype=np.float64)
+    if dim == 3:
+        c = np.cross(f, u)
+        left = -c / np.linalg.norm(c)
+    else:
+        left = np.array(camera.left[:dim], dtype=np.float64)
+    phi = 2.0 * np.pi * ((np.arange(width, dtype=np.float64) + 0.5) / width - 0.5)
+    theta = np.pi * ((np.arange(height, dtype=np.float64) + 0.5) / height - 0.5)
+    ct, st = np.cos(theta)[:, None, None], np.sin(theta)[:, None, None]
+    cp, sp = np.cos(phi)[None, :, None], np.sin(phi)[None, :, None]
+    directions = ct * (cp * f - sp * left) + st * u
+    origins = np.broadcast_to(np.array(camera.location[:dim], dtype=np.float64), directions.shape).copy()
+    return origins, np.ascontiguousarray(directions)
+
+
+def _ray_arrays(origins, directions, dim: int) -> Tuple[np.ndarray, np.ndarray, Tuple[int, ...]]:
+    """float64 C-contiguous copies (when needed) of two (..., dim) arrays of one shape, and their leading shape."""
+    o = np.ascontiguousarray(origins, dtype=np.float64)
+    d = np.ascontiguousarray(directions, dtype=np.float64)
+    if o.shape != d.shape:
+        raise ValueError(f"origins {o.shape} and directions {d.shape} must have the same shape")
+    if o.ndim < 1 or o.shape[-1] != dim:
+        raise ValueError(f"rays must have shape (..., {dim}) for this {dim}-D scene, got {o.shape}")
+    lead = o.shape[:-1]
+    if int(np.prod(lead, dtype=np.int64)) < 1 or int(np.prod(lead, dtype=np.int64)) > 0x7FFFFFFF:
+        raise ValueError("trace_rays needs 1 .. 2^31 - 1 rays")
+    return o, d, lead
+
+
+def _ray_struct(n: int, width: int, max_depth: int, pipeline: int, time: float, profile: bool, origins: int = 0,
+                directions: int = 0) -> EuclRays:
+    width = max(int(width), 1)
+    if n % width:
+        raise ValueError(f"width {width} does not divide the {n} rays")
+    if int(max_depth) < 0 or int(max_depth) + 1 > _capi.EUCL_MAX_LEVELS:
+        raise ValueError(f"max_depth must be 0 .. {_capi.EUCL_MAX_LEVELS - 1}")
+    return EuclRays(origins=origins, directions=directions, n=n, width=width, max_depth=int(max_depth), pipeline=pipeline,
+                    time_seconds=float(time), profile=int(profile))
 
 
 # Per-pixel auxiliary outputs (include/euclider_b200.h, EuclAovs): name -> (dtype, one value per pixel or `dim` values).
@@ -283,6 +344,47 @@ class Environment:
             check(lib().eucl_render_frames_device(self._device_scene(device), table, len(table), C.byref(opts),
                                                   C.c_void_p(d_out_rgb8), C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None,
                                                   C.byref(stats)))
+        return stats_to_dict(stats)
+
+    # -- caller-supplied rays: custom projections, picking, probes -----------------------------------
+    def trace_rays(self, origins, directions, time: float = 0.0, *, max_depth: Optional[int] = None,
+                   width: Optional[int] = None, device: int = 0, want_hit_ids: bool = True, aovs=None,
+                   out: Optional[np.ndarray] = None, profile: bool = False) -> RawRays:
+        """Traces one ray per origin / direction pair (eucl_trace_rays): arrays of shape (..., dim), converted to
+        float64.  Directions are used as given (not normalised).  Ray i gives what a pixel whose camera ray is
+        (origins[i], directions[i]) gives -- its RGB8 value, primary hit and AOV planes -- and an origin in no entity gives
+        the checkerboard of grid cell (i % width, i // width).  `width` (rays per grid row) defaults to the last leading
+        dimension of an (H, W, dim) grid and to 1 for a flat (N, dim) list; `max_depth` to the camera's.  Tracing the
+        camera's own rays of a w x h frame with width w reproduces `render((w, h), time)` bit for bit."""
+        o, d, lead = _ray_arrays(origins, directions, self.dim)
+        n = int(np.prod(lead, dtype=np.int64))
+        if width is None:
+            width = lead[-1] if len(lead) >= 2 else 1
+        rays = _ray_struct(n, width, self.camera.max_depth if max_depth is None else max_depth, self.pipeline, time, profile,
+                           o.ctypes.data, d.ctypes.data)
+        if out is None:
+            out = np.zeros(lead + (3,), dtype=np.uint8)
+        if out.dtype != np.uint8 or out.shape != lead + (3,) or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {lead + (3,)}")
+        hit = np.full(lead, -3, dtype=np.int32) if want_hit_ids else None
+        planes = _aov_arrays(aovs, lead, self.dim) if aovs else None
+        stats = EuclStats()
+        aov = C.byref(_aov_struct({k: a.ctypes.data for k, a in planes.items()})) if planes else None
+        check(lib().eucl_trace_rays(self._device_scene(device), C.byref(rays), out.ctypes.data,
+                                    hit.ctypes.data if hit is not None else None, aov, C.byref(stats)))
+        return RawRays(out, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
+
+    def trace_rays_device(self, d_origins: int, d_directions: int, n: int, d_out_rgb8: int, time: float = 0.0, *,
+                          max_depth: Optional[int] = None, width: int = 1, device: int = 0, d_out_hit_ids: int = 0,
+                          d_aovs: Optional[Mapping[str, int]] = None, profile: bool = False) -> dict:
+        """trace_rays with DEVICE arrays: `n` rays of `dim` float64 each at d_origins / d_directions, n * 3 bytes of RGB8,
+        n int32 hit ids and the AOV planes of `d_aovs` (name -> device pointer).  Returns the stats."""
+        rays = _ray_struct(int(n), width, self.camera.max_depth if max_depth is None else max_depth, self.pipeline, time,
+                           profile, int(d_origins), int(d_directions))
+        stats = EuclStats()
+        aov = C.byref(_device_aovs(d_aovs)) if d_aovs else None
+        check(lib().eucl_trace_rays_device(self._device_scene(device), C.byref(rays), C.c_void_p(d_out_rgb8),
+                                           C.c_void_p(d_out_hit_ids) if d_out_hit_ids else None, aov, C.byref(stats)))
         return stats_to_dict(stats)
 
     def trace_path_unknown(self, location: Sequence[float], direction: Sequence[float], distance: float, *,

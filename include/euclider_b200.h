@@ -389,6 +389,47 @@ int eucl_render_aovs(EuclScene* scene, const EuclFrame* frames, uint32_t n_frame
 int eucl_render_aovs_device(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
                             void* d_out_rgb8, void* d_out_hit_ids, const EuclAovs* d_aovs, EuclStats* stats);
 
+/* Caller-supplied rays instead of a camera: custom projections (panoramas, fisheyes, stereo pairs), jittered or
+ * supersampled primaries, picking and probes.  Ray i has origin o = origins[i] and direction d = directions[i] (`dim`
+ * doubles each; an f32 scene narrows them once).  d is used AS GIVEN, not normalised, like the vector of
+ * Universe::trace_unknown (mod.rs:253-271).  The outputs of ray i are those of a pixel whose camera ray is (o, d):
+ *   e = material_at(o) >= 0: the colour of trace(max_depth, e, o, material_enter(e, d)) composited over opaque white,
+ *       the primary hit entity (-1: a miss), and the AOV planes of the primary ray (o, d') with d' = material_enter(e, d)
+ *       (depth in units of |d'|);
+ *   e < 0: the reference's checkerboard (mod.rs:387-395) at grid cell (x, y) = (i % W, i / W) with W = `width`, hit id
+ *       -2, depth / position / normal NaN, segments / levels 0; counted in EuclStats.pixels and in no level count.
+ * Tracing the w x h camera rays of a pose (W = w, every origin the camera location) gives eucl_render's frame, hit
+ * ids, AOVs and counted EuclStats bit for bit.  One time (Perlin only) and one max_depth per call.
+ * The rays form a virtual frame of n / W rows of W and are chunked, split across pipelines and graph-replayed like a
+ * frame; a row is never split across chunks, so keep W moderate (a flat list: W = 1).  There is no band split and no
+ * compact layout: a ray list is split by the caller. */
+typedef struct EuclRays {
+    const double* origins;    /* [n][dim] */
+    const double* directions; /* [n][dim], used as given (not normalised) */
+    uint32_t n;               /* 1 .. 2^31 - 1 */
+    uint32_t width;           /* rays per grid row; 0 or 1 = a flat list; must divide n */
+    uint32_t max_depth;       /* as EuclCamera.max_depth */
+    int32_t pipeline;         /* EuclPipeline */
+    double time_seconds;      /* Perlin only, truncated to whole ms as for a frame */
+    int32_t profile;          /* as EuclRenderOpts.profile */
+    int32_t _pad;
+} EuclRays;                   /* 48 bytes */
+
+/* Traces `rays` (host arrays) into HOST outputs in ray order: n * 3 bytes of RGB8, and -- each optional -- n int32 hit
+ * ids (entity of the primary hit, -1 a miss, -2 an origin in no entity) and the planes of `aovs` (n entries each, as
+ * EuclAovs; an `aovs` without any plane counts as NULL).  The rays are copied to a scene-owned device buffer, stream-ordered
+ * before the first launch.  Synchronous.  EUCL_ERR_INVALID_ARGUMENT, before any device work, for n == 0 or n > 2^31 - 1,
+ * null origins, directions or output, a width that does not divide n, max_depth + 1 > EUCL_MAX_LEVELS and an unknown
+ * pipeline; the megakernel pipeline with max_depth > 24 fails with EUCL_ERR_SCENE_LIMIT. */
+int eucl_trace_rays(EuclScene* scene, const EuclRays* rays, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs,
+                    EuclStats* stats);
+
+/* Same, with DEVICE arrays on the scene's device: the rays' origins and directions, the output, the hit ids and every plane
+ * of `d_aovs` (the two structs themselves are read on the host).  A repeated call replays its CUDA graph and reads the
+ * arrays' current contents. */
+int eucl_trace_rays_device(EuclScene* scene, const EuclRays* rays, void* d_out_rgb8, void* d_out_hit_ids,
+                           const EuclAovs* d_aovs, EuclStats* stats);
+
 /* Universe::trace_path_unknown (src/universe/mod.rs:273-286): moves `location` by `distance` along
  * `direction` THROUGH the universe -- surfaces are crossed with the material transitions of the
  * entities on either side, so a step through a LinearSpace void is stretched or shrunk.  The

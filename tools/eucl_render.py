@@ -14,6 +14,11 @@ rendered --batch at a time (default: all in one call, Environment.render_frames)
 Per-pixel auxiliary outputs with --aov depth,position,normal,segments,levels: next to each image `out.png` the tool writes
 `out.<plane>.npy` (the plane as the library returns it, row 0 = bottom) and, for the scalar planes, a greyscale preview
 `out.<plane>.png` (top-down; depth and levels linear, segments on a log scale; pixels without a value black).
+
+A 360 x 180 degree panorama of the camera's position with --projection equirect (Environment.trace_rays of
+euclider_b200.equirect_rays; the centre column looks forward).  The default, perspective, is the camera's own projection.
+
+    python tools/eucl_render.py assets/scenes/3d_room.json pano.png --size 2048 1024 --projection equirect
 """
 import argparse
 import os
@@ -39,6 +44,8 @@ def parse_args(argv=None):
     ap.add_argument("--max-depth", type=int)
     ap.add_argument("--resolution", type=int, default=1, help="the reference's resolution divisor")
     ap.add_argument("--pipeline", default="wavefront", choices=["wavefront", "megakernel"])
+    ap.add_argument("--projection", default="perspective", choices=["perspective", "equirect"],
+                    help="equirect: a 360 x 180 degree panorama from the camera's position (single frames only)")
     seq = ap.add_argument_group("image sequences (per-frame motion; angles in radians)")
     seq.add_argument("--frames", type=int, default=1, help="frames to render")
     seq.add_argument("--batch", type=int, help="frames per render call (default: all)")
@@ -63,6 +70,8 @@ def parse_args(argv=None):
         ap.error("--plane4: A and B are axis indices")
     if args.frames > 1 and "%" not in args.output:
         ap.error("--frames > 1 needs an output pattern such as out_%04d.ppm")
+    if args.projection != "perspective" and is_sequence(args):
+        ap.error("--projection equirect renders single frames only")
     return args
 
 
@@ -129,6 +138,15 @@ def main(argv=None):
         env.camera.max_depth = args.max_depth
     env.pipeline = eb.EUCL_PIPELINE_MEGAKERNEL if args.pipeline == "megakernel" else eb.EUCL_PIPELINE_WAVEFRONT
     context = eb.SimulationContext(resolution=args.resolution)
+    if args.projection == "equirect":
+        w, h = args.size[0] // args.resolution, args.size[1] // args.resolution
+        res = env.trace_rays(*eb.equirect_rays(env.camera, w, h), args.time, want_hit_ids=False, aovs=args.aov or None)
+        eb.RawImage2d(res.data, w, h).save(args.output)
+        if args.aov:
+            write_aovs(args.output, res.aovs)
+        st = res.stats
+        print(f"{args.output}: {w}x{h} equirect, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
+        return
     if not is_sequence(args):
         img = env.render(tuple(args.size), args.time, context=context, aovs=args.aov or None)
         img.save(args.output)
