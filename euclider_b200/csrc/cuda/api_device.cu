@@ -11,6 +11,7 @@
 #include <cstring>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -47,27 +48,36 @@ int env_int(const char* name, int fallback) {
     return v && *v ? std::atoi(v) : fallback;
 }
 
-struct DeviceBuffer {
+// Grow-only device memory, or pinned host memory (kPinned), freed with its owner.
+template <bool kPinned>
+struct Buffer {
     void* ptr = nullptr;
     size_t bytes = 0;
+    Buffer() = default;
+    Buffer(const Buffer&) = delete;
+    Buffer& operator=(const Buffer&) = delete;
+    ~Buffer() { release(); }
     cudaError_t ensure(size_t want) {
         if (want <= bytes) return cudaSuccess;
-        if (ptr) cudaFree(ptr);
-        ptr = nullptr;
-        bytes = 0;
-        cudaError_t e = cudaMalloc(&ptr, want);
+        release();
+        cudaError_t e = kPinned ? cudaMallocHost(&ptr, want) : cudaMalloc(&ptr, want);
         if (e == cudaSuccess) bytes = want;
         return e;
     }
     void release() {
-        if (ptr) cudaFree(ptr);
+        if (ptr) {
+            if (kPinned) cudaFreeHost(ptr);
+            else cudaFree(ptr);
+        }
         ptr = nullptr;
         bytes = 0;
     }
 };
+using DeviceBuffer = Buffer<false>;
+using PinnedBuffer = Buffer<true>;
 
-// One helper thread per split scene: runs the second pipeline's host side (enqueue, stream synchronise, retry loop)
-// next to the caller's thread.  Kept alive between frames: waking it costs microseconds, creating it tens.
+// One helper thread per further pipeline of a split frame: runs that pipeline's host side (enqueue, stream synchronise,
+// retry loop) next to the caller's thread.  Kept alive between frames: waking it costs microseconds, creating it tens.
 struct Worker {
     std::thread th;
     std::mutex m;
@@ -100,7 +110,7 @@ struct Worker {
         std::unique_lock<std::mutex> lk(m);
         cv.wait(lk, [this] { return done; });
     }
-    void stop() {
+    ~Worker() {
         if (!th.joinable()) return;
         {
             std::lock_guard<std::mutex> lk(m);
@@ -111,43 +121,63 @@ struct Worker {
     }
 };
 
+// One pipeline of a frame: the streams a launch sequence runs on, its workspace and its CUDA graph.  Pipeline 0 renders
+// every call; a split frame (render_split) adds more, each rendering every k-th band next to it over the scene's blob.
+struct Pipeline {
+    cudaStream_t stream = nullptr;      // the stream kernels run on (own_stream unless the caller set one for pipeline 0)
+    cudaStream_t own_stream = nullptr;
+    cudaStream_t side_stream = nullptr; // light builds of a level's kernels run here, next to the heavy ones
+    cudaEvent_t ev[2] = {nullptr, nullptr}; // start and end of this pipeline's part of a call (timed)
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    std::vector<cudaEvent_t> prof_events;   // per-launch events, profile mode only
+    // workspace (grow-only)
+    DeviceBuffer nodes;        // the node arena
+    DeviceBuffer small;        // counters
+    DeviceBuffer order;        // per-bin node lists of the level being shaded
+    DeviceBuffer rorder;       // per-reach-key node lists of the next level
+    DeviceBuffer frame_entity; // a batch of frames: the frames' camera entities ...
+    DeviceBuffer node_frame;   // ... and the frame tag of every node
+    DeviceBuffer node_cost;    // (segments, levels) per node of the arena: AOV renders that want either plane
+    PinnedBuffer h_small;      // pinned mirror of the counters
+    int arena_capacity = 0;
+    double arena_factor = 0.0; // nodes per pixel the arena is sized for (learned from earlier frames)
+    int list_capacity = 0;     // entries per index list (bins, reach keys): the largest LEVEL a chunk may have
+    double list_factor = 1.0;  // ... in nodes per pixel (level 0 has exactly one; deeper levels are smaller in every shipped scene)
+    cudaGraphExec_t graph_exec = nullptr; // the last repeated chunk as a CUDA graph (render_impl)
+    uint64_t graph_key = 0, seen_key = 0; // parameter hash of graph_exec / of the previous direct launch sequence
+    uint32_t graph_launches = 0;
+
+    ~Pipeline() {
+        if (graph_exec) cudaGraphExecDestroy(graph_exec);
+        for (cudaEvent_t e : {ev[0], ev[1], ev_fork, ev_join})
+            if (e) cudaEventDestroy(e);
+        for (cudaEvent_t e : prof_events) cudaEventDestroy(e);
+        if (side_stream) cudaStreamDestroy(side_stream);
+        if (own_stream) cudaStreamDestroy(own_stream);
+    }
+};
+
 } // namespace
 
 struct EuclScene {
     int device = 0;
     int dim = 3;
     int sm_count = 148;
-    int blob_bytes = 0;
     size_t smem_bytes = 0;  // staged scene + plane_chain scratch
     size_t smem_scene = 0;  // staged scene only
     unsigned long long shade_light_mask = 1ull, shade_heavy_mask = 0ull;
-    uint8_t* d_blob = nullptr;
+    DeviceBuffer blob;
     std::vector<cudaArray_t> arrays;
     std::vector<cudaTextureObject_t> tex_objects;
-    cudaStream_t stream = nullptr;     // the stream kernels run on (own_stream unless the caller set one)
-    cudaStream_t own_stream = nullptr;
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    cudaStream_t side_stream = nullptr;                  // light builds of a level's kernels run here, next to the heavy ones
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    std::vector<cudaEvent_t> prof_events; // per-launch events, profile mode only
-    // workspace (grow-only)
-    DeviceBuffer nodes;    // the node arena
-    DeviceBuffer small;    // counters
-    DeviceBuffer frame;    // device frame buffer for eucl_render (host output)
-    DeviceBuffer hit_ids;  // device hit-id map for eucl_render
-    DeviceBuffer order;    // per-bin node lists of the level being shaded
-    DeviceBuffer path_io;  // eucl_trace_path staging
-    DeviceBuffer rorder;   // per-reach-key node lists of the next level
-    // a batch of frames (eucl_render_frames*): the per-frame constants (leader only; its twins read them), their pinned
-    // host staging, and per pipeline the frames' camera entities and the frame tag of every node
-    DeviceBuffer frame_table;
-    FrameParams* h_frame_table = nullptr;
-    uint32_t h_frame_table_cap = 0;
-    DeviceBuffer frame_entity;
-    DeviceBuffer node_frame;
-    DeviceBuffer node_cost; // (segments, levels) per node of this pipeline's arena: AOV renders that want either plane
+    // host-output staging (grow-only)
+    DeviceBuffer frame;     // device frame buffer for eucl_render (host output)
+    DeviceBuffer hit_ids;   // device hit-id map for eucl_render
     DeviceBuffer aov_stage; // device copies of the AOV planes for eucl_render_aovs (host output)
     DeviceBuffer ray_stage; // device copy of the rays of eucl_trace_rays (host input), refilled by every call
+    DeviceBuffer path_io;   // eucl_trace_path staging
+    // a batch of frames (eucl_render_frames*): the per-frame constants, read by every pipeline, and their pinned host staging
+    DeviceBuffer frame_table;
+    PinnedBuffer h_frame_table;
     int n_cull = 0;
     int light_capable = 0;
     // Grouping rays by reach key pays on scenes whose deep levels bounce around a few bounded objects
@@ -162,21 +192,17 @@ struct EuclScene {
     int warm_frames = 0;         // frames rendered so far
     int n_entities = 0;
     int real_bytes = 8;        // 8: f64 kernels (the reference's default `type F = f64`); 4: f32 kernels (`low_precision`)
-    int arena_capacity = 0;
-    double arena_factor = 0.0; // nodes per pixel the arena is sized for (learned from earlier frames)
-    cudaGraphExec_t graph_exec = nullptr; // the last repeated chunk as a CUDA graph (render_impl)
-    uint64_t graph_key = 0, seen_key = 0; // parameter hash of graph_exec / of the previous direct launch sequence
-    uint32_t graph_launches = 0;
-    int list_capacity = 0;     // entries per index list (bins, reach keys): the largest LEVEL a chunk may have
-    double list_factor = 1.0;  // ... in nodes per pixel (level 0 has exactly one; deeper levels are smaller in every shipped scene)
-    int32_t* h_small = nullptr; // pinned mirror of the counters
-    // Further pipelines of a split frame (render_split): scenes of their own -- streams, arena, counters, graph --
-    // over the same uploaded blob and textures, each rendering every k-th band next to this one.
-    std::vector<EuclScene*> twins;
-    std::vector<Worker*> workers; // one host thread per twin
-    bool is_twin = false;
-    cudaEvent_t ev_split[3] = {nullptr, nullptr, nullptr}; // start (timed), fork, end (timed)
-    cudaEvent_t ev_done = nullptr;                         // twin: its part of the frame is on its stream
+    std::vector<std::unique_ptr<Pipeline>> pipes; // [0] always exists; render_split adds the others
+    std::vector<std::unique_ptr<Worker>> workers; // one host thread per pipeline after the first
+    cudaEvent_t ev_split[3] = {nullptr, nullptr, nullptr}; // a split frame: start (timed), fork, end (timed)
+
+    cudaStream_t stream() const { return pipes[0]->stream; } // where calls stage their inputs and read back their outputs
+    ~EuclScene() {
+        for (cudaEvent_t e : ev_split)
+            if (e) cudaEventDestroy(e);
+        for (auto t : tex_objects) cudaDestroyTextureObject(t);
+        for (auto a : arrays) cudaFreeArray(a);
+    }
 };
 
 namespace {
@@ -641,6 +667,21 @@ struct BlobWriter {
     }
 };
 
+// One more pipeline: its streams, events and pinned counters; its workspace grows with the frames it renders.
+int add_pipeline(EuclScene* s) {
+    auto p = std::make_unique<Pipeline>();
+    EUCL_CUDA(cudaStreamCreateWithFlags(&p->own_stream, cudaStreamNonBlocking));
+    p->stream = p->own_stream;
+    EUCL_CUDA(cudaEventCreate(&p->ev[0]));
+    EUCL_CUDA(cudaEventCreate(&p->ev[1]));
+    EUCL_CUDA(cudaStreamCreateWithFlags(&p->side_stream, cudaStreamNonBlocking));
+    EUCL_CUDA(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
+    EUCL_CUDA(cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming));
+    EUCL_CUDA(p->h_small.ensure(sizeof(int32_t) * kSmallInts));
+    s->pipes.push_back(std::move(p));
+    return EUCL_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -657,41 +698,8 @@ int eucl_device_count(void) {
 void eucl_scene_destroy(EuclScene* s) {
     if (!s) return;
     cudaSetDevice(s->device);
-    for (Worker* w : s->workers) {
-        w->stop();
-        delete w;
-    }
-    for (EuclScene* t : s->twins) eucl_scene_destroy(t);
-    if (s->ev_done) cudaEventDestroy(s->ev_done);
-    if (s->stream) cudaStreamSynchronize(s->stream);
-    for (auto& e : s->ev_split)
-        if (e) cudaEventDestroy(e);
-    for (auto t : s->tex_objects) cudaDestroyTextureObject(t);
-    for (auto a : s->arrays) cudaFreeArray(a);
-    if (s->d_blob && !s->is_twin) cudaFree(s->d_blob);
-    s->nodes.release();
-    s->small.release();
-    s->frame.release();
-    s->hit_ids.release();
-    s->order.release();
-    s->path_io.release();
-    s->rorder.release();
-    s->frame_table.release();
-    s->frame_entity.release();
-    s->node_frame.release();
-    s->node_cost.release();
-    s->aov_stage.release();
-    s->ray_stage.release();
-    if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
-    if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
-    if (s->h_small) cudaFreeHost(s->h_small);
-    for (auto& e : s->ev)
-        if (e) cudaEventDestroy(e);
-    for (auto& e : s->prof_events) cudaEventDestroy(e);
-    if (s->ev_fork) cudaEventDestroy(s->ev_fork);
-    if (s->ev_join) cudaEventDestroy(s->ev_join);
-    if (s->side_stream) cudaStreamDestroy(s->side_stream);
-    if (s->own_stream) cudaStreamDestroy(s->own_stream);
+    s->workers.clear();
+    for (const auto& p : s->pipes) cudaStreamSynchronize(p->stream);
     delete s;
 }
 
@@ -717,40 +725,25 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     if (device < 0 || device >= n_dev) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_scene_create: device index out of range");
 
     EUCL_CUDA(cudaSetDevice(device));
-    EuclScene* s = new EuclScene();
+    auto s = std::make_unique<EuclScene>(); // freed with everything it holds on any early return
     s->device = device;
     s->real_bytes = precision == EUCL_PRECISION_F32 ? 4 : 8;
     s->dim = flat->dim;
     s->n_entities = flat->n_entities;
     cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device);
-    auto bail = [&](int st, const std::string& msg) {
-        eucl_scene_destroy(s);
-        return fail(st, msg);
-    };
-#define EUCL_CUDA_S(expr)                                                                                   \
-    do {                                                                                                    \
-        cudaError_t _e = (expr);                                                                            \
-        if (_e != cudaSuccess)                                                                              \
-            return bail(_e == cudaErrorMemoryAllocation ? EUCL_ERR_OUT_OF_MEMORY : EUCL_ERR_CUDA,           \
-                        std::string(#expr) + ": " + cudaGetErrorString(_e));                                \
-    } while (0)
-
-    EUCL_CUDA_S(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
-    s->stream = s->own_stream;
-    EUCL_CUDA_S(cudaEventCreate(&s->ev[0]));
-    EUCL_CUDA_S(cudaEventCreate(&s->ev[1]));
-    EUCL_CUDA_S(cudaStreamCreateWithFlags(&s->side_stream, cudaStreamNonBlocking));
-    EUCL_CUDA_S(cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming));
-    EUCL_CUDA_S(cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming));
+    status = add_pipeline(s.get());
+    if (status != EUCL_OK) return status;
+    for (int k = 0; k < 3; ++k)
+        EUCL_CUDA(cudaEventCreateWithFlags(&s->ev_split[k], k == 1 ? cudaEventDisableTiming : cudaEventDefault));
 
     // textures -> CUDA arrays + point-sampled texture objects
     for (int t = 0; t < flat->n_textures; ++t) {
         const EuclTexture& tx = flat->textures[t];
         cudaChannelFormatDesc desc = cudaCreateChannelDesc<uchar4>();
         cudaArray_t arr = nullptr;
-        EUCL_CUDA_S(cudaMallocArray(&arr, &desc, tx.width, tx.height));
+        EUCL_CUDA(cudaMallocArray(&arr, &desc, tx.width, tx.height));
         s->arrays.push_back(arr);
-        EUCL_CUDA_S(cudaMemcpy2DToArray(arr, 0, 0, flat->texels + tx.texel_offset, (size_t)tx.width * 4,
+        EUCL_CUDA(cudaMemcpy2DToArray(arr, 0, 0, flat->texels + tx.texel_offset, (size_t)tx.width * 4,
                                         (size_t)tx.width * 4, tx.height, cudaMemcpyHostToDevice));
         cudaResourceDesc rd{};
         rd.resType = cudaResourceTypeArray;
@@ -761,7 +754,7 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
         td.readMode = cudaReadModeElementType;
         td.normalizedCoords = 0;
         cudaTextureObject_t obj = 0;
-        EUCL_CUDA_S(cudaCreateTextureObject(&obj, &rd, &td, nullptr));
+        EUCL_CUDA(cudaCreateTextureObject(&obj, &rd, &td, nullptr));
         s->tex_objects.push_back(obj);
     }
 
@@ -832,7 +825,7 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
         de.node_root = (int)mb.out.size() - 1;
         int peak = 0, depth = 0;
         if (!mb.fits(de.node_first, de.node_root, &peak, &depth))
-            return bail(EUCL_ERR_SCENE_LIMIT, "entity " + std::to_string(e) + ": CSG program too large for the device evaluator (" +
+            return fail(EUCL_ERR_SCENE_LIMIT, "entity " + std::to_string(e) + ": CSG program too large for the device evaluator (" +
                                                   std::to_string(peak) + " arena slots of " + std::to_string(CSG_ARENA) + ", nesting " +
                                                   std::to_string(depth) + ")");
         dev_entities[(size_t)e] = de;
@@ -897,7 +890,6 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     h.max_entity_nodes = max_nodes;
     h.blob_bytes = (int)w.bytes.size();
     std::memcpy(w.bytes.data(), &h, sizeof h);
-    s->blob_bytes = h.blob_bytes;
     // staged scene + the per-thread plane_chain scratch columns (kernels.cu: plane_scratch)
     s->smem_scene = scene_smem_bytes(h.blob_bytes);
     s->smem_bytes = s->smem_scene + sizeof(double) * kPlaneChainMax * kBlock;
@@ -920,14 +912,12 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     int smem_optin = 0;
     cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
     if (s->smem_bytes > (size_t)smem_optin)
-        return bail(EUCL_ERR_SCENE_LIMIT, "scene tables (" + std::to_string(s->smem_bytes) +
+        return fail(EUCL_ERR_SCENE_LIMIT, "scene tables (" + std::to_string(s->smem_bytes) +
                                               " B) exceed the shared memory of one CTA (" + std::to_string(smem_optin) + " B)");
-    EUCL_CUDA_S(cudaMalloc((void**)&s->d_blob, w.bytes.size()));
-    EUCL_CUDA_S(cudaMemcpy(s->d_blob, w.bytes.data(), w.bytes.size(), cudaMemcpyHostToDevice));
-    EUCL_CUDA_S(EUCL_PREC(configure_kernels)(s->smem_bytes, s->smem_scene));
-    EUCL_CUDA_S(cudaMallocHost((void**)&s->h_small, sizeof(int32_t) * kSmallInts));
-#undef EUCL_CUDA_S
-    *out = s;
+    EUCL_CUDA(s->blob.ensure(w.bytes.size()));
+    EUCL_CUDA(cudaMemcpy(s->blob.ptr, w.bytes.data(), w.bytes.size(), cudaMemcpyHostToDevice));
+    EUCL_CUDA(EUCL_PREC(configure_kernels)(s->smem_bytes, s->smem_scene));
+    *out = s.release();
     return EUCL_OK;
 }
 
@@ -939,10 +929,11 @@ namespace {
 // T = the scalar the camera arithmetic runs in: double, or float for the reference's `low_precision` feature (the
 // results are stored as doubles either way; the f32 kernels narrow them back without loss)
 template <typename T>
-void frame_params_t(const EuclCamera& cam, const EuclRenderOpts& o, FrameParams* fp) {
+void frame_params_t(const EuclFrame& f, uint32_t width, uint32_t height, FrameParams* fp) {
+    const EuclCamera& cam = f.camera;
     const int D = cam.dim;
     std::memset(fp, 0, sizeof *fp);
-    const T w = (T)o.width, h = (T)o.height;
+    const T w = (T)width, h = (T)height;
     const T pi = (T)3.14159265358979323846264338327950288;
     const T fov_rad = pi * (T)cam.fov_deg / (T)180.0;
     volatile T diag = std::sqrt(w * w + h * h);
@@ -975,14 +966,14 @@ void frame_params_t(const EuclCamera& cam, const EuclRenderOpts& o, FrameParams*
         fp->right[k] = right[k];
     }
     // Duration * 1000 -> whole seconds -> / 1000 (d3/entity/surface.rs:32); `as F` narrows the f64 quotient
-    fp->time_millis = (T)(std::floor(o.time_seconds * 1000.0) / 1000.0);
-    fp->width = (int)o.width;
-    fp->height = (int)o.height;
+    fp->time_millis = (T)(std::floor(f.time_seconds * 1000.0) / 1000.0);
+    fp->width = (int)width;
+    fp->height = (int)height;
     fp->max_depth = (int)cam.max_depth;
 }
-void frame_params(const EuclCamera& cam, const EuclRenderOpts& o, int real_bytes, FrameParams* fp) {
-    if (real_bytes == 4) frame_params_t<float>(cam, o, fp);
-    else frame_params_t<double>(cam, o, fp);
+void frame_params(const EuclFrame& f, uint32_t width, uint32_t height, int real_bytes, FrameParams* fp) {
+    if (real_bytes == 4) frame_params_t<float>(f, width, height, fp);
+    else frame_params_t<double>(f, width, height, fp);
 }
 
 size_t arena_bytes(int dim, int real_bytes, size_t cap) {
@@ -990,46 +981,129 @@ size_t arena_bytes(int dim, int real_bytes, size_t cap) {
     return per * cap + 16 * 16;
 }
 
-// The frames of one call.  A single frame (eucl_render*) is a batch of one and renders exactly as it always did;
-// K > 1 frames (eucl_render_frames*) are ONE virtual frame of K * rows rows -- chunks, bands and pipelines split it
-// like any other frame -- whose per-pixel constants the kernels look up in a device table by virtual row.
+// FNV-1a over `bytes` bytes, continuing from `h`
+uint64_t fnv1a(const void* data, size_t bytes, uint64_t h = 1469598103934665603ull) {
+    const unsigned char* b = (const unsigned char*)data;
+    for (size_t k = 0; k < bytes; ++k) h = (h ^ b[k]) * 1099511628211ull;
+    return h;
+}
+
+// What one call renders.  Camera frames: K frames (eucl_render*: K = 1) are ONE virtual frame of K * rows rows -- chunks,
+// bands and pipelines split it like any other frame -- whose per-pixel constants the kernels look up in a device table by
+// virtual row; a single frame has no table and renders exactly as it always did.  Rays (eucl_trace_rays*): the rays on
+// the device in place of a camera, as a virtual frame of n / width rows of width.
 struct FrameBatch {
-    const EuclFrame* frames;
-    uint32_t n;                      // K
-    uint32_t rows;                   // rows per frame
-    const FrameParams* d_table;      // K > 1: [K] frame constants on the device, uploaded before the first launch
-    uint64_t table_key;              // K > 1: hash of the table contents, part of the graph key
-    // eucl_trace_rays*: the rays on the device ([n][dim] each) in place of a camera (K = 1; frames[0] carries only
-    // max_depth and the time), null for camera frames.  The virtual frame has n / width rows of width rays.
-    const double* ray_origins = nullptr;
-    const double* ray_directions = nullptr;
+    uint32_t n;                    // K (rays: 1)
+    uint32_t rows;                 // rows per frame
+    uint32_t max_depth;            // (every frame of a batch has this one)
+    FrameParams fp;                // frame 0's constants; rays: only the grid, the depth and the time
+    const FrameParams* d_table;    // K > 1: [K] frame constants on the device, uploaded before the first launch
+    uint64_t table_key;            // K > 1: hash of the table contents, part of the graph key
+    const double* ray_origins;     // rays: [n][dim] each; null for camera frames
+    const double* ray_directions;
 };
 
-Workspace carve(EuclScene* s, int dim, int cap, int list_cap, const FrameBatch& fb) {
+// The batch of `n` camera frames (arguments checked) and `virt`, the virtual frame they form.  K > 1: the frame constants
+// are computed on the host like a single frame's and uploaded on pipeline 0's stream, before the first launch and outside
+// any graph capture.
+int camera_batch(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, FrameBatch* fb, EuclRenderOpts* virt) {
+    *fb = FrameBatch{};
+    fb->n = n;
+    fb->rows = o->height;
+    fb->max_depth = frames[0].camera.max_depth;
+    frame_params(frames[0], o->width, o->height, s->real_bytes, &fb->fp);
+    *virt = *o;
+    virt->height = n * o->height;
+    if (n == 1) return EUCL_OK;
+    const size_t bytes = sizeof(FrameParams) * n;
+    EUCL_CUDA(s->h_frame_table.ensure(bytes));
+    FrameParams* table = (FrameParams*)s->h_frame_table.ptr;
+    for (uint32_t k = 0; k < n; ++k) frame_params(frames[k], o->width, o->height, s->real_bytes, &table[k]);
+    EUCL_CUDA(s->frame_table.ensure(bytes));
+    EUCL_CUDA(cudaMemcpyAsync(s->frame_table.ptr, table, bytes, cudaMemcpyHostToDevice, s->stream()));
+    fb->d_table = (const FrameParams*)s->frame_table.ptr;
+    fb->table_key = fnv1a(table, bytes);
+    return EUCL_OK;
+}
+
+// The batch of a ray call (arguments checked, rays on the device) and `o`, its virtual frame.  There is no camera: `fp`
+// carries the grid, the depth and the time (truncated as for a frame, then `as F`).
+FrameBatch ray_batch(const EuclScene* s, const EuclRays* r, const double* d_origins, const double* d_directions, bool want_hit,
+                     EuclRenderOpts* o) {
+    *o = EuclRenderOpts{};
+    o->width = r->width > 1 ? r->width : 1;
+    o->height = r->n / o->width;
+    o->time_seconds = r->time_seconds;
+    o->pipeline = r->pipeline;
+    o->want_hit_ids = want_hit ? 1 : 0;
+    o->profile = r->profile;
+    FrameBatch fb{};
+    fb.n = 1;
+    fb.rows = o->height;
+    fb.max_depth = r->max_depth;
+    const double millis = std::floor(r->time_seconds * 1000.0) / 1000.0;
+    fb.fp.time_millis = s->real_bytes == 4 ? (double)(float)millis : millis;
+    fb.fp.width = (int)o->width;
+    fb.fp.height = (int)o->height;
+    fb.fp.max_depth = (int)r->max_depth;
+    fb.ray_origins = d_origins;
+    fb.ray_directions = d_directions;
+    return fb;
+}
+
+// The launch configuration of `pipe`.  Queue kernels run as ONE wave of resident CTAs (512 threads per SM at 128
+// registers) walking their level with a grid stride: measured faster than 2-8 waves on glass scenes (3d_room 20.7 ->
+// 20.0 ms), equal elsewhere.
+Launch make_launch(const EuclScene* s, const Pipeline& pipe, const EuclRenderOpts& o) {
+    const int sms = s->sm_count;
+    Launch l{};
+    l.stream = pipe.stream;
+    l.blob = (const uint8_t*)s->blob.ptr;
+    l.smem_bytes = s->smem_bytes;
+    l.smem_scene = s->smem_scene;
+    l.grid_max = sms * std::max(1, env_int("EUCL_BLOCKS_PER_SM", kResidentThreads / kBlock));
+    l.grid_light = sms * std::max(1, env_int("EUCL_LIGHT_BLOCKS_PER_SM", kLightResidentBlocks));
+    l.grid_shade = sms * std::max(1, env_int("EUCL_SHADE_BLOCKS_PER_SM", kShadeResidentBlocks));
+    l.grid_mem = sms * std::max(1, env_int("EUCL_MEM_BLOCKS_PER_SM", 8));
+    l.shade_light_mask = s->shade_light_mask;
+    l.shade_heavy_mask = s->shade_heavy_mask;
+    l.grid_light_k2 = sms * std::max(1, env_int("EUCL_LIGHT_K2_BLOCKS_PER_SM", kLightK2ResidentBlocks));
+    l.light_capable = s->light_capable;
+    l.n_cull = s->n_cull;
+    // per-launch profiling and the debugging modes keep everything on one stream
+    l.side = (o.profile || env_int("EUCL_DEBUG_SYNC", 0) || !env_int("EUCL_CONCURRENT", 1)) ? nullptr : pipe.side_stream;
+    l.ev_fork = pipe.ev_fork;
+    l.ev_join = pipe.ev_join;
+    l.grid_background = sms * std::max(1, env_int("EUCL_BACKGROUND_BLOCKS_PER_SM", EUCL_BACKGROUND_MIN_BLOCKS));
+    return l;
+}
+
+Workspace carve(const EuclScene* s, const Pipeline& pipe, const FrameBatch& fb) {
+    const int cap = pipe.arena_capacity;
     Workspace ws{};
     ws.capacity = cap;
-    ws.list_cap = list_cap;
+    ws.list_cap = pipe.list_capacity;
     ws.n_frames = (int32_t)fb.n;
     ws.frame_rows = (int32_t)fb.rows;
     if (fb.n > 1) {
         ws.frames = fb.d_table;
-        ws.frame_entity = (int32_t*)s->frame_entity.ptr;
-        ws.node_frame = (int32_t*)s->node_frame.ptr;
+        ws.frame_entity = (int32_t*)pipe.frame_entity.ptr;
+        ws.node_frame = (int32_t*)pipe.node_frame.ptr;
     }
-    if (fb.n > 1 || fb.ray_origins) ws.untraced = (int32_t*)s->small.ptr + SmallLayout::untraced;
-    uint8_t* p = (uint8_t*)s->nodes.ptr;
+    if (fb.n > 1 || fb.ray_origins) ws.untraced = (int32_t*)pipe.small.ptr + SmallLayout::untraced;
+    uint8_t* p = (uint8_t*)pipe.nodes.ptr;
     auto take = [&](size_t bytes) {
         uint8_t* r = p;
         p += align16(bytes);
         return r;
     };
     const size_t rb = (size_t)s->real_bytes;
-    ws.ray = take((size_t)ray_reals(dim, s->real_bytes) * rb * cap);
+    ws.ray = take((size_t)ray_reals(s->dim, s->real_bytes) * rb * cap);
     ws.hit = take((size_t)kHitReals * rb * cap);
     ws.res = take((size_t)4 * rb * cap);
     ws.meta = (NodeMeta*)take(sizeof(NodeMeta) * (size_t)cap);
     ws.ray_cur = (int32_t*)take((size_t)4 * cap);
-    int32_t* small = (int32_t*)s->small.ptr;
+    int32_t* small = (int32_t*)pipe.small.ptr;
     ws.count = small + SmallLayout::count;
     ws.level_off = small + SmallLayout::level_off;
     ws.overflow = small + SmallLayout::overflow;
@@ -1037,12 +1111,12 @@ Workspace carve(EuclScene* s, int dim, int cap, int list_cap, const FrameBatch& 
     ws.undefined_count = (unsigned long long*)(small + SmallLayout::undefined64);
     ws.mega_level_counts = (unsigned long long*)(small + SmallLayout::mega64);
     ws.bin_count = small + SmallLayout::bins;
-    ws.order = (int32_t*)s->order.ptr;
-    const bool bin = s->order.ptr != nullptr;
+    ws.order = (int32_t*)pipe.order.ptr;
+    const bool bin = pipe.order.ptr != nullptr;
     ws.n_bins = bin ? kBinsPerEntity * s->n_entities + 1 : 1;
     ws.rbin_count = small + SmallLayout::rbins;
-    ws.rorder = (int32_t*)s->rorder.ptr;
-    ws.ray_bins = s->rorder.ptr != nullptr && s->ray_bins_now ? 1 : 0;
+    ws.rorder = (int32_t*)pipe.rorder.ptr;
+    ws.ray_bins = pipe.rorder.ptr != nullptr && s->ray_bins_now ? 1 : 0;
     return ws;
 }
 
@@ -1074,413 +1148,408 @@ void tune_grouping(EuclScene* s, const EuclStats& st, int pipeline) {
     }
 }
 
-// Renders this rank's rows of `o` (all of them, or -- sub_stride > 1 -- the bands that `o` names, which are every
-// sub_stride-th band of the caller's rank starting at sub_offset: render_split).
-// `o` describes the (virtual) frame: o->height = fb.n * fb.rows.
-int render_impl(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
-                const AovPlanes& aov_out, EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
-    const int dim = s->dim;
-    const EuclCamera* cam = &fb.frames[0].camera; // (every frame of a batch has this max_depth)
-    const bool rays = fb.ray_origins != nullptr;
-    FrameParams fp;
-    if (rays) { // no camera: the grid, the depth and the time (truncated as for a frame, then `as F`)
-        std::memset(&fp, 0, sizeof fp);
-        const double millis = std::floor(fb.frames[0].time_seconds * 1000.0) / 1000.0;
-        fp.time_millis = s->real_bytes == 4 ? (double)(float)millis : millis;
-        fp.width = (int)o->width;
-        fp.height = (int)o->height;
-        fp.max_depth = (int)cam->max_depth;
-    } else {
-        EuclRenderOpts first = *o;
-        first.height = fb.rows;
-        first.time_seconds = fb.frames[0].time_seconds;
-        frame_params(*cam, first, s->real_bytes, &fp);
+// The index lists and per-node buffers a call's workspace holds next to the node arena.
+struct WorkspaceNeeds {
+    bool rorder; // reach-key lists of the next level
+    bool order;  // shade-coherence bins: one node list per hit entity (+ miss), each able to hold a whole level
+    bool cost;   // the COST builds' (segments, levels) pair per node
+    bool frames; // a batch: the frame tag of every node
+};
+
+// Leaves a consistent, empty workspace: the next chunk allocates it again.
+void release_workspace(Pipeline& pipe) {
+    pipe.nodes.release();
+    pipe.order.release();
+    pipe.rorder.release();
+    pipe.node_cost.release();
+    pipe.arena_capacity = 0;
+    pipe.list_capacity = 0;
+}
+
+// Grows `pipe`'s workspace for chunks of *rows rows of `width` pixels at its learned factors.  The chunk shrinks by half
+// while its workspace does not fit: more than 2^31 nodes, over the memory budget, or an allocation failure.
+int reserve_workspace(const EuclScene* s, Pipeline& pipe, const WorkspaceNeeds& need, int pipeline, int width, int* rows) {
+    const size_t n_bins = (size_t)(kBinsPerEntity * s->n_entities + 1);
+    const size_t n_lists = (need.rorder ? (size_t)kRayBins : 0) + (need.order ? n_bins : 0);
+    for (;;) {
+        long long want = (long long)std::ceil((double)*rows * (double)width * pipe.arena_factor) + 1024;
+        long long want_list = (long long)std::ceil((double)*rows * (double)width * pipe.list_factor) + 1024;
+        if (pipeline == EUCL_PIPELINE_MEGAKERNEL) want = want_list = 16;
+        bool too_big = want > 0x7fff0000ll || want_list > 0x7fff0000ll;
+        if (!too_big && ((int)want > pipe.arena_capacity || (int)want_list > pipe.list_capacity)) {
+            EUCL_CUDA(cudaStreamSynchronize(pipe.stream));
+            want = std::max<long long>(want, pipe.arena_capacity);
+            want_list = std::max<long long>(want_list, pipe.list_capacity);
+            size_t free_b = 0, total_b = 0;
+            EUCL_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            const size_t held = pipe.nodes.bytes + pipe.order.bytes + pipe.rorder.bytes + pipe.node_cost.bytes;
+            size_t budget = (size_t)((double)(free_b + held) * 0.85);
+            const int cap_mb = env_int("EUCL_ARENA_MAX_MB", 0);
+            if (cap_mb > 0) budget = std::min(budget, (size_t)cap_mb << 20);
+            const size_t bytes = arena_bytes(s->dim, s->real_bytes, (size_t)want) + sizeof(int32_t) * n_lists * (size_t)want_list +
+                                 (need.cost ? sizeof(uint2) * (size_t)want : 0);
+            too_big = bytes > budget;
+            if (!too_big) {
+                cudaError_t e = pipe.nodes.ensure(arena_bytes(s->dim, s->real_bytes, (size_t)want));
+                if (e == cudaSuccess && need.rorder) e = pipe.rorder.ensure(sizeof(int32_t) * (size_t)kRayBins * (size_t)want_list);
+                if (e == cudaSuccess && need.order) e = pipe.order.ensure(sizeof(int32_t) * n_bins * (size_t)want_list);
+                if (e == cudaSuccess) {
+                    pipe.arena_capacity = (int)want;
+                    pipe.list_capacity = (int)want_list;
+                } else { // try a smaller chunk
+                    cudaGetLastError();
+                    release_workspace(pipe);
+                    if (e != cudaErrorMemoryAllocation) return fail(EUCL_ERR_CUDA, std::string("workspace allocation: ") + cudaGetErrorString(e));
+                    too_big = true;
+                }
+            }
+        }
+        if (!too_big) break;
+        if (*rows <= 1) return fail(EUCL_ERR_OUT_OF_MEMORY, "the node arena of a single row of pixels does not fit in device memory");
+        *rows = (*rows + 1) / 2;
     }
+    if (need.frames) EUCL_CUDA(pipe.node_frame.ensure(sizeof(int32_t) * (size_t)pipe.arena_capacity));
+    if (need.cost) EUCL_CUDA(pipe.node_cost.ensure(sizeof(uint2) * (size_t)pipe.arena_capacity));
+    return EUCL_OK;
+}
+
+// A frame that had to grow its arena over-shot (capacity grows by half each retry).  Now that the frame's real node count
+// is known, the pipeline keeps that plus a few per cent and gives the rest back, and with it the graph that points into
+// the old workspace: the next frame of this size allocates once more, exactly, and nothing afterwards.
+void trim_workspace(Pipeline& pipe, const EuclStats& st) {
+    if (st.retries == 0 || st.pixels == 0 || st.nodes == 0) return;
+    uint64_t max_level = 0;
+    for (uint32_t lv = 0; lv < st.levels; ++lv) max_level = std::max<uint64_t>(max_level, st.level_counts[lv]);
+    const double tight = (double)st.nodes / (double)st.pixels * 1.03 + 0.02;
+    const double tight_list = std::max(1.0, (double)max_level / (double)st.pixels * 1.03);
+    if ((double)pipe.arena_capacity > ((double)st.pixels * tight + 1024) * 1.08) {
+        pipe.arena_factor = tight;
+        pipe.list_factor = tight_list;
+        release_workspace(pipe);
+        if (pipe.graph_exec) cudaGraphExecDestroy(pipe.graph_exec);
+        pipe.graph_exec = nullptr;
+        pipe.graph_key = pipe.seen_key = 0;
+    }
+}
+
+// Everything the launch sequence of one chunk reads.
+struct ChunkLaunch {
+    const FrameBatch& fb;
+    int pipeline; // EuclPipeline
+    Launch l;
+    ChunkParams cp;
+    Workspace ws;
+    AovPlanes aov; // the planes a chunk writes (null = not wanted) and the cost buffer
+    uint8_t* d_rgb;
+    int32_t* d_hit;
+};
+
+// The diagnostic modes of one chunk.  Profile mode records an event after every launch (family -1 start, 0 raygen,
+// 1 intersect, 2 shade, 3 resolve).  EUCL_DEBUG_SYNC=1 synchronises after every launch and names the one that faulted.
+// EUCL_POISON=1 fills the work buffers with 0x7F bytes (huge positive indices) first, so that a read of anything this
+// frame did not write turns into a deterministic fault instead of depending on stale data.
+struct ChunkDebug {
+    bool profile, sync, poison;
+    std::vector<int> prof_family;
+    std::string fault;
+};
+
+// Everything one chunk puts on the stream: counters reset, kernels, counters back to the pinned mirror.  Returns the
+// number of kernels.
+uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c, ChunkDebug& dbg) {
+    const int dim = s->dim;
+    const FrameBatch& fb = c.fb;
+    const Launch& l = c.l;
+    auto mark = [&](int family) {
+        if (!dbg.profile) return;
+        if (pipe.prof_events.size() <= dbg.prof_family.size()) {
+            cudaEvent_t e = nullptr;
+            cudaEventCreate(&e);
+            pipe.prof_events.push_back(e);
+        }
+        cudaEventRecord(pipe.prof_events[dbg.prof_family.size()], pipe.stream);
+        dbg.prof_family.push_back(family);
+    };
+    auto check = [&](const char* what, int level) {
+        if (!dbg.sync || !dbg.fault.empty()) return;
+        cudaError_t e = cudaStreamSynchronize(pipe.stream);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) dbg.fault = std::string(what) + " level " + std::to_string(level) + ": " + cudaGetErrorString(e);
+    };
+    uint32_t launches = 0;
+    cudaMemsetAsync(pipe.small.ptr, 0, sizeof(int32_t) * kSmallInts, pipe.stream);
+    if (dbg.poison) {
+        cudaMemsetAsync(pipe.nodes.ptr, 0x7F, pipe.nodes.bytes, pipe.stream);
+        if (pipe.order.ptr) cudaMemsetAsync(pipe.order.ptr, 0x7F, pipe.order.bytes, pipe.stream);
+        if (pipe.rorder.ptr) cudaMemsetAsync(pipe.rorder.ptr, 0x7F, pipe.rorder.bytes, pipe.stream);
+    }
+    mark(-1);
+    if (c.pipeline == EUCL_PIPELINE_MEGAKERNEL) {
+        if (!fb.ray_origins) {
+            EUCL_PREC(launch_camera_entity)(dim, l, fb.fp, c.ws);
+            check("k_camera_entity", 0);
+            launches += 1;
+        }
+        EUCL_PREC(launch_megakernel)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.d_hit, c.aov, fb.ray_origins, fb.ray_directions);
+        mark(1);
+        launches += 1;
+    } else {
+        if (c.ws.frames) {
+            EUCL_PREC(launch_camera_entity)(dim, l, fb.fp, c.ws);
+            check("k_camera_entity", 0);
+            launches += 1;
+        }
+        if (fb.ray_origins) EUCL_PREC(launch_raygen_rays)(dim, l, fb.fp, c.cp, c.ws, c.d_hit, fb.ray_origins, fb.ray_directions);
+        else EUCL_PREC(launch_raygen)(dim, l, fb.fp, c.cp, c.ws, c.d_hit);
+        check("k_raygen", 0);
+        mark(0);
+        for (int level = 0; level < (int)fb.max_depth; ++level) {
+            launches += EUCL_PREC(launch_intersect)(dim, l, c.ws, level);
+            check("k_intersect", level);
+            mark(1);
+            launches += EUCL_PREC(launch_shade)(dim, l, fb.fp, c.cp, c.ws, level, c.d_hit);
+            check("k_shade", level);
+            mark(2);
+        }
+        // the nodes of the last level are background lookups (depth 0: mod.rs:157,183).  Measured and not kept:
+        // finishing them inside k_shade of the level above, from the child direction in registers (one launch
+        // and one ray record per node less, but the lookups then run at the heavy kernel's occupancy:
+        // 3d_room shade 7.14 + 0.47 -> 7.34 + 0.67 ms)
+        launches += EUCL_PREC(launch_shade)(dim, l, fb.fp, c.cp, c.ws, (int)fb.max_depth, c.d_hit);
+        check("k_shade", (int)fb.max_depth);
+        mark(2);
+        launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.aov);
+        check("k_resolve / k_final", 0);
+        mark(3);
+        launches += 1; // raygen
+    }
+    cudaMemcpyAsync(pipe.h_small.ptr, pipe.small.ptr, sizeof(int32_t) * kSmallInts, cudaMemcpyDeviceToHost, pipe.stream);
+    return launches;
+}
+
+// The CUDA-graph key of a chunk: a hash of everything its launches read
+uint64_t graph_key(const ChunkLaunch& c) {
+    const FrameBatch& fb = c.fb;
+    uint64_t key = fnv1a(&fb.fp, sizeof fb.fp);
+    auto mix = [&](const void* data, size_t bytes) { key = fnv1a(data, bytes, key); };
+    mix(&c.cp, sizeof c.cp);
+    mix(&c.ws, sizeof c.ws);
+    {   // the members of Launch one by one (the struct has padding bytes)
+        const Launch& l = c.l;
+        const void* ptrs[] = {l.stream, l.blob, l.side};
+        const unsigned long long nums[] = {l.smem_bytes, l.smem_scene, (unsigned long long)l.grid_max, (unsigned long long)l.grid_light,
+                                           (unsigned long long)l.grid_shade, (unsigned long long)l.grid_mem, l.shade_light_mask,
+                                           l.shade_heavy_mask, (unsigned long long)l.grid_light_k2,
+                                           (unsigned long long)l.light_capable, (unsigned long long)l.n_cull,
+                                           (unsigned long long)l.grid_background};
+        mix(ptrs, sizeof ptrs);
+        mix(nums, sizeof nums);
+    }
+    mix(&c.d_rgb, sizeof c.d_rgb);
+    mix(&c.d_hit, sizeof c.d_hit);
+    // the AOV planes and the cost buffer: a graph captured with or without them never stands in for the other
+    mix(&c.aov, sizeof c.aov);
+    mix(&c.pipeline, sizeof c.pipeline);
+    mix(&fb.max_depth, sizeof fb.max_depth);
+    // a batch: the graph reads the table the caller's poses were uploaded to, and it is keyed by its contents too, so
+    // that a changed pose or time is never taken for a repeated batch
+    if (fb.n > 1) mix(&fb.table_key, sizeof fb.table_key);
+    // a ray call: tagged, so that a ray call and a render whose other parameters coincide never stand in for each
+    // other, and keyed by the arrays it reads (their contents are read at replay time)
+    if (fb.ray_origins) {
+        const uint64_t ray_id[] = {0x52415953ull /* "RAYS" */, (uint64_t)(uintptr_t)fb.ray_origins, (uint64_t)(uintptr_t)fb.ray_directions,
+                                   (uint64_t)fb.fp.height * (uint64_t)fb.fp.width, (uint64_t)fb.fp.width};
+        mix(ray_id, sizeof ray_id);
+    }
+    return key;
+}
+
+// A chunk whose launch parameters repeat (a fixed pose rendered again: benchmarks, a paused camera, every rank of a
+// band-split frame) is replayed as ONE CUDA graph launch: the ~50 kernels of a frame then cost one driver call on the
+// host and run back to back on the device.  The first sighting of a parameter set launches directly, the second
+// captures, later ones replay.  Without `use_graph` every chunk launches directly.
+int launch_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c, ChunkDebug& dbg, bool use_graph, EuclStats* st) {
+    const uint64_t key = graph_key(c);
+    if (use_graph && pipe.graph_exec && pipe.graph_key == key) {
+        EUCL_CUDA(cudaGraphLaunch(pipe.graph_exec, pipe.stream));
+        st->launches += pipe.graph_launches;
+        st->graph_replays += 1;
+    } else if (use_graph && pipe.seen_key == key) {
+        if (pipe.graph_exec) cudaGraphExecDestroy(pipe.graph_exec);
+        pipe.graph_exec = nullptr;
+        cudaGraph_t graph = nullptr;
+        // one capture at a time in the process (the pipelines of a split frame capture in the same frame)
+        static std::mutex capture_mutex;
+        std::unique_lock<std::mutex> capture_lock(capture_mutex);
+        EUCL_CUDA(cudaStreamBeginCapture(pipe.stream, cudaStreamCaptureModeThreadLocal));
+        const uint32_t launches = enqueue_chunk(s, pipe, c, dbg);
+        cudaError_t ce = cudaStreamEndCapture(pipe.stream, &graph);
+        if (ce == cudaSuccess) ce = cudaGraphInstantiate(&pipe.graph_exec, graph, 0);
+        capture_lock.unlock();
+        if (graph) cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) { // not capturable here (e.g. a caller's stream in a state that forbids it): launch directly
+            cudaGetLastError();
+            pipe.graph_exec = nullptr;
+            pipe.seen_key = 0;
+            st->launches += enqueue_chunk(s, pipe, c, dbg);
+        } else {
+            pipe.graph_key = key;
+            pipe.graph_launches = launches;
+            EUCL_CUDA(cudaGraphLaunch(pipe.graph_exec, pipe.stream));
+            st->launches += launches;
+            st->graph_replays += 1;
+        }
+    } else {
+        pipe.seen_key = key;
+        st->launches += enqueue_chunk(s, pipe, c, dbg);
+    }
+    return EUCL_OK;
+}
+
+// Waits for a launched chunk and reads its counters back.  A level that overflowed the arena or the index lists grows
+// the learned factor and sets `*retry`; a chunk that fit adds its pixels and level counts to `st`.
+int read_back_chunk(Pipeline& pipe, const ChunkLaunch& c, const ChunkDebug& dbg, EuclStats* st, bool* retry) {
+    if (!dbg.fault.empty()) return fail(EUCL_ERR_CUDA, "EUCL_DEBUG_SYNC: " + dbg.fault);
+    EUCL_CUDA(cudaStreamSynchronize(pipe.stream));
+    EUCL_CUDA(cudaGetLastError());
+    const int32_t* h = (const int32_t*)pipe.h_small.ptr;
+    const uint32_t depth = c.fb.max_depth;
+    for (size_t k = 1; k < dbg.prof_family.size(); ++k) {
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, pipe.prof_events[k - 1], pipe.prof_events[k]);
+        float* slot = dbg.prof_family[k] == 0 ? &st->ms_raygen : dbg.prof_family[k] == 1 ? &st->ms_intersect
+                      : dbg.prof_family[k] == 2 ? &st->ms_shade : &st->ms_resolve;
+        *slot += ms;
+    }
+    if (env_int("EUCL_DUMP_LEVELS", 0) && !h[SmallLayout::overflow]) { // diagnostics: per-level counts, bins, launch times
+        for (uint32_t lv = 0; lv <= depth; ++lv) {
+            fprintf(stderr, "level %2u count %9d | bins", lv, h[SmallLayout::count + lv]);
+            for (int b = 0; b < c.ws.n_bins && c.ws.n_bins > 1; ++b) fprintf(stderr, " %d", h[SmallLayout::bins + lv * kMaxBins + b]);
+            fprintf(stderr, " | rbins");
+            for (int b = 0; b < kRayBins; ++b) fprintf(stderr, " %d", h[SmallLayout::rbins + lv * kRayBins + b]);
+            fprintf(stderr, "\n");
+        }
+        for (size_t k = 1; k < dbg.prof_family.size(); ++k) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, pipe.prof_events[k - 1], pipe.prof_events[k]);
+            fprintf(stderr, "launch %2zu family %d %.3f ms\n", k, dbg.prof_family[k], ms);
+        }
+    }
+    if (h[SmallLayout::overflow] == 2) return fail(EUCL_ERR_CUDA, "internal error: a queue index list and its level count disagree");
+    *retry = h[SmallLayout::overflow] != 0;
+    if (*retry) {
+        // levels after the overflowing one were skipped, so the counts are a lower bound only
+        long long need = 0;
+        for (uint32_t lv = 0; lv <= depth; ++lv) need += h[SmallLayout::count + lv];
+        if (h[SmallLayout::overflow] == 3) { // a level outgrew the index lists (they hold one level each)
+            pipe.list_factor = std::max(pipe.list_factor * 1.5, 1.0);
+        } else {
+            double factor = (double)need / (double)c.cp.n_pixels * 1.05 + 0.05;
+            pipe.arena_factor = std::max(pipe.arena_factor * 1.5, factor);
+        }
+        st->retries += 1;
+        if (st->retries > 32) return fail(EUCL_ERR_OUT_OF_MEMORY, "node arena keeps overflowing");
+        return EUCL_OK;
+    }
+    st->pixels += (uint64_t)c.cp.n_pixels;
+    // camera in no entity: checkerboard pixels, Universe::trace is never called (mod.rs:385-396).  In a batch with
+    // some frames traced, level 0 holds the checkerboard pixels of the others: they are not counted either.
+    const bool traced = h[SmallLayout::cam_entity] >= 0;
+    for (uint32_t lv = 0; traced && lv <= depth; ++lv) {
+        uint64_t n = c.pipeline == EUCL_PIPELINE_MEGAKERNEL ? ((const unsigned long long*)(h + SmallLayout::mega64))[lv]
+                                                            : (uint64_t)h[SmallLayout::count + lv];
+        if (lv == 0) n -= (uint64_t)h[SmallLayout::untraced];
+        st->level_counts[lv] += n;
+        st->nodes += n;
+        if (lv < depth) st->segments += n;
+    }
+    return EUCL_OK;
+}
+
+// Renders this rank's rows of `o` on `pipe`: all of them, or -- sub_stride > 1 -- the bands that `o` names, which are
+// every sub_stride-th band of the caller's rank starting at sub_offset (render_split).  `o` describes the (virtual)
+// frame: o->height = fb.n * fb.rows.
+int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
+                const AovPlanes& aov_out, EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
     const int width = (int)o->width;
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
+    const bool wavefront = o->pipeline == EUCL_PIPELINE_WAVEFRONT;
     EuclStats st{};
-    st.levels = cam->max_depth + 1;
-    if (!s->is_twin) choose_grouping(s); // a twin renders with its leader's setting
-    if (fb.n > 1) EUCL_CUDA(s->frame_entity.ensure(sizeof(int32_t) * fb.n));
-    EUCL_CUDA(cudaEventRecord(s->ev[0], s->stream));
+    st.levels = fb.max_depth + 1;
+    if (sub_stride <= 1) choose_grouping(s); // (render_split chooses for a split frame)
+    if (fb.n > 1) EUCL_CUDA(pipe.frame_entity.ensure(sizeof(int32_t) * fb.n));
+    EUCL_CUDA(cudaEventRecord(pipe.ev[0], pipe.stream));
     if (my_rows > 0) {
+        if ((long long)width > (1ll << 30)) return fail(EUCL_ERR_INVALID_ARGUMENT, "frame rows too wide");
+        if (!wavefront && fb.max_depth > 24) return fail(EUCL_ERR_SCENE_LIMIT, "megakernel pipeline supports max_depth <= 24");
+        EUCL_CUDA(pipe.small.ensure(sizeof(int32_t) * kSmallInts));
+        if (pipe.arena_factor <= 0.0) pipe.arena_factor = std::max(1.0, (double)env_int("EUCL_ARENA_FACTOR_X10", 45) / 10.0);
+        const WorkspaceNeeds need{wavefront && s->n_cull > 0 && env_int("EUCL_BIN_RAYS", 1),
+                                  wavefront && kBinsPerEntity * s->n_entities + 1 <= kMaxBins && env_int("EUCL_BIN_SHADE", 1),
+                                  wavefront && (aov_out.segments || aov_out.levels), fb.n > 1};
         // chunking: whole local rows, about EUCL_CHUNK_PIXELS primaries per chunk.  Large chunks are faster (longer
         // levels, fewer host round trips: 4d_room 7680x4320 renders 10 % faster as one chunk than as eight), so the
-        // default covers an 8K frame; the chunk shrinks by itself when its arena would not fit (2^31 nodes, the
-        // memory budget, or an allocation failure).
+        // default covers an 8K frame; the chunk shrinks by itself when its workspace does not fit (reserve_workspace).
         const long long chunk_pixels_target = std::max(1, env_int("EUCL_CHUNK_PIXELS", 1 << 25));
         int rows_per_chunk = (int)std::max<long long>(1, chunk_pixels_target / width);
         rows_per_chunk = std::min<int>(rows_per_chunk, (int)my_rows);
-        if ((long long)width > (1ll << 30)) return fail(EUCL_ERR_INVALID_ARGUMENT, "frame rows too wide");
-        EUCL_CUDA(s->small.ensure(sizeof(int32_t) * kSmallInts));
-        if (s->arena_factor <= 0.0) s->arena_factor = std::max(1.0, (double)env_int("EUCL_ARENA_FACTOR_X10", 45) / 10.0);
-        // queue kernels run as ONE wave of resident CTAs (512 threads per SM at 128 registers) walking their level with a grid
-        // stride: measured faster than 2-8 waves on glass scenes (3d_room 20.7 -> 20.0 ms), equal elsewhere
-        Launch l{s->stream, s->d_blob, s->smem_bytes, s->smem_scene,
-                 s->sm_count * std::max(1, env_int("EUCL_BLOCKS_PER_SM", kResidentThreads / kBlock)),
-                 s->sm_count * std::max(1, env_int("EUCL_LIGHT_BLOCKS_PER_SM", kLightResidentBlocks)),
-                 s->sm_count * std::max(1, env_int("EUCL_SHADE_BLOCKS_PER_SM", kShadeResidentBlocks)),
-                 s->sm_count * std::max(1, env_int("EUCL_MEM_BLOCKS_PER_SM", 8)),
-                 s->shade_light_mask, s->shade_heavy_mask,
-                 s->sm_count * std::max(1, env_int("EUCL_LIGHT_K2_BLOCKS_PER_SM", kLightK2ResidentBlocks)), s->light_capable, s->n_cull,
-                 // per-launch profiling and the debugging modes keep everything on one stream
-                 (o->profile || env_int("EUCL_DEBUG_SYNC", 0) || !env_int("EUCL_CONCURRENT", 1)) ? nullptr : s->side_stream, s->ev_fork,
-                 s->ev_join, s->sm_count * std::max(1, env_int("EUCL_BACKGROUND_BLOCKS_PER_SM", EUCL_BACKGROUND_MIN_BLOCKS))};
-        const bool want_rorder = o->pipeline == EUCL_PIPELINE_WAVEFRONT && s->n_cull > 0 && env_int("EUCL_BIN_RAYS", 1);
-        // shade-coherence bins: one node list per hit entity (+ miss), each able to hold a whole level
-        const bool want_order = o->pipeline == EUCL_PIPELINE_WAVEFRONT && kBinsPerEntity * s->n_entities + 1 <= kMaxBins && env_int("EUCL_BIN_SHADE", 1);
-        const size_t n_lists = (want_rorder ? (size_t)kRayBins : 0) + (want_order ? (size_t)(kBinsPerEntity * s->n_entities + 1) : 0);
-        // the COST builds keep a (segments, levels) pair per node next to the arena
-        const bool want_cost = o->pipeline == EUCL_PIPELINE_WAVEFRONT && (aov_out.segments || aov_out.levels);
-        auto workspace_bytes = [&](size_t cap, size_t list_cap) {
-            return arena_bytes(dim, s->real_bytes, cap) + sizeof(int32_t) * n_lists * list_cap + (want_cost ? sizeof(uint2) * cap : 0);
-        };
-
-        for (int row0 = 0; row0 < (int)my_rows;) {
-            ChunkParams cp{};
-            cp.local_row0 = row0;
-            cp.band_rows = o->band_rows ? (int)o->band_rows : (int)o->height;
-            cp.band_rank = (int)o->band_rank;
-            cp.band_world = o->band_world ? (int)o->band_world : 1;
-            cp.compact_rows = o->compact_rows;
-            cp.sub_stride = sub_stride;
-            cp.sub_offset = sub_offset;
-            for (;;) { // retry with a larger arena when a level overflowed, with a smaller chunk when the arena cannot grow
-                cp.n_rows = std::min<int>(rows_per_chunk, (int)my_rows - row0);
-                cp.n_pixels = cp.n_rows * width;
-                long long want = (long long)std::ceil((double)rows_per_chunk * (double)width * s->arena_factor) + 1024;
-                if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL) want = 16;
-                long long want_list = (long long)std::ceil((double)rows_per_chunk * (double)width * s->list_factor) + 1024;
-                if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL) want_list = 16;
-                bool too_big = want > 0x7fff0000ll || want_list > 0x7fff0000ll;
-                if (!too_big && ((int)want > s->arena_capacity || (int)want_list > s->list_capacity)) {
-                    EUCL_CUDA(cudaStreamSynchronize(s->stream));
-                    want = std::max<long long>(want, s->arena_capacity);
-                    want_list = std::max<long long>(want_list, s->list_capacity);
-                    size_t free_b = 0, total_b = 0;
-                    EUCL_CUDA(cudaMemGetInfo(&free_b, &total_b));
-                    const size_t held = s->nodes.bytes + s->order.bytes + s->rorder.bytes + s->node_cost.bytes;
-                    size_t budget = (size_t)((double)(free_b + held) * 0.85);
-                    const int cap_mb = env_int("EUCL_ARENA_MAX_MB", 0);
-                    if (cap_mb > 0) budget = std::min(budget, (size_t)cap_mb << 20);
-                    too_big = workspace_bytes((size_t)want, (size_t)want_list) > budget;
-                    if (!too_big) {
-                        cudaError_t e = s->nodes.ensure(arena_bytes(dim, s->real_bytes, (size_t)want));
-                        if (e == cudaSuccess && want_rorder) e = s->rorder.ensure(sizeof(int32_t) * (size_t)kRayBins * (size_t)want_list);
-                        if (e == cudaSuccess && want_order) e = s->order.ensure(sizeof(int32_t) * (size_t)(kBinsPerEntity * s->n_entities + 1) * (size_t)want_list);
-                        if (e == cudaSuccess) {
-                            s->arena_capacity = (int)want;
-                            s->list_capacity = (int)want_list;
-                        } else { // leave a consistent (empty) workspace behind and try a smaller chunk
-                            cudaGetLastError();
-                            s->nodes.release();
-                            s->rorder.release();
-                            s->order.release();
-                            s->node_cost.release();
-                            s->arena_capacity = 0;
-                            s->list_capacity = 0;
-                            if (e != cudaErrorMemoryAllocation) return fail(EUCL_ERR_CUDA, std::string("workspace allocation: ") + cudaGetErrorString(e));
-                            too_big = true;
-                        }
-                    }
-                }
-                if (too_big) {
-                    if (rows_per_chunk <= 1)
-                        return fail(EUCL_ERR_OUT_OF_MEMORY, "the node arena of a single row of pixels does not fit in device memory");
-                    rows_per_chunk = (rows_per_chunk + 1) / 2;
-                    continue;
-                }
-                if (fb.n > 1) EUCL_CUDA(s->node_frame.ensure(sizeof(int32_t) * (size_t)s->arena_capacity));
-                if (want_cost) EUCL_CUDA(s->node_cost.ensure(sizeof(uint2) * (size_t)s->arena_capacity));
-                Workspace ws = carve(s, dim, s->arena_capacity, s->list_capacity, fb);
-                AovPlanes aov = aov_out;
-                aov.cost = want_cost ? (uint2*)s->node_cost.ptr : nullptr;
-                // profile mode: one event after every launch; family = 0 raygen, 1 intersect, 2 shade, 3 resolve
-                std::vector<int> prof_family;
-                auto mark = [&](int family) {
-                    if (!o->profile) return;
-                    if (s->prof_events.size() <= prof_family.size()) {
-                        cudaEvent_t e = nullptr;
-                        cudaEventCreate(&e);
-                        s->prof_events.push_back(e);
-                    }
-                    cudaEventRecord(s->prof_events[prof_family.size()], s->stream);
-                    prof_family.push_back(family);
-                };
-                // EUCL_DEBUG_SYNC=1: synchronise after every launch and name the one that faulted;
-                // EUCL_POISON=1: fill the work buffers with 0x7F bytes (huge positive indices) first, so that a read of anything this
-                // frame did not write turns into a deterministic fault instead of depending on stale data
-                const bool debug_sync = env_int("EUCL_DEBUG_SYNC", 0) != 0;
-                const bool poison = env_int("EUCL_POISON", 0) != 0;
-                std::string fault;
-                auto dbg = [&](const char* what, int level) {
-                    if (!debug_sync || !fault.empty()) return;
-                    cudaError_t e = cudaStreamSynchronize(s->stream);
-                    if (e == cudaSuccess) e = cudaGetLastError();
-                    if (e != cudaSuccess) fault = std::string(what) + " level " + std::to_string(level) + ": " + cudaGetErrorString(e);
-                };
-                if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL && cam->max_depth > 24)
-                    return fail(EUCL_ERR_SCENE_LIMIT, "megakernel pipeline supports max_depth <= 24");
-                // everything one chunk puts on the stream: counters reset, kernels, counters back to the pinned mirror
-                auto enqueue = [&]() -> uint32_t {
-                    uint32_t launches = 0;
-                    cudaMemsetAsync(s->small.ptr, 0, sizeof(int32_t) * kSmallInts, s->stream);
-                    if (poison) {
-                        cudaMemsetAsync(s->nodes.ptr, 0x7F, s->nodes.bytes, s->stream);
-                        if (s->order.ptr) cudaMemsetAsync(s->order.ptr, 0x7F, s->order.bytes, s->stream);
-                        if (s->rorder.ptr) cudaMemsetAsync(s->rorder.ptr, 0x7F, s->rorder.bytes, s->stream);
-                    }
-                    mark(-1);
-                    if (o->pipeline == EUCL_PIPELINE_MEGAKERNEL) {
-                        if (!rays) {
-                            EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
-                            dbg("k_camera_entity", 0);
-                            launches += 1;
-                        }
-                        EUCL_PREC(launch_megakernel)(dim, l, fp, cp, ws, d_rgb, d_hit, aov, fb.ray_origins, fb.ray_directions);
-                        mark(1);
-                        launches += 1;
-                    } else {
-                        if (ws.frames) {
-                            EUCL_PREC(launch_camera_entity)(dim, l, fp, ws);
-                            dbg("k_camera_entity", 0);
-                            launches += 1;
-                        }
-                        if (rays) EUCL_PREC(launch_raygen_rays)(dim, l, fp, cp, ws, d_hit, fb.ray_origins, fb.ray_directions);
-                        else EUCL_PREC(launch_raygen)(dim, l, fp, cp, ws, d_hit);
-                        dbg("k_raygen", 0);
-                        mark(0);
-                        for (int level = 0; level < (int)cam->max_depth; ++level) {
-                            launches += EUCL_PREC(launch_intersect)(dim, l, ws, level);
-                            dbg("k_intersect", level);
-                            mark(1);
-                            launches += EUCL_PREC(launch_shade)(dim, l, fp, cp, ws, level, d_hit);
-                            dbg("k_shade", level);
-                            mark(2);
-                        }
-                        // the nodes of the last level are background lookups (depth 0: mod.rs:157,183).  Measured and not kept:
-                        // finishing them inside k_shade of the level above, from the child direction in registers (one launch
-                        // and one ray record per node less, but the lookups then run at the heavy kernel's occupancy:
-                        // 3d_room shade 7.14 + 0.47 -> 7.34 + 0.67 ms)
-                        launches += EUCL_PREC(launch_shade)(dim, l, fp, cp, ws, (int)cam->max_depth, d_hit);
-                        dbg("k_shade", (int)cam->max_depth);
-                        mark(2);
-                        launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fp, cp, ws, d_rgb, aov);
-                        dbg("k_resolve / k_final", 0);
-                        mark(3);
-                        launches += 1; // raygen
-                    }
-                    cudaMemcpyAsync(s->h_small, s->small.ptr, sizeof(int32_t) * kSmallInts, cudaMemcpyDeviceToHost, s->stream);
-                    return launches;
-                };
-                // A chunk whose launch parameters repeat (a fixed pose rendered again: benchmarks, a paused camera, every rank
-                // of a band-split frame) is replayed as ONE CUDA graph launch: the ~50 kernels of a frame then cost one
-                // driver call on the host and run back to back on the device.  The first sighting of a parameter set
-                // launches directly, the second captures, later ones replay.  EUCL_GRAPH=0 disables.
-                uint64_t key = 1469598103934665603ull;
-                auto mix = [&](const void* data, size_t bytes) {
-                    const unsigned char* b = (const unsigned char*)data;
-                    for (size_t k = 0; k < bytes; ++k) key = (key ^ b[k]) * 1099511628211ull;
-                };
-                mix(&fp, sizeof fp);
-                mix(&cp, sizeof cp);
-                mix(&ws, sizeof ws);
-                {   // the members of Launch one by one (the struct has padding bytes)
-                    const void* ptrs[] = {l.stream, l.blob, l.side};
-                    const unsigned long long nums[] = {l.smem_bytes, l.smem_scene, (unsigned long long)l.grid_max, (unsigned long long)l.grid_light,
-                                                       (unsigned long long)l.grid_shade, (unsigned long long)l.grid_mem, l.shade_light_mask,
-                                                       l.shade_heavy_mask, (unsigned long long)l.grid_light_k2,
-                                                       (unsigned long long)l.light_capable, (unsigned long long)l.n_cull,
-                                                       (unsigned long long)l.grid_background};
-                    mix(ptrs, sizeof ptrs);
-                    mix(nums, sizeof nums);
-                }
-                mix(&d_rgb, sizeof d_rgb);
-                mix(&d_hit, sizeof d_hit);
-                // the AOV planes a chunk writes (null = not wanted) and the cost buffer: a graph captured with or without
-                // them never stands in for the other
-                mix(&aov, sizeof aov);
-                const int pipeline_id = o->pipeline;
-                mix(&pipeline_id, sizeof pipeline_id);
-                const uint32_t depth_id = cam->max_depth;
-                mix(&depth_id, sizeof depth_id);
-                // a batch: the graph reads the table the caller's poses were uploaded to, and it is keyed by its contents
-                // too, so that a changed pose or time is never taken for a repeated batch
-                if (fb.n > 1) mix(&fb.table_key, sizeof fb.table_key);
-                // a ray call: tagged, so that a ray call and a render whose other parameters coincide never stand in for
-                // each other, and keyed by the arrays it reads (their contents are read at replay time)
-                if (rays) {
-                    const uint64_t ray_id[] = {0x52415953ull /* "RAYS" */, (uint64_t)(uintptr_t)fb.ray_origins,
-                                               (uint64_t)(uintptr_t)fb.ray_directions, (uint64_t)o->height * o->width, o->width};
-                    mix(ray_id, sizeof ray_id);
-                }
-                // (not while the scene is still choosing its ray-grouping mode: capture time would distort the comparison;
-                // ray calls take no part in that choice)
-                const bool graph_ok = env_int("EUCL_GRAPH", 1) && !o->profile && !debug_sync && !poison &&
-                                      (s->ray_bins_mode >= 0 || o->pipeline != EUCL_PIPELINE_WAVEFRONT || rays);
-                if (graph_ok && s->graph_exec && s->graph_key == key) {
-                    EUCL_CUDA(cudaGraphLaunch(s->graph_exec, s->stream));
-                    st.launches += s->graph_launches;
-                    st.graph_replays += 1;
-                } else if (graph_ok && s->seen_key == key) {
-                    if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
-                    s->graph_exec = nullptr;
-                    cudaGraph_t graph = nullptr;
-                    // one capture at a time in the process (the pipelines of a split frame capture in the same frame)
-                    static std::mutex capture_mutex;
-                    std::unique_lock<std::mutex> capture_lock(capture_mutex);
-                    EUCL_CUDA(cudaStreamBeginCapture(s->stream, cudaStreamCaptureModeThreadLocal));
-                    const uint32_t launches = enqueue();
-                    cudaError_t ce = cudaStreamEndCapture(s->stream, &graph);
-                    if (ce == cudaSuccess) ce = cudaGraphInstantiate(&s->graph_exec, graph, 0);
-                    capture_lock.unlock();
-                    if (graph) cudaGraphDestroy(graph);
-                    if (ce != cudaSuccess) { // not capturable here (e.g. a caller's stream in a state that forbids it): launch directly
-                        cudaGetLastError();
-                        s->graph_exec = nullptr;
-                        s->seen_key = 0;
-                        st.launches += enqueue();
-                    } else {
-                        s->graph_key = key;
-                        s->graph_launches = launches;
-                        EUCL_CUDA(cudaGraphLaunch(s->graph_exec, s->stream));
-                        st.launches += launches;
-                        st.graph_replays += 1;
-                    }
-                } else {
-                    s->seen_key = key;
-                    st.launches += enqueue();
-                }
-                if (!fault.empty()) return fail(EUCL_ERR_CUDA, "EUCL_DEBUG_SYNC: " + fault);
-                EUCL_CUDA(cudaStreamSynchronize(s->stream));
-                EUCL_CUDA(cudaGetLastError());
-                for (size_t k = 1; k < prof_family.size(); ++k) {
-                    float ms = 0.f;
-                    cudaEventElapsedTime(&ms, s->prof_events[k - 1], s->prof_events[k]);
-                    float* slot = prof_family[k] == 0 ? &st.ms_raygen : prof_family[k] == 1 ? &st.ms_intersect
-                                  : prof_family[k] == 2 ? &st.ms_shade : &st.ms_resolve;
-                    *slot += ms;
-                }
-                if (env_int("EUCL_DUMP_LEVELS", 0) && !s->h_small[SmallLayout::overflow]) { // diagnostics: per-level counts, bins, launch times
-                    for (uint32_t lv = 0; lv <= cam->max_depth; ++lv) {
-                        fprintf(stderr, "level %2u count %9d | bins", lv, s->h_small[SmallLayout::count + lv]);
-                        for (int b = 0; b < ws.n_bins && ws.n_bins > 1; ++b) fprintf(stderr, " %d", s->h_small[SmallLayout::bins + lv * kMaxBins + b]);
-                        fprintf(stderr, " | rbins");
-                        for (int b = 0; b < kRayBins; ++b) fprintf(stderr, " %d", s->h_small[SmallLayout::rbins + lv * kRayBins + b]);
-                        fprintf(stderr, "\n");
-                    }
-                    for (size_t k = 1; k < prof_family.size(); ++k) {
-                        float ms = 0.f;
-                        cudaEventElapsedTime(&ms, s->prof_events[k - 1], s->prof_events[k]);
-                        fprintf(stderr, "launch %2zu family %d %.3f ms\n", k, prof_family[k], ms);
-                    }
-                }
-                if (s->h_small[SmallLayout::overflow] == 2)
-                    return fail(EUCL_ERR_CUDA, "internal error: a queue index list and its level count disagree");
-                if (s->h_small[SmallLayout::overflow]) {
-                    // levels after the overflowing one were skipped, so the counts are a lower bound only
-                    long long need = 0;
-                    for (uint32_t lv = 0; lv <= cam->max_depth; ++lv) need += s->h_small[SmallLayout::count + lv];
-                    if (s->h_small[SmallLayout::overflow] == 3) { // a level outgrew the index lists (they hold one level each)
-                        s->list_factor = std::max(s->list_factor * 1.5, 1.0);
-                    } else {
-                        double factor = (double)need / (double)cp.n_pixels * 1.05 + 0.05;
-                        s->arena_factor = std::max(s->arena_factor * 1.5, factor);
-                    }
-                    st.retries += 1;
-                    if (st.retries > 32) return fail(EUCL_ERR_OUT_OF_MEMORY, "node arena keeps overflowing");
-                    continue;
-                }
-                break;
-            }
-            row0 += cp.n_rows;
-            st.pixels += (uint64_t)cp.n_pixels;
-            // camera in no entity: checkerboard pixels, Universe::trace is never called (mod.rs:385-396).  In a batch with
-            // some frames traced, level 0 holds the checkerboard pixels of the others: they are not counted either.
-            const bool traced = s->h_small[SmallLayout::cam_entity] >= 0;
-            for (uint32_t lv = 0; traced && lv <= cam->max_depth; ++lv) {
-                uint64_t c = o->pipeline == EUCL_PIPELINE_MEGAKERNEL
-                                 ? ((const unsigned long long*)(s->h_small + SmallLayout::mega64))[lv]
-                                 : (uint64_t)s->h_small[SmallLayout::count + lv];
-                if (lv == 0) c -= (uint64_t)s->h_small[SmallLayout::untraced];
-                st.level_counts[lv] += c;
-                st.nodes += c;
-                if (lv < cam->max_depth) st.segments += c;
+        const bool debug_sync = env_int("EUCL_DEBUG_SYNC", 0) != 0;
+        const bool poison = env_int("EUCL_POISON", 0) != 0;
+        // (no graph while the scene is still choosing its ray grouping: capture time would distort the comparison; ray
+        // calls take no part in that choice)
+        const bool use_graph = env_int("EUCL_GRAPH", 1) && !o->profile && !debug_sync && !poison &&
+                               (s->ray_bins_mode >= 0 || !wavefront || fb.ray_origins);
+        ChunkLaunch c{fb, o->pipeline, make_launch(s, pipe, *o), ChunkParams{}, Workspace{}, aov_out, d_rgb, d_hit};
+        c.cp.band_rows = o->band_rows ? (int)o->band_rows : (int)o->height;
+        c.cp.band_rank = (int)o->band_rank;
+        c.cp.band_world = o->band_world ? (int)o->band_world : 1;
+        c.cp.compact_rows = o->compact_rows;
+        c.cp.sub_stride = sub_stride;
+        c.cp.sub_offset = sub_offset;
+        for (int row0 = 0; row0 < (int)my_rows; row0 += c.cp.n_rows) {
+            c.cp.local_row0 = row0;
+            for (bool retry = true; retry;) { // a larger arena when a level overflowed
+                int rc = reserve_workspace(s, pipe, need, o->pipeline, width, &rows_per_chunk);
+                if (rc != EUCL_OK) return rc;
+                c.cp.n_rows = std::min<int>(rows_per_chunk, (int)my_rows - row0);
+                c.cp.n_pixels = c.cp.n_rows * width;
+                c.ws = carve(s, pipe, fb);
+                c.aov.cost = need.cost ? (uint2*)pipe.node_cost.ptr : nullptr;
+                ChunkDebug dbg{o->profile != 0, debug_sync, poison, {}, {}};
+                rc = launch_chunk(s, pipe, c, dbg, use_graph, &st);
+                if (rc == EUCL_OK) rc = read_back_chunk(pipe, c, dbg, &st, &retry);
+                if (rc != EUCL_OK) return rc;
             }
         }
     }
-    EUCL_CUDA(cudaEventRecord(s->ev[1], s->stream));
-    EUCL_CUDA(cudaEventSynchronize(s->ev[1]));
-    EUCL_CUDA(cudaEventElapsedTime(&st.ms_total, s->ev[0], s->ev[1]));
-    // A frame that had to grow its arena over-shot (capacity grows by half each retry).  Now that the frame's real node
-    // count is known, the scene keeps that plus a few per cent and gives the rest back: the next frame of this size
-    // allocates once more, exactly, and nothing afterwards.
-    if (st.retries > 0 && st.pixels > 0 && st.nodes > 0 && o->pipeline == EUCL_PIPELINE_WAVEFRONT && st.pixels == (uint64_t)my_rows * width) {
-        uint64_t max_level = 0;
-        for (uint32_t lv = 0; lv <= cam->max_depth; ++lv) max_level = std::max<uint64_t>(max_level, st.level_counts[lv]);
-        const double tight = (double)st.nodes / (double)st.pixels * 1.03 + 0.02;
-        const double tight_list = std::max(1.0, (double)max_level / (double)st.pixels * 1.03);
-        if ((double)s->arena_capacity > ((double)st.pixels * tight + 1024) * 1.08) {
-            s->arena_factor = tight;
-            s->list_factor = tight_list;
-            s->nodes.release();
-            s->order.release();
-            s->rorder.release();
-            s->node_cost.release();
-            s->arena_capacity = 0;
-            s->list_capacity = 0;
-            if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
-            s->graph_exec = nullptr;
-            s->graph_key = s->seen_key = 0;
-        }
-    }
+    EUCL_CUDA(cudaEventRecord(pipe.ev[1], pipe.stream));
+    EUCL_CUDA(cudaEventSynchronize(pipe.ev[1]));
+    EUCL_CUDA(cudaEventElapsedTime(&st.ms_total, pipe.ev[0], pipe.ev[1]));
+    if (wavefront && st.pixels == (uint64_t)my_rows * width) trim_workspace(pipe, st);
     // (a split frame is judged as a whole: render_split).  A ray batch is not a frame of its size: it never tunes.
-    if (!rays) {
-        if (sub_stride <= 1) tune_grouping(s, st, o->pipeline);
+    if (sub_stride <= 1 && !fb.ray_origins) {
+        tune_grouping(s, st, o->pipeline);
         s->warm_frames++;
     }
-    st.ray_grouping = s->ray_bins_now && s->rorder.ptr != nullptr && o->pipeline == EUCL_PIPELINE_WAVEFRONT ? 1u : 0u;
+    st.ray_grouping = s->ray_bins_now && pipe.rorder.ptr != nullptr && wavefront ? 1u : 0u;
     if (stats) *stats = st;
     return EUCL_OK;
 }
 
-// One more scene over the leader's uploaded blob and textures, with streams, events, counters and (later) an arena of its own.
-int add_twin(EuclScene* s) {
-    EuclScene* t = new EuclScene();
-    t->is_twin = true;
-    t->device = s->device;
-    t->dim = s->dim;
-    t->sm_count = s->sm_count;
-    t->blob_bytes = s->blob_bytes;
-    t->smem_bytes = s->smem_bytes;
-    t->smem_scene = s->smem_scene;
-    t->shade_light_mask = s->shade_light_mask;
-    t->shade_heavy_mask = s->shade_heavy_mask;
-    t->d_blob = s->d_blob;
-    t->n_cull = s->n_cull;
-    t->light_capable = s->light_capable;
-    t->n_entities = s->n_entities;
-    t->real_bytes = s->real_bytes;
-    cudaError_t e = cudaStreamCreateWithFlags(&t->own_stream, cudaStreamNonBlocking);
-    t->stream = t->own_stream;
-    if (e == cudaSuccess) e = cudaEventCreate(&t->ev[0]);
-    if (e == cudaSuccess) e = cudaEventCreate(&t->ev[1]);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&t->side_stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&t->ev_fork, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&t->ev_join, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&t->ev_done, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaMallocHost((void**)&t->h_small, sizeof(int32_t) * kSmallInts);
-    for (int k = 0; k < 3 && e == cudaSuccess; ++k)
-        if (!s->ev_split[k]) e = cudaEventCreateWithFlags(&s->ev_split[k], k == 1 ? cudaEventDisableTiming : cudaEventDefault);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        eucl_scene_destroy(t);
-        return fail(e == cudaErrorMemoryAllocation ? EUCL_ERR_OUT_OF_MEMORY : EUCL_ERR_CUDA, std::string("split pipeline: ") + cudaGetErrorString(e));
-    }
-    s->twins.push_back(t);
-    s->workers.push_back(new Worker());
-    s->workers.back()->start();
-    return EUCL_OK;
+// `part`, rendered next to `st` as another part of the same frame, added to it: counts and times add up, and a chunk
+// counts as replayed where every part replayed.
+void add_stats(EuclStats* st, const EuclStats& part) {
+    st->pixels += part.pixels;
+    st->segments += part.segments;
+    st->nodes += part.nodes;
+    for (uint32_t lv = 0; lv < EUCL_MAX_LEVELS; ++lv) st->level_counts[lv] += part.level_counts[lv];
+    st->launches += part.launches;
+    st->retries += part.retries;
+    st->graph_replays = std::min(st->graph_replays, part.graph_replays);
+    st->ms_raygen += part.ms_raygen;
+    st->ms_intersect += part.ms_intersect;
+    st->ms_shade += part.ms_shade;
+    st->ms_resolve += part.ms_resolve;
 }
 
 constexpr int kMaxSplit = 8;
@@ -1504,74 +1573,58 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     int k = std::min(kMaxSplit, env_int("EUCL_SPLIT", EUCL_SPLIT_DEFAULT));
     k = (int)std::min<uint32_t>((uint32_t)std::max(k, 1), my_rows / band); // a band or more for every pipeline
     if (o->pipeline != EUCL_PIPELINE_WAVEFRONT || (long long)my_rows * o->width < (long long)env_int("EUCL_SPLIT_MIN_PIXELS", 1 << 16)) k = 1;
-    if (k <= 1) return render_impl(s, fb, o, d_rgb, d_hit, aov, stats);
-    while ((int)s->twins.size() < k - 1) {
-        int rc = add_twin(s);
-        if (rc != EUCL_OK) return rc;
+    if (k <= 1) return render_impl(s, *s->pipes[0], fb, o, d_rgb, d_hit, aov, stats);
+    while ((int)s->pipes.size() < k) {
+        const int rc = add_pipeline(s);
+        if (rc != EUCL_OK) {
+            cudaGetLastError(); // (a failed allocation must not fail the scene's next call)
+            return rc;
+        }
+        s->workers.push_back(std::make_unique<Worker>());
+        s->workers.back()->start();
     }
     choose_grouping(s);
     EuclRenderOpts opts[kMaxSplit];
-    EuclStats part[kMaxSplit];
-    int rc[kMaxSplit];
+    EuclStats part[kMaxSplit] = {};
+    int rc[kMaxSplit] = {}; // EUCL_OK
     std::string err[kMaxSplit];
     for (int p = 0; p < k; ++p) {
         opts[p] = *o;
         opts[p].band_rows = band;
         opts[p].band_world = (uint32_t)k * world;
         opts[p].band_rank = rank + (uint32_t)p * world;
-        part[p] = EuclStats{};
-        rc[p] = EUCL_OK;
     }
-    EUCL_CUDA(cudaEventRecord(s->ev_split[0], s->stream));
-    EUCL_CUDA(cudaEventRecord(s->ev_split[1], s->stream)); // the other pipelines start after whatever the caller's stream holds
+    const cudaStream_t lead = s->stream();
+    EUCL_CUDA(cudaEventRecord(s->ev_split[0], lead));
+    EUCL_CUDA(cudaEventRecord(s->ev_split[1], lead)); // the other pipelines start after whatever the caller's stream holds
+    for (int p = 1; p < k; ++p) EUCL_CUDA(cudaStreamWaitEvent(s->pipes[p]->stream, s->ev_split[1], 0));
     // per-launch profiling and the debugging modes run the pipelines one after the other on the caller's thread
     const bool serial = o->profile || env_int("EUCL_DEBUG_SYNC", 0) || env_int("EUCL_POISON", 0);
-    auto pipeline = [&](int p) {
-        EuclScene* t = s->twins[p - 1];
-        cudaSetDevice(t->device);
-        rc[p] = render_impl(t, fb, &opts[p], d_rgb, d_hit, aov, &part[p], k, p);
+    auto run = [&](int p) {
+        cudaSetDevice(s->device);
+        rc[p] = render_impl(s, *s->pipes[p], fb, &opts[p], d_rgb, d_hit, aov, &part[p], k, p);
         if (rc[p] != EUCL_OK) err[p] = eucl_last_error();
     };
-    for (int p = 1; p < k; ++p) {
-        EuclScene* t = s->twins[p - 1];
-        t->ray_bins_mode = s->ray_bins_mode;
-        t->ray_bins_now = s->ray_bins_now;
-        EUCL_CUDA(cudaStreamWaitEvent(t->stream, s->ev_split[1], 0));
-    }
     // (no early return between here and the last wait(): the helper threads work on this frame's locals)
-    for (int p = 1; p < k && !serial; ++p) s->workers[p - 1]->run([&pipeline, p] { pipeline(p); });
-    rc[0] = render_impl(s, fb, &opts[0], d_rgb, d_hit, aov, &part[0], k, 0);
+    for (int p = 1; p < k && !serial; ++p) s->workers[p - 1]->run([&run, p] { run(p); });
+    run(0);
     for (int p = 1; p < k; ++p) {
-        if (serial) pipeline(p);
+        if (serial) run(p);
         else s->workers[p - 1]->wait();
     }
-    if (rc[0] != EUCL_OK) return rc[0];
-    for (int p = 1; p < k; ++p)
+    for (int p = 0; p < k; ++p)
         if (rc[p] != EUCL_OK) return fail(rc[p], err[p]);
-    for (int p = 1; p < k; ++p) { // the caller's stream continues after every pipeline
-        EuclScene* t = s->twins[p - 1];
-        EUCL_CUDA(cudaEventRecord(t->ev_done, t->stream));
-        EUCL_CUDA(cudaStreamWaitEvent(s->stream, t->ev_done, 0));
-    }
-    EUCL_CUDA(cudaEventRecord(s->ev_split[2], s->stream));
+    for (int p = 1; p < k; ++p) // the caller's stream continues after every pipeline (ev[1]: the end of its part)
+        EUCL_CUDA(cudaStreamWaitEvent(lead, s->pipes[p]->ev[1], 0));
+    EUCL_CUDA(cudaEventRecord(s->ev_split[2], lead));
     EUCL_CUDA(cudaEventSynchronize(s->ev_split[2]));
     EuclStats st = part[0];
     EUCL_CUDA(cudaEventElapsedTime(&st.ms_total, s->ev_split[0], s->ev_split[2]));
-    for (int p = 1; p < k; ++p) {
-        const EuclStats& b = part[p];
-        st.pixels += b.pixels;
-        st.segments += b.segments;
-        st.nodes += b.nodes;
-        for (uint32_t lv = 0; lv < EUCL_MAX_LEVELS; ++lv) st.level_counts[lv] += b.level_counts[lv];
-        st.launches += b.launches;
-        st.retries += b.retries;
-        st.graph_replays = std::min(st.graph_replays, b.graph_replays);
-        st.ms_raygen += b.ms_raygen;
-        st.ms_intersect += b.ms_intersect;
-        st.ms_shade += b.ms_shade;
-        st.ms_resolve += b.ms_resolve;
+    for (int p = 1; p < k; ++p) add_stats(&st, part[p]);
+    if (!fb.ray_origins) {
+        tune_grouping(s, st, o->pipeline);
+        s->warm_frames++;
     }
-    if (!fb.ray_origins) tune_grouping(s, st, o->pipeline);
     if (stats) *stats = st;
     return EUCL_OK;
 }
@@ -1606,48 +1659,6 @@ int check_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const
     return EUCL_OK;
 }
 
-// The batch of `n` frames and the virtual frame they form.  K > 1: the frame constants are computed on the host like
-// a single frame's and uploaded, stream-ordered before the first launch (and outside any graph capture).
-int prepare_batch(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, FrameBatch* fb,
-                  EuclRenderOpts* virt) {
-    *fb = FrameBatch{frames, n, o->height, nullptr, 0};
-    *virt = *o;
-    virt->height = n * o->height;
-    if (n == 1) return EUCL_OK;
-    if (s->h_frame_table_cap < n) {
-        if (s->h_frame_table) cudaFreeHost(s->h_frame_table);
-        s->h_frame_table = nullptr;
-        s->h_frame_table_cap = 0;
-        EUCL_CUDA(cudaMallocHost((void**)&s->h_frame_table, sizeof(FrameParams) * n));
-        s->h_frame_table_cap = n;
-    }
-    uint64_t key = 1469598103934665603ull;
-    for (uint32_t k = 0; k < n; ++k) {
-        EuclRenderOpts one = *o;
-        one.time_seconds = frames[k].time_seconds;
-        frame_params(frames[k].camera, one, s->real_bytes, &s->h_frame_table[k]);
-        const unsigned char* b = (const unsigned char*)&s->h_frame_table[k];
-        for (size_t i = 0; i < sizeof(FrameParams); ++i) key = (key ^ b[i]) * 1099511628211ull;
-    }
-    EUCL_CUDA(s->frame_table.ensure(sizeof(FrameParams) * n));
-    EUCL_CUDA(cudaMemcpyAsync(s->frame_table.ptr, s->h_frame_table, sizeof(FrameParams) * n, cudaMemcpyHostToDevice, s->stream));
-    fb->d_table = (const FrameParams*)s->frame_table.ptr;
-    fb->table_key = key;
-    return EUCL_OK;
-}
-
-// Device-output render of `n` frames (eucl_render_device: n = 1), or -- `rays` -- of a ray call's virtual frame (`o` then
-// is that frame and `frames` is rays->frames).
-int render_frames_to_device(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* d_rgb,
-                            int32_t* d_hit, const AovPlanes& aov, EuclStats* stats, const FrameBatch* rays = nullptr) {
-    if (rays) return render_split(s, *rays, o, d_rgb, d_hit, aov, stats);
-    FrameBatch fb;
-    EuclRenderOpts virt;
-    const int st = prepare_batch(s, frames, n, o, &fb, &virt);
-    if (st != EUCL_OK) return st;
-    return render_split(s, fb, &virt, d_rgb, d_hit, aov, stats);
-}
-
 // eucl_render_aovs*: at least one plane.  Checked before any device is touched.
 int check_aovs(const EuclAovs* a, const char* fn) {
     if (!a || !(a->depth || a->position || a->normal || a->segments || a->levels))
@@ -1659,16 +1670,43 @@ AovPlanes aov_planes(const EuclAovs* a) {
     return AovPlanes{a->depth, a->position, a->normal, a->segments, a->levels, nullptr};
 }
 
-// Host-output render of `n` frames (arguments already checked): rendered into the scene's device buffers, then copied out.
+// One frame: what eucl_render accepts; K > 1 frames: what eucl_render_frames accepts.
+int check_aov_call(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, const EuclAovs* aovs,
+                   const char* fn) {
+    int st = n_frames == 1 ? check_args(s, frames ? &frames[0].camera : nullptr, o) : check_frames(s, frames, n_frames, o);
+    if (st == EUCL_OK) st = check_aovs(aovs, fn);
+    return st;
+}
+
+static_assert(sizeof(EuclRays) == 48, "EuclRays is part of the C ABI");
+
+// eucl_trace_rays*: checked before any device is touched.
+int check_rays(EuclScene* s, const EuclRays* r, const void* out, const char* fn) {
+    const std::string f(fn);
+    if (!s || !r) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null argument");
+    if (r->n == 0 || r->n > 0x7fffffffu) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n must be 1 .. 2^31 - 1");
+    if (!r->origins || !r->directions) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null ray array");
+    if (!out) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null output");
+    if (r->width > 1 && r->n % r->width != 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": width does not divide n");
+    if (r->max_depth + 1ull > EUCL_MAX_LEVELS) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": max_depth too large");
+    if (r->pipeline != EUCL_PIPELINE_WAVEFRONT && r->pipeline != EUCL_PIPELINE_MEGAKERNEL)
+        return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": unknown pipeline");
+    return EUCL_OK;
+}
+
+const EuclAovs* any_plane(const EuclAovs* a) {
+    return a && (a->depth || a->position || a->normal || a->segments || a->levels) ? a : nullptr;
+}
+
+// Host-output render of a batch whose virtual frame is `o`: rendered into the scene's device buffers, then copied out.
 // A rank of a band-split render (band_world > 1, a single frame) renders its rows compactly on the device and then copies
 // each band to its place in the caller's frame: rows of other ranks are never read or written, so N ranks can fill ONE
 // host frame (shared pinned memory) over their own PCIe links at the same time.  The AOV planes go the same way.
-int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const EuclRenderOpts* o, uint8_t* out_rgb8,
-                   int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats, const FrameBatch* rays = nullptr) {
-    EUCL_CUDA(cudaSetDevice(s->device));
+int render_to_host(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
+                   const EuclAovs* aovs, EuclStats* stats) {
     const bool scatter = !o->compact_rows && o->band_world > 1;
     const size_t my_rows = eucl_band_rows_for_rank(o);
-    const size_t rows = (o->compact_rows || scatter) ? my_rows : (size_t)n * o->height;
+    const size_t rows = (o->compact_rows || scatter) ? my_rows : (size_t)o->height;
     const size_t pixels = rows * (size_t)o->width;
     const bool want_hit = o->want_hit_ids && out_hit_ids;
     EUCL_CUDA(s->frame.ensure(std::max<size_t>(pixels, 1) * 3));
@@ -1694,14 +1732,14 @@ int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const Eucl
     EuclRenderOpts opts = *o;
     opts.want_hit_ids = want_hit ? 1 : 0;
     if (scatter) opts.compact_rows = 1;
-    const int st = render_frames_to_device(s, frames, n, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr,
-                                           d_aov, stats, rays);
+    const int st = render_split(s, fb, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, d_aov, stats);
     if (st != EUCL_OK) return st;
+    const cudaStream_t stream = s->stream();
     if (!scatter) {
-        EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, s->stream));
-        if (want_hit) EUCL_CUDA(cudaMemcpyAsync(out_hit_ids, s->hit_ids.ptr, pixels * 4, cudaMemcpyDeviceToHost, s->stream));
+        EUCL_CUDA(cudaMemcpyAsync(out_rgb8, s->frame.ptr, pixels * 3, cudaMemcpyDeviceToHost, stream));
+        if (want_hit) EUCL_CUDA(cudaMemcpyAsync(out_hit_ids, s->hit_ids.ptr, pixels * 4, cudaMemcpyDeviceToHost, stream));
         for (int k = 0; k < 5; ++k)
-            if (host[k]) EUCL_CUDA(cudaMemcpyAsync(host[k], dev[k], pixels * px_bytes[k], cudaMemcpyDeviceToHost, s->stream));
+            if (host[k]) EUCL_CUDA(cudaMemcpyAsync(host[k], dev[k], pixels * px_bytes[k], cudaMemcpyDeviceToHost, stream));
     } else if (my_rows > 0) {
         // band k of this rank: compact rows [k * band, ...) -> frame rows [(k * world + rank) * band, ...)
         const size_t band = o->band_rows ? o->band_rows : o->height, world = o->band_world;
@@ -1710,10 +1748,10 @@ int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const Eucl
             const size_t band_bytes = band * o->width * px_bytes;
             uint8_t* d = (uint8_t*)dst + (size_t)o->band_rank * band_bytes;
             cudaError_t e = cudaSuccess;
-            if (full) e = cudaMemcpy2DAsync(d, world * band_bytes, src, band_bytes, band_bytes, full, cudaMemcpyDeviceToHost, s->stream);
+            if (full) e = cudaMemcpy2DAsync(d, world * band_bytes, src, band_bytes, band_bytes, full, cudaMemcpyDeviceToHost, stream);
             if (e == cudaSuccess && tail)
                 e = cudaMemcpyAsync(d + full * world * band_bytes, (const uint8_t*)src + full * band_bytes, tail * o->width * px_bytes,
-                                    cudaMemcpyDeviceToHost, s->stream);
+                                    cudaMemcpyDeviceToHost, stream);
             return e;
         };
         EUCL_CUDA(copy_bands(out_rgb8, s->frame.ptr, 3));
@@ -1721,7 +1759,7 @@ int render_to_host(EuclScene* s, const EuclFrame* frames, uint32_t n, const Eucl
         for (int k = 0; k < 5; ++k)
             if (host[k]) EUCL_CUDA(copy_bands(host[k], dev[k], px_bytes[k]));
     }
-    EUCL_CUDA(cudaStreamSynchronize(s->stream));
+    EUCL_CUDA(cudaStreamSynchronize(stream));
     return EUCL_OK;
 }
 
@@ -1736,8 +1774,10 @@ int eucl_render_device(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts
     if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_device: null output");
     EUCL_CUDA(cudaSetDevice(s->device));
     const EuclFrame frame{*cam, o->time_seconds};
-    return render_frames_to_device(s, &frame, 1, o, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr,
-                                   AovPlanes{}, stats);
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, &frame, 1, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
 }
 
 int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o,
@@ -1746,8 +1786,10 @@ int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_
     if (st != EUCL_OK) return st;
     if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames_device: null output");
     EUCL_CUDA(cudaSetDevice(s->device));
-    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
-                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
 }
 
 int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
@@ -1755,7 +1797,11 @@ int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames,
     int st = check_frames(s, frames, n_frames, o);
     if (st != EUCL_OK) return st;
     if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_frames: null output");
-    return render_to_host(s, frames, n_frames, o, out_rgb8, out_hit_ids, nullptr, stats);
+    EUCL_CUDA(cudaSetDevice(s->device));
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_to_host(s, fb, &virt, out_rgb8, out_hit_ids, nullptr, stats);
 }
 
 int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
@@ -1763,103 +1809,54 @@ int eucl_render(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts* o, ui
     int st = check_args(s, cam, o);
     if (st != EUCL_OK) return st;
     if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render: null output");
+    EUCL_CUDA(cudaSetDevice(s->device));
     const EuclFrame frame{*cam, o->time_seconds};
-    return render_to_host(s, &frame, 1, o, out_rgb8, out_hit_ids, nullptr, stats);
-}
-
-// One frame: what eucl_render accepts; K > 1 frames: what eucl_render_frames accepts.
-static int check_aov_call(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, const EuclAovs* aovs,
-                          const char* fn) {
-    int st = n_frames == 1 ? check_args(s, frames ? &frames[0].camera : nullptr, o) : check_frames(s, frames, n_frames, o);
-    if (st == EUCL_OK) st = check_aovs(aovs, fn);
-    return st;
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, &frame, 1, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_to_host(s, fb, &virt, out_rgb8, out_hit_ids, nullptr, stats);
 }
 
 int eucl_render_aovs(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
                      int32_t* out_hit_ids, const EuclAovs* aovs, EuclStats* stats) {
-    const int st = check_aov_call(s, frames, n_frames, o, aovs, "eucl_render_aovs");
+    int st = check_aov_call(s, frames, n_frames, o, aovs, "eucl_render_aovs");
     if (st != EUCL_OK) return st;
     if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_aovs: null output");
-    return render_to_host(s, frames, n_frames, o, out_rgb8, out_hit_ids, aovs, stats);
+    EUCL_CUDA(cudaSetDevice(s->device));
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_to_host(s, fb, &virt, out_rgb8, out_hit_ids, aovs, stats);
 }
 
 int eucl_render_aovs_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, void* d_out_rgb8,
                             void* d_out_hit_ids, const EuclAovs* d_aovs, EuclStats* stats) {
-    const int st = check_aov_call(s, frames, n_frames, o, d_aovs, "eucl_render_aovs_device");
+    int st = check_aov_call(s, frames, n_frames, o, d_aovs, "eucl_render_aovs_device");
     if (st != EUCL_OK) return st;
     if (!d_out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_render_aovs_device: null output");
     EUCL_CUDA(cudaSetDevice(s->device));
-    return render_frames_to_device(s, frames, n_frames, o, (uint8_t*)d_out_rgb8,
-                                   o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, aov_planes(d_aovs), stats);
-}
-
-} // extern "C"
-
-namespace {
-
-static_assert(sizeof(EuclRays) == 48, "EuclRays is part of the C ABI");
-
-// eucl_trace_rays*: checked before any device is touched.
-int check_rays(EuclScene* s, const EuclRays* r, const void* out, const char* fn) {
-    const std::string f(fn);
-    if (!s || !r) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null argument");
-    if (r->n == 0 || r->n > 0x7fffffffu) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n must be 1 .. 2^31 - 1");
-    if (!r->origins || !r->directions) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null ray array");
-    if (!out) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null output");
-    if (r->width > 1 && r->n % r->width != 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": width does not divide n");
-    if (r->max_depth + 1ull > EUCL_MAX_LEVELS) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": max_depth too large");
-    if (r->pipeline != EUCL_PIPELINE_WAVEFRONT && r->pipeline != EUCL_PIPELINE_MEGAKERNEL)
-        return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": unknown pipeline");
-    return EUCL_OK;
-}
-
-// The virtual frame of a ray call (n / width rows of width) and its batch: one "frame" that carries the depth and the
-// time, and the device rays.
-struct RayCall {
-    EuclFrame frame;
-    EuclRenderOpts opts;
     FrameBatch fb;
-    RayCall(const EuclScene* s, const EuclRays* r, const double* d_origins, const double* d_directions, bool want_hit) {
-        std::memset(&frame, 0, sizeof frame);
-        frame.camera.dim = s->dim;
-        frame.camera.max_depth = r->max_depth;
-        frame.time_seconds = r->time_seconds;
-        const uint32_t w = r->width > 1 ? r->width : 1;
-        opts = EuclRenderOpts{};
-        opts.width = w;
-        opts.height = r->n / w;
-        opts.time_seconds = r->time_seconds;
-        opts.pipeline = r->pipeline;
-        opts.want_hit_ids = want_hit ? 1 : 0;
-        opts.profile = r->profile;
-        fb = FrameBatch{&frame, 1, opts.height, nullptr, 0};
-        fb.ray_origins = d_origins;
-        fb.ray_directions = d_directions;
-    }
-};
-
-const EuclAovs* any_plane(const EuclAovs* a) {
-    return a && (a->depth || a->position || a->normal || a->segments || a->levels) ? a : nullptr;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, aov_planes(d_aovs),
+                        stats);
 }
-
-} // namespace
-
-extern "C" {
 
 int eucl_trace_rays(EuclScene* s, const EuclRays* r, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs,
                     EuclStats* stats) {
     const int st = check_rays(s, r, out_rgb8, "eucl_trace_rays");
     if (st != EUCL_OK) return st;
     EUCL_CUDA(cudaSetDevice(s->device));
-    // staged before the first launch, on the scene's stream and outside any graph capture: a replayed graph reads them
+    // staged before the first launch, on pipeline 0's stream and outside any graph capture: a replayed graph reads them
     const size_t bytes = sizeof(double) * (size_t)s->dim * r->n;
     EUCL_CUDA(s->ray_stage.ensure(2 * bytes));
     double* d_o = (double*)s->ray_stage.ptr;
     double* d_d = (double*)((uint8_t*)s->ray_stage.ptr + bytes);
-    EUCL_CUDA(cudaMemcpyAsync(d_o, r->origins, bytes, cudaMemcpyHostToDevice, s->stream));
-    EUCL_CUDA(cudaMemcpyAsync(d_d, r->directions, bytes, cudaMemcpyHostToDevice, s->stream));
-    RayCall call(s, r, d_o, d_d, out_hit_ids != nullptr);
-    return render_to_host(s, &call.frame, 1, &call.opts, out_rgb8, out_hit_ids, any_plane(aovs), stats, &call.fb);
+    EUCL_CUDA(cudaMemcpyAsync(d_o, r->origins, bytes, cudaMemcpyHostToDevice, s->stream()));
+    EUCL_CUDA(cudaMemcpyAsync(d_d, r->directions, bytes, cudaMemcpyHostToDevice, s->stream()));
+    EuclRenderOpts o;
+    const FrameBatch fb = ray_batch(s, r, d_o, d_d, out_hit_ids != nullptr, &o);
+    return render_to_host(s, fb, &o, out_rgb8, out_hit_ids, any_plane(aovs), stats);
 }
 
 int eucl_trace_rays_device(EuclScene* s, const EuclRays* r, void* d_out_rgb8, void* d_out_hit_ids, const EuclAovs* d_aovs,
@@ -1867,18 +1864,18 @@ int eucl_trace_rays_device(EuclScene* s, const EuclRays* r, void* d_out_rgb8, vo
     const int st = check_rays(s, r, d_out_rgb8, "eucl_trace_rays_device");
     if (st != EUCL_OK) return st;
     EUCL_CUDA(cudaSetDevice(s->device));
-    RayCall call(s, r, r->origins, r->directions, d_out_hit_ids != nullptr);
-    return render_frames_to_device(s, &call.frame, 1, &call.opts, (uint8_t*)d_out_rgb8, (int32_t*)d_out_hit_ids,
-                                   aov_planes(any_plane(d_aovs)), stats, &call.fb);
+    EuclRenderOpts o;
+    const FrameBatch fb = ray_batch(s, r, r->origins, r->directions, d_out_hit_ids != nullptr, &o);
+    return render_split(s, fb, &o, (uint8_t*)d_out_rgb8, (int32_t*)d_out_hit_ids, aov_planes(any_plane(d_aovs)), stats);
 }
 
 int eucl_scene_memory(const EuclScene* s, uint64_t* arena_bytes, uint64_t* list_bytes, uint64_t* node_capacity) {
     if (!s) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_scene_memory: null scene");
-    uint64_t arena = s->nodes.bytes, lists = s->order.bytes + s->rorder.bytes, cap = (uint64_t)s->arena_capacity;
-    for (const EuclScene* t : s->twins) { // a split scene holds one arena per pipeline
-        arena += t->nodes.bytes;
-        lists += t->order.bytes + t->rorder.bytes;
-        cap += (uint64_t)t->arena_capacity;
+    uint64_t arena = 0, lists = 0, cap = 0;
+    for (const auto& p : s->pipes) { // a split scene holds one arena per pipeline
+        arena += p->nodes.bytes;
+        lists += p->order.bytes + p->rorder.bytes;
+        cap += (uint64_t)p->arena_capacity;
     }
     if (arena_bytes) *arena_bytes = arena;
     if (list_bytes) *list_bytes = lists;
@@ -1889,8 +1886,9 @@ int eucl_scene_memory(const EuclScene* s, uint64_t* arena_bytes, uint64_t* list_
 int eucl_scene_set_stream(EuclScene* s, void* cuda_stream) {
     if (!s) return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_scene_set_stream: null scene");
     EUCL_CUDA(cudaSetDevice(s->device));
-    EUCL_CUDA(cudaStreamSynchronize(s->stream));
-    s->stream = cuda_stream ? (cudaStream_t)cuda_stream : s->own_stream;
+    Pipeline& p = *s->pipes[0];
+    EUCL_CUDA(cudaStreamSynchronize(p.stream));
+    p.stream = cuda_stream ? (cudaStream_t)cuda_stream : p.own_stream;
     return EUCL_OK;
 }
 
@@ -1900,6 +1898,7 @@ int eucl_trace_path(EuclScene* s, const double* location, const double* directio
         return fail(EUCL_ERR_INVALID_ARGUMENT, "eucl_trace_path: null argument");
     EUCL_CUDA(cudaSetDevice(s->device));
     const int D = s->dim;
+    const cudaStream_t stream = s->stream();
     EUCL_CUDA(s->path_io.ensure(sizeof(double) * 4 * EUCL_MAX_DIM + 16));
     double* d_in = (double*)s->path_io.ptr;
     double* d_out = d_in + 2 * EUCL_MAX_DIM;
@@ -1909,14 +1908,13 @@ int eucl_trace_path(EuclScene* s, const double* location, const double* directio
         h_in[k] = location[k];
         h_in[D + k] = direction[k];
     }
-    EUCL_CUDA(cudaMemcpyAsync(d_in, h_in, sizeof h_in, cudaMemcpyHostToDevice, s->stream));
-    Launch l{s->stream, s->d_blob, s->smem_bytes, s->smem_scene, 1, 1, 1, 1, 1ull, 0ull, 1, 0, 0, nullptr, nullptr, nullptr};
-    EUCL_PREC(launch_trace_path)(D, l, d_in, distance, d_out, d_found);
+    EUCL_CUDA(cudaMemcpyAsync(d_in, h_in, sizeof h_in, cudaMemcpyHostToDevice, stream));
+    EUCL_PREC(launch_trace_path)(D, make_launch(s, *s->pipes[0], EuclRenderOpts{}), d_in, distance, d_out, d_found);
     double h_out[2 * EUCL_MAX_DIM];
     int h_found = 0;
-    EUCL_CUDA(cudaMemcpyAsync(h_out, d_out, sizeof h_out, cudaMemcpyDeviceToHost, s->stream));
-    EUCL_CUDA(cudaMemcpyAsync(&h_found, d_found, sizeof h_found, cudaMemcpyDeviceToHost, s->stream));
-    EUCL_CUDA(cudaStreamSynchronize(s->stream));
+    EUCL_CUDA(cudaMemcpyAsync(h_out, d_out, sizeof h_out, cudaMemcpyDeviceToHost, stream));
+    EUCL_CUDA(cudaMemcpyAsync(&h_found, d_found, sizeof h_found, cudaMemcpyDeviceToHost, stream));
+    EUCL_CUDA(cudaStreamSynchronize(stream));
     EUCL_CUDA(cudaGetLastError());
     if (h_found < 0) return fail(EUCL_ERR_SCENE_LIMIT, "eucl_trace_path: more than 100000 surface crossings");
     if (h_found == 0) return 1; /* the start point lies in no entity: Option::None in the reference */
