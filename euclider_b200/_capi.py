@@ -86,6 +86,18 @@ class EuclRays(C.Structure):
                 ("_pad", C.c_int32)]
 
 
+class EuclTreeNode(C.Structure):
+    _fields_ = [("parent", C.c_int32), ("level", C.c_int32), ("kind", C.c_int32), ("medium", C.c_int32),
+                ("hit_entity", C.c_int32), ("exiting", C.c_int32), ("flags", C.c_uint32), ("surface_rgba8", C.c_uint32),
+                ("ratio", C.c_double), ("t", C.c_double), ("origin", c_double4), ("direction", c_double4),
+                ("normal", c_double4), ("color", C.c_double * 4)]
+
+
+class EuclTreeQuery(C.Structure):
+    _fields_ = [("items", C.c_void_p), ("n_items", C.c_uint32), ("capacity", C.c_uint32), ("nodes", C.c_void_p),
+                ("counts", C.c_void_p)]
+
+
 class EuclFlatScene(C.Structure):
     _fields_ = [("dim", C.c_int32),
                 ("n_prims", C.c_int32), ("n_nodes", C.c_int32), ("n_entities", C.c_int32),
@@ -120,6 +132,11 @@ EUCL_OK = 0
 EUCL_PIPELINE_WAVEFRONT = 0
 EUCL_PIPELINE_MEGAKERNEL = 1
 EUCL_PRECISION_F64, EUCL_PRECISION_F32 = 0, 1
+EUCL_TREE_ROOT, EUCL_TREE_TRANSMITTED, EUCL_TREE_REFLECTED = range(3)
+EUCL_TREE_BACKGROUND, EUCL_TREE_SURFACE, EUCL_TREE_OPAQUE, EUCL_TREE_NO_DESTINATION, EUCL_TREE_UNDEFINED, EUCL_TREE_CHECKERBOARD = (
+    1, 2, 4, 8, 16, 32)
+EUCL_TREE_MAX_ITEMS = 65536
+EUCL_TREE_MAX_NODES = 1 << 24
 PRIM_VOID, PRIM_SPHERE, PRIM_HYPERPLANE, PRIM_HALFSPACE, PRIM_CYLINDER = range(5)
 CSG_LEAF, CSG_UNION, CSG_INTERSECTION, CSG_COMPLEMENT, CSG_SYMDIFF = range(5)
 MAT_VACUUM, MAT_LINEAR_SPACE = range(2)
@@ -167,6 +184,10 @@ PROTOTYPES = {
                                   C.POINTER(EuclStats)]),
     "eucl_trace_rays_device": (C.c_int, [C.c_void_p, C.POINTER(EuclRays), C.c_void_p, C.c_void_p, C.POINTER(EuclAovs),
                                          C.POINTER(EuclStats)]),
+    "eucl_render_trees": (C.c_int, [C.c_void_p, C.POINTER(EuclFrame), C.c_uint32, C.POINTER(EuclRenderOpts), C.c_void_p,
+                                    C.c_void_p, C.POINTER(EuclTreeQuery), C.POINTER(EuclStats)]),
+    "eucl_trace_ray_trees": (C.c_int, [C.c_void_p, C.POINTER(EuclRays), C.c_void_p, C.c_void_p, C.POINTER(EuclTreeQuery),
+                                       C.POINTER(EuclStats)]),
     "eucl_trace_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,
                                   C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "eucl_camera_rotate_yaw": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),

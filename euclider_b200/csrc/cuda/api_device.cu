@@ -174,6 +174,7 @@ struct EuclScene {
     DeviceBuffer hit_ids;   // device hit-id map for eucl_render
     DeviceBuffer aov_stage; // device copies of the AOV planes for eucl_render_aovs (host output)
     DeviceBuffer ray_stage; // device copy of the rays of eucl_trace_rays (host input), refilled by every call
+    DeviceBuffer tree_stage; // a tree call: its query and the nodes and counts every pipeline exports into (host output)
     DeviceBuffer path_io;   // eucl_trace_path staging
     // a batch of frames (eucl_render_frames*): the per-frame constants, read by every pipeline, and their pinned host staging
     DeviceBuffer frame_table;
@@ -1001,6 +1002,7 @@ struct FrameBatch {
     uint64_t table_key;            // K > 1: hash of the table contents, part of the graph key
     const double* ray_origins;     // rays: [n][dim] each; null for camera frames
     const double* ray_directions;
+    TreeQuery tree;                // a tree call: the items whose trees the chunks export (n_items 0: none)
 };
 
 // The batch of `n` camera frames (arguments checked) and `virt`, the virtual frame they form.  K > 1: the frame constants
@@ -1290,7 +1292,7 @@ uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c,
             check("k_camera_entity", 0);
             launches += 1;
         }
-        EUCL_PREC(launch_megakernel)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.d_hit, c.aov, fb.ray_origins, fb.ray_directions);
+        EUCL_PREC(launch_megakernel)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.d_hit, c.aov, fb.ray_origins, fb.ray_directions, fb.tree);
         mark(1);
         launches += 1;
     } else {
@@ -1320,6 +1322,10 @@ uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c,
         mark(2);
         launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.aov);
         check("k_resolve / k_final", 0);
+        if (fb.tree.n_items) {
+            launches += EUCL_PREC(launch_tree_export)(dim, l, fb.fp, c.cp, c.ws, fb.tree);
+            check("k_tree_export", 0);
+        }
         mark(3);
         launches += 1; // raygen
     }
@@ -1369,6 +1375,10 @@ uint64_t graph_key(const ChunkLaunch& c) {
 // host and run back to back on the device.  The first sighting of a parameter set launches directly, the second
 // captures, later ones replay.  Without `use_graph` every chunk launches directly.
 int launch_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c, ChunkDebug& dbg, bool use_graph, EuclStats* st) {
+    if (c.fb.tree.n_items) { // a tree call launches directly and leaves the plain calls' graph and keys as they were
+        st->launches += enqueue_chunk(s, pipe, c, dbg);
+        return EUCL_OK;
+    }
     const uint64_t key = graph_key(c);
     if (use_graph && pipe.graph_exec && pipe.graph_key == key) {
         EUCL_CUDA(cudaGraphLaunch(pipe.graph_exec, pipe.stream));
@@ -1526,8 +1536,9 @@ int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRe
     EUCL_CUDA(cudaEventSynchronize(pipe.ev[1]));
     EUCL_CUDA(cudaEventElapsedTime(&st.ms_total, pipe.ev[0], pipe.ev[1]));
     if (wavefront && st.pixels == (uint64_t)my_rows * width) trim_workspace(pipe, st);
-    // (a split frame is judged as a whole: render_split).  A ray batch is not a frame of its size: it never tunes.
-    if (sub_stride <= 1 && !fb.ray_origins) {
+    // (a split frame is judged as a whole: render_split).  A ray batch is not a frame of its size, and a tree call pays
+    // for its export: neither tunes.
+    if (sub_stride <= 1 && !fb.ray_origins && !fb.tree.n_items) {
         tune_grouping(s, st, o->pipeline);
         s->warm_frames++;
     }
@@ -1621,7 +1632,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     EuclStats st = part[0];
     EUCL_CUDA(cudaEventElapsedTime(&st.ms_total, s->ev_split[0], s->ev_split[2]));
     for (int p = 1; p < k; ++p) add_stats(&st, part[p]);
-    if (!fb.ray_origins) {
+    if (!fb.ray_origins && !fb.tree.n_items) {
         tune_grouping(s, st, o->pipeline);
         s->warm_frames++;
     }
@@ -1691,6 +1702,80 @@ int check_rays(EuclScene* s, const EuclRays* r, const void* out, const char* fn)
     if (r->max_depth + 1ull > EUCL_MAX_LEVELS) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": max_depth too large");
     if (r->pipeline != EUCL_PIPELINE_WAVEFRONT && r->pipeline != EUCL_PIPELINE_MEGAKERNEL)
         return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": unknown pipeline");
+    return EUCL_OK;
+}
+
+// The host rays of a ray call, copied to the scene's device buffer before the first launch, on pipeline 0's stream and
+// outside any graph capture: a replayed graph reads them.
+int stage_rays(EuclScene* s, const EuclRays* r, double** d_origins, double** d_directions) {
+    const size_t bytes = sizeof(double) * (size_t)s->dim * r->n;
+    EUCL_CUDA(s->ray_stage.ensure(2 * bytes));
+    *d_origins = (double*)s->ray_stage.ptr;
+    *d_directions = (double*)((uint8_t*)s->ray_stage.ptr + bytes);
+    EUCL_CUDA(cudaMemcpyAsync(*d_origins, r->origins, bytes, cudaMemcpyHostToDevice, s->stream()));
+    EUCL_CUDA(cudaMemcpyAsync(*d_directions, r->directions, bytes, cudaMemcpyHostToDevice, s->stream()));
+    return EUCL_OK;
+}
+
+static_assert(sizeof(EuclTreeNode) == 176, "EuclTreeNode is part of the C ABI");
+static_assert(sizeof(EuclTreeQuery) == 32, "EuclTreeQuery is part of the C ABI");
+
+// eucl_render_trees / eucl_trace_ray_trees: the query against a virtual frame of `cells` cells.  Checked before any device
+// is touched.
+int check_tree_query(const EuclTreeQuery* q, uint64_t cells, const char* fn) {
+    const std::string f(fn);
+    if (!q || q->n_items == 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": no tree query (use the plain entry point)");
+    if (q->n_items > EUCL_TREE_MAX_ITEMS) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": more than EUCL_TREE_MAX_ITEMS items");
+    if (!q->items || !q->nodes || !q->counts) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null items, nodes or counts");
+    if (q->capacity == 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": capacity must be at least 1");
+    if ((uint64_t)q->n_items * q->capacity > EUCL_TREE_MAX_NODES)
+        return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n_items * capacity above EUCL_TREE_MAX_NODES");
+    for (uint32_t i = 0; i < q->n_items; ++i)
+        if (q->items[i] >= cells)
+            return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": item " + std::to_string(i) + " (" + std::to_string(q->items[i]) +
+                                                       ") is outside the virtual frame of " + std::to_string(cells) + " cells");
+    return EUCL_OK;
+}
+
+// The device side of a checked query, staged on pipeline 0's stream before the first launch: the distinct items, sorted,
+// each with its first request slot, and the slots' nodes (zeroed) and counts that the pipelines export into -- every item
+// by exactly one chunk of one pipeline.
+int stage_tree_query(EuclScene* s, const EuclTreeQuery* q, std::vector<uint32_t>* order, TreeQuery* out) {
+    order->resize(q->n_items);
+    for (uint32_t i = 0; i < q->n_items; ++i) (*order)[i] = i;
+    std::stable_sort(order->begin(), order->end(), [q](uint32_t a, uint32_t b) { return q->items[a] < q->items[b]; });
+    std::vector<uint32_t> items, slots;
+    for (uint32_t i : *order)
+        if (items.empty() || items.back() != q->items[i]) {
+            items.push_back(q->items[i]);
+            slots.push_back(i);
+        }
+    const size_t node_bytes = align16(sizeof(EuclTreeNode) * q->n_items * (size_t)q->capacity);
+    const size_t list_bytes = align16(sizeof(uint32_t) * q->n_items);
+    EUCL_CUDA(s->tree_stage.ensure(node_bytes + 3 * list_bytes));
+    uint8_t* p = (uint8_t*)s->tree_stage.ptr;
+    *out = TreeQuery{(const uint32_t*)(p + node_bytes + list_bytes), (const uint32_t*)(p + node_bytes + 2 * list_bytes),
+                     (int32_t)items.size(), (int32_t)q->capacity, (EuclTreeNode*)p, (uint32_t*)(p + node_bytes)};
+    const cudaStream_t stream = s->stream();
+    EUCL_CUDA(cudaMemsetAsync(p, 0, node_bytes + list_bytes, stream));
+    EUCL_CUDA(cudaMemcpyAsync((void*)out->items, items.data(), sizeof(uint32_t) * items.size(), cudaMemcpyHostToDevice, stream));
+    EUCL_CUDA(cudaMemcpyAsync((void*)out->slots, slots.data(), sizeof(uint32_t) * slots.size(), cudaMemcpyHostToDevice, stream));
+    return EUCL_OK;
+}
+
+// After a tree call has rendered (its pipelines joined): the staged nodes and counts to the caller's arrays, then every
+// duplicate slot from the first slot of its item (`order`: the slots sorted by item, stable).
+int read_back_trees(EuclScene* s, const EuclTreeQuery* q, const std::vector<uint32_t>& order, const TreeQuery& tq) {
+    const size_t per_slot = sizeof(EuclTreeNode) * (size_t)q->capacity;
+    EUCL_CUDA(cudaMemcpyAsync(q->nodes, tq.nodes, per_slot * q->n_items, cudaMemcpyDeviceToHost, s->stream()));
+    EUCL_CUDA(cudaMemcpyAsync(q->counts, tq.counts, sizeof(uint32_t) * q->n_items, cudaMemcpyDeviceToHost, s->stream()));
+    EUCL_CUDA(cudaStreamSynchronize(s->stream()));
+    for (size_t k = 1; k < order.size(); ++k) { // a duplicate follows its item's first slot (or an earlier duplicate)
+        const uint32_t prev = order[k - 1], slot = order[k];
+        if (q->items[slot] != q->items[prev]) continue;
+        std::memcpy(q->nodes + (size_t)slot * q->capacity, q->nodes + (size_t)prev * q->capacity, per_slot);
+        q->counts[slot] = q->counts[prev];
+    }
     return EUCL_OK;
 }
 
@@ -1844,19 +1929,50 @@ int eucl_render_aovs_device(EuclScene* s, const EuclFrame* frames, uint32_t n_fr
 
 int eucl_trace_rays(EuclScene* s, const EuclRays* r, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs,
                     EuclStats* stats) {
-    const int st = check_rays(s, r, out_rgb8, "eucl_trace_rays");
+    int st = check_rays(s, r, out_rgb8, "eucl_trace_rays");
     if (st != EUCL_OK) return st;
     EUCL_CUDA(cudaSetDevice(s->device));
-    // staged before the first launch, on pipeline 0's stream and outside any graph capture: a replayed graph reads them
-    const size_t bytes = sizeof(double) * (size_t)s->dim * r->n;
-    EUCL_CUDA(s->ray_stage.ensure(2 * bytes));
-    double* d_o = (double*)s->ray_stage.ptr;
-    double* d_d = (double*)((uint8_t*)s->ray_stage.ptr + bytes);
-    EUCL_CUDA(cudaMemcpyAsync(d_o, r->origins, bytes, cudaMemcpyHostToDevice, s->stream()));
-    EUCL_CUDA(cudaMemcpyAsync(d_d, r->directions, bytes, cudaMemcpyHostToDevice, s->stream()));
+    double *d_o, *d_d;
+    if ((st = stage_rays(s, r, &d_o, &d_d)) != EUCL_OK) return st;
     EuclRenderOpts o;
     const FrameBatch fb = ray_batch(s, r, d_o, d_d, out_hit_ids != nullptr, &o);
     return render_to_host(s, fb, &o, out_rgb8, out_hit_ids, any_plane(aovs), stats);
+}
+
+int eucl_render_trees(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
+                      int32_t* out_hit_ids, const EuclTreeQuery* query, EuclStats* stats) {
+    const char* fn = "eucl_render_trees";
+    int st = n_frames == 1 ? check_args(s, frames ? &frames[0].camera : nullptr, o) : check_frames(s, frames, n_frames, o);
+    if (st != EUCL_OK) return st;
+    if (o->band_world > 1 || o->compact_rows)
+        return fail(EUCL_ERR_INVALID_ARGUMENT, std::string(fn) + ": band-split and compact-row tree calls are not supported");
+    if (!out_rgb8) return fail(EUCL_ERR_INVALID_ARGUMENT, std::string(fn) + ": null output");
+    if ((st = check_tree_query(query, (uint64_t)n_frames * o->height * o->width, fn)) != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    FrameBatch fb;
+    EuclRenderOpts virt;
+    if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
+    std::vector<uint32_t> order;
+    if ((st = stage_tree_query(s, query, &order, &fb.tree)) != EUCL_OK) return st;
+    if ((st = render_to_host(s, fb, &virt, out_rgb8, out_hit_ids, nullptr, stats)) != EUCL_OK) return st;
+    return read_back_trees(s, query, order, fb.tree);
+}
+
+int eucl_trace_ray_trees(EuclScene* s, const EuclRays* r, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclTreeQuery* query,
+                         EuclStats* stats) {
+    const char* fn = "eucl_trace_ray_trees";
+    int st = check_rays(s, r, out_rgb8, fn);
+    if (st != EUCL_OK) return st;
+    if ((st = check_tree_query(query, r->n, fn)) != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    double *d_o, *d_d;
+    if ((st = stage_rays(s, r, &d_o, &d_d)) != EUCL_OK) return st;
+    EuclRenderOpts o;
+    FrameBatch fb = ray_batch(s, r, d_o, d_d, out_hit_ids != nullptr, &o);
+    std::vector<uint32_t> order;
+    if ((st = stage_tree_query(s, query, &order, &fb.tree)) != EUCL_OK) return st;
+    if ((st = render_to_host(s, fb, &o, out_rgb8, out_hit_ids, nullptr, stats)) != EUCL_OK) return st;
+    return read_back_trees(s, query, order, fb.tree);
 }
 
 int eucl_trace_rays_device(EuclScene* s, const EuclRays* r, void* d_out_rgb8, void* d_out_hit_ids, const EuclAovs* d_aovs,

@@ -931,6 +931,144 @@ __global__ void __launch_bounds__(256) k_aov_primary(FrameParams fp, ChunkParams
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// ray-tree export (eucl_render_trees, eucl_trace_ray_trees; DESIGN.md §5.3)
+
+// Request slot of virtual-frame cell `item`, or -1 when the query does not name it: binary search of the sorted items.
+__device__ __forceinline__ int tree_slot(const TreeQuery& tq, uint32_t item) {
+    int lo = 0, hi = tq.n_items;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (tq.items[mid] < item) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo < tq.n_items && tq.items[lo] == item ? (int)tq.slots[lo] : -1;
+}
+
+// One Universe::trace call of an item's tree as the wavefront arena and the megakernel walk both know it.
+template <int D>
+struct TreeRecord {
+    int parent, level, kind, medium, hit;
+    bool exiting, checkerboard;
+    unsigned flags, q;
+    real ratio, t;
+    Vec<D> o, d, n_raw; // n_raw: the intersector's normal (normal_closer = exiting ? -n_raw : n_raw)
+};
+
+// EUCL_TREE_* flags of a node from its shading outcome: `last` = level max_depth, `hit` entity or -1, NODE_* flags,
+// `has_t` = a transmitted child exists.
+__device__ __forceinline__ unsigned tree_flags(bool last, int hit, real ratio, unsigned node_flags, bool has_t) {
+    if (last || hit < 0) return EUCL_TREE_BACKGROUND;
+    unsigned f = 0u;
+    if (!(ratio >= R(1.0))) {
+        f |= EUCL_TREE_SURFACE;
+        if (node_flags & NODE_HAS_SC) f |= EUCL_TREE_OPAQUE;
+        else if (!has_t) f |= EUCL_TREE_NO_DESTINATION;
+    }
+    if (node_flags & NODE_UNDEFINED) f |= EUCL_TREE_UNDEFINED;
+    return f;
+}
+
+// Everything of a node but its colour, widened to double; components beyond D are 0.
+template <int D>
+__device__ __forceinline__ void tree_store(EuclTreeNode* out, const TreeRecord<D>& r) {
+    const double nan = __longlong_as_double(0x7ff8000000000000ll), inf = __longlong_as_double(0x7ff0000000000000ll);
+    const bool hit = r.hit >= 0 && !r.checkerboard;
+    out->parent = r.parent;
+    out->level = r.level;
+    out->kind = r.kind;
+    out->medium = r.checkerboard ? -1 : r.medium;
+    out->hit_entity = hit ? r.hit : -1;
+    out->exiting = hit && r.exiting ? 1 : 0;
+    out->flags = r.checkerboard ? EUCL_TREE_CHECKERBOARD : r.flags;
+    out->surface_rgba8 = r.checkerboard ? 0u : r.q;
+    out->ratio = r.checkerboard ? 0.0 : (double)r.ratio;
+    out->t = r.checkerboard ? nan : (hit ? (double)r.t : inf);
+#pragma unroll
+    for (int k = 0; k < EUCL_MAX_DIM; ++k) {
+        const int j = k < D ? k : 0;
+        const real n = r.exiting ? -r.n_raw[j] : r.n_raw[j];
+        out->origin[k] = k >= D ? 0.0 : (r.checkerboard ? nan : (double)r.o[j]);
+        out->direction[k] = k >= D ? 0.0 : (r.checkerboard ? nan : (double)r.d[j]);
+        out->normal[k] = k >= D ? 0.0 : (hit ? (double)n : nan);
+    }
+}
+__device__ __forceinline__ void tree_store_color(EuclTreeNode* out, const Rgba& c) {
+    out->color[0] = (double)c.r;
+    out->color[1] = (double)c.g;
+    out->color[2] = (double)c.b;
+    out->color[3] = (double)c.a;
+}
+
+// K7 (tree calls only, after the resolve): the trees of the query's items that lie in this chunk, read from the arena, which
+// still holds every level of the chunk.  One thread per item walks its tree depth-first over tchild / rchild with an
+// explicit stack of at most max_depth + 1 entries (the reflected child is pushed first, so the transmitted subtree comes out
+// first: pre-order).  Resolved colours are in `res` for every level but 0, whose colour k_final composes without storing it.
+// Items of other chunks or of another pipeline's bands are skipped: their chunk writes them.
+template <int D>
+__global__ void __launch_bounds__(128) k_tree_export(FrameParams fp, ChunkParams cp, Workspace ws, TreeQuery tq) {
+    __shared__ real s_unit[256];
+    if (*ws.overflow) return; // the chunk is retried with a larger arena and exports then
+    fill_unit_table(s_unit);
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= tq.n_items) return;
+    const uint32_t item = tq.items[u];
+    const int row = (int)(item / (uint32_t)fp.width), x = (int)(item % (uint32_t)fp.width);
+    int local = row; // frame_row_of_local inverted: this pipeline's bands, then the chunk's local rows
+    if (cp.band_world > 1) {
+        const int band = row / cp.band_rows;
+        if (band % cp.band_world != cp.band_rank) return;
+        local = (band / cp.band_world) * cp.band_rows + row % cp.band_rows;
+    }
+    if (local < cp.local_row0 || local >= cp.local_row0 + cp.n_rows) return;
+    EuclTreeNode* out = tq.nodes + (size_t)tq.slots[u] * tq.capacity;
+    int st_node[EUCL_MAX_LEVELS], st_parent[EUCL_MAX_LEVELS], st_level_kind[EUCL_MAX_LEVELS];
+    st_node[0] = (local - cp.local_row0) * fp.width + x;
+    st_parent[0] = -1;
+    st_level_kind[0] = EUCL_TREE_ROOT;
+    int sp = 1;
+    uint32_t count = 0;
+    while (sp > 0) {
+        --sp;
+        const int node = st_node[sp], level = st_level_kind[sp] >> 2;
+        const int idx = (int)count++;
+        const NodeMeta m = ws.meta[node];
+        if (idx < tq.capacity) {
+            TreeRecord<D> r{};
+            r.parent = st_parent[sp];
+            r.level = level;
+            r.kind = st_level_kind[sp] & 3;
+            r.medium = ws.ray_cur[node];
+            r.checkerboard = (m.flags & NODE_FINAL_RGB) != 0;
+            r.hit = -1;
+            r.ratio = m.ratio;
+            r.q = m.q;
+            if (!r.checkerboard) {
+                load_ray<D>(ws, node, r.o, r.d);
+                if (level < fp.max_depth) { // level max_depth: a background lookup, never intersected
+                    const HitHead h = load_hit<D>(ws, node, r.n_raw);
+                    r.hit = h.entity;
+                    r.exiting = h.exiting != 0;
+                    r.t = h.t;
+                }
+                r.flags = tree_flags(level >= fp.max_depth, r.hit, m.ratio, m.flags, m.tchild >= 0);
+            }
+            tree_store<D>(out + idx, r);
+            tree_store_color(out + idx, level == 0 ? node_color(ws, m, node, s_unit) : load_res(ws, node));
+        }
+        const int children[2] = {m.rchild, m.tchild};
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            if (children[k] < 0 || sp >= EUCL_MAX_LEVELS) continue;
+            st_node[sp] = children[k];
+            st_parent[sp] = idx;
+            st_level_kind[sp] = ((level + 1) << 2) | (k == 0 ? EUCL_TREE_REFLECTED : EUCL_TREE_TRANSMITTED);
+            ++sp;
+        }
+    }
+    tq.counts[tq.slots[u]] = count;
+}
+
 // Cross-check pipeline: one thread walks the whole ray tree of its pixel depth-first with an
 // explicit stack (transmitted subtree first, then the reflected one, as the reference recurses).
 constexpr int kMegaMaxDepth = 24;
@@ -946,11 +1084,14 @@ struct MegaFrame {
 // AOV (k_megakernel_aov): also the AOV planes -- the level-0 geometry, and the segments and levels counted along the walk.
 // The cross-check of k_aov_primary and the COST builds of the wavefront.
 // RAYS (k_megakernel_rays*): the caller's rays of eucl_trace_rays* instead of a camera, addressed as in k_raygen_rays.
-template <int D, bool AOV, bool RAYS>
+// TREE (k_megakernel_tree, k_megakernel_rays_tree): also records the walk of the query's items, node by node as it descends
+// (pre-order) and each node's colour once it is known -- the cross-check of k_tree_export.
+template <int D, bool AOV, bool RAYS, bool TREE = false>
 __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ blob, const FrameParams& fp, const ChunkParams& cp,
                                                   const Workspace& ws, uint8_t* __restrict__ out_rgb8,
                                                   int32_t* __restrict__ hit_ids_out, const AovPlanes& aov,
-                                                  const double* __restrict__ origins, const double* __restrict__ directions) {
+                                                  const double* __restrict__ origins, const double* __restrict__ directions,
+                                                  const TreeQuery& tq = TreeQuery{}) {
     const SceneView& sv = stage_scene(blob);
     real* ts = plane_scratch(blob);
     const int cam_entity = *ws.cam_entity;
@@ -961,6 +1102,8 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
         const int x = i % fp.width;
         int y = frame_row_of_local(cp, local_row);
         const size_t opix = (size_t)out_row_of_local(cp, local_row) * fp.width + x;
+        const int slot = TREE ? tree_slot(tq, (uint32_t)y * (uint32_t)fp.width + (uint32_t)x) : -1;
+        EuclTreeNode* const tree_out = TREE && slot >= 0 ? tq.nodes + (size_t)slot * tq.capacity : nullptr;
         int belongs_to = cam_entity, f = 0;
         Vec<D> ray_o, ray_d;
         if (RAYS) {
@@ -976,6 +1119,14 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
             belongs_to = ws.frame_entity[f];
         }
         if (belongs_to < 0) {
+            if (TREE && tree_out) {
+                TreeRecord<D> r{};
+                r.parent = -1;
+                r.checkerboard = true;
+                tree_store<D>(tree_out, r);
+                tree_store_color(tree_out, checkerboard(x, y));
+                tq.counts[slot] = 1u;
+            }
             final_rgb8(checkerboard(x, y), false, out_rgb8 + opix * 3);
             if (hit_ids_out) hit_ids_out[opix] = -2;
             local_counts[0]++;
@@ -1003,6 +1154,10 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
         material_enter<D>(sv, belongs_to, d);
         int cur = belongs_to, level = 0;
         Rgba val{R(0.0), R(0.0), R(0.0), R(0.0)};
+        // TREE: pre-order index of the node open at each level, the kind of the node about to be evaluated, nodes so far
+        int tree_idx[TREE ? kMegaMaxDepth + 1 : 1];
+        int tree_kind = EUCL_TREE_ROOT;
+        uint32_t tree_count = 0u;
         for (;;) {
             // ---- descend: evaluate the node for ray (o, d, cur) at `level`
             bool leaf = true;
@@ -1018,11 +1173,34 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
                 aov_levels = max(aov_levels, (unsigned)level + 1u);
                 if (level == 0) write_primary<D>(aov, opix, true, ent >= 0, t_hit, p, exiting ? -n : n);
             }
+            // TREE: the node, but its colour, from what this step evaluated
+            auto record = [&](real ratio, unsigned q, unsigned node_flags, bool has_t) {
+                const int idx = (int)tree_count++;
+                tree_idx[TREE ? level : 0] = idx;
+                if (idx >= tq.capacity) return;
+                TreeRecord<D> r{};
+                r.parent = level > 0 ? tree_idx[TREE ? level - 1 : 0] : -1;
+                r.level = level;
+                r.kind = tree_kind;
+                r.medium = cur;
+                r.hit = ent;
+                r.exiting = ent >= 0 && exiting;
+                r.flags = tree_flags(level >= fp.max_depth, ent, ratio, node_flags, has_t);
+                r.q = q;
+                r.ratio = ratio;
+                r.t = t_hit;
+                r.o = o;
+                r.d = d;
+                if (ent >= 0) r.n_raw = n;
+                tree_store<D>(tree_out + idx, r);
+            };
             if (ent < 0) {
+                if (TREE && tree_out) record(R(0.0), 0u, NODE_LEAF, false);
                 val = mapped_color<D>(sv, sv.background, d);
             } else {
                 ShadeOut<D> so;
                 shade_hit<D, true>(sv, time_millis, d, cur, ent, exiting, cos_raw, angle_raw, p, n, so);
+                if (TREE && tree_out) record(so.ratio, so.q, so.flags, so.t_emit);
                 if (so.flags & NODE_UNDEFINED) {
                     val = Rgba{R(0.0), R(0.0), R(0.0), R(0.0)};
                     atomicAdd(ws.undefined_count, 1ull);
@@ -1041,6 +1219,7 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
                         f.r = so.r;
                         f.state |= 4u;
                     }
+                    tree_kind = so.t_emit ? EUCL_TREE_TRANSMITTED : EUCL_TREE_REFLECTED;
                     if (so.t_emit) {
                         o = so.t.o;
                         d = so.t.d;
@@ -1059,6 +1238,8 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
             // ---- ascend with `val` until a pending reflected child is found
             bool done = false;
             for (;;) {
+                // `val` is the colour of the node open at `level`
+                if (TREE && tree_out && tree_idx[TREE ? level : 0] < tq.capacity) tree_store_color(tree_out + tree_idx[TREE ? level : 0], val);
                 if (level == 0) {
                     done = true;
                     break;
@@ -1070,6 +1251,7 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
                     f.state |= 2u;
                     if (f.state & 4u) {
                         f.state |= 1u;
+                        tree_kind = EUCL_TREE_REFLECTED;
                         o = f.r.o;
                         d = f.r.d;
                         cur = f.r.cur;
@@ -1088,6 +1270,7 @@ __device__ __forceinline__ void megakernel_pixels(const uint8_t* __restrict__ bl
             if (aov.segments) aov.segments[opix] = aov_segments;
             if (aov.levels) aov.levels[opix] = aov_levels;
         }
+        if (TREE && tree_out) tq.counts[slot] = tree_count;
     }
     for (int l = 0; l <= fp.max_depth && l <= kMegaMaxDepth; ++l) {
         // per-level node counts, warp-reduced
@@ -1122,6 +1305,19 @@ __global__ void __launch_bounds__(kBlock) k_megakernel_rays_aov(const uint8_t* _
                                                                 const double* __restrict__ origins,
                                                                 const double* __restrict__ directions) {
     megakernel_pixels<D, true, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, aov, origins, directions);
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel_tree(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                            Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                            int32_t* __restrict__ hit_ids_out, TreeQuery tq) {
+    megakernel_pixels<D, false, false, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{}, nullptr, nullptr, tq);
+}
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_megakernel_rays_tree(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
+                                                                 Workspace ws, uint8_t* __restrict__ out_rgb8,
+                                                                 int32_t* __restrict__ hit_ids_out, const double* __restrict__ origins,
+                                                                 const double* __restrict__ directions, TreeQuery tq) {
+    megakernel_pixels<D, false, true, true>(blob, fp, cp, ws, out_rgb8, hit_ids_out, AovPlanes{}, origins, directions, tq);
 }
 
 // Universe::trace_path_unknown / trace_path (mod.rs:186-227,273-286) with Surface::get_path
@@ -1352,8 +1548,22 @@ int launch_resolve_and_final(int dim, const Launch& l, const FrameParams& fp, co
 }
 void launch_megakernel(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
                        uint8_t* out_rgb8, int32_t* hit_ids_out, const AovPlanes& aov, const double* origins,
-                       const double* directions) {
+                       const double* directions, const TreeQuery& tree) {
     const int grid = grid_for(cp.n_pixels, kBlock, 1 << 30);
+    if (tree.n_items && origins) {
+        EUCL_DISPATCH_DIM(dim,
+                          (k_megakernel_rays_tree<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                              origins, directions, tree)),
+                          (k_megakernel_rays_tree<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
+                                                                                              origins, directions, tree)));
+        return;
+    }
+    if (tree.n_items) {
+        EUCL_DISPATCH_DIM(
+            dim, (k_megakernel_tree<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, tree)),
+            (k_megakernel_tree<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, tree)));
+        return;
+    }
     const bool want_aov = aov.depth || aov.position || aov.normal || aov.segments || aov.levels;
     if (origins && want_aov) {
         EUCL_DISPATCH_DIM(dim,
@@ -1380,6 +1590,15 @@ void launch_megakernel(int dim, const Launch& l, const FrameParams& fp, const Ch
     EUCL_DISPATCH_DIM(
         dim, (k_megakernel<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)),
         (k_megakernel<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)));
+}
+
+// The trees of the query's items in this chunk (after launch_resolve_and_final, while the arena is intact).  Returns 1.
+int launch_tree_export(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
+                       const TreeQuery& tree) {
+    const int grid = grid_for(tree.n_items, 128, 1 << 30);
+    EUCL_DISPATCH_DIM(dim, (k_tree_export<3><<<grid, 128, 0, l.stream>>>(fp, cp, ws, tree)),
+                      (k_tree_export<4><<<grid, 128, 0, l.stream>>>(fp, cp, ws, tree)));
+    return 1;
 }
 
 void launch_trace_path(int dim, const Launch& l, const double* d_in, double distance, double* d_out, int* d_found) {
@@ -1448,6 +1667,10 @@ cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene) {
     EUCL_CONF(k_megakernel_rays<4>, smem_bytes, heavy);
     EUCL_CONF(k_megakernel_rays_aov<3>, smem_bytes, heavy);
     EUCL_CONF(k_megakernel_rays_aov<4>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_tree<3>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_tree<4>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_rays_tree<3>, smem_bytes, heavy);
+    EUCL_CONF(k_megakernel_rays_tree<4>, smem_bytes, heavy);
     EUCL_CONF(k_trace_path<3>, smem_bytes, 1);
     EUCL_CONF(k_trace_path<4>, smem_bytes, 1);
 #undef EUCL_CONF

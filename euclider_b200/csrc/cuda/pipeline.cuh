@@ -129,6 +129,18 @@ struct AovPlanes {
     uint2* cost;
 };
 
+// Ray-tree export of a tree call (eucl_render_trees, eucl_trace_ray_trees; DESIGN.md §5.3): the device view of the query.
+// The distinct items, sorted, each with the first request slot that names it; the host copies that slot's tree to the
+// slots of its duplicates.  n_items == 0: no tree call (k_tree_export and the TREE megakernels are builds of their own).
+struct TreeQuery {
+    const uint32_t* items; // [n_items] distinct virtual-frame cells, ascending
+    const uint32_t* slots; // [n_items] request slot of each
+    int32_t n_items;
+    int32_t capacity;      // nodes kept per slot
+    EuclTreeNode* nodes;   // [request slots][capacity]
+    uint32_t* counts;      // [request slots] nodes of the whole tree
+};
+
 struct Launch {
     cudaStream_t stream;
     const uint8_t* blob;
@@ -203,7 +215,9 @@ constexpr int kMaxBins = 64; // shade-coherence bins (miss, then kBinsPerEntity 
                                  const eucl::Workspace& ws, uint8_t* out_rgb8, const eucl::AovPlanes& aov);                    \
     void launch_megakernel(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
                            const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out, const eucl::AovPlanes& aov,     \
-                           const double* origins, const double* directions);                                               \
+                           const double* origins, const double* directions, const eucl::TreeQuery& tree);                  \
+    int launch_tree_export(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
+                           const eucl::Workspace& ws, const eucl::TreeQuery& tree);                                        \
     void launch_trace_path(int dim, const eucl::Launch& l, const double* d_in, double distance, double* d_out, int* d_found); \
     cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);                                                       \
     }

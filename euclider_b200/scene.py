@@ -12,13 +12,13 @@ import ctypes as C
 import os
 from dataclasses import dataclass, field
 from pathlib import Path
-from typing import Dict, Mapping, Optional, Sequence, Tuple, Union
+from typing import Dict, List, Mapping, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
 from . import _capi
 from ._capi import (EuclAovs, EuclCamera, EuclError, EuclFlatScene, EuclFrame, EuclRays, EuclRenderOpts, EuclStats,
-                    EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, check, lib)
+                    EuclTreeQuery, EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, check, lib)
 
 ParserError = EuclError  # the reference's `ParserError` (src/scene.rs:524-552); see EuclError.status
 
@@ -44,6 +44,7 @@ class RawImage2d:
     hit_ids: Optional[np.ndarray] = None  # int32 (height, width): primary hit entity, -1 background, -2 checkerboard
     stats: Optional[dict] = None
     aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name (AOV_NAMES), rows as `data`
+    trees: Optional[List["RayTree"]] = None  # requested ray trees, in request order
 
     def to_top_down(self) -> np.ndarray:
         return self.data[::-1]
@@ -68,6 +69,7 @@ class RawFrames:
     hit_ids: Optional[np.ndarray] = None  # int32 (K, height, width), as RawImage2d.hit_ids
     stats: Optional[dict] = None  # summed over the K frames
     aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name, frame k at index k
+    trees: Optional[List["RayTree"]] = None  # requested ray trees, in request order
 
     def __len__(self) -> int:
         return int(self.data.shape[0])
@@ -85,6 +87,7 @@ class RawRays:
     hit_ids: Optional[np.ndarray] = None  # int32 (...): primary hit entity, -1 a miss, -2 an origin in no entity
     stats: Optional[dict] = None
     aovs: Optional[Dict[str, np.ndarray]] = None  # requested AOV planes by name, leading shape as `data`
+    trees: Optional[List["RayTree"]] = None  # requested ray trees, in request order
 
 
 def equirect_rays(camera: EuclCamera, width: int, height: int) -> Tuple[np.ndarray, np.ndarray]:
@@ -185,6 +188,92 @@ def _device_aovs(d_aovs: Mapping[str, int]) -> EuclAovs:
     return _aov_struct(d_aovs)
 
 
+# Ray-tree nodes (include/euclider_b200.h, EuclTreeNode): the C layout, 176 bytes.
+TREE_NODE_DTYPE = np.dtype([("parent", "<i4"), ("level", "<i4"), ("kind", "<i4"), ("medium", "<i4"), ("hit_entity", "<i4"),
+                            ("exiting", "<i4"), ("flags", "<u4"), ("surface_rgba8", "<u4"), ("ratio", "<f8"), ("t", "<f8"),
+                            ("origin", "<f8", (4,)), ("direction", "<f8", (4,)), ("normal", "<f8", (4,)), ("color", "<f8", (4,))])
+TREE_KINDS = ("root", "transmitted", "reflected")
+TREE_FLAGS = (("background", _capi.EUCL_TREE_BACKGROUND), ("surface", _capi.EUCL_TREE_SURFACE), ("opaque", _capi.EUCL_TREE_OPAQUE),
+              ("no_destination", _capi.EUCL_TREE_NO_DESTINATION), ("undefined", _capi.EUCL_TREE_UNDEFINED),
+              ("checkerboard", _capi.EUCL_TREE_CHECKERBOARD))
+
+
+@dataclass
+class RayTree:
+    """The ray tree behind one pixel or ray: one node per Universe::trace call, in pre-order (a node, its transmitted
+    subtree, its reflected subtree).  Field meanings are those of EuclTreeNode in include/euclider_b200.h."""
+    nodes: np.ndarray  # TREE_NODE_DTYPE: the first min(count, capacity) nodes
+    count: int         # nodes of the whole tree
+    dim: int
+    precision: str = "f64"  # the scene's real: every float field holds a value of this type
+
+    @property
+    def truncated(self) -> bool:
+        return self.count > len(self.nodes)
+
+    def children(self, j: int) -> List[int]:
+        """Indices of node j's stored children: the transmitted one first, then the reflected one."""
+        return [int(i) for i in np.flatnonzero(self.nodes["parent"] == int(j))]
+
+    def locations(self) -> np.ndarray:
+        """Hit locations o + d * t in the scene's precision (the intersectors' expression), (n, dim) float64; NaN where a
+        node has no hit."""
+        ft = np.float32 if self.precision == "f32" else np.float64
+        o = self.nodes["origin"][:, :self.dim].astype(ft)
+        d = self.nodes["direction"][:, :self.dim].astype(ft)
+        t = self.nodes["t"].astype(ft)[:, None]
+        with np.errstate(invalid="ignore", over="ignore"):
+            p = (o + d * t).astype(np.float64)
+        p[self.nodes["hit_entity"] < 0] = np.nan
+        return p
+
+    def format(self) -> str:
+        """An indented text view, one line per node."""
+        lines = []
+        for j, nd in enumerate(self.nodes):
+            flags = "|".join(name for name, bit in TREE_FLAGS if int(nd["flags"]) & bit) or "-"
+            what = f"hit {int(nd['hit_entity'])} t={float(nd['t']):.6g}" if nd["hit_entity"] >= 0 else "miss"
+            if nd["hit_entity"] >= 0:
+                what += f" {'exiting' if nd['exiting'] else 'entering'} ratio={float(nd['ratio']):.4g}"
+            if int(nd["flags"]) & _capi.EUCL_TREE_SURFACE:
+                what += f" surface=#{int(nd['surface_rgba8']):08x}"
+            rgba = ", ".join(f"{float(c):.4f}" for c in nd["color"])
+            lines.append(f"{'  ' * int(nd['level'])}[{j}] {TREE_KINDS[int(nd['kind'])]} level {int(nd['level'])} "
+                         f"in {int(nd['medium'])}: {what} [{flags}] colour ({rgba})")
+        if self.truncated:
+            lines.append(f"... {self.count - len(self.nodes)} more nodes (capacity {len(self.nodes)})")
+        return "\n".join(lines)
+
+
+def default_tree_capacity(max_depth: int) -> int:
+    """Nodes kept per tree unless asked otherwise: a full binary tree of max_depth + 1 levels, at most 4096."""
+    return min(2 ** (int(max_depth) + 1) - 1, 4096)
+
+
+def _tree_query(items: Sequence[int], capacity: int):
+    """EuclTreeQuery over host arrays, and the arrays (kept alive by the caller): items, nodes, counts."""
+    items = np.ascontiguousarray(items, dtype=np.uint32)
+    capacity = int(capacity)
+    if capacity < 1:
+        raise ValueError("tree_capacity must be at least 1")
+    if not 1 <= len(items) <= _capi.EUCL_TREE_MAX_ITEMS:
+        raise ValueError(f"trees: 1 .. {_capi.EUCL_TREE_MAX_ITEMS} items")
+    if len(items) * capacity > _capi.EUCL_TREE_MAX_NODES:
+        raise ValueError(f"trees: {len(items)} items x capacity {capacity} exceed {_capi.EUCL_TREE_MAX_NODES} nodes")
+    nodes = np.zeros((len(items), capacity), TREE_NODE_DTYPE)
+    counts = np.zeros(len(items), np.uint32)
+    query = EuclTreeQuery(items=items.ctypes.data, n_items=len(items), capacity=capacity, nodes=nodes.ctypes.data,
+                          counts=counts.ctypes.data)
+    return query, (items, nodes, counts)
+
+
+def _cell(value, extent: int, what: str) -> int:
+    v = int(value)
+    if not 0 <= v < extent:
+        raise ValueError(f"tree {what} {v} out of range 0 .. {extent - 1}")
+    return v
+
+
 def _frame_table(cameras: Sequence[EuclCamera], times) -> C.Array:
     """EuclFrame[K] from K cameras and a time per frame (or one time for all)."""
     cameras = list(cameras)
@@ -246,14 +335,18 @@ class Environment:
     def render(self, dimensions: Tuple[int, int], time: float = 0.0, threads: int = 0,
                context: Optional[SimulationContext] = None, *, device: int = 0, want_hit_ids: bool = False,
                band_rows: int = 0, band_rank: int = 0, band_world: int = 1, out: Optional[np.ndarray] = None,
-               profile: bool = False, aovs=None) -> RawImage2d:
+               profile: bool = False, aovs=None, trees: Optional[Sequence[Tuple[int, int]]] = None,
+               tree_capacity: Optional[int] = None) -> RawImage2d:
         """Environment::render.  `time` is seconds since start (the reference passes a Duration);
         `threads` is accepted for signature parity and ignored (the GPU schedules the pixels).
         `aovs`: per-pixel auxiliary planes to return in `.aovs` (names from AOV_NAMES, or a mapping name -> array to
-        render into); the frame, hit ids and stats are the same with or without them."""
+        render into); the frame, hit ids and stats are the same with or without them.
+        `trees`: pixels (x, y), row 0 at the bottom, whose ray trees to return in `.trees` (RayTree, in request order),
+        keeping up to `tree_capacity` nodes each (default: default_tree_capacity(max_depth)); not with `aovs`."""
         del threads
         context = context or SimulationContext()
         width, height = int(dimensions[0]) // context.resolution, int(dimensions[1]) // context.resolution
+        items = self._tree_items(trees, aovs, lambda c: _cell(c[1], height, "y") * width + _cell(c[0], width, "x"))
         opts = EuclRenderOpts(width=width, height=height, time_seconds=float(time), band_rows=band_rows,
                               band_rank=band_rank, band_world=band_world, pipeline=self.pipeline, compact_rows=0,
                               want_hit_ids=int(want_hit_ids), profile=int(profile))
@@ -263,15 +356,22 @@ class Environment:
         hit = np.full((height, width), -3, dtype=np.int32) if want_hit_ids else None
         planes = _aov_arrays(aovs, (height, width), self.dim) if aovs else None
         stats = EuclStats()
+        result = None
         if planes:
             table = _frame_table([self.camera], float(time))
             check(lib().eucl_render_aovs(self._device_scene(device), table, 1, C.byref(opts), out.ctypes.data,
                                          hit.ctypes.data if hit is not None else None,
                                          C.byref(_aov_struct({n: a.ctypes.data for n, a in planes.items()})), C.byref(stats)))
+        elif items is not None:
+            query, result = _tree_query(items, self._tree_capacity(tree_capacity, self.camera.max_depth))
+            check(lib().eucl_render_trees(self._device_scene(device), _frame_table([self.camera], float(time)), 1, C.byref(opts),
+                                          out.ctypes.data, hit.ctypes.data if hit is not None else None, C.byref(query),
+                                          C.byref(stats)))
         else:
             check(lib().eucl_render(self._device_scene(device), C.byref(self.camera), C.byref(opts), out.ctypes.data,
                                     hit.ctypes.data if hit is not None else None, C.byref(stats)))
-        return RawImage2d(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
+        return RawImage2d(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes,
+                          trees=self._ray_trees(result))
 
     # -- device-resident variant (inputs and outputs stay in HBM) --------------------------------
     def render_device(self, d_out_rgb8: int, dimensions: Tuple[int, int], time: float = 0.0, *, device: int = 0,
@@ -298,15 +398,19 @@ class Environment:
     # -- many frames per call: camera paths and animations -------------------------------------------
     def render_frames(self, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera], times=0.0,
                       context: Optional[SimulationContext] = None, *, device: int = 0, want_hit_ids: bool = False,
-                      out: Optional[np.ndarray] = None, profile: bool = False, aovs=None) -> RawFrames:
+                      out: Optional[np.ndarray] = None, profile: bool = False, aovs=None,
+                      trees: Optional[Sequence[Tuple[int, int, int]]] = None, tree_capacity: Optional[int] = None) -> RawFrames:
         """Renders one frame per camera pose in ONE call (eucl_render_frames): frame k equals
         `render(dimensions, times[k])` with `self.camera` set to `cameras[k]`, bit for bit.  `times` is one time for
         every frame or a sequence of one per frame.  Batching pays the fixed cost of a frame once per call.
-        `aovs` as for `render`; plane k of the result belongs to frame k."""
+        `aovs` as for `render`; plane k of the result belongs to frame k.  `trees`: pixels (k, x, y) of frame k, as for
+        `render`."""
         table = _frame_table(cameras, times)
         context = context or SimulationContext()
         width, height = int(dimensions[0]) // context.resolution, int(dimensions[1]) // context.resolution
         k = len(table)
+        items = self._tree_items(trees, aovs, lambda c: ((_cell(c[0], k, "frame") * height + _cell(c[2], height, "y")) * width
+                                                         + _cell(c[1], width, "x")))
         if out is None:
             out = np.zeros((k, height, width, 3), dtype=np.uint8)
         if out.dtype != np.uint8 or out.shape != (k, height, width, 3) or not out.flags["C_CONTIGUOUS"]:
@@ -316,14 +420,19 @@ class Environment:
         hit = np.full((k, height, width), -3, dtype=np.int32) if want_hit_ids else None
         planes = _aov_arrays(aovs, (k, height, width), self.dim) if aovs else None
         stats = EuclStats()
+        result = None
         if planes:
             check(lib().eucl_render_aovs(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
                                          hit.ctypes.data if hit is not None else None,
                                          C.byref(_aov_struct({n: a.ctypes.data for n, a in planes.items()})), C.byref(stats)))
+        elif items is not None:
+            query, result = _tree_query(items, self._tree_capacity(tree_capacity, table[0].camera.max_depth))
+            check(lib().eucl_render_trees(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
+                                          hit.ctypes.data if hit is not None else None, C.byref(query), C.byref(stats)))
         else:
             check(lib().eucl_render_frames(self._device_scene(device), table, k, C.byref(opts), out.ctypes.data,
                                            hit.ctypes.data if hit is not None else None, C.byref(stats)))
-        return RawFrames(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
+        return RawFrames(out, width, height, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes, trees=self._ray_trees(result))
 
     def render_frames_device(self, d_out_rgb8: int, dimensions: Tuple[int, int], cameras: Sequence[EuclCamera],
                              times=0.0, *, device: int = 0, d_out_hit_ids: int = 0, profile: bool = False,
@@ -349,15 +458,20 @@ class Environment:
     # -- caller-supplied rays: custom projections, picking, probes -----------------------------------
     def trace_rays(self, origins, directions, time: float = 0.0, *, max_depth: Optional[int] = None,
                    width: Optional[int] = None, device: int = 0, want_hit_ids: bool = True, aovs=None,
-                   out: Optional[np.ndarray] = None, profile: bool = False) -> RawRays:
+                   out: Optional[np.ndarray] = None, profile: bool = False, trees=None,
+                   tree_capacity: Optional[int] = None) -> RawRays:
         """Traces one ray per origin / direction pair (eucl_trace_rays): arrays of shape (..., dim), converted to
         float64.  Directions are used as given (not normalised).  Ray i gives what a pixel whose camera ray is
         (origins[i], directions[i]) gives -- its RGB8 value, primary hit and AOV planes -- and an origin in no entity gives
         the checkerboard of grid cell (i % width, i // width).  `width` (rays per grid row) defaults to the last leading
         dimension of an (H, W, dim) grid and to 1 for a flat (N, dim) list; `max_depth` to the camera's.  Tracing the
-        camera's own rays of a w x h frame with width w reproduces `render((w, h), time)` bit for bit."""
+        camera's own rays of a w x h frame with width w reproduces `render((w, h), time)` bit for bit.
+        `trees`: rays whose ray trees to return in `.trees` (RayTree, in request order), each a flat ray index or an index
+        tuple into the rays' leading shape; `tree_capacity` as for `render`; not with `aovs`."""
         o, d, lead = _ray_arrays(origins, directions, self.dim)
         n = int(np.prod(lead, dtype=np.int64))
+        items = self._tree_items(trees, aovs, lambda c: (int(np.ravel_multi_index(tuple(int(v) for v in c), lead))
+                                                         if isinstance(c, (tuple, list)) else _cell(c, n, "ray index")))
         if width is None:
             width = lead[-1] if len(lead) >= 2 else 1
         rays = _ray_struct(n, width, self.camera.max_depth if max_depth is None else max_depth, self.pipeline, time, profile,
@@ -369,10 +483,16 @@ class Environment:
         hit = np.full(lead, -3, dtype=np.int32) if want_hit_ids else None
         planes = _aov_arrays(aovs, lead, self.dim) if aovs else None
         stats = EuclStats()
-        aov = C.byref(_aov_struct({k: a.ctypes.data for k, a in planes.items()})) if planes else None
-        check(lib().eucl_trace_rays(self._device_scene(device), C.byref(rays), out.ctypes.data,
-                                    hit.ctypes.data if hit is not None else None, aov, C.byref(stats)))
-        return RawRays(out, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes)
+        result = None
+        if items is not None:
+            query, result = _tree_query(items, self._tree_capacity(tree_capacity, rays.max_depth))
+            check(lib().eucl_trace_ray_trees(self._device_scene(device), C.byref(rays), out.ctypes.data,
+                                             hit.ctypes.data if hit is not None else None, C.byref(query), C.byref(stats)))
+        else:
+            aov = C.byref(_aov_struct({k: a.ctypes.data for k, a in planes.items()})) if planes else None
+            check(lib().eucl_trace_rays(self._device_scene(device), C.byref(rays), out.ctypes.data,
+                                        hit.ctypes.data if hit is not None else None, aov, C.byref(stats)))
+        return RawRays(out, hit_ids=hit, stats=stats_to_dict(stats), aovs=planes, trees=self._ray_trees(result))
 
     def trace_rays_device(self, d_origins: int, d_directions: int, n: int, d_out_rgb8: int, time: float = 0.0, *,
                           max_depth: Optional[int] = None, width: int = 1, device: int = 0, d_out_hit_ids: int = 0,
@@ -437,6 +557,30 @@ class Environment:
         check(lib().eucl_camera_rotate_plane4(C.byref(self.camera), int(axis_a), int(axis_b), float(angle)))
 
     # -- plumbing ----------------------------------------------------------------------------------
+    @staticmethod
+    def _tree_items(trees, aovs, item_of) -> Optional[List[int]]:
+        """The virtual-frame cells of the requested trees (None: no tree call); ValueError with AOVs or for an empty or
+        out-of-range request."""
+        if trees is None:
+            return None
+        if aovs:
+            raise ValueError("trees and aovs cannot be asked for in one call")
+        items = [item_of(c) for c in trees]
+        if not items:
+            raise ValueError("trees names no item")
+        return items
+
+    @staticmethod
+    def _tree_capacity(tree_capacity: Optional[int], max_depth: int) -> int:
+        return default_tree_capacity(max_depth) if tree_capacity is None else int(tree_capacity)
+
+    def _ray_trees(self, result) -> Optional[List[RayTree]]:
+        if result is None:
+            return None
+        _, nodes, counts = result
+        cap = nodes.shape[1]
+        return [RayTree(nodes[i, :min(int(c), cap)], int(c), self.dim, self.precision) for i, c in enumerate(counts)]
+
     @property
     def flat(self) -> EuclFlatScene:
         return lib().eucl_parsed_flat(self._parsed).contents

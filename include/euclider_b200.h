@@ -430,6 +430,63 @@ int eucl_trace_rays(EuclScene* scene, const EuclRays* rays, uint8_t* out_rgb8, i
 int eucl_trace_rays_device(EuclScene* scene, const EuclRays* rays, void* d_out_rgb8, void* d_out_hit_ids,
                            const EuclAovs* d_aovs, EuclStats* stats);
 
+/* Ray-tree inspection: the whole ray tree behind chosen pixels or rays, node by node.  An ITEM is one cell of a call's
+ * virtual frame: row * width + x for a camera call (row 0 at the bottom; frame k of a batch uses rows k*height + y), the
+ * ray index for a ray call.  The item's TREE lists the Universe::trace calls made for it (mod.rs:149-184), one node per
+ * call, in PRE-ORDER: a node, then its transmitted subtree, then its reflected subtree -- the order in which the reference
+ * evaluates them (get_intersection_color before get_reflection_color, surface.rs:144-162).  Float fields hold the scene's
+ * real widened to double (an f32 scene gives f32 values).  Two rules tie a tree to the other outputs: the root colour
+ * composited over opaque white and quantised is the pixel, and the nodes with level < max_depth are the pixel's
+ * `segments` AOV (largest level + 1: its `levels`). */
+#define EUCL_TREE_ROOT 0
+#define EUCL_TREE_TRANSMITTED 1
+#define EUCL_TREE_REFLECTED 2
+
+#define EUCL_TREE_BACKGROUND 1u     /* colour = background.get_color(direction): a miss, or level == max_depth */
+#define EUCL_TREE_SURFACE 2u        /* the surface colour was evaluated (a hit with ratio < 1) */
+#define EUCL_TREE_OPAQUE 4u         /* the surface colour's alpha quantises to 255: it is the transmitted term, no transmitted ray */
+#define EUCL_TREE_NO_DESTINATION 8u /* no transmitted ray: its origin lies in no entity */
+#define EUCL_TREE_UNDEFINED 16u     /* neither term exists (the reference would panic): transparent black */
+#define EUCL_TREE_CHECKERBOARD 32u  /* root of an item whose origin lies in no entity: origin, direction, normal and t are NaN */
+
+typedef struct EuclTreeNode {
+    int32_t parent;         /* index in this item's list; -1 for the root */
+    int32_t level;          /* 0 = primary ray; a node at level max_depth is a background lookup, never intersected */
+    int32_t kind;           /* EUCL_TREE_ROOT, EUCL_TREE_TRANSMITTED, EUCL_TREE_REFLECTED */
+    int32_t medium;         /* entity the ray travels in (trace's belongs_to); -1 for a checkerboard root */
+    int32_t hit_entity;     /* entity of the closest hit, -1 none */
+    int32_t exiting;        /* 1: normal_closer = -normal */
+    uint32_t flags;         /* EUCL_TREE_* flags */
+    uint32_t surface_rgba8; /* to_pixel4(surface colour), r | g<<8 | b<<16 | a<<24; valid with EUCL_TREE_SURFACE, else 0 */
+    double ratio;           /* clamped reflection ratio; 0 without a hit */
+    double t;               /* hit distance; +inf without a hit; NaN for a checkerboard root */
+    double origin[EUCL_MAX_DIM], direction[EUCL_MAX_DIM]; /* the ray as traced (after material transitions) */
+    double normal[EUCL_MAX_DIM]; /* normal_closer; NaN without a hit */
+    double color[4];        /* what Universe::trace returns for this node (RGBA); root: before compositing over white */
+} EuclTreeNode;             /* 176 bytes */
+
+#define EUCL_TREE_MAX_ITEMS 65536u
+#define EUCL_TREE_MAX_NODES (1u << 24) /* n_items * capacity: 2816 MiB of nodes (4096 items of a full depth-10 tree fit) */
+
+typedef struct EuclTreeQuery {
+    const uint32_t* items; /* [n_items]; duplicates allowed */
+    uint32_t n_items;      /* 1 .. EUCL_TREE_MAX_ITEMS */
+    uint32_t capacity;     /* nodes kept per item, >= 1 */
+    EuclTreeNode* nodes;   /* [n_items][capacity], host */
+    uint32_t* counts;      /* [n_items]: nodes in the whole tree; > capacity = truncated to the first `capacity` in pre-order */
+} EuclTreeQuery;           /* 32 bytes */
+
+/* eucl_render_frames (n_frames == 1: eucl_render of frames[0]) and eucl_trace_rays that also export the trees of
+ * query->items.  HOST buffers, synchronous.  The RGB8 output, the hit ids and the counted EuclStats equal the plain call's;
+ * `launches` includes the export kernels.  A tree call is never captured or replayed as a CUDA graph and leaves the plain
+ * calls' graphs alone, and it never feeds the ray-grouping tuner.  EUCL_ERR_INVALID_ARGUMENT, before any device work, for
+ * a null or empty query, null items, nodes or counts, capacity 0, an item outside the virtual frame, n_items * capacity
+ * above EUCL_TREE_MAX_NODES, band_world > 1 or compact_rows, and everything the plain entry point rejects. */
+int eucl_render_trees(EuclScene* scene, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* opts,
+                      uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclTreeQuery* query, EuclStats* stats);
+int eucl_trace_ray_trees(EuclScene* scene, const EuclRays* rays, uint8_t* out_rgb8, int32_t* out_hit_ids,
+                         const EuclTreeQuery* query, EuclStats* stats);
+
 /* Universe::trace_path_unknown (src/universe/mod.rs:273-286): moves `location` by `distance` along
  * `direction` THROUGH the universe -- surfaces are crossed with the material transitions of the
  * entities on either side, so a step through a LinearSpace void is stretched or shrunk.  The

@@ -19,8 +19,16 @@ A 360 x 180 degree panorama of the camera's position with --projection equirect 
 euclider_b200.equirect_rays; the centre column looks forward).  The default, perspective, is the camera's own projection.
 
     python tools/eucl_render.py assets/scenes/3d_room.json pano.png --size 2048 1024 --projection equirect
+
+The ray tree behind chosen pixels with --inspect X,Y (repeatable; `center` is the pixel (width / 2, height / 2), the
+reference's debug pixel): every Universe::trace call of the pixel, printed as an indented tree and written to
+`out.tree_X_Y.json` (the nodes of EuclTreeNode, include/euclider_b200.h; pixel (X, Y) with row 0 at the bottom).  Single
+frames only, perspective or equirect, and not together with --aov.
+
+    python tools/eucl_render.py assets/scenes/3d_room.json out.png --size 640 360 --inspect center --inspect 100,40
 """
 import argparse
+import json
 import os
 import sys
 from pathlib import Path
@@ -59,6 +67,8 @@ def parse_args(argv=None):
     seq.add_argument("--time-step", type=float, default=0.0, help="seconds added to the time per frame")
     ap.add_argument("--aov", type=aov_list, default=[], metavar="P,Q,..",
                     help=f"also write these per-pixel planes, from {','.join(eb.AOV_NAMES)}")
+    ap.add_argument("--inspect", type=inspect_spec, action="append", default=[], metavar="X,Y|center",
+                    help="print the ray tree of this pixel and write it to out.tree_X_Y.json (repeatable)")
     args = ap.parse_args(argv)
     if args.frames < 1:
         ap.error("--frames must be at least 1")
@@ -72,7 +82,52 @@ def parse_args(argv=None):
         ap.error("--frames > 1 needs an output pattern such as out_%04d.ppm")
     if args.projection != "perspective" and is_sequence(args):
         ap.error("--projection equirect renders single frames only")
+    if args.inspect and is_sequence(args):
+        ap.error("--inspect works on single frames only")
+    if args.inspect and args.aov:
+        ap.error("--inspect and --aov cannot be used together")
     return args
+
+
+def inspect_spec(text: str):
+    """`center` or `X,Y` (integers)."""
+    if text == "center":
+        return text
+    try:
+        x, y = (int(v) for v in text.split(","))
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"--inspect takes X,Y or center, not {text!r}") from None
+    return (x, y)
+
+
+def inspect_pixels(specs, width: int, height: int) -> list:
+    return [(width // 2, height // 2) if s == "center" else s for s in specs]
+
+
+def tree_to_json(tree: "eb.RayTree", pixel) -> dict:
+    fields = eb.TREE_NODE_DTYPE.names
+    nodes = [{f: (nd[f][:tree.dim].tolist() if nd[f].ndim else nd[f].item()) if f in ("origin", "direction", "normal")
+              else (nd[f].tolist() if nd[f].ndim else nd[f].item()) for f in fields} for nd in tree.nodes]
+    return {"pixel": list(pixel), "count": tree.count, "truncated": tree.truncated, "precision": tree.precision, "nodes": nodes}
+
+
+def tree_from_json(doc: dict, dim: int) -> "eb.RayTree":
+    nodes = np.zeros(len(doc["nodes"]), eb.TREE_NODE_DTYPE)
+    for j, nd in enumerate(doc["nodes"]):
+        for f, v in nd.items():
+            if f in ("origin", "direction", "normal"):
+                nodes[j][f][:dim] = v
+            else:
+                nodes[j][f] = v
+    return eb.RayTree(nodes, int(doc["count"]), dim, doc.get("precision", "f64"))
+
+
+def write_trees(image_path: str, pixels, trees) -> None:
+    for (x, y), tree in zip(pixels, trees):
+        print(f"pixel ({x}, {y}): {tree.count} nodes")
+        print(tree.format())
+        with open(aov_path(image_path, f"tree_{x}_{y}", ".json"), "w") as f:
+            json.dump(tree_to_json(tree, (x, y)), f, indent=1)
 
 
 def aov_list(text: str) -> list:
@@ -140,18 +195,25 @@ def main(argv=None):
     context = eb.SimulationContext(resolution=args.resolution)
     if args.projection == "equirect":
         w, h = args.size[0] // args.resolution, args.size[1] // args.resolution
-        res = env.trace_rays(*eb.equirect_rays(env.camera, w, h), args.time, want_hit_ids=False, aovs=args.aov or None)
+        pixels = inspect_pixels(args.inspect, w, h)
+        res = env.trace_rays(*eb.equirect_rays(env.camera, w, h), args.time, want_hit_ids=False, aovs=args.aov or None,
+                             trees=[(y, x) for x, y in pixels] if pixels else None)
         eb.RawImage2d(res.data, w, h).save(args.output)
         if args.aov:
             write_aovs(args.output, res.aovs)
+        if pixels:
+            write_trees(args.output, pixels, res.trees)
         st = res.stats
         print(f"{args.output}: {w}x{h} equirect, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
         return
     if not is_sequence(args):
-        img = env.render(tuple(args.size), args.time, context=context, aovs=args.aov or None)
+        pixels = inspect_pixels(args.inspect, args.size[0] // args.resolution, args.size[1] // args.resolution)
+        img = env.render(tuple(args.size), args.time, context=context, aovs=args.aov or None, trees=pixels or None)
         img.save(args.output)
         if args.aov:
             write_aovs(args.output, img.aovs)
+        if pixels:
+            write_trees(args.output, pixels, img.trees)
         st = img.stats
         print(f"{args.output}: {img.width}x{img.height}, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
         return
