@@ -35,9 +35,6 @@ using namespace eucl;
                         std::string(#expr) + ": " + cudaGetErrorString(_e));                              \
     } while (0)
 
-// the launcher of the scene's precision: namespace eucl holds the f64 build of kernels.cu, eucl_f32 the f32 build
-#define EUCL_PREC(fn) (s->real_bytes == 4 ? eucl_f32::fn : eucl::fn)
-
 // pipelines a rank's share of a frame is rendered as (render_split); EUCL_SPLIT overrides
 #ifndef EUCL_SPLIT_DEFAULT
 #define EUCL_SPLIT_DEFAULT 2
@@ -193,6 +190,7 @@ struct EuclScene {
     int warm_frames = 0;         // frames rendered so far
     int n_entities = 0;
     int real_bytes = 8;        // 8: f64 kernels (the reference's default `type F = f64`); 4: f32 kernels (`low_precision`)
+    const Kernels* k = nullptr; // the launchers of the build of that precision, for this scene's dimension
     std::vector<std::unique_ptr<Pipeline>> pipes; // [0] always exists; render_split adds the others
     std::vector<std::unique_ptr<Worker>> workers; // one host thread per pipeline after the first
     cudaEvent_t ev_split[3] = {nullptr, nullptr, nullptr}; // a split frame: start (timed), fork, end (timed)
@@ -728,8 +726,10 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     EUCL_CUDA(cudaSetDevice(device));
     auto s = std::make_unique<EuclScene>(); // freed with everything it holds on any early return
     s->device = device;
-    s->real_bytes = precision == EUCL_PRECISION_F32 ? 4 : 8;
+    const bool f32 = precision == EUCL_PRECISION_F32;
+    s->real_bytes = f32 ? 4 : 8;
     s->dim = flat->dim;
+    s->k = f32 ? &eucl_f32::kernels(s->dim) : &eucl::kernels(s->dim);
     s->n_entities = flat->n_entities;
     cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device);
     status = add_pipeline(s.get());
@@ -917,7 +917,8 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
                                               " B) exceed the shared memory of one CTA (" + std::to_string(smem_optin) + " B)");
     EUCL_CUDA(s->blob.ensure(w.bytes.size()));
     EUCL_CUDA(cudaMemcpy(s->blob.ptr, w.bytes.data(), w.bytes.size(), cudaMemcpyHostToDevice));
-    EUCL_CUDA(EUCL_PREC(configure_kernels)(s->smem_bytes, s->smem_scene));
+    const auto configure_kernels = f32 ? eucl_f32::configure_kernels : eucl::configure_kernels;
+    EUCL_CUDA(configure_kernels(s->smem_bytes, s->smem_scene));
     *out = s.release();
     return EUCL_OK;
 }
@@ -1003,6 +1004,7 @@ struct FrameBatch {
     const double* ray_origins;     // rays: [n][dim] each; null for camera frames
     const double* ray_directions;
     TreeQuery tree;                // a tree call: the items whose trees the chunks export (n_items 0: none)
+    AovPlanes aov;                 // the device planes the call writes (null = not wanted); `cost` stays null here
 };
 
 // The batch of `n` camera frames (arguments checked) and `virt`, the virtual frame they form.  K > 1: the frame constants
@@ -1241,7 +1243,7 @@ struct ChunkLaunch {
     Launch l;
     ChunkParams cp;
     Workspace ws;
-    AovPlanes aov; // the planes a chunk writes (null = not wanted) and the cost buffer
+    uint2* cost;   // the pipeline's per-node (segments, levels) buffer when the call wants either (AovPlanes::cost)
     uint8_t* d_rgb;
     int32_t* d_hit;
 };
@@ -1259,8 +1261,9 @@ struct ChunkDebug {
 // Everything one chunk puts on the stream: counters reset, kernels, counters back to the pinned mirror.  Returns the
 // number of kernels.
 uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c, ChunkDebug& dbg) {
-    const int dim = s->dim;
     const FrameBatch& fb = c.fb;
+    AovPlanes aov = fb.aov;
+    aov.cost = c.cost;
     const Launch& l = c.l;
     auto mark = [&](int family) {
         if (!dbg.profile) return;
@@ -1288,28 +1291,27 @@ uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c,
     mark(-1);
     if (c.pipeline == EUCL_PIPELINE_MEGAKERNEL) {
         if (!fb.ray_origins) {
-            EUCL_PREC(launch_camera_entity)(dim, l, fb.fp, c.ws);
+            s->k->camera_entity(l, fb.fp, c.ws);
             check("k_camera_entity", 0);
             launches += 1;
         }
-        EUCL_PREC(launch_megakernel)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.d_hit, c.aov, fb.ray_origins, fb.ray_directions, fb.tree);
+        s->k->megakernel(l, fb.fp, c.cp, c.ws, c.d_rgb, c.d_hit, aov, fb.ray_origins, fb.ray_directions, fb.tree);
         mark(1);
         launches += 1;
     } else {
         if (c.ws.frames) {
-            EUCL_PREC(launch_camera_entity)(dim, l, fb.fp, c.ws);
+            s->k->camera_entity(l, fb.fp, c.ws);
             check("k_camera_entity", 0);
             launches += 1;
         }
-        if (fb.ray_origins) EUCL_PREC(launch_raygen_rays)(dim, l, fb.fp, c.cp, c.ws, c.d_hit, fb.ray_origins, fb.ray_directions);
-        else EUCL_PREC(launch_raygen)(dim, l, fb.fp, c.cp, c.ws, c.d_hit);
+        s->k->raygen(l, fb.fp, c.cp, c.ws, c.d_hit, fb.ray_origins, fb.ray_directions);
         check("k_raygen", 0);
         mark(0);
         for (int level = 0; level < (int)fb.max_depth; ++level) {
-            launches += EUCL_PREC(launch_intersect)(dim, l, c.ws, level);
+            launches += s->k->intersect(l, c.ws, level);
             check("k_intersect", level);
             mark(1);
-            launches += EUCL_PREC(launch_shade)(dim, l, fb.fp, c.cp, c.ws, level, c.d_hit);
+            launches += s->k->shade(l, fb.fp, c.cp, c.ws, level, c.d_hit);
             check("k_shade", level);
             mark(2);
         }
@@ -1317,13 +1319,13 @@ uint32_t enqueue_chunk(const EuclScene* s, Pipeline& pipe, const ChunkLaunch& c,
         // finishing them inside k_shade of the level above, from the child direction in registers (one launch
         // and one ray record per node less, but the lookups then run at the heavy kernel's occupancy:
         // 3d_room shade 7.14 + 0.47 -> 7.34 + 0.67 ms)
-        launches += EUCL_PREC(launch_shade)(dim, l, fb.fp, c.cp, c.ws, (int)fb.max_depth, c.d_hit);
+        launches += s->k->shade(l, fb.fp, c.cp, c.ws, (int)fb.max_depth, c.d_hit);
         check("k_shade", (int)fb.max_depth);
         mark(2);
-        launches += EUCL_PREC(launch_resolve_and_final)(dim, l, fb.fp, c.cp, c.ws, c.d_rgb, c.aov);
+        launches += s->k->resolve_and_final(l, fb.fp, c.cp, c.ws, c.d_rgb, aov);
         check("k_resolve / k_final", 0);
         if (fb.tree.n_items) {
-            launches += EUCL_PREC(launch_tree_export)(dim, l, fb.fp, c.cp, c.ws, fb.tree);
+            launches += s->k->tree_export(l, fb.fp, c.cp, c.ws, fb.tree);
             check("k_tree_export", 0);
         }
         mark(3);
@@ -1354,7 +1356,8 @@ uint64_t graph_key(const ChunkLaunch& c) {
     mix(&c.d_rgb, sizeof c.d_rgb);
     mix(&c.d_hit, sizeof c.d_hit);
     // the AOV planes and the cost buffer: a graph captured with or without them never stands in for the other
-    mix(&c.aov, sizeof c.aov);
+    mix(&fb.aov, sizeof fb.aov);
+    mix(&c.cost, sizeof c.cost);
     mix(&c.pipeline, sizeof c.pipeline);
     mix(&fb.max_depth, sizeof fb.max_depth);
     // a batch: the graph reads the table the caller's poses were uploaded to, and it is keyed by its contents too, so
@@ -1480,7 +1483,7 @@ int read_back_chunk(Pipeline& pipe, const ChunkLaunch& c, const ChunkDebug& dbg,
 // every sub_stride-th band of the caller's rank starting at sub_offset (render_split).  `o` describes the (virtual)
 // frame: o->height = fb.n * fb.rows.
 int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit,
-                const AovPlanes& aov_out, EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
+                EuclStats* stats, int sub_stride = 1, int sub_offset = 0) {
     const int width = (int)o->width;
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
     const bool wavefront = o->pipeline == EUCL_PIPELINE_WAVEFRONT;
@@ -1496,7 +1499,7 @@ int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRe
         if (pipe.arena_factor <= 0.0) pipe.arena_factor = std::max(1.0, (double)env_int("EUCL_ARENA_FACTOR_X10", 45) / 10.0);
         const WorkspaceNeeds need{wavefront && s->n_cull > 0 && env_int("EUCL_BIN_RAYS", 1),
                                   wavefront && kBinsPerEntity * s->n_entities + 1 <= kMaxBins && env_int("EUCL_BIN_SHADE", 1),
-                                  wavefront && (aov_out.segments || aov_out.levels), fb.n > 1};
+                                  wavefront && (fb.aov.segments || fb.aov.levels), fb.n > 1};
         // chunking: whole local rows, about EUCL_CHUNK_PIXELS primaries per chunk.  Large chunks are faster (longer
         // levels, fewer host round trips: 4d_room 7680x4320 renders 10 % faster as one chunk than as eight), so the
         // default covers an 8K frame; the chunk shrinks by itself when its workspace does not fit (reserve_workspace).
@@ -1509,7 +1512,7 @@ int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRe
         // calls take no part in that choice)
         const bool use_graph = env_int("EUCL_GRAPH", 1) && !o->profile && !debug_sync && !poison &&
                                (s->ray_bins_mode >= 0 || !wavefront || fb.ray_origins);
-        ChunkLaunch c{fb, o->pipeline, make_launch(s, pipe, *o), ChunkParams{}, Workspace{}, aov_out, d_rgb, d_hit};
+        ChunkLaunch c{fb, o->pipeline, make_launch(s, pipe, *o), ChunkParams{}, Workspace{}, nullptr, d_rgb, d_hit};
         c.cp.band_rows = o->band_rows ? (int)o->band_rows : (int)o->height;
         c.cp.band_rank = (int)o->band_rank;
         c.cp.band_world = o->band_world ? (int)o->band_world : 1;
@@ -1524,7 +1527,7 @@ int render_impl(EuclScene* s, Pipeline& pipe, const FrameBatch& fb, const EuclRe
                 c.cp.n_rows = std::min<int>(rows_per_chunk, (int)my_rows - row0);
                 c.cp.n_pixels = c.cp.n_rows * width;
                 c.ws = carve(s, pipe, fb);
-                c.aov.cost = need.cost ? (uint2*)pipe.node_cost.ptr : nullptr;
+                c.cost = need.cost ? (uint2*)pipe.node_cost.ptr : nullptr;
                 ChunkDebug dbg{o->profile != 0, debug_sync, poison, {}, {}};
                 rc = launch_chunk(s, pipe, c, dbg, use_graph, &st);
                 if (rc == EUCL_OK) rc = read_back_chunk(pipe, c, dbg, &st, &retry);
@@ -1572,8 +1575,7 @@ constexpr int kMaxSplit = 8;
 // 3d_room frame whatever its size (profiles/r2_band_scaling.txt) -- 3 % of a 4K frame on one GPU, 20 % of an
 // eighth of it.  Independent pipelines, each on every k-th 16-row band and on streams of its own, fill each other's
 // tails.  The picture cannot depend on it: pixels are independent (mod.rs:316-348).
-int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, const AovPlanes& aov,
-                 EuclStats* stats) {
+int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* d_rgb, int32_t* d_hit, EuclStats* stats) {
     const uint32_t my_rows = eucl_band_rows_for_rank(o);
     uint32_t world = o->band_world > 1 ? o->band_world : 1, rank = world > 1 ? o->band_rank : 0, band = o->band_rows;
     if (band == 0) { // one band: the frame belongs to rank 0
@@ -1584,7 +1586,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     int k = std::min(kMaxSplit, env_int("EUCL_SPLIT", EUCL_SPLIT_DEFAULT));
     k = (int)std::min<uint32_t>((uint32_t)std::max(k, 1), my_rows / band); // a band or more for every pipeline
     if (o->pipeline != EUCL_PIPELINE_WAVEFRONT || (long long)my_rows * o->width < (long long)env_int("EUCL_SPLIT_MIN_PIXELS", 1 << 16)) k = 1;
-    if (k <= 1) return render_impl(s, *s->pipes[0], fb, o, d_rgb, d_hit, aov, stats);
+    if (k <= 1) return render_impl(s, *s->pipes[0], fb, o, d_rgb, d_hit, stats);
     while ((int)s->pipes.size() < k) {
         const int rc = add_pipeline(s);
         if (rc != EUCL_OK) {
@@ -1613,7 +1615,7 @@ int render_split(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, ui
     const bool serial = o->profile || env_int("EUCL_DEBUG_SYNC", 0) || env_int("EUCL_POISON", 0);
     auto run = [&](int p) {
         cudaSetDevice(s->device);
-        rc[p] = render_impl(s, *s->pipes[p], fb, &opts[p], d_rgb, d_hit, aov, &part[p], k, p);
+        rc[p] = render_impl(s, *s->pipes[p], fb, &opts[p], d_rgb, d_hit, &part[p], k, p);
         if (rc[p] != EUCL_OK) err[p] = eucl_last_error();
     };
     // (no early return between here and the last wait(): the helper threads work on this frame's locals)
@@ -1787,7 +1789,7 @@ const EuclAovs* any_plane(const EuclAovs* a) {
 // A rank of a band-split render (band_world > 1, a single frame) renders its rows compactly on the device and then copies
 // each band to its place in the caller's frame: rows of other ranks are never read or written, so N ranks can fill ONE
 // host frame (shared pinned memory) over their own PCIe links at the same time.  The AOV planes go the same way.
-int render_to_host(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
+int render_to_host(EuclScene* s, FrameBatch fb, const EuclRenderOpts* o, uint8_t* out_rgb8, int32_t* out_hit_ids,
                    const EuclAovs* aovs, EuclStats* stats) {
     const bool scatter = !o->compact_rows && o->band_world > 1;
     const size_t my_rows = eucl_band_rows_for_rank(o);
@@ -1813,11 +1815,11 @@ int render_to_host(EuclScene* s, const FrameBatch& fb, const EuclRenderOpts* o, 
                 p += align16(std::max<size_t>(pixels, 1) * px_bytes[k]);
             }
     }
-    const AovPlanes d_aov{(float*)dev[0], (float*)dev[1], (float*)dev[2], (uint32_t*)dev[3], (uint32_t*)dev[4], nullptr};
+    fb.aov = AovPlanes{(float*)dev[0], (float*)dev[1], (float*)dev[2], (uint32_t*)dev[3], (uint32_t*)dev[4], nullptr};
     EuclRenderOpts opts = *o;
     opts.want_hit_ids = want_hit ? 1 : 0;
     if (scatter) opts.compact_rows = 1;
-    const int st = render_split(s, fb, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, d_aov, stats);
+    const int st = render_split(s, fb, &opts, (uint8_t*)s->frame.ptr, want_hit ? (int32_t*)s->hit_ids.ptr : nullptr, stats);
     if (st != EUCL_OK) return st;
     const cudaStream_t stream = s->stream();
     if (!scatter) {
@@ -1862,7 +1864,7 @@ int eucl_render_device(EuclScene* s, const EuclCamera* cam, const EuclRenderOpts
     FrameBatch fb;
     EuclRenderOpts virt;
     if ((st = camera_batch(s, &frame, 1, o, &fb, &virt)) != EUCL_OK) return st;
-    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
 }
 
 int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o,
@@ -1874,7 +1876,7 @@ int eucl_render_frames_device(EuclScene* s, const EuclFrame* frames, uint32_t n_
     FrameBatch fb;
     EuclRenderOpts virt;
     if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
-    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, AovPlanes{}, stats);
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
 }
 
 int eucl_render_frames(EuclScene* s, const EuclFrame* frames, uint32_t n_frames, const EuclRenderOpts* o, uint8_t* out_rgb8,
@@ -1923,8 +1925,8 @@ int eucl_render_aovs_device(EuclScene* s, const EuclFrame* frames, uint32_t n_fr
     FrameBatch fb;
     EuclRenderOpts virt;
     if ((st = camera_batch(s, frames, n_frames, o, &fb, &virt)) != EUCL_OK) return st;
-    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, aov_planes(d_aovs),
-                        stats);
+    fb.aov = aov_planes(d_aovs);
+    return render_split(s, fb, &virt, (uint8_t*)d_out_rgb8, o->want_hit_ids ? (int32_t*)d_out_hit_ids : nullptr, stats);
 }
 
 int eucl_trace_rays(EuclScene* s, const EuclRays* r, uint8_t* out_rgb8, int32_t* out_hit_ids, const EuclAovs* aovs,
@@ -1981,8 +1983,9 @@ int eucl_trace_rays_device(EuclScene* s, const EuclRays* r, void* d_out_rgb8, vo
     if (st != EUCL_OK) return st;
     EUCL_CUDA(cudaSetDevice(s->device));
     EuclRenderOpts o;
-    const FrameBatch fb = ray_batch(s, r, r->origins, r->directions, d_out_hit_ids != nullptr, &o);
-    return render_split(s, fb, &o, (uint8_t*)d_out_rgb8, (int32_t*)d_out_hit_ids, aov_planes(any_plane(d_aovs)), stats);
+    FrameBatch fb = ray_batch(s, r, r->origins, r->directions, d_out_hit_ids != nullptr, &o);
+    fb.aov = aov_planes(any_plane(d_aovs));
+    return render_split(s, fb, &o, (uint8_t*)d_out_rgb8, (int32_t*)d_out_hit_ids, stats);
 }
 
 int eucl_scene_memory(const EuclScene* s, uint64_t* arena_bytes, uint64_t* list_bytes, uint64_t* node_capacity) {
@@ -2025,7 +2028,7 @@ int eucl_trace_path(EuclScene* s, const double* location, const double* directio
         h_in[D + k] = direction[k];
     }
     EUCL_CUDA(cudaMemcpyAsync(d_in, h_in, sizeof h_in, cudaMemcpyHostToDevice, stream));
-    EUCL_PREC(launch_trace_path)(D, make_launch(s, *s->pipes[0], EuclRenderOpts{}), d_in, distance, d_out, d_found);
+    s->k->trace_path(make_launch(s, *s->pipes[0], EuclRenderOpts{}), d_in, distance, d_out, d_found);
     double h_out[2 * EUCL_MAX_DIM];
     int h_found = 0;
     EUCL_CUDA(cudaMemcpyAsync(h_out, d_out, sizeof h_out, cudaMemcpyDeviceToHost, stream));

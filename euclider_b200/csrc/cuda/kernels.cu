@@ -355,6 +355,23 @@ __device__ __forceinline__ int frame_of_row(const Workspace& ws, int& y) {
     return f;
 }
 
+// K1 (k_raygen, k_raygen_rays) with ws.ray_bins: primary ray i joins the reach-key list of its key when it is traced (one
+// atomicAdd per warp and key).  Every lane of the warp calls it.
+template <int D>
+__device__ __forceinline__ void bin_primary(const SceneView& sv, const Workspace& ws, int i, unsigned lane, bool traced,
+                                            const Vec<D>& o, const Vec<D>& dir) {
+    const unsigned active = __ballot_sync(0xffffffffu, traced);
+    if (traced) {
+        const int key = reach_key<D>(sv, o, dir);
+        const unsigned peers = __match_any_sync(active, key);
+        const int leader = __ffs(peers) - 1;
+        int s2 = 0;
+        if ((int)lane == leader) s2 = atomicAdd(&ws.rbin_count[key], __popc(peers));
+        s2 = __shfl_sync(peers, s2, leader);
+        ws.rorder[(size_t)key * ws.list_cap + s2 + __popc(peers & ((1u << lane) - 1u))] = i;
+    }
+}
+
 // K1: one primary ray per pixel of the chunk; level 0 of the node arena is the pixel order.
 template <int D>
 __global__ void __launch_bounds__(kBlock) k_raygen(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp,
@@ -409,18 +426,7 @@ __global__ void __launch_bounds__(kBlock) k_raygen(const uint8_t* __restrict__ b
         Vec<D> dir = batch ? camera_ray<D>(ws.frames[f], x, y) : camera_ray<D>(fp, x, y);
         if (traced) material_enter<D>(sv, belongs_to, dir);
         if (valid) store_ray<D>(ws, i, loc, dir, traced ? belongs_to : -1);
-        if (ws.ray_bins) { // group the primary rays by reach key like k_shade groups the children (one atomicAdd per warp and key)
-            const unsigned active = __ballot_sync(0xffffffffu, valid && traced);
-            if (valid && traced) {
-                const int key = reach_key<D>(sv, loc, dir);
-                const unsigned peers = __match_any_sync(active, key);
-                const int leader = __ffs(peers) - 1;
-                int s2 = 0;
-                if ((int)lane == leader) s2 = atomicAdd(&ws.rbin_count[key], __popc(peers));
-                s2 = __shfl_sync(peers, s2, leader);
-                ws.rorder[(size_t)key * ws.list_cap + s2 + __popc(peers & ((1u << lane) - 1u))] = i;
-            }
-        }
+        if (ws.ray_bins) bin_primary<D>(sv, ws, i, lane, valid && traced, loc, dir); // like k_shade groups the children
     }
 }
 
@@ -465,18 +471,7 @@ __global__ void __launch_bounds__(kBlock) k_raygen_rays(const uint8_t* __restric
         // ray_cur -1 keeps k_shade off it
         if (traced) material_enter<D>(sv, belongs_to, dir);
         if (valid) store_ray<D>(ws, i, o, dir, traced ? belongs_to : -1);
-        if (ws.ray_bins) { // as k_raygen
-            const unsigned active = __ballot_sync(0xffffffffu, valid && traced);
-            if (valid && traced) {
-                const int key = reach_key<D>(sv, o, dir);
-                const unsigned peers = __match_any_sync(active, key);
-                const int leader = __ffs(peers) - 1;
-                int s2 = 0;
-                if ((int)lane == leader) s2 = atomicAdd(&ws.rbin_count[key], __popc(peers));
-                s2 = __shfl_sync(peers, s2, leader);
-                ws.rorder[(size_t)key * ws.list_cap + s2 + __popc(peers & ((1u << lane) - 1u))] = i;
-            }
-        }
+        if (ws.ray_bins) bin_primary<D>(sv, ws, i, lane, valid && traced, o, dir);
     }
 }
 
@@ -1414,120 +1409,91 @@ inline int grid_for(int n, int block, int grid_max) {
     return (int)g;
 }
 
-} // namespace
-
-#define EUCL_DISPATCH_DIM(dim, CALL3, CALL4) \
-    do {                                     \
-        if ((dim) == 3) { CALL3; }           \
-        else { CALL4; }                      \
-    } while (0)
-
-// (a batch: in front of k_raygen as well, one thread per frame)
-void launch_camera_entity(int dim, const Launch& l, const FrameParams& fp, const Workspace& ws) {
-    EUCL_DISPATCH_DIM(dim, (k_camera_entity<3><<<1, 32, l.smem_scene, l.stream>>>(l.blob, fp, ws)),
-                      (k_camera_entity<4><<<1, 32, l.smem_scene, l.stream>>>(l.blob, fp, ws)));
+// The light and the heavy build of a level's kernel, each when wanted; returns the number launched.  When both run and
+// there is a side stream, the light one runs there: it waits for everything enqueued on the main stream so far (fork), and
+// the main stream waits for it (join).
+template <typename LaunchLight, typename LaunchHeavy>
+int launch_light_and_heavy(const Launch& l, bool light, bool heavy, LaunchLight launch_light, LaunchHeavy launch_heavy) {
+    const bool fork = light && heavy && l.side != nullptr;
+    if (fork) {
+        cudaEventRecord(l.ev_fork, l.stream);
+        cudaStreamWaitEvent(l.side, l.ev_fork, 0);
+    }
+    if (light) launch_light(fork ? l.side : l.stream);
+    if (heavy) launch_heavy();
+    if (fork) {
+        cudaEventRecord(l.ev_join, l.side);
+        cudaStreamWaitEvent(l.stream, l.ev_join, 0);
+    }
+    return (int)light + (int)heavy;
 }
-void launch_raygen(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                   int32_t* hit_ids_out) {
+
+// The builds of k_shade by [GLASS][RAY_BINS][FRAMES]
+template <int D>
+auto shade_build(bool glass, bool ray_bins, bool frames) {
+    static const decltype(&k_shade<D, false, false, false>) builds[2][2][2] = {
+        {{k_shade<D, false, false, false>, k_shade<D, false, false, true>}, {k_shade<D, true, false, false>, k_shade<D, true, false, true>}},
+        {{k_shade<D, false, true, false>, k_shade<D, false, true, true>}, {k_shade<D, true, true, false>, k_shade<D, true, true, true>}}};
+    return builds[glass][ray_bins][frames];
+}
+
+template <int D>
+void launch_camera_entity(const Launch& l, const FrameParams& fp, const Workspace& ws) {
+    k_camera_entity<D><<<1, 32, l.smem_scene, l.stream>>>(l.blob, fp, ws);
+}
+template <int D>
+void launch_raygen(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, int32_t* hit_ids_out,
+                   const double* origins, const double* directions) {
     const int grid = grid_for(cp.n_pixels, kBlock, l.grid_mem);
-    EUCL_DISPATCH_DIM(dim, (k_raygen<3><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out)),
-                      (k_raygen<4><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out)));
-}
-void launch_raygen_rays(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                        int32_t* hit_ids_out, const double* origins, const double* directions) {
-    const int grid = grid_for(cp.n_pixels, kBlock, l.grid_mem);
-    EUCL_DISPATCH_DIM(
-        dim, (k_raygen_rays<3><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out, origins, directions)),
-        (k_raygen_rays<4><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out, origins, directions)));
-}
-// fork: the side stream waits for everything enqueued on the main stream so far; join: the main stream waits for the side
-static void fork_side(const Launch& l) {
-    cudaEventRecord(l.ev_fork, l.stream);
-    cudaStreamWaitEvent(l.side, l.ev_fork, 0);
-}
-static void join_side(const Launch& l) {
-    cudaEventRecord(l.ev_join, l.side);
-    cudaStreamWaitEvent(l.stream, l.ev_join, 0);
+    if (origins) k_raygen_rays<D><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out, origins, directions);
+    else k_raygen<D><<<grid, kBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, hit_ids_out);
 }
 
-int launch_intersect(int dim, const Launch& l, const Workspace& ws, int level) {
+template <int D>
+int launch_intersect(const Launch& l, const Workspace& ws, int level) {
     // grouped level of a light-capable scene: key 0 -> light build, the other keys -> heavy build;
     // a light-capable scene without cull roots (every ray has key 0) runs the light build in node order
     const bool light_all = l.light_capable && l.n_cull == 0;
     const bool split = l.light_capable && ws.ray_bins != 0;
     const size_t smem_light = l.smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block;
-    const bool light = light_all || split, heavy = !light_all;
-    const bool fork = light && heavy && l.side != nullptr;
-    cudaStream_t light_stream = fork ? l.side : l.stream;
-    if (fork) fork_side(l);
-    int launches = 0;
-    if (light) {
-        EUCL_DISPATCH_DIM(dim, (k_intersect<3, true><<<l.grid_light_k2, kLightK2Block, smem_light, light_stream>>>(l.blob, ws, level, 1u)),
-                          (k_intersect<4, true><<<l.grid_light_k2, kLightK2Block, smem_light, light_stream>>>(l.blob, ws, level, 1u)));
-        ++launches;
-    }
-    if (heavy) {
-        const unsigned mask = split ? 0xfffeu : 0xffffu;
-        EUCL_DISPATCH_DIM(dim, (k_intersect<3, false><<<l.grid_max, kBlock, l.smem_bytes, l.stream>>>(l.blob, ws, level, mask)),
-                          (k_intersect<4, false><<<l.grid_max, kBlock, l.smem_bytes, l.stream>>>(l.blob, ws, level, mask)));
-        ++launches;
-    }
-    if (fork) join_side(l);
-    return launches;
+    const unsigned heavy_mask = split ? 0xfffeu : 0xffffu;
+    return launch_light_and_heavy(
+        l, light_all || split, !light_all,
+        [&](cudaStream_t stream) { k_intersect<D, true><<<l.grid_light_k2, kLightK2Block, smem_light, stream>>>(l.blob, ws, level, 1u); },
+        [&] { k_intersect<D, false><<<l.grid_max, kBlock, l.smem_bytes, l.stream>>>(l.blob, ws, level, heavy_mask); });
 }
-template <int D, bool RAY_BINS, bool GLASS, bool FRAMES>
-static void launch_shade_build(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                               int level, unsigned long long mask, int32_t* hit_ids_out) {
-    if (GLASS) k_shade<D, RAY_BINS, true, FRAMES><<<l.grid_shade, kShadeBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
-    else k_shade<D, RAY_BINS, false, FRAMES><<<l.grid_light, kLightBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level, mask, hit_ids_out);
-}
-template <int D, bool RAY_BINS, bool GLASS>
-static void launch_shade_one(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                             int level, unsigned long long mask, int32_t* hit_ids_out) {
-    if (ws.node_frame) launch_shade_build<D, RAY_BINS, GLASS, true>(l, stream, fp, cp, ws, level, mask, hit_ids_out);
-    else launch_shade_build<D, RAY_BINS, GLASS, false>(l, stream, fp, cp, ws, level, mask, hit_ids_out);
-}
-template <int D, bool GLASS>
-static void launch_shade_dim(const Launch& l, cudaStream_t stream, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                             int level, unsigned long long mask, int32_t* hit_ids_out) {
-    if (ws.ray_bins && level + 1 < fp.max_depth) launch_shade_one<D, true, GLASS>(l, stream, fp, cp, ws, level, mask, hit_ids_out); // the next level will be intersected: group its rays
-    else launch_shade_one<D, false, GLASS>(l, stream, fp, cp, ws, level, mask, hit_ids_out);
-}
-int launch_shade(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, int level,
+
+template <int D>
+int launch_shade(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, int level,
                  int32_t* hit_ids_out) {
-    const bool last_level = level >= fp.max_depth;
-    unsigned long long light = l.shade_light_mask, heavy = l.shade_heavy_mask;
-    if (last_level) { // background lookups only
-        const int grid = l.grid_background;
-        EUCL_DISPATCH_DIM(dim, (k_background<3><<<grid, 256, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level, hit_ids_out)),
-                          (k_background<4><<<grid, 256, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level, hit_ids_out)));
+    if (level >= fp.max_depth) { // last level: background lookups only
+        k_background<D><<<l.grid_background, 256, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level, hit_ids_out);
         return 1;
-    } else if (ws.n_bins <= 1) { // not binned: one kernel that can shade everything
+    }
+    unsigned long long light = l.shade_light_mask, heavy = l.shade_heavy_mask;
+    if (ws.n_bins <= 1) { // not binned: one kernel that can shade everything
         light = 0ull;
         heavy = ~0ull;
     }
-    int launches = 0;
-    const bool fork = light && heavy && l.side != nullptr;
-    cudaStream_t light_stream = fork ? l.side : l.stream;
-    if (fork) fork_side(l);
-    if (light) {
-        EUCL_DISPATCH_DIM(dim, (launch_shade_dim<3, false>(l, light_stream, fp, cp, ws, level, light, hit_ids_out)),
-                          (launch_shade_dim<4, false>(l, light_stream, fp, cp, ws, level, light, hit_ids_out)));
-        ++launches;
-    }
-    if (heavy) {
-        EUCL_DISPATCH_DIM(dim, (launch_shade_dim<3, true>(l, l.stream, fp, cp, ws, level, heavy, hit_ids_out)),
-                          (launch_shade_dim<4, true>(l, l.stream, fp, cp, ws, level, heavy, hit_ids_out)));
-        ++launches;
-    }
-    if (fork) join_side(l);
-    return launches;
+    const bool ray_bins = ws.ray_bins && level + 1 < fp.max_depth; // the next level will be intersected: group its rays
+    const bool frames = ws.node_frame != nullptr;
+    return launch_light_and_heavy(
+        l, light != 0ull, heavy != 0ull,
+        [&](cudaStream_t stream) {
+            shade_build<D>(false, ray_bins, frames)<<<l.grid_light, kLightBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level,
+                                                                                                       light, hit_ids_out);
+        },
+        [&] {
+            shade_build<D>(true, ray_bins, frames)<<<l.grid_shade, kShadeBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level,
+                                                                                                       heavy, hit_ids_out);
+        });
 }
+
 // Bottom-up resolve of the ray tree (level max_depth holds leaves only) and the RGB8 pack of level 0.
-// Returns the number of kernels launched.
 // With AOVs: the COST builds when segments or levels are wanted, and k_aov_primary for the primary-hit planes.
-int launch_resolve_and_final(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                             uint8_t* out_rgb8, const AovPlanes& aov) {
+template <int D>
+int launch_resolve_and_final(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, uint8_t* out_rgb8,
+                             const AovPlanes& aov) {
     const bool cost = aov.segments || aov.levels;
     int launches = 0;
     for (int level = fp.max_depth - 1; level >= 1; --level) {
@@ -1540,73 +1506,47 @@ int launch_resolve_and_final(int dim, const Launch& l, const FrameParams& fp, co
     else k_final<<<grid, 256, 0, l.stream>>>(fp, cp, ws, out_rgb8);
     ++launches;
     if (aov.depth || aov.position || aov.normal) {
-        EUCL_DISPATCH_DIM(dim, (k_aov_primary<3><<<grid, 256, 0, l.stream>>>(fp, cp, ws, aov)),
-                          (k_aov_primary<4><<<grid, 256, 0, l.stream>>>(fp, cp, ws, aov)));
+        k_aov_primary<D><<<grid, 256, 0, l.stream>>>(fp, cp, ws, aov);
         ++launches;
     }
     return launches;
 }
-void launch_megakernel(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                       uint8_t* out_rgb8, int32_t* hit_ids_out, const AovPlanes& aov, const double* origins,
-                       const double* directions, const TreeQuery& tree) {
+
+// The build of the megakernel: a tree call records the walk (and writes no AOV plane), else AOVs if any plane is wanted;
+// each with or without the caller's rays.
+template <int D>
+void launch_megakernel(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, uint8_t* out_rgb8,
+                       int32_t* hit_ids_out, const AovPlanes& aov, const double* origins, const double* directions,
+                       const TreeQuery& tree) {
     const int grid = grid_for(cp.n_pixels, kBlock, 1 << 30);
-    if (tree.n_items && origins) {
-        EUCL_DISPATCH_DIM(dim,
-                          (k_megakernel_rays_tree<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                              origins, directions, tree)),
-                          (k_megakernel_rays_tree<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                              origins, directions, tree)));
-        return;
-    }
-    if (tree.n_items) {
-        EUCL_DISPATCH_DIM(
-            dim, (k_megakernel_tree<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, tree)),
-            (k_megakernel_tree<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, tree)));
-        return;
-    }
+    const auto launch = [&](auto kernel, auto... extra) {
+        kernel<<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, extra...);
+    };
     const bool want_aov = aov.depth || aov.position || aov.normal || aov.segments || aov.levels;
-    if (origins && want_aov) {
-        EUCL_DISPATCH_DIM(dim,
-                          (k_megakernel_rays_aov<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                             aov, origins, directions)),
-                          (k_megakernel_rays_aov<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                             aov, origins, directions)));
-        return;
-    }
-    if (origins) {
-        EUCL_DISPATCH_DIM(dim,
-                          (k_megakernel_rays<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                         origins, directions)),
-                          (k_megakernel_rays<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out,
-                                                                                         origins, directions)));
-        return;
-    }
-    if (want_aov) {
-        EUCL_DISPATCH_DIM(
-            dim, (k_megakernel_aov<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)),
-            (k_megakernel_aov<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out, aov)));
-        return;
-    }
-    EUCL_DISPATCH_DIM(
-        dim, (k_megakernel<3><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)),
-        (k_megakernel<4><<<grid, kBlock, l.smem_bytes, l.stream>>>(l.blob, fp, cp, ws, out_rgb8, hit_ids_out)));
+    if (tree.n_items && origins) launch(k_megakernel_rays_tree<D>, origins, directions, tree);
+    else if (tree.n_items) launch(k_megakernel_tree<D>, tree);
+    else if (origins && want_aov) launch(k_megakernel_rays_aov<D>, aov, origins, directions);
+    else if (origins) launch(k_megakernel_rays<D>, origins, directions);
+    else if (want_aov) launch(k_megakernel_aov<D>, aov);
+    else launch(k_megakernel<D>);
 }
 
-// The trees of the query's items in this chunk (after launch_resolve_and_final, while the arena is intact).  Returns 1.
-int launch_tree_export(int dim, const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
-                       const TreeQuery& tree) {
-    const int grid = grid_for(tree.n_items, 128, 1 << 30);
-    EUCL_DISPATCH_DIM(dim, (k_tree_export<3><<<grid, 128, 0, l.stream>>>(fp, cp, ws, tree)),
-                      (k_tree_export<4><<<grid, 128, 0, l.stream>>>(fp, cp, ws, tree)));
+// The trees of the query's items in this chunk (after launch_resolve_and_final, while the arena is intact).
+template <int D>
+int launch_tree_export(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, const TreeQuery& tree) {
+    k_tree_export<D><<<grid_for(tree.n_items, 128, 1 << 30), 128, 0, l.stream>>>(fp, cp, ws, tree);
     return 1;
 }
 
-void launch_trace_path(int dim, const Launch& l, const double* d_in, double distance, double* d_out, int* d_found) {
-    EUCL_DISPATCH_DIM(dim, (k_trace_path<3><<<1, 32, l.smem_bytes, l.stream>>>(l.blob, d_in, distance, d_out, d_found)),
-                      (k_trace_path<4><<<1, 32, l.smem_bytes, l.stream>>>(l.blob, d_in, distance, d_out, d_found)));
+template <int D>
+void launch_trace_path(const Launch& l, const double* d_in, double distance, double* d_out, int* d_found) {
+    k_trace_path<D><<<1, 32, l.smem_bytes, l.stream>>>(l.blob, d_in, distance, d_out, d_found);
 }
 
-namespace {
+template <int D>
+const Kernels kKernels{launch_camera_entity<D>, launch_raygen<D>,      launch_intersect<D>,   launch_shade<D>,
+                       launch_resolve_and_final<D>, launch_megakernel<D>, launch_tree_export<D>, launch_trace_path<D>};
+
 template <typename K>
 cudaError_t configure_one(K kernel, size_t smem, int resident_ctas) {
     // Shared-memory carveout: just what the kernel's resident CTAs need, the rest of the 256 KB stays L1 for
@@ -1621,60 +1561,46 @@ cudaError_t configure_one(K kernel, size_t smem, int resident_ctas) {
     pct = pct < 0 ? 0 : (pct > 100 ? 100 : pct);
     cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     if (smem <= 48 * 1024) return cudaSuccess;
+    // The limit belongs to the kernel, not to the scene, and is shared by every scene of the process: it only ever
+    // grows, so that a scene created later with smaller tables cannot fail the launches of a larger one.
+    cudaFuncAttributes attr{};
+    cudaError_t e = cudaFuncGetAttributes(&attr, kernel);
+    if (e != cudaSuccess || (size_t)attr.maxDynamicSharedSizeBytes >= smem) return e;
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
+
+template <int D>
+cudaError_t configure_dim(size_t smem_bytes, size_t smem_scene) {
+    cudaError_t e = cudaSuccess;
+    const auto conf = [&](auto kernel, size_t smem, int resident_ctas) {
+        if (e == cudaSuccess) e = configure_one(kernel, smem, resident_ctas);
+    };
+    const int heavy = kResidentThreads / kBlock;
+    conf(k_camera_entity<D>, smem_scene, 1);
+    conf(k_raygen<D>, smem_scene, 2);
+    conf(k_raygen_rays<D>, smem_scene, 2);
+    conf(k_intersect<D, false>, smem_bytes, heavy);
+    conf(k_intersect<D, true>, smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
+    for (int b = 0; b < 8; ++b) // [GLASS][RAY_BINS][FRAMES]
+        conf(shade_build<D>(b & 4, b & 2, b & 1), smem_scene, (b & 4) ? kShadeResidentBlocks : kLightResidentBlocks);
+    conf(k_background<D>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
+    conf(k_megakernel<D>, smem_bytes, heavy);
+    conf(k_megakernel_aov<D>, smem_bytes, heavy);
+    conf(k_megakernel_rays<D>, smem_bytes, heavy);
+    conf(k_megakernel_rays_aov<D>, smem_bytes, heavy);
+    conf(k_megakernel_tree<D>, smem_bytes, heavy);
+    conf(k_megakernel_rays_tree<D>, smem_bytes, heavy);
+    conf(k_trace_path<D>, smem_bytes, 1);
+    return e;
+}
+
 } // namespace
 
+const Kernels& kernels(int dim) { return dim == 3 ? kKernels<3> : kKernels<4>; }
+
 cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene) {
-    cudaError_t e;
-    const int heavy = kResidentThreads / kBlock;
-#define EUCL_CONF(K, SMEM, CTAS) \
-    if ((e = configure_one(K, SMEM, CTAS)) != cudaSuccess) return e
-    EUCL_CONF(k_camera_entity<3>, smem_scene, 1);
-    EUCL_CONF(k_camera_entity<4>, smem_scene, 1);
-    EUCL_CONF(k_raygen<3>, smem_scene, 2);
-    EUCL_CONF(k_raygen<4>, smem_scene, 2);
-    EUCL_CONF((k_intersect<3, false>), smem_bytes, heavy);
-    EUCL_CONF((k_intersect<4, false>), smem_bytes, heavy);
-    const size_t smem_light = smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block;
-    EUCL_CONF((k_intersect<3, true>), smem_light, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
-    EUCL_CONF((k_intersect<4, true>), smem_light, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
-    EUCL_CONF((k_shade<3, true, true, false>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, true, true, false>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, false, true, false>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, false, true, false>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, true, false, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, true, false, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<3, false, false, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, false, false, false>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<3, true, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, true, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, false, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<4, false, true, true>), smem_scene, kShadeResidentBlocks);
-    EUCL_CONF((k_shade<3, true, false, true>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, true, false, true>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<3, false, false, true>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF((k_shade<4, false, false, true>), smem_scene, kLightResidentBlocks);
-    EUCL_CONF(k_background<3>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
-    EUCL_CONF(k_background<4>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
-    EUCL_CONF(k_megakernel<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel<4>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_aov<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_aov<4>, smem_bytes, heavy);
-    EUCL_CONF(k_raygen_rays<3>, smem_scene, 2);
-    EUCL_CONF(k_raygen_rays<4>, smem_scene, 2);
-    EUCL_CONF(k_megakernel_rays<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_rays<4>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_rays_aov<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_rays_aov<4>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_tree<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_tree<4>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_rays_tree<3>, smem_bytes, heavy);
-    EUCL_CONF(k_megakernel_rays_tree<4>, smem_bytes, heavy);
-    EUCL_CONF(k_trace_path<3>, smem_bytes, 1);
-    EUCL_CONF(k_trace_path<4>, smem_bytes, 1);
-#undef EUCL_CONF
-    return cudaSuccess;
+    const cudaError_t e = configure_dim<3>(smem_bytes, smem_scene);
+    return e != cudaSuccess ? e : configure_dim<4>(smem_bytes, smem_scene);
 }
 
 #if EUCL_REAL_IS_DOUBLE

@@ -197,32 +197,35 @@ constexpr int kRayBins = 16; // 2^4 reach keys
 constexpr int kBinsPerEntity = 3; // entering, exiting, exiting with total internal reflection predicted
 constexpr int kMaxBins = 64; // shade-coherence bins (miss, then kBinsPerEntity per entity); larger scenes shade unbinned
 
+// The launchers of one build of kernels.cu for one dimension.  `origins` / `directions`: the rays of eucl_trace_rays*,
+// null for camera frames.  The int-returning launchers return the number of kernels they launched.
+struct Kernels {
+    void (*camera_entity)(const Launch& l, const FrameParams& fp, const Workspace& ws); // (a batch: in front of raygen too)
+    void (*raygen)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, int32_t* hit_ids_out,
+                   const double* origins, const double* directions);
+    int (*intersect)(const Launch& l, const Workspace& ws, int level);
+    int (*shade)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, int level,
+                 int32_t* hit_ids_out);
+    int (*resolve_and_final)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws,
+                             uint8_t* out_rgb8, const AovPlanes& aov);
+    void (*megakernel)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, uint8_t* out_rgb8,
+                       int32_t* hit_ids_out, const AovPlanes& aov, const double* origins, const double* directions,
+                       const TreeQuery& tree);
+    int (*tree_export)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, const TreeQuery& tree);
+    void (*trace_path)(const Launch& l, const double* d_in, double distance, double* d_out, int* d_found);
+};
+
 } // namespace eucl
 
 // kernels.cu, compiled twice: namespace eucl (real = double) and namespace eucl_f32 (real = float, the reference's
-// `low_precision` feature).  The structs above are shared.
-#define EUCL_DECLARE_LAUNCHERS(NS)                                                                                             \
-    namespace NS {                                                                                                             \
-    void launch_camera_entity(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::Workspace& ws);        \
-    void launch_raygen(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,              \
-                       const eucl::Workspace& ws, int32_t* hit_ids_out);                                                       \
-    void launch_raygen_rays(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,         \
-                            const eucl::Workspace& ws, int32_t* hit_ids_out, const double* origins, const double* directions); \
-    int launch_intersect(int dim, const eucl::Launch& l, const eucl::Workspace& ws, int level);                                \
-    int launch_shade(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,                \
-                     const eucl::Workspace& ws, int level, int32_t* hit_ids_out);                                              \
-    int launch_resolve_and_final(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,    \
-                                 const eucl::Workspace& ws, uint8_t* out_rgb8, const eucl::AovPlanes& aov);                    \
-    void launch_megakernel(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
-                           const eucl::Workspace& ws, uint8_t* out_rgb8, int32_t* hit_ids_out, const eucl::AovPlanes& aov,     \
-                           const double* origins, const double* directions, const eucl::TreeQuery& tree);                  \
-    int launch_tree_export(int dim, const eucl::Launch& l, const eucl::FrameParams& fp, const eucl::ChunkParams& cp,          \
-                           const eucl::Workspace& ws, const eucl::TreeQuery& tree);                                        \
-    void launch_trace_path(int dim, const eucl::Launch& l, const double* d_in, double distance, double* d_out, int* d_found); \
-    cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);                                                       \
-    }
-EUCL_DECLARE_LAUNCHERS(eucl)
-EUCL_DECLARE_LAUNCHERS(eucl_f32)
+// `low_precision` feature).  The structs above are shared; a scene picks its table once (EuclScene::k), so no launch
+// can reach the other precision's build.  configure_kernels sets up every kernel of the build, both dimensions.
 namespace eucl {
+const Kernels& kernels(int dim);
+cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);
 int fp64_peak(double* dadd, double* dmul, double* dfma); // T op/s on the current device (f64 build only)
 } // namespace eucl
+namespace eucl_f32 {
+const eucl::Kernels& kernels(int dim);
+cudaError_t configure_kernels(size_t smem_bytes, size_t smem_scene);
+} // namespace eucl_f32
