@@ -8,7 +8,7 @@ from pathlib import Path
 
 from ._capi import EuclAovs, EuclCamera, EuclError, EuclFrame, EuclRays, EuclRenderOpts, EuclStats, EUCL_PIPELINE_MEGAKERNEL, EUCL_PIPELINE_WAVEFRONT, lib
 from .scene import (AOV_NAMES, TREE_NODE_DTYPE, Environment, Parser, ParserError, RawFrames, RawImage2d, RawRays, RayTree,
-                    SimulationContext, default_tree_capacity, equirect_rays)
+                    SimulationContext, camera_step, default_tree_capacity, equirect_rays)
 
 ROOT = Path(__file__).resolve().parent.parent
 ASSET_ROOT = ROOT / "assets"  # the reference scenes, restated, and stand-in textures (assets/make_assets.py)
@@ -19,6 +19,6 @@ def load_reference_scene(name: str) -> Environment:
     return Parser.default(resource_root=ASSET_ROOT).parse_file(ASSET_ROOT / "scenes" / f"{name}.json")
 
 
-__all__ = ["Parser", "Environment", "SimulationContext", "RawImage2d", "RawFrames", "RawRays", "EuclFrame", "EuclAovs", "EuclRays", "equirect_rays", "AOV_NAMES", "RayTree", "TREE_NODE_DTYPE", "default_tree_capacity", "ParserError", "EuclError", "EuclCamera",
+__all__ = ["Parser", "Environment", "SimulationContext", "RawImage2d", "RawFrames", "RawRays", "EuclFrame", "EuclAovs", "EuclRays", "equirect_rays", "camera_step", "AOV_NAMES", "RayTree", "TREE_NODE_DTYPE", "default_tree_capacity", "ParserError", "EuclError", "EuclCamera",
            "EuclRenderOpts", "EuclStats", "EUCL_PIPELINE_WAVEFRONT", "EUCL_PIPELINE_MEGAKERNEL", "lib",
            "load_reference_scene", "ASSET_ROOT", "ROOT"]

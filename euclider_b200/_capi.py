@@ -190,6 +190,12 @@ PROTOTYPES = {
                                        C.POINTER(EuclStats)]),
     "eucl_trace_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,
                                   C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "eucl_locate_points": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
+    "eucl_locate_points_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
+    "eucl_trace_paths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p,
+                                   C.c_void_p, C.c_void_p]),
+    "eucl_trace_paths_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]),
     "eucl_camera_rotate_yaw": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),
     "eucl_camera_rotate_pitch": (C.c_int, [C.POINTER(EuclCamera), C.c_double, C.c_int]),
     "eucl_camera_rotate_roll": (C.c_int, [C.POINTER(EuclCamera), C.c_double]),

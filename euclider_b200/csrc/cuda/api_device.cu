@@ -173,6 +173,7 @@ struct EuclScene {
     DeviceBuffer ray_stage; // device copy of the rays of eucl_trace_rays (host input), refilled by every call
     DeviceBuffer tree_stage; // a tree call: its query and the nodes and counts every pipeline exports into (host output)
     DeviceBuffer path_io;   // eucl_trace_path staging
+    DeviceBuffer query_io;  // eucl_locate_points / eucl_trace_paths staging: one chunk of host items at a time
     // a batch of frames (eucl_render_frames*): the per-frame constants, read by every pipeline, and their pinned host staging
     DeviceBuffer frame_table;
     PinnedBuffer h_frame_table;
@@ -1850,6 +1851,26 @@ int render_to_host(EuclScene* s, FrameBatch fb, const EuclRenderOpts* o, uint8_t
     return EUCL_OK;
 }
 
+// The universe queries (eucl_locate_points*, eucl_trace_paths*): checked before any device work.
+int check_query(const EuclScene* s, bool arrays, uint32_t n, uint32_t steps, const char* fn) {
+    const std::string f(fn);
+    if (!s || !arrays) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": null argument");
+    if (n == 0 || steps == 0) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n and steps must be at least 1");
+    if ((uint64_t)n * steps > 0x7FFFFFFFull) return fail(EUCL_ERR_INVALID_ARGUMENT, f + ": n * steps above 2^31 - 1");
+    return EUCL_OK;
+}
+
+// Points, or walker steps, that a host query stages through query_io per round trip: the buffer stays at a few tens of
+// MB whatever n is.  A walker's steps are never split, so one walker of more steps takes a chunk of its own.
+constexpr uint32_t kQueryChunk = 1u << 18;
+
+// Waits for the queries' kernels and reports a launch or execution error.
+int finish_query(EuclScene* s) {
+    EUCL_CUDA(cudaStreamSynchronize(s->stream()));
+    EUCL_CUDA(cudaGetLastError());
+    return EUCL_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -2042,6 +2063,77 @@ int eucl_trace_path(EuclScene* s, const double* location, const double* directio
         out_direction[k] = h_out[D + k];
     }
     return EUCL_OK;
+}
+
+int eucl_locate_points_device(EuclScene* s, const double* d_points, uint32_t n, int32_t* d_out_entity) {
+    const int st = check_query(s, d_points && d_out_entity, n, 1, "eucl_locate_points_device");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    s->k->locate(make_launch(s, *s->pipes[0], EuclRenderOpts{}), d_points, n, d_out_entity);
+    return finish_query(s);
+}
+
+int eucl_locate_points(EuclScene* s, const double* points, uint32_t n, int32_t* out_entity) {
+    const int st = check_query(s, points && out_entity, n, 1, "eucl_locate_points");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    const size_t D = (size_t)s->dim, chunk = std::min(n, kQueryChunk);
+    EUCL_CUDA(s->query_io.ensure(chunk * (sizeof(double) * D + sizeof(int32_t))));
+    double* d_points = (double*)s->query_io.ptr;
+    int32_t* d_out = (int32_t*)(d_points + chunk * D);
+    const Launch l = make_launch(s, *s->pipes[0], EuclRenderOpts{});
+    for (size_t i0 = 0; i0 < n; i0 += chunk) { // stream-ordered: a chunk's copies wait for the previous chunk's kernel
+        const uint32_t m = (uint32_t)std::min(chunk, (size_t)n - i0);
+        EUCL_CUDA(cudaMemcpyAsync(d_points, points + i0 * D, sizeof(double) * D * m, cudaMemcpyHostToDevice, l.stream));
+        s->k->locate(l, d_points, m, d_out);
+        EUCL_CUDA(cudaMemcpyAsync(out_entity + i0, d_out, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, l.stream));
+    }
+    return finish_query(s);
+}
+
+int eucl_trace_paths_device(EuclScene* s, const double* d_locations, const double* d_directions, const double* d_distances,
+                            uint32_t n, uint32_t steps, double* d_out_locations, double* d_out_directions, int32_t* d_out_status) {
+    const int st = check_query(s, d_locations && d_directions && d_distances && d_out_locations && d_out_status, n, steps,
+                               "eucl_trace_paths_device");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    s->k->trace_paths(make_launch(s, *s->pipes[0], EuclRenderOpts{}), d_locations, d_directions, d_distances, n, steps,
+                      d_out_locations, d_out_directions, d_out_status);
+    return finish_query(s);
+}
+
+int eucl_trace_paths(EuclScene* s, const double* locations, const double* directions, const double* distances, uint32_t n,
+                     uint32_t steps, double* out_locations, double* out_directions, int32_t* out_status) {
+    const int st = check_query(s, locations && directions && distances && out_locations && out_status, n, steps,
+                               "eucl_trace_paths");
+    if (st != EUCL_OK) return st;
+    EUCL_CUDA(cudaSetDevice(s->device));
+    const size_t D = (size_t)s->dim, walkers = std::min<size_t>(n, std::max<uint32_t>(1u, kQueryChunk / steps));
+    const size_t items = walkers * steps;
+    const bool dirs = out_directions != nullptr;
+    EUCL_CUDA(s->query_io.ensure(sizeof(double) * walkers * (2 * D + 1) + sizeof(double) * items * D * (dirs ? 2 : 1) +
+                                 sizeof(int32_t) * items));
+    double* d_loc = (double*)s->query_io.ptr;
+    double* d_dir = d_loc + walkers * D;
+    double* d_dist = d_dir + walkers * D;
+    double* d_out_loc = d_dist + walkers;
+    double* d_out_dir = dirs ? d_out_loc + items * D : nullptr;
+    int32_t* d_status = (int32_t*)(d_out_loc + items * D * (dirs ? 2 : 1));
+    const Launch l = make_launch(s, *s->pipes[0], EuclRenderOpts{});
+    for (size_t i0 = 0; i0 < n; i0 += walkers) {
+        const size_t m = std::min(walkers, (size_t)n - i0), o = i0 * steps;
+        EUCL_CUDA(cudaMemcpyAsync(d_loc, locations + i0 * D, sizeof(double) * D * m, cudaMemcpyHostToDevice, l.stream));
+        EUCL_CUDA(cudaMemcpyAsync(d_dir, directions + i0 * D, sizeof(double) * D * m, cudaMemcpyHostToDevice, l.stream));
+        EUCL_CUDA(cudaMemcpyAsync(d_dist, distances + i0, sizeof(double) * m, cudaMemcpyHostToDevice, l.stream));
+        s->k->trace_paths(l, d_loc, d_dir, d_dist, (uint32_t)m, steps, d_out_loc, d_out_dir, d_status);
+        EUCL_CUDA(cudaMemcpyAsync(out_locations + o * D, d_out_loc, sizeof(double) * D * m * steps, cudaMemcpyDeviceToHost,
+                                  l.stream));
+        if (dirs)
+            EUCL_CUDA(cudaMemcpyAsync(out_directions + o * D, d_out_dir, sizeof(double) * D * m * steps, cudaMemcpyDeviceToHost,
+                                      l.stream));
+        EUCL_CUDA(cudaMemcpyAsync(out_status + o, d_status, sizeof(int32_t) * m * steps, cudaMemcpyDeviceToHost, l.stream));
+    }
+    return finish_query(s);
 }
 
 int eucl_device_malloc(int device, uint64_t bytes, void** d_ptr) {

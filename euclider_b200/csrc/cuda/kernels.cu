@@ -1377,6 +1377,99 @@ __global__ void __launch_bounds__(32) k_trace_path(const uint8_t* __restrict__ b
     *out_found = found;
 }
 
+// The walk of k_trace_path above for one thread of a larger CTA (k_trace_paths): `ts` / `ts_stride` are the thread's
+// plane_chain scratch column.  Returns 1 moved (loc, dir: the end point and the direction there), 0 the start lies in no
+// entity (loc and dir untouched), -1 more than 100000 surface crossings (loc and dir: where the walk stopped).
+// k_trace_path keeps a copy of its own, and this one is not inlined: k_trace_path's resources are pinned
+// (tests/golden/kernel_resources.json), and with an inlined copy in k_trace_path, or in k_trace_paths, its 3-D f64 build
+// grows from 4512 to 4528 bytes of stack (CUDA 12.9).
+template <int D>
+__device__ __noinline__ int walk_path(const SceneView& sv, Vec<D>& loc, Vec<D>& dir, real distance, real* ts, int ts_stride) {
+    int belongs_to = material_at<D>(sv, loc);
+    if (belongs_to < 0) return 0;
+    material_enter<D>(sv, belongs_to, dir);
+    for (int step = 0; step < 100000; ++step) {
+        const ClosestHit h = closest_hit<D>(sv, loc, dir, ts, ts_stride);
+        bool moved = false;
+        if (h.entity >= 0 && !(distance - h.t <= R(0.0))) { // get_path: Some
+            Vec<D> p, n_raw;
+            hit_geometry<D>(sv, h.prim, h.flags, loc, dir, h.t, p, n_raw);
+            const bool exiting = angle_from_cos(angle_cos(dir, n_raw)) < kFracPi2;
+            const Vec<D> n_closer = exiting ? -n_raw : n_raw;
+            const Vec<D> new_origin = p + (-n_closer) * kApproxEpsilon * R(128.0);
+            const int dest = exiting ? material_at<D>(sv, new_origin) : h.entity;
+            if (dest >= 0) {
+                Vec<D> nd = dir;
+                material_exit<D>(sv, belongs_to, nd);
+                material_enter<D>(sv, dest, nd);
+                distance = distance - h.t;
+                belongs_to = dest;
+                loc = new_origin;
+                dir = nd;
+                moved = true;
+            }
+        }
+        if (!moved) { // Material::trace_path (material.rs:54-56,144-146), then exit
+            loc = loc + dir * distance;
+            material_exit<D>(sv, belongs_to, dir);
+            return 1;
+        }
+    }
+    return -1;
+}
+
+// eucl_trace_paths*: one walker per thread, `steps` walks each.  Step j starts where step j-1 ended (step 0 at the
+// walker's location) and walks the walker's own distance along its own direction (the move_camera rule).  Outputs
+// [n][steps]: status 1 the end point and direction; 0 the start (the walker stays: step 0 gives the location as given,
+// not narrowed) and NaN, repeated by every later step; -1 NaN and NaN, and the walker stops (every later step is -1
+// too).  out_dir may be null.
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_trace_paths(const uint8_t* __restrict__ blob, const double* __restrict__ locations,
+                                                        const double* __restrict__ directions,
+                                                        const double* __restrict__ distances, uint32_t n, uint32_t steps,
+                                                        double* __restrict__ out_loc, double* __restrict__ out_dir,
+                                                        int32_t* __restrict__ out_status) {
+    const SceneView& sv = stage_scene(blob);
+    real* ts = plane_scratch(blob);
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    Vec<D> loc, dir0;
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+        loc[k] = R(locations[(size_t)i * D + k]);
+        dir0[k] = R(directions[(size_t)i * D + k]);
+    }
+    const real distance = R(distances[i]);
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    int status = 1;
+    bool moved = false;
+    for (uint32_t j = 0; j < steps; ++j) {
+        Vec<D> dir = dir0;
+        if (status == 1) status = walk_path<D>(sv, loc, dir, distance, ts, (int)blockDim.x);
+        moved = moved || status == 1;
+        const size_t o = ((size_t)i * steps + j) * D;
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            out_loc[o + k] = status < 0 ? nan : moved ? (double)loc[k] : locations[(size_t)i * D + k];
+            if (out_dir) out_dir[o + k] = status == 1 ? (double)dir[k] : nan;
+        }
+        out_status[(size_t)i * steps + j] = status;
+    }
+}
+
+// eucl_locate_points*: Universe::material_at of each point (narrowed once), -1 in no entity.  Grid-stride over the points.
+template <int D>
+__global__ void __launch_bounds__(kBlock) k_locate(const uint8_t* __restrict__ blob, const double* __restrict__ points, uint32_t n,
+                                                   int32_t* __restrict__ out) {
+    const SceneView& sv = stage_scene(blob);
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        Vec<D> p;
+#pragma unroll
+        for (int k = 0; k < D; ++k) p[k] = R(points[(size_t)i * D + k]);
+        out[i] = material_at<D>(sv, p);
+    }
+}
+
 #if EUCL_REAL_IS_DOUBLE
 // BEGIN_KEEP64
 // FP64 issue-rate microbenchmark: 8 independent dependency chains per thread
@@ -1544,8 +1637,21 @@ void launch_trace_path(const Launch& l, const double* d_in, double distance, dou
 }
 
 template <int D>
+void launch_trace_paths(const Launch& l, const double* d_locations, const double* d_directions, const double* d_distances,
+                        uint32_t n, uint32_t steps, double* d_out_locations, double* d_out_directions, int32_t* d_out_status) {
+    k_trace_paths<D><<<grid_for((int)n, kBlock, 1 << 30), kBlock, l.smem_bytes, l.stream>>>(
+        l.blob, d_locations, d_directions, d_distances, n, steps, d_out_locations, d_out_directions, d_out_status);
+}
+
+template <int D>
+void launch_locate(const Launch& l, const double* d_points, uint32_t n, int32_t* d_out) {
+    k_locate<D><<<grid_for((int)n, kBlock, l.grid_mem), kBlock, l.smem_scene, l.stream>>>(l.blob, d_points, n, d_out);
+}
+
+template <int D>
 const Kernels kKernels{launch_camera_entity<D>, launch_raygen<D>,      launch_intersect<D>,   launch_shade<D>,
-                       launch_resolve_and_final<D>, launch_megakernel<D>, launch_tree_export<D>, launch_trace_path<D>};
+                       launch_resolve_and_final<D>, launch_megakernel<D>, launch_tree_export<D>, launch_trace_path<D>,
+                       launch_trace_paths<D>,   launch_locate<D>};
 
 template <typename K>
 cudaError_t configure_one(K kernel, size_t smem, int resident_ctas) {
@@ -1591,6 +1697,8 @@ cudaError_t configure_dim(size_t smem_bytes, size_t smem_scene) {
     conf(k_megakernel_tree<D>, smem_bytes, heavy);
     conf(k_megakernel_rays_tree<D>, smem_bytes, heavy);
     conf(k_trace_path<D>, smem_bytes, 1);
+    conf(k_trace_paths<D>, smem_bytes, heavy);
+    conf(k_locate<D>, smem_scene, 2);
     return e;
 }
 

@@ -144,7 +144,7 @@ struct TreeQuery {
 struct Launch {
     cudaStream_t stream;
     const uint8_t* blob;
-    size_t smem_bytes; // staged scene + the per-thread plane_chain scratch of a kBlock-thread CTA (k_intersect, k_megakernel, k_trace_path)
+    size_t smem_bytes; // staged scene + the per-thread plane_chain scratch of a kBlock-thread CTA (k_intersect, k_megakernel, k_trace_path*)
     size_t smem_scene; // staged scene only (the other kernels)
     int grid_max;   // blocks of the heavy queue kernels (k_intersect, k_shade<GLASS>): resident CTAs per SM x SMs, one wave
     int grid_light; // blocks of the light shade kernel (kLightBlock threads each), one wave
@@ -213,6 +213,10 @@ struct Kernels {
                        const TreeQuery& tree);
     int (*tree_export)(const Launch& l, const FrameParams& fp, const ChunkParams& cp, const Workspace& ws, const TreeQuery& tree);
     void (*trace_path)(const Launch& l, const double* d_in, double distance, double* d_out, int* d_found);
+    // the universe queries (eucl_trace_paths*, eucl_locate_points*), every array on the device
+    void (*trace_paths)(const Launch& l, const double* d_locations, const double* d_directions, const double* d_distances,
+                        uint32_t n, uint32_t steps, double* d_out_locations, double* d_out_directions, int32_t* d_out_status);
+    void (*locate)(const Launch& l, const double* d_points, uint32_t n, int32_t* d_out);
 };
 
 } // namespace eucl

@@ -131,6 +131,26 @@ def _ray_arrays(origins, directions, dim: int) -> Tuple[np.ndarray, np.ndarray, 
     return o, d, lead
 
 
+def _point_array(values, dim: int, what: str) -> Tuple[np.ndarray, Tuple[int, ...]]:
+    """A float64 C-contiguous copy (when needed) of a (..., dim) array, and its leading shape."""
+    a = np.ascontiguousarray(values, dtype=np.float64)
+    if a.ndim < 1 or a.shape[-1] != dim:
+        raise ValueError(f"{what} must have shape (..., {dim}) for this {dim}-D scene, got {a.shape}")
+    n = int(np.prod(a.shape[:-1], dtype=np.int64))
+    if n < 1 or n > 0x7FFFFFFF:
+        raise ValueError(f"{what}: 1 .. 2^31 - 1 items")
+    return a, a.shape[:-1]
+
+
+def camera_step(direction: Sequence[float], distance: float, dim: int) -> Optional[Tuple[List[float], float]]:
+    """The normalisation of Environment.move_camera: (direction / |direction|, distance * |direction|) as the walk's
+    direction and length, or None for a zero direction (the camera does not move)."""
+    norm = sum(float(v) * float(v) for v in direction[:dim]) ** 0.5
+    if norm == 0.0:
+        return None
+    return [float(v) / norm for v in direction[:dim]], distance * norm
+
+
 def _ray_struct(n: int, width: int, max_depth: int, pipeline: int, time: float, profile: bool, origins: int = 0,
                 directions: int = 0) -> EuclRays:
     width = max(int(width), 1)
@@ -529,16 +549,66 @@ class Environment:
         (The reference additionally turns the view when the void bends the path; it labels that code
         "not tested", and it is not reproduced here.)  Returns False when the camera is in no entity."""
         dim = self.dim
-        norm = sum(float(v) * float(v) for v in direction[:dim]) ** 0.5
-        if norm == 0.0:
+        step = camera_step(direction, distance, dim)
+        if step is None:
             return True
-        unit = [float(v) / norm for v in direction[:dim]]
-        res = self.trace_path_unknown([self.camera.location[k] for k in range(dim)], unit, distance * norm, device=device)
+        res = self.trace_path_unknown([self.camera.location[k] for k in range(dim)], step[0], step[1], device=device)
         if res is None:
             return False
         for k in range(dim):
             self.camera.location[k] = res[0][k]
         return True
+
+    # -- universe queries in bulk: one device call for many points or walkers -------------------------
+    def locate(self, points, *, device: int = 0) -> np.ndarray:
+        """Universe::material_at (mod.rs:229-251) of every point (eucl_locate_points): an array of shape (..., dim) gives
+        int32 (...), the first entity in list order whose shape contains the point, -1 when none does."""
+        p, lead = _point_array(points, self.dim, "points")
+        out = np.empty(lead, np.int32)
+        check(lib().eucl_locate_points(self._device_scene(device), p.ctypes.data, out.size, out.ctypes.data))
+        return out
+
+    def locate_device(self, d_points: int, n: int, d_out: int, *, device: int = 0) -> None:
+        """locate with DEVICE arrays: n points of `dim` float64 at d_points, n int32 entities at d_out."""
+        check(lib().eucl_locate_points_device(self._device_scene(device), C.c_void_p(int(d_points)), int(n),
+                                              C.c_void_p(int(d_out))))
+
+    def trace_paths(self, locations, directions, distances, steps: int = 1, *,
+                    device: int = 0) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Universe::trace_path_unknown for many walkers, `steps` steps each (eucl_trace_paths): locations and directions
+        of shape (..., dim), distances a scalar or of the leading shape.  Step j starts where step j-1 ended and walks the
+        walker's own distance along its own direction (used as given), as `move_camera` steps a camera.  Returns
+        (locations (..., steps, dim), directions (..., steps, dim), status (..., steps)): status 1 moved; 0 the step's
+        start lies in no entity (the walker stays, direction NaN, later steps alike); -1 more than 100000 surface
+        crossings (NaN, and the walker stops)."""
+        loc, lead = _point_array(locations, self.dim, "locations")
+        dirs, dlead = _point_array(directions, self.dim, "directions")
+        if dlead != lead:
+            raise ValueError(f"locations {loc.shape} and directions {dirs.shape} must have the same shape")
+        dist = np.asarray(distances, dtype=np.float64)
+        if dist.shape not in ((), lead):
+            raise ValueError(f"distances must be a scalar or of shape {lead}, got {dist.shape}")
+        dist = np.ascontiguousarray(np.broadcast_to(dist, lead))
+        steps = int(steps)
+        n = int(np.prod(lead, dtype=np.int64))
+        if steps < 1 or n * steps > 0x7FFFFFFF:
+            raise ValueError("trace_paths needs steps >= 1 and n * steps <= 2^31 - 1")
+        out_loc = np.empty(lead + (steps, self.dim), np.float64)
+        out_dir = np.empty_like(out_loc)
+        status = np.empty(lead + (steps,), np.int32)
+        check(lib().eucl_trace_paths(self._device_scene(device), loc.ctypes.data, dirs.ctypes.data, dist.ctypes.data, n, steps,
+                                     out_loc.ctypes.data, out_dir.ctypes.data, status.ctypes.data))
+        return out_loc, out_dir, status
+
+    def trace_paths_device(self, d_locations: int, d_directions: int, d_distances: int, n: int, steps: int,
+                           d_out_locations: int, d_out_status: int, d_out_directions: int = 0, *, device: int = 0) -> None:
+        """trace_paths with DEVICE arrays: n walkers (dim float64 locations and directions, one float64 distance each),
+        outputs [n][steps] ([n][steps][dim] float64 locations and, unless 0, directions; int32 status)."""
+        check(lib().eucl_trace_paths_device(self._device_scene(device), C.c_void_p(int(d_locations)),
+                                            C.c_void_p(int(d_directions)), C.c_void_p(int(d_distances)), int(n), int(steps),
+                                            C.c_void_p(int(d_out_locations)),
+                                            C.c_void_p(int(d_out_directions)) if d_out_directions else None,
+                                            C.c_void_p(int(d_out_status))))
 
     # The view-turning part of the reference's camera `update` (d3/entity/camera.rs:94-145,303-350;
     # d4/entity/camera.rs:68-130).  The reference derives the angles from mouse deltas and held keys;

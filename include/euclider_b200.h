@@ -497,6 +497,35 @@ int eucl_trace_ray_trees(EuclScene* scene, const EuclRays* rays, uint8_t* out_rg
 int eucl_trace_path(EuclScene* scene, const double* location, const double* direction, double distance,
                     double* out_location, double* out_direction);
 
+/* Universe queries in bulk: the scene's geometry without a render, one launch and one thread per item.  They run on the
+ * scene's stream (eucl_scene_set_stream), read nothing but the scene, and leave the render calls' CUDA graphs alone.  The
+ * host variants stage their arrays through a scene-owned device buffer in chunks of a bounded number of items, so device
+ * memory does not grow with n.  EUCL_ERR_INVALID_ARGUMENT, before any device work, for a null required pointer, n == 0,
+ * steps == 0 and n * steps > 2^31 - 1.
+ *
+ * Universe::material_at (mod.rs:229-251) for n points: out_entity[i] = the first entity in list order whose shape
+ * contains points[i] (dim doubles each; an f32 scene narrows them once), -1 when none does.  Synchronous. */
+int eucl_locate_points(EuclScene* scene, const double* points, uint32_t n, int32_t* out_entity);
+/* Same, with DEVICE arrays on the scene's device. */
+int eucl_locate_points_device(EuclScene* scene, const double* d_points, uint32_t n, int32_t* d_out_entity);
+
+/* Universe::trace_path_unknown for n walkers, `steps` steps each.  Step j of walker i starts where step j-1 ended
+ * (step 0 at locations[i]) and moves distances[i] along directions[i] (used as given, not normalised), exactly as
+ * eucl_trace_path(scene, start, directions[i], distances[i], ...) would.  This is the camera rule of
+ * Environment.move_camera: every step uses the walker's own direction, not the direction returned by the previous step.
+ * Outputs [n][steps]: the location and direction eucl_trace_path returns, and a status:
+ *   1  moved;
+ *   0  the step's start lies in no entity: the location is the start (the walker stays), the direction is NaN, and the
+ *      later steps repeat the same result;
+ *  -1  more than 100000 surface crossings: the location and direction are NaN, and the walker stops (the later steps are -1 too).
+ * out_directions may be NULL.  One walker's status never fails the call.  Synchronous. */
+int eucl_trace_paths(EuclScene* scene, const double* locations, const double* directions, const double* distances,
+                     uint32_t n, uint32_t steps, double* out_locations, double* out_directions, int32_t* out_status);
+/* Same, with DEVICE arrays on the scene's device (d_out_directions may be NULL). */
+int eucl_trace_paths_device(EuclScene* scene, const double* d_locations, const double* d_directions, const double* d_distances,
+                            uint32_t n, uint32_t steps, double* d_out_locations, double* d_out_directions,
+                            int32_t* d_out_status);
+
 /* Camera rotations: the view-turning part of the reference's per-frame Camera::update, on an EuclCamera pose
  * (host arithmetic; the translation part is eucl_trace_path).  Angles in radians.  Replaces
  * PitchYawCamera3::rotate_yaw_static / rotate_pitch_static (src/universe/d3/entity/camera.rs:110-136),

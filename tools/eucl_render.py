@@ -5,8 +5,9 @@
         [--resource-root assets] [--location x y z [w]] [--max-depth N] [--pipeline megakernel]
 
 Image sequences -- a camera path, a turntable, a Perlin animation -- with --frames N: frame k is the pose after k steps
-of the per-frame motion and the time --time + k * --time-step; the output name takes a printf pattern.  Frames are
-rendered --batch at a time (default: all in one call, Environment.render_frames).
+of the per-frame motion and the time --time + k * --time-step; the output name takes a printf pattern.  The translations
+of the whole camera path are one Environment.trace_paths call.  Frames are rendered --batch at a time (default: all in one
+call, Environment.render_frames).
 
     python tools/eucl_render.py assets/scenes/3d_room.json out_%04d.ppm --size 128 96 --frames 64 \\
         --move 0 0.05 0 --yaw 0.02 --time-step 0.04
@@ -26,6 +27,13 @@ reference's debug pixel): every Universe::trace call of the pixel, printed as an
 frames only, perspective or equirect, and not together with --aov.
 
     python tools/eucl_render.py assets/scenes/3d_room.json out.png --size 640 360 --inspect center --inspect 100,40
+
+A map of which entity owns each point of a plane, with no ray tracing, with --section EXTENT (Environment.locate): the
+plane through the camera location spanned by the camera's right axis (image right) and forward axis (image up), EXTENT
+scene units wide at the output size, sampled at pixel centres.  Each entity index has a fixed colour, points in no entity
+are black; `out.entity.npy` holds the entity map as locate returns it (int32, row 0 = bottom).  Single frames only.
+
+    python tools/eucl_render.py assets/scenes/4d_room.json section.png --size 800 800 --section 30
 """
 import argparse
 import json
@@ -69,6 +77,9 @@ def parse_args(argv=None):
                     help=f"also write these per-pixel planes, from {','.join(eb.AOV_NAMES)}")
     ap.add_argument("--inspect", type=inspect_spec, action="append", default=[], metavar="X,Y|center",
                     help="print the ray tree of this pixel and write it to out.tree_X_Y.json (repeatable)")
+    ap.add_argument("--section", type=float, metavar="EXTENT",
+                    help="write the entity map of the plane through the camera (right x forward), EXTENT units wide, "
+                         "instead of rendering")
     args = ap.parse_args(argv)
     if args.frames < 1:
         ap.error("--frames must be at least 1")
@@ -86,6 +97,11 @@ def parse_args(argv=None):
         ap.error("--inspect works on single frames only")
     if args.inspect and args.aov:
         ap.error("--inspect and --aov cannot be used together")
+    if args.section is not None:
+        if args.aov or args.inspect or is_sequence(args) or args.projection != "perspective":
+            ap.error("--section writes single entity maps: not with --aov, --inspect, --projection equirect or a sequence")
+        if not args.section > 0.0:
+            ap.error("--section takes a positive extent")
     return args
 
 
@@ -169,10 +185,46 @@ def is_sequence(args) -> bool:
             or args.plane4 is not None or args.time_step or "%" in args.output)
 
 
-def step_camera(env, args) -> None:
-    """One frame's motion: the translation through the universe, then the turns."""
-    if args.move is not None and not env.move_camera(args.move, 1.0):
-        print("warning: the camera is in no entity; it stays where it is", file=sys.stderr)
+# --section: a colour per entity index (cycled), black for points in no entity
+SECTION_PALETTE = np.array([[230, 25, 75], [60, 180, 75], [255, 225, 25], [0, 130, 200], [245, 130, 48], [145, 30, 180],
+                            [70, 240, 240], [240, 50, 230], [210, 245, 60], [250, 190, 212], [0, 128, 128], [220, 190, 255],
+                            [170, 110, 40], [255, 250, 200], [128, 0, 0], [170, 255, 195]], dtype=np.uint8)
+
+
+def section_points(camera, dim: int, width: int, height: int, extent: float) -> np.ndarray:
+    """(height, width, dim) float64 points of the plane through the camera location spanned by the right axis (x, image
+    right) and the forward axis (y, image up), `extent` units wide, at pixel centres, row 0 at the bottom.  The right
+    axis is normalize(forward x up) in 3-D and -left in 4-D, as for the camera's own rays."""
+    f = np.array(camera.forward[:dim], dtype=np.float64)
+    if dim == 3:
+        c = np.cross(f, np.array(camera.up[:dim], dtype=np.float64))
+        right = c / np.linalg.norm(c)
+    else:
+        right = -np.array(camera.left[:dim], dtype=np.float64)
+    pixel = extent / width
+    xs = ((np.arange(width, dtype=np.float64) + 0.5) - width / 2.0) * pixel
+    ys = ((np.arange(height, dtype=np.float64) + 0.5) - height / 2.0) * pixel
+    loc = np.array(camera.location[:dim], dtype=np.float64)
+    return loc + xs[None, :, None] * right + ys[:, None, None] * f
+
+
+def section_image(entity: np.ndarray) -> np.ndarray:
+    """RGB8 of an entity map: SECTION_PALETTE by entity index, black for -1."""
+    rgb = SECTION_PALETTE[np.maximum(entity, 0) % len(SECTION_PALETTE)]
+    rgb[entity < 0] = 0
+    return rgb
+
+
+def write_section(env, args) -> None:
+    w, h = args.size[0] // args.resolution, args.size[1] // args.resolution
+    entity = env.locate(section_points(env.camera, env.dim, w, h, args.section))
+    eb.RawImage2d(section_image(entity), w, h).save(args.output)
+    np.save(aov_path(args.output, "entity", ".npy"), entity)
+    print(f"{args.output}: {w}x{h} entity map, {args.section:g} units wide, entities {sorted(set(np.unique(entity).tolist()))}")
+
+
+def turn_camera(env, args) -> None:
+    """One frame's turns, after its translation."""
     if args.yaw:
         env.rotate_yaw(args.yaw)
     if args.pitch:
@@ -181,6 +233,34 @@ def step_camera(env, args) -> None:
         env.rotate_roll(args.roll)
     if args.plane4 is not None:
         env.rotate_plane4(int(args.plane4[0]), int(args.plane4[1]), args.plane4[2])
+
+
+def camera_path(env, args) -> list:
+    """The cameras of the frames: frame k is the pose after k steps of the per-frame motion, each step the translation
+    through the universe (as Environment.move_camera makes it), then the turns.  Turns do not move the camera, so the
+    translations of all the steps are one Environment.trace_paths call: one walker at the camera location, with the
+    direction and length move_camera normalises --move to."""
+    steps = args.frames - 1
+    dim = env.dim
+    status = None
+    if args.move is not None and steps > 0:
+        step = eb.camera_step(args.move, 1.0, dim)
+        if step is not None:
+            unit = step[0] + [0.0] * (dim - len(step[0]))
+            locations, _, status = env.trace_paths([env.camera.location[k] for k in range(dim)], unit, step[1], steps=steps)
+    cameras = [env.camera.copy()]
+    for k in range(steps):
+        if status is not None:
+            if status[k] < 0:
+                raise eb.EuclError(-21, "the camera path crosses more than 100000 surfaces in one step")
+            if status[k] == 0:
+                print("warning: the camera is in no entity; it stays where it is", file=sys.stderr)
+            else:
+                for j in range(dim):
+                    env.camera.location[j] = locations[k, j]
+        turn_camera(env, args)
+        cameras.append(env.camera.copy())
+    return cameras
 
 
 def main(argv=None):
@@ -193,6 +273,9 @@ def main(argv=None):
         env.camera.max_depth = args.max_depth
     env.pipeline = eb.EUCL_PIPELINE_MEGAKERNEL if args.pipeline == "megakernel" else eb.EUCL_PIPELINE_WAVEFRONT
     context = eb.SimulationContext(resolution=args.resolution)
+    if args.section is not None:
+        write_section(env, args)
+        return
     if args.projection == "equirect":
         w, h = args.size[0] // args.resolution, args.size[1] // args.resolution
         pixels = inspect_pixels(args.inspect, w, h)
@@ -217,12 +300,8 @@ def main(argv=None):
         st = img.stats
         print(f"{args.output}: {img.width}x{img.height}, {st['segments']} ray segments, {st['ms_total']:.2f} ms on the device")
         return
-    cameras, times = [], []
-    for k in range(args.frames):
-        if k > 0:
-            step_camera(env, args)
-        cameras.append(env.camera.copy())
-        times.append(args.time + k * args.time_step)
+    cameras = camera_path(env, args)
+    times = [args.time + k * args.time_step for k in range(args.frames)]
     batch = args.batch or args.frames
     segments, ms = 0, 0.0
     for k0 in range(0, args.frames, batch):
