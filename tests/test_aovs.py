@@ -1,5 +1,5 @@
 """Per-pixel auxiliary outputs (eucl_render_aovs*, Environment.render(..., aovs=...)): depth, position and normal of the
-primary hit and the segments and levels of each pixel's ray tree equal the CPU oracle's planes (tests/oracle_aovs.cc)
+primary hit and the segments and levels of each pixel's ray tree equal the CPU oracle's planes (oracle/oracle_features.cc)
 bit for bit -- any NaN equals any NaN -- in every layout a render has (batches, bands, compact rows, two pipelines,
 chunks, retries, graph replays), on both pipelines and precisions; and asking for them changes nothing else.  The CPU
 tests cover the ABI struct, the oracle's own consistency, the Python argument checks and the tool's --aov option."""
@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 import euclider_b200 as eb
-import oracle_aovs_api as aov_oracle
+import oracle_api
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT / "tools"))
@@ -89,7 +89,7 @@ def check_oracle(env, size, time=0.0, camera=None, variant="det", rows=None):
         plain = env.render(size, time, want_hit_ids=True)
     finally:
         env.camera = saved
-    rgb, hit, planes, st = aov_oracle.render_aovs(env, w, h, time=time, camera=camera, variant=variant, rows=rows)
+    rgb, hit, planes, st = oracle_api.render_aovs(env, w, h, time=time, camera=camera, variant=variant, rows=rows)
     r0, r1 = rows or (0, h)
     assert np.array_equal(img.data[r0:r1], rgb) and np.array_equal(img.hit_ids[r0:r1], hit), "frame differs from the oracle"
     assert_planes({n: a[r0:r1] for n, a in img.aovs.items()}, planes)
@@ -331,7 +331,7 @@ def test_4k_rows_against_oracle(built_lib, monkeypatch):
     img = env.render((w, h), 0.0, want_hit_ids=True, aovs=ALL)
     assert int(img.aovs["segments"].sum(dtype=np.uint64)) == img.stats["segments"]
     for r0, r1 in [(0, 2), (99, 101), (1599, 1601), (2158, 2160)]:
-        rgb, hit, planes, _ = aov_oracle.render_aovs(env, w, h, rows=(r0, r1))
+        rgb, hit, planes, _ = oracle_api.render_aovs(env, w, h, rows=(r0, r1))
         assert np.array_equal(img.data[r0:r1], rgb) and np.array_equal(img.hit_ids[r0:r1], hit)
         assert_planes({n: a[r0:r1] for n, a in img.aovs.items()}, planes, what=f"rows {r0}-{r1}: ")
 
@@ -399,7 +399,7 @@ def test_aovs_struct_layout():
 def test_oracle_planes_are_consistent(oracle, name, size, variant):
     env = load(name)
     w, h = size
-    rgb, hit, planes, st = aov_oracle.render_aovs(env, w, h, time=0.5, variant=variant)
+    rgb, hit, planes, st = oracle_api.render_aovs(env, w, h, time=0.5, variant=variant)
     rgb0, hit0, st0 = oracle.render(env, w, h, time=0.5, variant=variant)
     assert np.array_equal(rgb, rgb0) and np.array_equal(hit, hit0)
     assert st["segments"] == st0["segments"] and st["level_counts"] == st0["level_counts"]

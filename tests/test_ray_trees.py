@@ -1,5 +1,5 @@
 """Ray-tree inspection (eucl_render_trees, eucl_trace_ray_trees; Environment.render / render_frames / trace_rays with
-`trees=`): the trees equal the CPU oracle's restatement of Tracer::trace (tests/oracle_trees.cc) node for node and bit for
+`trees=`): the trees equal the CPU oracle's restatement of Tracer::trace (oracle/oracle_features.cc) node for node and bit for
 bit, any NaN equal to any NaN, for both pipelines and both precisions; a tree call renders exactly what the plain call
 renders; every tree agrees with the pixel, the hit id and the AOV planes; and the trees survive the frame machinery (chunks,
 split pipelines, arena retries, duplicate items, graph replays around them).  The CPU tests pin the ABI layout, the Python
@@ -16,9 +16,7 @@ import numpy as np
 import pytest
 
 import euclider_b200 as eb
-import oracle_aovs_api as aov_oracle
-import oracle_rays_api as ray_oracle
-import oracle_trees_api as ot
+import oracle_api
 from euclider_b200 import _capi
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -57,7 +55,7 @@ def counted(stats):
 def assert_trees_equal(got, want, labels):
     assert len(got) == len(want) == len(labels)
     for label, a, b in zip(labels, got, want):
-        diff = ot.first_difference(a, b)
+        diff = oracle_api.first_difference(a, b)
         assert diff is None, f"item {label}: {diff}"
 
 
@@ -65,12 +63,12 @@ def check_consistency(env, trees, cells, rgb, hit, planes, max_depth):
     """Each tree against the other outputs of its item (`cells`: indices into rgb / hit / the planes): the composited root
     is the pixel, the root hit the hit id, the root t and normal the depth and normal planes after narrowing, and the
     node levels give segments and levels."""
-    variant = ot.variant_of(env)
+    variant = oracle_api.variant_of(env)
     for cell, tr in zip(cells, trees):
         root = tr.nodes[0]
         checker = bool(root["flags"] & _capi.EUCL_TREE_CHECKERBOARD)
         assert root["parent"] == -1 and root["level"] == 0 and root["kind"] == _capi.EUCL_TREE_ROOT
-        assert np.array_equal(ot.tree_pixel(root, variant), rgb[cell]), (cell, tr.format())
+        assert np.array_equal(oracle_api.tree_pixel(root, variant), rgb[cell]), (cell, tr.format())
         assert (-2 if checker else root["hit_entity"]) == hit[cell], cell
         with np.errstate(over="ignore"):  # narrowing, as the depth plane does
             assert same(np.float32(root["t"]), planes["depth"][cell]), cell
@@ -106,7 +104,7 @@ def check_render_trees(env, size, time=0.0, pixels=None, capacity=None, seed=0):
     assert len(got.trees) == len(pixels)
     check_consistency(env, got.trees, [(y, x) for x, y in pixels], plain.data, plain.hit_ids, plain.aovs, md)
     cap = eb.default_tree_capacity(md) if capacity is None else capacity
-    want = ot.pixel_trees(env, w, h, pixels, time, capacity=cap)
+    want = oracle_api.pixel_trees(env, w, h, pixels, time, capacity=cap)
     assert_trees_equal(got.trees, want, pixels)
     return got
 
@@ -147,7 +145,7 @@ def check_ray_trees(env, o, d, items, time=0.0, max_depth=None, width=None, capa
     w = max(int(w), 1)
     of, df = o.reshape(-1, env.dim), d.reshape(-1, env.dim)
     cap = eb.default_tree_capacity(md) if capacity is None else capacity
-    want = [ot.ray_tree(env, of[i], df[i], (i % w, i // w), md, time, cap) for i in flat]
+    want = [oracle_api.ray_tree(env, of[i], df[i], (i % w, i // w), md, time, cap) for i in flat]
     assert_trees_equal(got.trees, want, items)
     return got
 
@@ -236,7 +234,7 @@ def test_batch_of_traced_and_untraced_frames(built_lib, pipeline):
     assert counted(got.stats) == counted(plain.stats)
     check_consistency(env, got.trees, [(k, y, x) for k, x, y in items], plain.data, plain.hit_ids, plain.aovs,
                       int(env.camera.max_depth))
-    want = [ot.pixel_trees(env, w, h, [(x, y)], times[k], camera=cams[k], capacity=eb.default_tree_capacity(env.camera.max_depth))[0]
+    want = [oracle_api.pixel_trees(env, w, h, [(x, y)], times[k], camera=cams[k], capacity=eb.default_tree_capacity(env.camera.max_depth))[0]
             for k, x, y in items]
     assert_trees_equal(got.trees, want, items)
     kinds = {bool(t.nodes[0]["flags"] & _capi.EUCL_TREE_CHECKERBOARD) for t in got.trees}
@@ -291,7 +289,7 @@ def test_origins_in_no_entity_and_flat_list_against_grid(built_lib, pipeline):
     assert any(checker) and not all(checker)
     for a, b, c in zip(flat.trees, grid.trees, checker):  # only the checkerboard colour depends on the grid width
         if not c:
-            assert ot.first_difference(a, b) is None
+            assert oracle_api.first_difference(a, b) is None
 
 
 @pytest.mark.gpu
@@ -306,7 +304,7 @@ def test_truncation_keeps_prefixes(built_lib, pipeline):
         got = check_render_trees(env, (48, 30), pixels=pixels, capacity=cap)
         for a, b in zip(got.trees, full):
             assert a.count == b.count and len(a.nodes) == min(cap, b.count) and a.truncated == (b.count > cap)
-            assert ot.first_difference(a, eb.RayTree(b.nodes[:cap], b.count, b.dim, b.precision)) is None
+            assert oracle_api.first_difference(a, eb.RayTree(b.nodes[:cap], b.count, b.dim, b.precision)) is None
 
 
 @pytest.mark.gpu
@@ -350,7 +348,7 @@ def test_duplicate_items(built_lib, pipeline):
     env.pipeline = pipeline_id(pipeline)
     pixels = [(5, 7), (20, 11), (5, 7), (0, 0), (20, 11), (5, 7)]
     got = check_render_trees(env, (32, 20), pixels=pixels)
-    assert ot.first_difference(got.trees[0], got.trees[2]) is None and ot.first_difference(got.trees[0], got.trees[5]) is None
+    assert oracle_api.first_difference(got.trees[0], got.trees[2]) is None and oracle_api.first_difference(got.trees[0], got.trees[5]) is None
     o, d = random_rays(env, 500, seed=4)
     check_ray_trees(env, o, d, [3, 499, 3, 3, 17, 499])
 
@@ -446,7 +444,7 @@ def test_tool_inspect(built_lib, tmp_path):
         doc = json.loads((tmp_path / f"room.tree_{x}_{y}.json").read_text())
         assert doc["pixel"] == [x, y] and doc["count"] == tree.count
         back = eucl_render.tree_from_json(doc, env.dim)
-        assert ot.first_difference(back, tree) is None
+        assert oracle_api.first_difference(back, tree) is None
 
 
 # ---------------------------------------------------------------------------------------------------------------- CPU
@@ -514,14 +512,14 @@ def test_ray_tree_helpers():
     text = tree.format().splitlines()
     assert text[0].startswith("[0] root level 0") and text[2].startswith("    [2] reflected level 2") and "5 more" in text[-1]
     other = eb.RayTree(nodes.copy(), 9, 3)
-    assert ot.first_difference(tree, other) is None
+    assert oracle_api.first_difference(tree, other) is None
     other.nodes["t"][1] = np.nextafter(0.5, 1.0)
-    assert ot.first_difference(tree, other).startswith("node 1, level 1, transmitted: t 0x3fe0000000000000 vs 0x3fe0000000000001")
+    assert oracle_api.first_difference(tree, other).startswith("node 1, level 1, transmitted: t 0x3fe0000000000000 vs 0x3fe0000000000001")
     nan2 = eb.RayTree(nodes.copy(), 9, 3)
     nodes["t"][2] = np.nan
     nan2.nodes["t"][2] = -np.float64(np.nan)
-    assert ot.first_difference(eb.RayTree(nodes, 9, 3), nan2) is None
-    assert "node count 9 vs 8" in ot.first_difference(tree, eb.RayTree(nodes.copy(), 8, 3))
+    assert oracle_api.first_difference(eb.RayTree(nodes, 9, 3), nan2) is None
+    assert "node count 9 vs 8" in oracle_api.first_difference(tree, eb.RayTree(nodes.copy(), 8, 3))
 
 
 def test_tool_inspect_option_parsing():
@@ -545,14 +543,14 @@ def test_oracle_restatement_equals_oracle(name, variant):
     node counts the AOV oracle's segments / levels, and the Tracer's level counts those of oracle_render."""
     env = load(name)
     w, h = (16, 10) if variant == "det" else (8, 6)
-    rgb, hit, planes, stats = aov_oracle.render_aovs(env, w, h, time=0.5, variant=variant)
+    rgb, hit, planes, stats = oracle_api.render_aovs(env, w, h, time=0.5, variant=variant)
     pixels = [(x, y) for y in range(h) for x in range(w)]
-    trees = ot.pixel_trees(env, w, h, pixels, 0.5, capacity=1 << 14, variant=variant, level_counts=True)
+    trees = oracle_api.pixel_trees(env, w, h, pixels, 0.5, capacity=1 << 14, variant=variant, level_counts=True)
     md = int(env.camera.max_depth)
     total = np.zeros(md + 1, np.uint64)
     for (x, y), (tree, levels) in zip(pixels, trees):
         assert not tree.truncated
-        assert np.array_equal(ot.tree_pixel(tree.nodes[0], variant), rgb[y, x]), (x, y)
+        assert np.array_equal(oracle_api.tree_pixel(tree.nodes[0], variant), rgb[y, x]), (x, y)
         assert tree.nodes[0]["hit_entity"] == hit[y, x], (x, y)
         lv = tree.nodes["level"]
         assert np.array_equal(np.bincount(lv, minlength=md + 1), levels), (x, y)

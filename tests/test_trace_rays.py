@@ -1,6 +1,6 @@
 """Caller-supplied rays (eucl_trace_rays*, Environment.trace_rays): the camera's own rays reproduce eucl_render bit for
 bit, and arbitrary rays -- unnormalised, degenerate, starting in no entity or inside a LinearSpace void -- equal the CPU
-oracle's definition (tests/oracle_rays.cc) bit for bit, any NaN equal to any NaN, through every part of the machinery a
+oracle's definition (oracle/oracle_features.cc) bit for bit, any NaN equal to any NaN, through every part of the machinery a
 frame uses (chunks, retries, split pipelines, graph replays).  The CPU tests cover the ABI struct, the oracle exports, the
 Python argument checks, the equirect geometry and the tool's --projection option."""
 import ctypes as C
@@ -13,8 +13,7 @@ import numpy as np
 import pytest
 
 import euclider_b200 as eb
-import oracle_aovs_api as aov_oracle
-import oracle_rays_api as ray_oracle
+import oracle_api
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT / "tools"))
@@ -82,7 +81,7 @@ def random_rays(env, n, seed):
 def check_rays_oracle(env, origins, directions, time=0.0, max_depth=None, width=None, variant="det"):
     """One trace_rays call with every plane against the oracle; returns it."""
     got = env.trace_rays(origins, directions, time, max_depth=max_depth, width=width, aovs=ALL)
-    rgb, hit, planes, st = ray_oracle.trace_rays(env, origins, directions, time=time, max_depth=max_depth, width=width,
+    rgb, hit, planes, st = oracle_api.trace_rays(env, origins, directions, time=time, max_depth=max_depth, width=width,
                                                  variant=variant)
     assert_same_result(got, rgb, hit, planes)
     assert got.stats["segments"] == st["segments"] and got.stats["nodes"] == st["nodes"]
@@ -99,7 +98,7 @@ def check_identity(env, size, time=0.5, variant="det", camera=None):
         env.camera = camera.copy()
     try:
         img = env.render(size, time, want_hit_ids=True, aovs=ALL)
-        o, d = ray_oracle.camera_rays(env, w, h, variant=variant)
+        o, d = oracle_api.camera_rays(env, w, h, variant=variant)
         got = env.trace_rays(o, d, time, aovs=ALL)
     finally:
         env.camera = saved
@@ -241,7 +240,7 @@ def test_split_pipelines_equal_one(built_lib, monkeypatch, name):
         assert_same_result(r, results[0].data, results[0].hit_ids, results[0].aovs)
         assert {k: r.stats[k] for k in COUNTED} == {k: results[0].stats[k] for k in COUNTED}
     rows = slice(100, 104)  # a sample against the oracle
-    rgb, hit, planes, _ = ray_oracle.trace_rays(env, o[rows], d[rows], time=0.5)
+    rgb, hit, planes, _ = oracle_api.trace_rays(env, o[rows], d[rows], time=0.5)
     assert np.array_equal(results[2].data[rows], rgb) and np.array_equal(results[2].hit_ids[rows], hit)
 
 
@@ -262,7 +261,7 @@ def test_chunk_boundaries_inside_the_list(built_lib, monkeypatch, chunk_pixels):
 @pytest.mark.gpu
 def test_forced_arena_retry(built_lib, monkeypatch):
     env = load("3d_fresnel_2")
-    o, d = ray_oracle.camera_rays(env, 48, 31)
+    o, d = oracle_api.camera_rays(env, 48, 31)
     plain = env.trace_rays(o, d, aovs=ALL)
     monkeypatch.setenv("EUCL_ARENA_FACTOR_X10", "11")
     tight = load("3d_fresnel_2")
@@ -317,7 +316,7 @@ def test_device_entry_and_graph_replay(built_lib, pipeline):
         o, d = random_rays(env, n, seed)
         st = dev.trace(env, o, d, time=0.5)
         replays.append(st["graph_replays"])
-        rgb, hit, planes, ost = ray_oracle.trace_rays(env, o, d, time=0.5)
+        rgb, hit, planes, ost = oracle_api.trace_rays(env, o, d, time=0.5)
         assert_same_result(dev.result(), rgb, hit, planes, what=f"seed {seed}: ")
         assert st["level_counts"] == ost["level_counts"]
     assert replays[2] > 0
@@ -338,7 +337,7 @@ def test_host_entry_graph_replay(built_lib):
 def test_render_and_trace_rays_alternate(built_lib):
     env = load("3d_room")
     w, h = 64, 40
-    o, d = ray_oracle.camera_rays(env, w, h)
+    o, d = oracle_api.camera_rays(env, w, h)
     o2, d2 = o.copy(), d[::-1].copy()  # the same grid, other rays
     # the scene settles its ray-grouping mode (no graphs while it measures), then the render runs as a graph
     for _ in range(12):
@@ -514,7 +513,7 @@ def test_tool_projection_option_parsing():
 def test_oracle_camera_rays_equal_ray_vector(oracle, name, variant):
     env = load(name)
     w, h = 13, 7
-    o, d = ray_oracle.camera_rays(env, w, h, variant=variant)
+    o, d = oracle_api.camera_rays(env, w, h, variant=variant)
     assert np.array_equal(o, np.broadcast_to(o[0, 0], o.shape))
     if variant == "f32":  # float rays, widened
         assert np.array_equal(d.astype(np.float32).astype(np.float64), d)
@@ -533,9 +532,9 @@ def test_oracle_camera_rays_equal_ray_vector(oracle, name, variant):
 def test_oracle_trace_rays_of_camera_rays_equals_render(name, size, variant):
     env = load(name)
     w, h = size
-    o, d = ray_oracle.camera_rays(env, w, h, variant=variant)
-    rgb, hit, planes, st = ray_oracle.trace_rays(env, o, d, time=0.5, variant=variant)
-    rgb0, hit0, planes0, st0 = aov_oracle.render_aovs(env, w, h, time=0.5, variant=variant)
+    o, d = oracle_api.camera_rays(env, w, h, variant=variant)
+    rgb, hit, planes, st = oracle_api.trace_rays(env, o, d, time=0.5, variant=variant)
+    rgb0, hit0, planes0, st0 = oracle_api.render_aovs(env, w, h, time=0.5, variant=variant)
     assert np.array_equal(rgb, rgb0) and np.array_equal(hit, hit0)
     for n in ALL:
         assert same(planes[n], planes0[n]), n

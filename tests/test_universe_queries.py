@@ -1,6 +1,6 @@
 """Universe queries in bulk (eucl_locate_points*, eucl_trace_paths*; Environment.locate, Environment.trace_paths): many
 points located and many walkers moved through the universe in one device call.  On the GPU, bit for bit: locate equals the
-CPU oracle's Universe::material_at (tests/oracle_queries.cc) and what a render decides about a ray's origin, trace_paths
+CPU oracle's Universe::material_at (oracle/oracle_features.cc) and what a render decides about a ray's origin, trace_paths
 equals eucl_trace_path called once per walker and step and the oracle's trace_path_unknown, the host variants equal the
 device variants across chunk boundaries, a query leaves a render's graph replay alone, and the tool's camera path and
 entity sections equal their definitions.  The CPU tests cover the ABI, the argument checks and the tool's options."""
@@ -14,8 +14,6 @@ import pytest
 
 import euclider_b200 as eb
 import oracle_api
-import oracle_queries_api as query_oracle
-import oracle_rays_api as ray_oracle
 from test_negated_rooms import SHAPES as NEGATED_ROOMS, load as load_negated, scene as negated_scene
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -100,7 +98,7 @@ def test_locate_equals_oracle(built_lib, name, precision):
     env = load(name, precision)
     pts = query_points(env, 3000, seed=len(name))
     got = env.locate(pts)
-    want = query_oracle.locate(env, pts, variant(precision))
+    want = oracle_api.locate(env, pts, variant(precision))
     assert got.dtype == np.int32 and got.shape == (len(pts),)
     bad = np.flatnonzero(got != want)
     assert not len(bad), f"{len(bad)} points differ, first {pts[bad[0]]}: {got[bad[0]]} vs {want[bad[0]]}"
@@ -121,7 +119,7 @@ def test_locate_equals_the_renderers_origin_decision(built_lib, name):
     for shift in (0.0, 0.5 * ext, 2.0 * ext):  # the camera's rays from places in and out of the entities
         cam = env.camera.copy()
         cam.location[0] += shift
-        o, d = ray_oracle.camera_rays(env, w, h, camera=cam)
+        o, d = oracle_api.camera_rays(env, w, h, camera=cam)
         o = o + rng.normal(0.0, 0.2 * ext, (h, w, 1)) * (np.arange(dim) == 1)  # a different origin per ray
         res = env.trace_rays(o, d, max_depth=2)
         located = env.locate(o)
@@ -235,7 +233,7 @@ def test_locate_sizes_and_device_variant(built_lib, n):
     env.locate_device(dev.ptr("points"), n, dev.ptr("out"))
     assert np.array_equal(dev.get("out"), got)
     sample = np.arange(0, n, max(1, n // 3000))
-    assert np.array_equal(got[sample], query_oracle.locate(env, pts[sample]))
+    assert np.array_equal(got[sample], oracle_api.locate(env, pts[sample]))
     assert env.locate(pts[0]).shape == () and env.locate(pts[0]) == got[0]
     grid = query_points(env, 12, seed=1)[:12].reshape(3, 4, env.dim)
     assert np.array_equal(env.locate(grid), env.locate(grid.reshape(12, env.dim)).reshape(3, 4))
@@ -372,7 +370,7 @@ def test_tool_section_equals_locate(built_lib, tmp_path, name):
     ys = (np.arange(h) + 0.5 - h / 2) * (extent / w)
     pts = np.array(cam.location[:dim]) + xs[None, :, None] * right + ys[:, None, None] * f
     assert entity.dtype == np.int32 and entity.shape == (h, w)
-    assert np.array_equal(entity, query_oracle.locate(env, pts))
+    assert np.array_equal(entity, oracle_api.locate(env, pts))
     assert len(np.unique(entity)) > 1
     from PIL import Image
 

@@ -3,7 +3,7 @@
 against trace_rays_device of that frame's own camera rays (width = frame width), plus an equirect panorama of the same
 size, all into device buffers, in one process on one Environment per way.
 
-The camera rays come from the CPU oracle's Tracer::ray_vector (tests/oracle_rays.cc), which equals the device's camera
+The camera rays come from the CPU oracle's Tracer::ray_vector (oracle/oracle_features.cc), which equals the device's camera
 arithmetic bit for bit, so the frame and the traced rays must be equal bytes; the run fails otherwise.  After a warm-up
 (arena sizing, the ray-grouping tuner, graph capture) the three ways alternate call by call, --repeats times each; every
 call replays its way's CUDA graph.  Timed is the device time of each call (EuclStats.ms_total, CUDA events on the scene's
@@ -23,7 +23,7 @@ sys.path.insert(0, str(ROOT / "tools"))
 sys.path.insert(0, str(ROOT / "tests"))
 
 import euclider_b200 as eb  # noqa: E402
-import oracle_rays_api  # noqa: E402
+import oracle_api  # noqa: E402
 from batch_throughput import gpu_identity  # noqa: E402
 
 WORKLOADS = [("3d_room", 1920, 1080), ("4d_room", 1920, 1080)]
@@ -36,7 +36,7 @@ def measure(name, w, h, repeats):
     envs = {way: eb.load_reference_scene(name) for way in ("render", "rays", "equirect")}
     for env in envs.values():
         env.camera.max_depth = DEPTH
-    cam_o, cam_d = oracle_rays_api.camera_rays(envs["rays"], w, h)
+    cam_o, cam_d = oracle_api.camera_rays(envs["rays"], w, h)
     eq_o, eq_d = eb.equirect_rays(envs["equirect"].camera, w, h)
     rays = {"rays": (torch.from_numpy(cam_o).cuda(), torch.from_numpy(cam_d).cuda()),
             "equirect": (torch.from_numpy(eq_o).cuda(), torch.from_numpy(eq_d).cuda())}
