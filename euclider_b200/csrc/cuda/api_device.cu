@@ -179,6 +179,7 @@ struct EuclScene {
     PinnedBuffer h_frame_table;
     int n_cull = 0;
     int light_capable = 0;
+    int csg2_capable = 0;
     // Grouping rays by reach key pays on scenes whose deep levels bounce around a few bounded objects
     // (3d_room: -13 % frame time) and costs a little elsewhere, so it is auto-tuned per scene: the
     // first two retry-free frames run with and without it, the faster setting is kept.  The picture
@@ -848,9 +849,12 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     }
     s->n_cull = h.n_cull;
     // per-entity classification for the closest-hit loops; a scene is "light-capable" when a ray with reach key 0
-    // can only meet primitives and root plane chains (k_intersect<LIGHT>)
+    // can only meet primitives and root plane chains (k_intersect<LIGHT>), and "csg2-capable" when every surfaced entity
+    // is a primitive, a root plane chain or a two-leaf program (csg2_first): no closest-hit evaluation of the scene needs
+    // the hit arena, and k_intersect_csg2 walks the rays the heavy build would walk
     std::vector<int32_t> ent_flags((size_t)std::max(flat->n_entities, 1), 0);
-    bool light_capable = true;
+    bool light_capable = true, csg2_capable = true;
+    const auto plane_chain_node = [](const MNode& m) { return m.kind == M_CHAIN && (m.b & 0x4000) && (m.b & 0x3fff) <= kPlaneChainMax; };
     for (int e = 0; e < flat->n_entities; ++e) {
         const EuclEntity& de = dev_entities[(size_t)e];
         if (negated[(size_t)e]) ent_flags[(size_t)e] = ENT_NEGATED; // material_at needs it for entities without a surface too
@@ -858,15 +862,24 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
         const MNode& root = mb.out[(size_t)de.node_root];
         int fl = ENT_SURFACED | ent_flags[(size_t)e];
         if (root.kind == M_PRIM) fl |= ENT_PRIM;
-        else if (root.kind == M_CHAIN && de.node_first == de.node_root && (root.b & 0x4000) && (root.b & 0x3fff) <= kPlaneChainMax) fl |= ENT_ROOT_PLANES;
+        else if (de.node_first == de.node_root && plane_chain_node(root)) fl |= ENT_ROOT_PLANES;
+        else if (root.kind == M_OP && de.node_root == de.node_first + 2) {
+            const MNode& a = mb.out[(size_t)de.node_first];
+            const MNode& b = mb.out[(size_t)de.node_first + 1];
+            if ((a.kind == M_PRIM || plane_chain_node(a)) && b.kind == M_PRIM) fl |= ENT_CSG2;
+        }
         for (int k = 0; k < h.n_cull; ++k)
             if (h.cull_root[k] == de.node_root) fl |= ENT_CULL_ROOT;
         if (!(fl & (ENT_PRIM | ENT_ROOT_PLANES | ENT_CULL_ROOT))) light_capable = false;
+        if (!(fl & (ENT_PRIM | ENT_ROOT_PLANES | ENT_CSG2))) csg2_capable = false;
         ent_flags[(size_t)e] = fl;
     }
     if (!env_int("EUCL_INTERSECT_SPLIT", 1)) light_capable = false; // diagnostics: one build intersects every ray
+    if (!env_int("EUCL_CSG2", 1)) csg2_capable = false;              // A/B: the general heavy build instead
     h.light_capable = light_capable ? 1 : 0;
+    h.csg2_capable = csg2_capable ? 1 : 0;
     s->light_capable = h.light_capable;
+    s->csg2_capable = h.csg2_capable;
     h.off_ent_flags = w.put(ent_flags.data(), ent_flags.size());
     h.off_entities = w.put(dev_entities.data(), dev_entities.size());
     h.off_materials = w.put(flat->materials, (size_t)flat->n_materials);
@@ -1074,6 +1087,8 @@ Launch make_launch(const EuclScene* s, const Pipeline& pipe, const EuclRenderOpt
     l.shade_heavy_mask = s->shade_heavy_mask;
     l.grid_light_k2 = sms * std::max(1, env_int("EUCL_LIGHT_K2_BLOCKS_PER_SM", kLightK2ResidentBlocks));
     l.light_capable = s->light_capable;
+    l.grid_csg2 = sms * std::max(1, env_int("EUCL_CSG2_BLOCKS_PER_SM", csg2_resident_blocks(s->dim, s->real_bytes)));
+    l.csg2_capable = s->csg2_capable;
     l.n_cull = s->n_cull;
     // per-launch profiling and the debugging modes keep everything on one stream
     l.side = (o.profile || env_int("EUCL_DEBUG_SYNC", 0) || !env_int("EUCL_CONCURRENT", 1)) ? nullptr : pipe.side_stream;
@@ -1350,7 +1365,8 @@ uint64_t graph_key(const ChunkLaunch& c) {
                                            (unsigned long long)l.grid_shade, (unsigned long long)l.grid_mem, l.shade_light_mask,
                                            l.shade_heavy_mask, (unsigned long long)l.grid_light_k2,
                                            (unsigned long long)l.light_capable, (unsigned long long)l.n_cull,
-                                           (unsigned long long)l.grid_background};
+                                           (unsigned long long)l.grid_background, (unsigned long long)l.grid_csg2,
+                                           (unsigned long long)l.csg2_capable};
         mix(ptrs, sizeof ptrs);
         mix(nums, sizeof nums);
     }
@@ -1436,6 +1452,9 @@ int read_back_chunk(Pipeline& pipe, const ChunkLaunch& c, const ChunkDebug& dbg,
         *slot += ms;
     }
     if (env_int("EUCL_DUMP_LEVELS", 0) && !h[SmallLayout::overflow]) { // diagnostics: per-level counts, bins, launch times
+        // which intersect builds the levels ran: light for key 0, k_intersect_csg2 or the heavy build for the rest
+        fprintf(stderr, "intersect light_capable %d csg2_capable %d n_cull %d ray_bins %d\n", c.l.light_capable, c.l.csg2_capable,
+                c.l.n_cull, c.ws.ray_bins != 0 ? 1 : 0);
         for (uint32_t lv = 0; lv <= depth; ++lv) {
             fprintf(stderr, "level %2u count %9d | bins", lv, h[SmallLayout::count + lv]);
             for (int b = 0; b < c.ws.n_bins && c.ws.n_bins > 1; ++b) fprintf(stderr, " %d", h[SmallLayout::bins + lv * kMaxBins + b]);

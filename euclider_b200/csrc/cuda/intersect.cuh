@@ -601,6 +601,118 @@ __device__ __forceinline__ bool csg_first(const SceneView& sv, int first, int ro
     return false;
 }
 
+// csg_first of a two-leaf program (ENT_CSG2): three macro nodes [A, B, M_OP(op)] at first .. first + 2, A a primitive or a
+// chain of <= kPlaneChainMax half-spaces, B a primitive (3d_room's glass: Complement(cuboid, sphere)).  An exact
+// restatement: A's list is what csg_first stores in its arena -- the same bound check and plane_chain call (whole list,
+// distances in the scratch column `ts`, items as packed 4-bit leaf indices) or the same prim_roots -- and B's is prim_roots'
+// two values; the merge is csg_first's M_OP branch at limit 1 step for step (ties and NaN pick b, the has_a-only quirk of
+// Complement, the flag negations, the early ends), and node_inside of a leaf operand IS prim_inside / chain_inside, called
+// here directly.  Same IEEE operations on the same operands in the same order; only the bookkeeping moves from the
+// local-memory arena and the bit stack into registers, so a kernel built on this has no stack.
+template <int D>
+__device__ __forceinline__ bool csg2_first(const SceneView& sv, int first, const Vec<D>& o, const Vec<D>& d, real* ts,
+                                           int ts_stride, CHit& out) {
+    const MNode* mn = reinterpret_cast<const MNode*>(sv.nodes());
+    const MNode na = mn[first], nb = mn[first + 1];
+    const int op = mn[first + 2].a;
+    const bool a_chain = na.kind == M_CHAIN;
+    const int a_op = na.b >> 16, a_count = na.b & 0x3fff;
+    int al = 0;
+    real a0 = R(0.0), a1 = R(0.0);
+    unsigned long long a_list = 0ull;
+    if (!a_chain) {
+        al = prim_roots<D>(sv, na.a, o, d, a0, a1);
+    } else if (!ray_misses<D>(sv.bounds()[first], o, d, dot(d, d))) {
+        al = plane_chain<D>(sv, a_op, na.a, a_count, o, d, false, ts, ts_stride, a_list);
+    }
+    real b0 = R(0.0), b1 = R(0.0);
+    const int bl = prim_roots<D>(sv, nb.a, o, d, b0, b1);
+    const auto a_hit = [&](int i) -> CHit {
+        if (!a_chain) return CHit{i == 0 ? a0 : a1, na.a, i};
+        const int idx = (int)((a_list >> (4 * i)) & 15ull);
+        return CHit{ts[idx * ts_stride], na.a + idx, 0};
+    };
+    const auto inside_a = [&](const Vec<D>& p) {
+        return a_chain ? chain_inside<D>(sv, a_op, na.a, a_count, p) : prim_inside<D>(sv, na.a, p);
+    };
+    int ia = 0, ib = 0;
+    while (true) {
+        const bool has_a = ia < al, has_b = ib < bl;
+        if (!has_a && !has_b) return false;
+        CHit ha = a_hit(has_a ? ia : 0);
+        CHit hb{ib == 0 ? b0 : b1, nb.a, ib};
+        if (has_a && has_b) {
+            const bool a_closer = ha.t < hb.t; // ties (and NaN) pick b
+            if (op == EUCL_CSG_COMPLEMENT) {
+                if (a_closer) {
+                    ++ia;
+                    if (!prim_inside<D>(sv, nb.a, o + d * ha.t)) {
+                        out = ha;
+                        return true;
+                    }
+                } else {
+                    ++ib;
+                    if (inside_a(o + d * hb.t)) {
+                        hb.flags ^= 2;
+                        out = hb;
+                        return true;
+                    }
+                }
+            } else {
+                CHit closer = a_closer ? ha : hb;
+                if (a_closer) ++ia;
+                else ++ib;
+                const Vec<D> p = o + d * closer.t;
+                const bool in = a_closer ? prim_inside<D>(sv, nb.a, p) : inside_a(p);
+                if (op == EUCL_CSG_UNION) {
+                    if (!in) {
+                        out = closer;
+                        return true;
+                    }
+                } else if (op == EUCL_CSG_INTERSECTION) {
+                    if (in) {
+                        out = closer;
+                        return true;
+                    }
+                } else { // SymmetricDifference: always yields, flipped when inside the other
+                    if (in) closer.flags ^= 2;
+                    out = closer;
+                    return true;
+                }
+            }
+        } else if (has_a) {
+            if (op == EUCL_CSG_COMPLEMENT) { // emitted without advancing (reference quirk): it is the first item
+                out = ha;
+                return true;
+            }
+            const bool in = prim_inside<D>(sv, nb.a, o + d * ha.t);
+            if (op == EUCL_CSG_UNION) {
+                if (in) return false; // None
+            } else if (op == EUCL_CSG_INTERSECTION) {
+                if (!in) return false;
+            } else if (in) {
+                ha.flags ^= 2;
+            }
+            out = ha;
+            return true;
+        } else {
+            const bool in = inside_a(o + d * hb.t);
+            if (op == EUCL_CSG_UNION) {
+                if (in) return false; // None
+            } else if (op == EUCL_CSG_INTERSECTION) {
+                if (!in) return false;
+            } else if (op == EUCL_CSG_COMPLEMENT) {
+                if (!in) return false;
+                hb.flags ^= 2;
+            } else if (in) {
+                hb.flags ^= 2;
+            }
+            out = hb;
+            return true;
+        }
+    }
+}
+
 struct ClosestHit {
     int entity; // -1: no hit
     int prim;
@@ -661,6 +773,41 @@ __device__ __forceinline__ ClosestHit closest_hit_light(const SceneView& sv, con
             prim = root.a + idx;
         }
         if (found && (best.entity < 0 || best.t > t0)) best = ClosestHit{e, prim, (flags & ENT_NEGATED) ? 2 : 0, t0};
+    }
+    return best;
+}
+
+// trace_closest in a "csg2-capable" scene (SceneHeader::csg2_capable): every surfaced entity is one primitive, one root
+// chain of half-spaces or a two-leaf program, so closest_hit's loop runs with the light loop's root-chain shortcut and
+// csg2_first in place of the general evaluator: no hit arena, no stack.  Everything closest_hit does around an entity
+// stays: the bound check of every non-primitive root (a ray with some key bit set may still miss the other bounds), the
+// ENT_NEGATED flip and the strictly-closer rule.
+template <int D>
+__device__ __forceinline__ ClosestHit closest_hit_csg2(const SceneView& sv, const Vec<D>& o, const Vec<D>& d, real* ts,
+                                                       int ts_stride) {
+    ClosestHit best{-1, 0, 0, R(0.0)};
+    const real dd = dot(d, d);
+    for (int e = 0; e < sv.n_entities; ++e) {
+        const int flags = sv.ent_flags()[e];
+        if (!(flags & ENT_SURFACED)) continue;
+        const EuclEntity ent = sv.entities()[e];
+        if (!(flags & ENT_PRIM) && ray_misses<D>(sv.bounds()[ent.node_root], o, d, dd)) continue;
+        const MNode root = reinterpret_cast<const MNode*>(sv.nodes())[ent.node_root];
+        CHit h{R(0.0), root.a, 0};
+        bool found;
+        if (flags & ENT_PRIM) {
+            real t1 = R(0.0);
+            found = prim_roots<D>(sv, root.a, o, d, h.t, t1) > 0;
+        } else if (flags & ENT_ROOT_PLANES) {
+            unsigned long long L = 0ull;
+            found = plane_chain<D>(sv, root.b >> 16, root.a, root.b & 0x3fff, o, d, true, ts, ts_stride, L) > 0;
+            const int idx = (int)(L & 15ull);
+            h = CHit{ts[idx * ts_stride], root.a + idx, 0};
+        } else { // ENT_CSG2
+            found = csg2_first<D>(sv, ent.node_first, o, d, ts, ts_stride, h);
+        }
+        if (flags & ENT_NEGATED) h.flags ^= 2; // the `b`-only branch of ComplementIterator negates the normal
+        if (found && (best.entity < 0 || best.t > h.t)) best = ClosestHit{e, h.prim, h.flags, h.t};
     }
     return best;
 }

@@ -480,10 +480,12 @@ __global__ void __launch_bounds__(kBlock) k_raygen_rays(const uint8_t* __restric
 // Two builds share a level when its rays are grouped by reach key and the scene allows it (SceneHeader::light_capable):
 // the LIGHT one walks the rays with key 0 -- they can only hit primitives and root plane chains -- without the CSG
 // evaluator and its per-thread hit arena, at a fraction of the registers; the HEAVY one walks the other keys (or every
-// ray when the level is not grouped).  `key_mask` selects the reach-key lists of a launch.
-template <int D, bool LIGHT>
-__global__ void __launch_bounds__(LIGHT ? kLightK2Block : kBlock, LIGHT ? EUCL_INTERSECT_LIGHT_MIN_BLOCKS : EUCL_INTERSECT_MIN_BLOCKS)
-    k_intersect(const uint8_t* __restrict__ blob, Workspace ws, int level, unsigned key_mask) {
+// ray when the level is not grouped).  `key_mask` selects the reach-key lists of a launch.  In a csg2-capable scene
+// (SceneHeader::csg2_capable) k_intersect_csg2 takes the HEAVY one's place: closest_hit_csg2 instead of closest_hit, so
+// no hit arena and no stack.
+enum : int { K2_HEAVY = 0, K2_LIGHT = 1, K2_CSG2 = 2 };
+template <int D, int BUILD>
+__device__ __forceinline__ void intersect_level(const uint8_t* __restrict__ blob, const Workspace& ws, int level, unsigned key_mask) {
     // an earlier level did not fit: the host grows the arena and retries.  One decision per block (see k_shade).
     __shared__ int s_skip, s_total;
     __shared__ int s_rprefix[kRayBins + 1];
@@ -540,7 +542,9 @@ __global__ void __launch_bounds__(LIGHT ? kLightK2Block : kBlock, LIGHT ? EUCL_I
         if (valid) {
             Vec<D> o, d;
             load_ray<D>(ws, node, o, d);
-            const ClosestHit h = LIGHT ? closest_hit_light<D>(sv, o, d, ts, (int)blockDim.x) : closest_hit<D>(sv, o, d, ts, (int)blockDim.x);
+            const ClosestHit h = BUILD == K2_LIGHT  ? closest_hit_light<D>(sv, o, d, ts, (int)blockDim.x)
+                                 : BUILD == K2_CSG2 ? closest_hit_csg2<D>(sv, o, d, ts, (int)blockDim.x)
+                                                    : closest_hit<D>(sv, o, d, ts, (int)blockDim.x);
             HitHead rec{R(0.0), R(0.0), R(0.0), -1, 0};
             Vec<D> n;
 #pragma unroll
@@ -584,6 +588,18 @@ __global__ void __launch_bounds__(LIGHT ? kLightK2Block : kBlock, LIGHT ? EUCL_I
             }
         }
     }
+}
+
+template <int D, bool LIGHT>
+__global__ void __launch_bounds__(LIGHT ? kLightK2Block : kBlock, LIGHT ? EUCL_INTERSECT_LIGHT_MIN_BLOCKS : EUCL_INTERSECT_MIN_BLOCKS)
+    k_intersect(const uint8_t* __restrict__ blob, Workspace ws, int level, unsigned key_mask) {
+    intersect_level<D, LIGHT ? K2_LIGHT : K2_HEAVY>(blob, ws, level, key_mask);
+}
+
+template <int D>
+__global__ void __launch_bounds__(kCsg2Block, csg2_resident_blocks(D, (int)sizeof(real)))
+    k_intersect_csg2(const uint8_t* __restrict__ blob, Workspace ws, int level, unsigned key_mask) {
+    intersect_level<D, K2_CSG2>(blob, ws, level, key_mask);
 }
 
 // K3: shade every node of one level and append its children to the next level.  Children are
@@ -1548,12 +1564,17 @@ int launch_intersect(const Launch& l, const Workspace& ws, int level) {
     // a light-capable scene without cull roots (every ray has key 0) runs the light build in node order
     const bool light_all = l.light_capable && l.n_cull == 0;
     const bool split = l.light_capable && ws.ray_bins != 0;
+    // a csg2-capable scene walks the heavy build's rays, grouped or not, with k_intersect_csg2
     const size_t smem_light = l.smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block;
+    const size_t smem_csg2 = l.smem_scene + sizeof(real) * kPlaneChainMax * kCsg2Block;
     const unsigned heavy_mask = split ? 0xfffeu : 0xffffu;
     return launch_light_and_heavy(
         l, light_all || split, !light_all,
         [&](cudaStream_t stream) { k_intersect<D, true><<<l.grid_light_k2, kLightK2Block, smem_light, stream>>>(l.blob, ws, level, 1u); },
-        [&] { k_intersect<D, false><<<l.grid_max, kBlock, l.smem_bytes, l.stream>>>(l.blob, ws, level, heavy_mask); });
+        [&] {
+            if (l.csg2_capable) k_intersect_csg2<D><<<l.grid_csg2, kCsg2Block, smem_csg2, l.stream>>>(l.blob, ws, level, heavy_mask);
+            else k_intersect<D, false><<<l.grid_max, kBlock, l.smem_bytes, l.stream>>>(l.blob, ws, level, heavy_mask);
+        });
 }
 
 template <int D>
@@ -1687,6 +1708,7 @@ cudaError_t configure_dim(size_t smem_bytes, size_t smem_scene) {
     conf(k_raygen_rays<D>, smem_scene, 2);
     conf(k_intersect<D, false>, smem_bytes, heavy);
     conf(k_intersect<D, true>, smem_scene + sizeof(real) * kPlaneChainMax * kLightK2Block, EUCL_INTERSECT_LIGHT_MIN_BLOCKS);
+    conf(k_intersect_csg2<D>, smem_scene + sizeof(real) * kPlaneChainMax * kCsg2Block, csg2_resident_blocks(D, (int)sizeof(real)));
     for (int b = 0; b < 8; ++b) // [GLASS][RAY_BINS][FRAMES]
         conf(shade_build<D>(b & 4, b & 2, b & 1), smem_scene, (b & 4) ? kShadeResidentBlocks : kLightResidentBlocks);
     conf(k_background<D>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);

@@ -159,6 +159,8 @@ struct Launch {
     cudaStream_t side;  // nullptr: launch one after the other on `stream`
     cudaEvent_t ev_fork, ev_join;
     int grid_background; // blocks of the last level's kernel (256 threads each), one wave
+    int grid_csg2;       // blocks of k_intersect_csg2 (kCsg2Block threads each), one wave
+    int csg2_capable;    // SceneHeader::csg2_capable: k_intersect_csg2 replaces the heavy intersect build
 };
 
 #ifndef EUCL_BLOCK
@@ -193,6 +195,13 @@ constexpr int kLightResidentBlocks = EUCL_SHADE_LIGHT_MIN_BLOCKS; // ... and CTA
 #endif
 constexpr int kLightK2Block = EUCL_LIGHT_K2_BLOCK; // threads per CTA of the light intersect kernel
 constexpr int kLightK2ResidentBlocks = EUCL_INTERSECT_LIGHT_MIN_BLOCKS;
+#ifndef EUCL_CSG2_BLOCK
+#define EUCL_CSG2_BLOCK 128
+#endif
+constexpr int kCsg2Block = EUCL_CSG2_BLOCK; // threads per CTA of k_intersect_csg2
+// ... and CTAs per SM its register budget allows: 5 (<= 96 registers, no spills) except 4-D f64, which spills 140 B at
+// 96 registers and runs at 4 (128).  3d_room 4K, one B200 at 1000 W, one call: 13.62 ms per frame at 5 CTAs, 13.81 at 4.
+constexpr int csg2_resident_blocks(int dim, int real_bytes) { return dim == 4 && real_bytes == 8 ? 4 : 5; }
 constexpr int kRayBins = 16; // 2^4 reach keys
 constexpr int kBinsPerEntity = 3; // entering, exiting, exiting with total internal reflection predicted
 constexpr int kMaxBins = 64; // shade-coherence bins (miss, then kBinsPerEntity per entity); larger scenes shade unbinned

@@ -34,6 +34,8 @@ struct SceneHeader {
     int32_t off_ent_flags; // per entity: EntFlags
     int32_t light_capable; // 1: every surfaced entity is a primitive, a root plane chain or a cull root (see k_intersect<LIGHT>)
     int32_t off_lin_rows;  // LinRow table, 2 * EUCL_MAX_DIM rows per transform
+    int32_t csg2_capable;  // 1: every surfaced entity is a primitive, a root plane chain or a two-leaf program (k_intersect_csg2)
+    int32_t _pad[3];
 };
 
 // LinearSpace in table form.  eucl_scene_create recognises component expressions that are sums of terms
@@ -61,7 +63,8 @@ enum EntFlags : int32_t {
     ENT_PRIM = 2,       // the shape is one primitive
     ENT_ROOT_PLANES = 4, // the shape is one chain of <= kPlaneChainMax half-spaces
     ENT_CULL_ROOT = 8,  // owns a reach-key bit: rays with key 0 cannot hit it
-    ENT_NEGATED = 16    // Complement(VoidShape, X) lowered to X: hits flip their normal, membership is inverted
+    ENT_NEGATED = 16,   // Complement(VoidShape, X) lowered to X: hits flip their normal, membership is inverted
+    ENT_CSG2 = 32       // the shape is M_OP(A, B): A a primitive or a chain of <= kPlaneChainMax half-spaces, B a primitive
 };
 static_assert(sizeof(SceneHeader) % 16 == 0, "header must keep 16-byte alignment");
 
