@@ -162,7 +162,7 @@ struct EuclScene {
     int sm_count = 148;
     size_t smem_bytes = 0;  // staged scene + plane_chain scratch
     size_t smem_scene = 0;  // staged scene only
-    unsigned long long shade_light_mask = 1ull, shade_heavy_mask = 0ull;
+    unsigned long long shade_light_mask = 1ull, shade_heavy_mask = 0ull, shade_glass_mask = 0ull;
     DeviceBuffer blob;
     std::vector<cudaArray_t> arrays;
     std::vector<cudaTextureObject_t> tex_objects;
@@ -909,20 +909,26 @@ int eucl_scene_create_precision(const EuclFlatScene* flat, int device, int preci
     s->smem_scene = scene_smem_bytes(h.blob_bytes);
     s->smem_bytes = s->smem_scene + sizeof(double) * kPlaneChainMax * kBlock;
     // shade bins of the light build of k_shade: the miss bin and the bins of every entity whose surface has a uniform
-    // reflection ratio and the identity threshold direction; the heavy build (Fresnel, Snell) shades the others
+    // reflection ratio and the identity threshold direction; the others (Fresnel, Snell) go to k_shade_glass when their
+    // colour program is one constant, else to the heavy build
     s->shade_light_mask = 1ull;
     s->shade_heavy_mask = 0ull;
+    s->shade_glass_mask = 0ull;
+    const bool shade_glass = env_int("EUCL_SHADE_GLASS", 1) != 0; // 0: the heavy build shades them all (A/B in one library)
     if (kBinsPerEntity * flat->n_entities + 1 <= kMaxBins)
         for (int e = 0; e < flat->n_entities; ++e) {
             const int sf = flat->entities[e].surface;
             if (sf < 0) continue;
-            const bool simple = flat->surfaces[sf].ratio_op == EUCL_RATIO_UNIFORM && flat->surfaces[sf].thr_op == EUCL_THR_IDENTITY;
+            const EuclSurface& surf = flat->surfaces[sf];
+            const bool simple = surf.ratio_op == EUCL_RATIO_UNIFORM && surf.thr_op == EUCL_THR_IDENTITY;
+            const bool uniform_sc = surf.color_len == 1 && flat->color_ops[surf.color_first].op == EUCL_COL_UNIFORM;
             const unsigned long long bits = ((1ull << kBinsPerEntity) - 1ull) << (1 + kBinsPerEntity * e);
-            (simple ? s->shade_light_mask : s->shade_heavy_mask) |= bits;
+            (simple ? s->shade_light_mask : shade_glass && uniform_sc ? s->shade_glass_mask : s->shade_heavy_mask) |= bits;
         }
     if (env_int("EUCL_SHADE_SPLIT", 1) == 0) { // one build shades every bin (diagnostics)
-        s->shade_heavy_mask |= s->shade_light_mask;
+        s->shade_heavy_mask |= s->shade_light_mask | s->shade_glass_mask;
         s->shade_light_mask = 0ull;
+        s->shade_glass_mask = 0ull;
     }
     int smem_optin = 0;
     cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
@@ -1085,6 +1091,9 @@ Launch make_launch(const EuclScene* s, const Pipeline& pipe, const EuclRenderOpt
     l.grid_mem = sms * std::max(1, env_int("EUCL_MEM_BLOCKS_PER_SM", 8));
     l.shade_light_mask = s->shade_light_mask;
     l.shade_heavy_mask = s->shade_heavy_mask;
+    l.shade_glass_mask = s->shade_glass_mask;
+    for (int rb = 0; rb < 2; ++rb)
+        l.grid_shade_glass[rb] = sms * std::max(1, env_int("EUCL_SHADE_GLASS_BLOCKS_PER_SM", shade_glass_resident_blocks(rb != 0, s->real_bytes)));
     l.grid_light_k2 = sms * std::max(1, env_int("EUCL_LIGHT_K2_BLOCKS_PER_SM", kLightK2ResidentBlocks));
     l.light_capable = s->light_capable;
     l.grid_csg2 = sms * std::max(1, env_int("EUCL_CSG2_BLOCKS_PER_SM", csg2_resident_blocks(s->dim, s->real_bytes)));
@@ -1366,7 +1375,8 @@ uint64_t graph_key(const ChunkLaunch& c) {
                                            l.shade_heavy_mask, (unsigned long long)l.grid_light_k2,
                                            (unsigned long long)l.light_capable, (unsigned long long)l.n_cull,
                                            (unsigned long long)l.grid_background, (unsigned long long)l.grid_csg2,
-                                           (unsigned long long)l.csg2_capable};
+                                           (unsigned long long)l.csg2_capable, l.shade_glass_mask,
+                                           (unsigned long long)l.grid_shade_glass[0], (unsigned long long)l.grid_shade_glass[1]};
         mix(ptrs, sizeof ptrs);
         mix(nums, sizeof nums);
     }
@@ -1455,6 +1465,9 @@ int read_back_chunk(Pipeline& pipe, const ChunkLaunch& c, const ChunkDebug& dbg,
         // which intersect builds the levels ran: light for key 0, k_intersect_csg2 or the heavy build for the rest
         fprintf(stderr, "intersect light_capable %d csg2_capable %d n_cull %d ray_bins %d\n", c.l.light_capable, c.l.csg2_capable,
                 c.l.n_cull, c.ws.ray_bins != 0 ? 1 : 0);
+        // which shade builds take the bins of a binned level: light, k_shade_glass, heavy
+        fprintf(stderr, "shade bins light %#llx glass %#llx heavy %#llx\n", c.l.shade_light_mask, c.l.shade_glass_mask,
+                c.l.shade_heavy_mask);
         for (uint32_t lv = 0; lv <= depth; ++lv) {
             fprintf(stderr, "level %2u count %9d | bins", lv, h[SmallLayout::count + lv]);
             for (int b = 0; b < c.ws.n_bins && c.ws.n_bins > 1; ++b) fprintf(stderr, " %d", h[SmallLayout::bins + lv * kMaxBins + b]);

@@ -174,6 +174,8 @@ struct ShadeOut {
 // Step 1, shade_decide: reflection ratio, surface colour and its u8 quantisation, and WHICH children exist.
 // GLASS = false compiles the Fresnel / Snell providers out: the light shade kernel only ever sees surfaces
 // with a uniform reflection ratio and the identity threshold direction (the host routes the bins).
+// UNIFORM_SC: the surface's colour program is one EUCL_COL_UNIFORM op (the host routes the bins, k_shade_glass); its colour
+// is read from the op, the value surface_color would push and pop, without the program interpreter and its stack.
 template <int D>
 struct ShadeDecision {
     real ratio;
@@ -184,7 +186,7 @@ struct ShadeDecision {
     real from_theta; // angle_between(direction, -normal_closer); Fresnel / Snell surfaces only
     RefractionCache rc;
 };
-template <int D, bool GLASS>
+template <int D, bool GLASS, bool UNIFORM_SC = false>
 __device__ __forceinline__ void shade_decide(const SceneView& sv, real time_millis, int ent, bool exiting, real cos_raw,
                                              real angle_raw, const Vec<D>& p, const Vec<D>& n_raw, ShadeDecision<D>& out,
                                              Rgba& sc_out) {
@@ -207,7 +209,8 @@ __device__ __forceinline__ void shade_decide(const SceneView& sv, real time_mill
     out.dest = -1;
     bool have_t = false;
     if (!(ratio >= R(1.0))) { // get_intersection_color
-        const Rgba sc = surface_color<D>(sv, sf, p, n_raw, cos_raw, angle_raw, exiting, time_millis);
+        const Rgba sc = UNIFORM_SC ? uniform_surface_color(sv, sf)
+                                   : surface_color<D>(sv, sf, p, n_raw, cos_raw, angle_raw, exiting, time_millis);
         const unsigned q = to_pixel4(sc);
         out.q = q;
         if ((q >> 24) == 255u) {
@@ -613,10 +616,12 @@ __global__ void __launch_bounds__(kCsg2Block, csg2_resident_blocks(D, (int)sizeo
 //
 // FRAMES: a batch of frames (Workspace::node_frame): Perlin time from the node's frame, children tagged with it.  A build of
 // its own so that the single-frame builds carry none of it.
-template <int D, bool RAY_BINS, bool GLASS, bool FRAMES>
-__global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUCL_SHADE_MIN_BLOCKS : EUCL_SHADE_LIGHT_MIN_BLOCKS)
-    k_shade(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp, Workspace ws, int level, unsigned long long bin_mask,
-            int32_t* __restrict__ hit_ids_out) {
+//
+// k_shade_glass is the heavy build for the bins of Fresnel / Snell surfaces whose colour program is one constant
+// (UNIFORM_SC): the same code without the colour-program interpreter, so that it needs fewer registers and no colour stack.
+template <int D, bool RAY_BINS, bool GLASS, bool FRAMES, bool UNIFORM_SC>
+__device__ __forceinline__ void shade_level(const uint8_t* __restrict__ blob, const FrameParams& fp, const ChunkParams& cp,
+                                            const Workspace& ws, int level, unsigned long long bin_mask, int32_t* __restrict__ hit_ids_out) {
     const int off = ws.level_off[level], cnt = ws.count[level];
     const bool last_level = level >= fp.max_depth; // depth 0: background without intersecting (mod.rs:157,183)
     // binned levels: position g of the concatenated bins of this launch -> (bin, index) through the bin prefix sums
@@ -699,7 +704,7 @@ __global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUC
                 const Vec<D> p = o + d * ei.t; // the intersectors' expression for the hit location (shape.rs:700,795,993)
                 Rgba sc;
                 const real time_millis = R(FRAMES ? ws.frames[ws.node_frame[node]].time_millis : fp.time_millis);
-                shade_decide<D, GLASS>(sv, time_millis, ei.entity, ei.exiting != 0, ei.cos_raw, ei.angle_raw, p, n, dec, sc);
+                shade_decide<D, GLASS, UNIFORM_SC>(sv, time_millis, ei.entity, ei.exiting != 0, ei.cos_raw, ei.angle_raw, p, n, dec, sc);
                 if (dec.flags & NODE_HAS_SC) {
                     store_res(ws, node, sc);
                     if (!dec.r_emit) dec.flags |= NODE_LEAF; // opaque without a mirror term: the colour is final
@@ -772,6 +777,18 @@ __global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUC
             bin_child(rchild, rkey);
         }
     }
+}
+template <int D, bool RAY_BINS, bool GLASS, bool FRAMES>
+__global__ void __launch_bounds__(GLASS ? kShadeBlock : kLightBlock, GLASS ? EUCL_SHADE_MIN_BLOCKS : EUCL_SHADE_LIGHT_MIN_BLOCKS)
+    k_shade(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp, Workspace ws, int level, unsigned long long bin_mask,
+            int32_t* __restrict__ hit_ids_out) {
+    shade_level<D, RAY_BINS, GLASS, FRAMES, false>(blob, fp, cp, ws, level, bin_mask, hit_ids_out);
+}
+template <int D, bool RAY_BINS, bool FRAMES>
+__global__ void __launch_bounds__(kShadeGlassBlock, shade_glass_resident_blocks(RAY_BINS, (int)sizeof(real)))
+    k_shade_glass(const uint8_t* __restrict__ blob, FrameParams fp, ChunkParams cp, Workspace ws, int level,
+                  unsigned long long bin_mask, int32_t* __restrict__ hit_ids_out) {
+    shade_level<D, RAY_BINS, true, FRAMES, true>(blob, fp, cp, ws, level, bin_mask, hit_ids_out);
 }
 
 // K3 of the LAST level: depth 0, `background.get_color(direction)` without intersecting (mod.rs:157,183).  A kernel of its
@@ -1545,6 +1562,13 @@ auto shade_build(bool glass, bool ray_bins, bool frames) {
         {{k_shade<D, false, true, false>, k_shade<D, false, true, true>}, {k_shade<D, true, true, false>, k_shade<D, true, true, true>}}};
     return builds[glass][ray_bins][frames];
 }
+// ... and of k_shade_glass by [RAY_BINS][FRAMES]
+template <int D>
+auto shade_glass_build(bool ray_bins, bool frames) {
+    static const decltype(&k_shade_glass<D, false, false>) builds[2][2] = {
+        {k_shade_glass<D, false, false>, k_shade_glass<D, false, true>}, {k_shade_glass<D, true, false>, k_shade_glass<D, true, true>}};
+    return builds[ray_bins][frames];
+}
 
 template <int D>
 void launch_camera_entity(const Launch& l, const FrameParams& fp, const Workspace& ws) {
@@ -1584,22 +1608,28 @@ int launch_shade(const Launch& l, const FrameParams& fp, const ChunkParams& cp, 
         k_background<D><<<l.grid_background, 256, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level, hit_ids_out);
         return 1;
     }
-    unsigned long long light = l.shade_light_mask, heavy = l.shade_heavy_mask;
+    unsigned long long light = l.shade_light_mask, glass = l.shade_glass_mask, heavy = l.shade_heavy_mask;
     if (ws.n_bins <= 1) { // not binned: one kernel that can shade everything
         light = 0ull;
+        glass = 0ull;
         heavy = ~0ull;
     }
     const bool ray_bins = ws.ray_bins && level + 1 < fp.max_depth; // the next level will be intersected: group its rays
     const bool frames = ws.node_frame != nullptr;
-    return launch_light_and_heavy(
-        l, light != 0ull, heavy != 0ull,
+    // k_shade_glass and the heavy build both run on the main stream, one after the other, when a level needs both
+    return (glass != 0ull && heavy != 0ull) + launch_light_and_heavy(
+        l, light != 0ull, (glass | heavy) != 0ull,
         [&](cudaStream_t stream) {
             shade_build<D>(false, ray_bins, frames)<<<l.grid_light, kLightBlock, l.smem_scene, stream>>>(l.blob, fp, cp, ws, level,
                                                                                                        light, hit_ids_out);
         },
         [&] {
-            shade_build<D>(true, ray_bins, frames)<<<l.grid_shade, kShadeBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level,
-                                                                                                       heavy, hit_ids_out);
+            if (glass)
+                shade_glass_build<D>(ray_bins, frames)<<<l.grid_shade_glass[ray_bins], kShadeGlassBlock, l.smem_scene, l.stream>>>(
+                    l.blob, fp, cp, ws, level, glass, hit_ids_out);
+            if (heavy)
+                shade_build<D>(true, ray_bins, frames)<<<l.grid_shade, kShadeBlock, l.smem_scene, l.stream>>>(l.blob, fp, cp, ws, level,
+                                                                                                           heavy, hit_ids_out);
         });
 }
 
@@ -1711,6 +1741,8 @@ cudaError_t configure_dim(size_t smem_bytes, size_t smem_scene) {
     conf(k_intersect_csg2<D>, smem_scene + sizeof(real) * kPlaneChainMax * kCsg2Block, csg2_resident_blocks(D, (int)sizeof(real)));
     for (int b = 0; b < 8; ++b) // [GLASS][RAY_BINS][FRAMES]
         conf(shade_build<D>(b & 4, b & 2, b & 1), smem_scene, (b & 4) ? kShadeResidentBlocks : kLightResidentBlocks);
+    for (int b = 0; b < 4; ++b) // [RAY_BINS][FRAMES]
+        conf(shade_glass_build<D>(b & 2, b & 1), smem_scene, shade_glass_resident_blocks(b & 2, (int)sizeof(real)));
     conf(k_background<D>, smem_scene, EUCL_BACKGROUND_MIN_BLOCKS);
     conf(k_megakernel<D>, smem_bytes, heavy);
     conf(k_megakernel_aov<D>, smem_bytes, heavy);

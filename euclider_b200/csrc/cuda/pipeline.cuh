@@ -161,6 +161,8 @@ struct Launch {
     int grid_background; // blocks of the last level's kernel (256 threads each), one wave
     int grid_csg2;       // blocks of k_intersect_csg2 (kCsg2Block threads each), one wave
     int csg2_capable;    // SceneHeader::csg2_capable: k_intersect_csg2 replaces the heavy intersect build
+    unsigned long long shade_glass_mask; // shade bins of k_shade_glass (Fresnel / Snell surfaces of one constant colour)
+    int grid_shade_glass[2];             // blocks of k_shade_glass by RAY_BINS (kShadeGlassBlock threads each), one wave
 };
 
 #ifndef EUCL_BLOCK
@@ -187,6 +189,17 @@ constexpr int kShadeBlock = EUCL_SHADE_BLOCK; // threads per CTA of the heavy sh
 constexpr int kShadeResidentBlocks = EUCL_SHADE_MIN_BLOCKS;
 constexpr int kLightBlock = EUCL_LIGHT_BLOCK; // threads per CTA of the light shade kernel
 constexpr int kLightResidentBlocks = EUCL_SHADE_LIGHT_MIN_BLOCKS; // ... and CTAs per SM its register budget allows
+#ifndef EUCL_SHADE_GLASS_BLOCK
+#define EUCL_SHADE_GLASS_BLOCK 128
+#endif
+constexpr int kShadeGlassBlock = EUCL_SHADE_GLASS_BLOCK; // threads per CTA of k_shade_glass
+// ... and CTAs per SM, by build.  Every setting below 128 registers spills.  The RAY_BINS builds (levels walked grouped by
+// reach key) wait on reach_key's bound tests and the key-list atomics, and more resident warps pay for the spills: f64 6
+// CTAs (80 registers), f32 5 (96).  The other builds spend their time in the shading arithmetic and keep 128 registers:
+// 4 CTAs.  One B200 at 1000 W, ms per frame: 3d_room 4K (grouped) f64 at 4 / 5 / 6 / 7 CTAs 13.31 - 13.33 / 13.21 - 13.26
+// / 13.12 - 13.13 / 13.17 - 13.19, f32 at 4 / 5 / 6 11.34 - 11.35 / 11.28 - 11.29 / 11.35 - 11.37; 3d_fresnel 1080p
+// (ungrouped) f64 at 4 / 5 1.65 / 1.74 (parent 1.73).
+constexpr int shade_glass_resident_blocks(bool ray_bins, int real_bytes) { return !ray_bins ? 4 : real_bytes == 8 ? 6 : 5; }
 #ifndef EUCL_LIGHT_K2_BLOCK
 #define EUCL_LIGHT_K2_BLOCK 128
 #endif

@@ -576,4 +576,10 @@ __device__ EUCL_SC_INLINE Rgba surface_color(const SceneView& sv, const EuclSurf
     return sp > 0 ? stack[sp - 1] : Rgba{R(0.0), R(0.0), R(0.0), R(0.0)};
 }
 
+// surface_color of a program that is one EUCL_COL_UNIFORM op (surface.rs:425-429): the op's constant
+__device__ __forceinline__ Rgba uniform_surface_color(const SceneView& sv, const EuclSurface& sf) {
+    const EuclColorOp& op = sv.color_ops()[sf.color_first];
+    return Rgba{R(op.f[0]), R(op.f[1]), R(op.f[2]), R(op.f[3])};
+}
+
 } // namespace EUCL_NS
